@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the hot path (Renderer::Accumulate x spp + Renderer::Render) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One STEP = one frame of the workload: ResetAccumulator, Accumulate() for the workload's sample count, Render(). In the device-timed pass
@@ -38,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "cpu-raytracing-experiments_b200")
 sys.path[:0] = [ROOT, PKG]
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (no __pycache__ next to the modules it imports)
 
 WORKLOADS = {
     # name: scene, width, height(internal, multiple of 16), spp, max_bounces, K
@@ -51,6 +52,7 @@ WORKLOADS = {
 STRONG_SPP = 128   # the `strong` record: this many samples per frame, split over the ranks by bucket
 METRIC, UNIT = "Mrays/s", "Mrays/s"
 DIGESTS = os.path.join(ROOT, "tests", "golden", "bench_digests.json")
+DUMP_BYTES = 64_000_000   # --dump-outputs: payload of all .npy files of one run together
 
 
 def make_scene(name):
@@ -380,6 +382,28 @@ class Bench:
         self.r.close()
 
 
+def device_frame(r, dev):
+    """The RGBA32F frame in the renderer's device framebuffer (where b2r_resolve_device / b2r_team_resolve leave it), copied to the host."""
+    import torch
+    from b2r_dist import _DevArray
+    r.sync()
+    ptr, nbytes = r.device_framebuffer()
+    return torch.as_tensor(_DevArray(ptr, nbytes // 4), device=dev).cpu().numpy().reshape(r.height, r.width, 4)
+
+
+def dump_array(out_dir, name, a, budget):
+    """Writes `a` as out_dir/name.npy; a frame larger than `budget` bytes is written as a fixed sample of its pixels instead (rows of the
+    flattened [pixel][channel] array at ascending indices drawn with RandomState(0), so two runs sample the same pixels). Returns the bytes
+    of payload written."""
+    import numpy as np
+    if a.nbytes > budget:
+        flat = a.reshape(-1, a.shape[-1])
+        keep = budget // flat[0].nbytes
+        a = flat[np.sort(np.random.RandomState(0).choice(len(flat), keep, replace=False))]
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    return a.nbytes
+
+
 def roofline(b, kt, pc, steps, hbm_peak, peak_src, sm_max):
     """Per-kernel roofline rows from the kernel-by-kernel pass (CUDA event pair around every launch) and the device counters of the same
     steps. Algorithmic bytes / flops: DESIGN.md §5. The top-level keys describe the dominant kernel; `kernels` lists every kernel of the step."""
@@ -480,6 +504,8 @@ def run_workload(args, name, rank, world, local, stream, dev, secondary=False):
         clocks.start()
     ms_total = b.timed(steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # the frame of the last timed step, before any other pass touches the framebuffer
+        args.dump_left -= dump_array(args.dump_outputs, f"{name}_frame", device_frame(r, dev), args.dump_left)
     rays_total, launches = b.rays(r.counters())
     secs = ms_total / 1e3
     value = rays_total / secs / 1e6
@@ -709,7 +735,17 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch kernel by kernel (for ncu); never used for a reported number")
     ap.add_argument("--reference-exact", action="store_true", help="brute-force workloads: B2R_FLAG_REFERENCE_EXACT (bit-identical to the reference's own renderer; one extra ranking kernel per bounce)")
     ap.add_argument("--combine", default="team", choices=["team", "p2p", "nccl"], help="multi-GPU frame combine: team = sliced resolve over NVLink with device-side hand-shakes (default); p2p = rank 0 resolves, host barriers (round 1); nccl = all-reduce then resolve")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps of each workload, write the RGBA32F frame of its last step as DIR/<workload>_frame.npy "
+                    "(float32 [height][width][4]; a frame that does not fit the 64 MB left for the run is written as a fixed sample of its pixels, [pixels][4]: "
+                    "the rows of the flattened [height*width][4] frame at the indices np.sort(np.random.RandomState(0).choice(height*width, pixels, replace=False)))")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs writes the GPU path's frames: --impl ours only")
+        os.makedirs(args.dump_outputs, exist_ok=True)
+    args.dump_left = DUMP_BYTES - 4096   # (4 KB for the .npy headers)
     args.warmup = max(args.warmup, 0)
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))

@@ -60,19 +60,19 @@ def test_live_bit_exact_and_schedule_independent(threads, monkeypatch):
         assert racted == acted and rframe.tobytes() == frame.tobytes(), name
 
 
-@live
 def test_canonical_mode_within_north_star_tolerance_of_reference():
-    """What the GPU computes (SIMD-FMA formula for every closest-hit ray) against the reference: divergent-path fraction and RMSE."""
+    """What the GPU computes (SIMD-FMA formula for every closest-hit ray) against the reference: divergent-path fraction and RMSE. The
+    reference's side — its first sample (bucket 1) and its 200-spp frame of this render — is tests/golden/reference_default_160x96_mb16.npz
+    (tests/gen_golden.py)."""
     sc = scenes.default_scene(); w, h, mb = 160, 96, 16
-    r = oracle_py.ReferenceRenderer(sc, w, h, mb); r.accumulate(1); one = r.buckets()[1].copy()  # sample index 1 lands in bucket 1 (Q1)
-    r.accumulate(199); racted, rframe = r.render(); r.close()
+    ref = np.load(os.path.join(G, "reference_default_160x96_mb16.npz")); one, rframe = ref["first_sample"], ref["frame_200spp"]  # sample index 1 lands in bucket 1 (Q1)
     o = oracle_py.Oracle(w, h, max_bounces=mb, K=5); o.set_scene(sc); o.accumulate(1, threads=1); mine = o.buckets()[1].copy()
     o.accumulate(199); rc, frame = o.render(); acted = rc == 0; o.close()
     rel = np.abs(mine - one) / np.maximum(np.abs(one), 1e-6)
     divergent = float((rel > 1e-4).any(axis=0).mean())
     rmse = float(np.sqrt(np.mean((frame[..., :3] - rframe[..., :3]) ** 2)))
     print(f"canonical oracle vs reference renderer: divergent per-sample pixel fraction {divergent:.3e}, converged (200 spp) tonemapped RMSE {rmse:.3e}")
-    assert racted and acted and divergent < 2e-3 and rmse < 1e-3
+    assert acted and divergent < 2e-3 and rmse < 1e-3
 
 
 # ---------------------------------------------------------------------------------------------- GGX closure (the reference's `#define BRDF 1` build)
