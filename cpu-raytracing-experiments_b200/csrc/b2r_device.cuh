@@ -664,8 +664,7 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p,
 			const PathState s0 = primary_path(p.frame, p.batch->cam, p.batch->acc[sl], sl, idx - sl * p.frame.npix);
 			store_path(p.q, 0, idx, s0); rad_zero(p.rad, p.frame.npix, s0.pid);
 			ox = s0.ox; oy = s0.oy; oz = s0.oz; dx[r] = s0.dx; dy[r] = s0.dy; dz[r] = s0.dz;   // (all camera rays leave the same point)
-			ix[r] = 1.0f / dx[r]; iy[r] = 1.0f / dy[r]; iz[r] = 1.0f / dz[r];
-			nx[r] = -(ox * ix[r]); ny[r] = -(oy * iy[r]); nz[r] = -(oz * iz[r]); ax[r] = fabsf(ix[r]); ay[r] = fabsf(iy[r]); az[r] = fabsf(iz[r]);
+			slab_setup(ox, oy, oz, dx[r], dy[r], dz[r], &ix[r], &iy[r], &iz[r], &nx[r], &ny[r], &nz[r], &ax[r], &ay[r], &az[r]);
 			best[r] = FLT_MAX; prim[r] = -1;
 		}
 		uint32_t node = 0u, sp = 0u;
@@ -683,7 +682,7 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p,
 				float tn[RPL]; bool h[RPL]; bool any = false; uint32_t tmin = 0xffffffffu;
 #pragma unroll
 				for (int r = 0; r < RPL; r++) {
-					slab(a, b, ix[r], iy[r], iz[r], nx[r], ny[r], nz[r], ax[r], ay[r], az[r], best[r], &tn[r], &h[r]);  // an empty slot's box (h = -1e30) is never hit
+					slab(a, b, ix[r], iy[r], iz[r], nx[r], ny[r], nz[r], ax[r], ay[r], az[r], best[r], &tn[r], &h[r]);  // an empty slot's box (h = -1e30) fails every constrained axis (camera rays keep at least one, slab_setup)
 					any = any || h[r]; tmin = min(tmin, h[r] ? __float_as_uint(tn[r]) : 0xffffffffu);
 				}
 				if (COUNT && l != kEmptyLink) c_box += RPL;
@@ -903,9 +902,7 @@ __global__ void __launch_bounds__(kTravBlock, 8) k_intersect_shadow(const Params
 			idx = got; active = true;
 			const float4 a = p.q.SA[idx], b = p.q.SB[idx];
 			ox = a.x; oy = a.y; oz = a.z; dx = a.w; dy = b.x; dz = b.y; tfar = b.z; pid = __float_as_uint(b.w);
-			ix = 1.0f / dx; iy = 1.0f / dy; iz = 1.0f / dz;
-			nx = -(ox * ix); ny = -(oy * iy); nz = -(oz * iz);
-			ax = fabsf(ix); ay = fabsf(iy); az = fabsf(iz);
+			slab_setup(ox, oy, oz, dx, dy, dz, &ix, &iy, &iz, &nx, &ny, &nz, &ax, &ay, &az);
 			node = root = p.q.SS[idx]; up = __ldg(parent + root); skip = kNoNode; stack.reset();
 		}
 		uint32_t live = __ballot_sync(0xffffffffu, active);

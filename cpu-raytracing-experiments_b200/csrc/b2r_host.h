@@ -11,7 +11,7 @@ namespace b2r {
 // 128-byte traversal node: four 32-byte child slots, each two float4 — a box as centre + half extents in EVERY slot:
 //   inner child : {c.x, c.y, c.z, 0  } {h.x, h.y, link = wide-node index (>= 0), h.z}
 //   leaf child  : {c.x, c.y, c.z, r^2} {H,   H,   link = ~prim_index      (< 0),  H  }   (sphere inlined: no leaf fetch)
-//   empty slot  : link = kEmptyLink, h = -1e30 (its box fails every slab test)
+//   empty slot  : link = kEmptyLink, h = -1e30 (its box fails the slab test of every ray that keeps an axis constrained, b2r_shade.h slab_setup)
 // A leaf's H is the half extent of a cube around the sphere that contains every ray the float sphere tests can report as a hit
 // (leaf_half_extent, b2r_shade.h); inner boxes are the padded union of their child node's slot boxes (refit_child_box), so the one
 // uniform slab pass of the traversal kernels is conservative for all four slots. The spheres are the reference's prims (BVH leaf

@@ -260,6 +260,33 @@ B2R_HD void rad_zero(float* rad, uint32_t npix, uint32_t pid) {
 struct Ray { float ox, oy, oz, dx, dy, dz; };
 
 constexpr float kSlabWiden = 1.0000008f;  // the exit distance is widened by ~7 ulp: rounding of the four operations per plane never rejects a box
+// Per-ray set-up of the slab test, shared by TravBase::arm, k_intersect_packet and k_intersect_shadow: i = 1/d, n = -o/d, a = |1/d| per axis.
+// Rule: an axis keeps n only while |1/d| * (|ox| + |oy| + |oz| + 2^64) <= 2^126; otherwise n is NaN, every term of that axis is NaN and drops
+// out of fminf / fmaxf, and the axis leaves every box unconstrained — exactly what a zero component (0 * inf) always did. Why it is safe:
+// - conservative: an unconstrained axis only accepts more boxes, and a box test never decides a result (the sphere tests do);
+// - no overflow on a kept axis: |n| <= 2^126 and, for box centres |c| <= 2^64, |c/d| <= 2^126, so t_centre is finite; a half extent h
+//   with |h/d| > FLT_MAX turns near into -inf and far into +inf, which only widens the box. Without the rule a finite 1/d with
+//   |o/d| > FLT_MAX (d = 1e-38 from o = 400) made n = -inf, every exit distance -inf, and the BVH rejected every box brute force hits;
+// - domain: box centres stay below 2^64 when sphere bounds and origins are below 2^61 (where |c - o|^2 is finite in the sphere tests); a
+//   direction with a component of at least 2^-60 keeps that axis, so an empty slot (h = -1e30) is still rejected. A finite origin with
+//   every |d| component below about 2^-61 (like d = 0, which did so before the rule) has no constrained axis: empty slots then pass and
+//   their zero sphere at the world origin is tested under the id ~kEmptyLink — outside the domain above;
+// - a non-finite origin makes the sum non-finite: all three axes are unconstrained and the walk tests every sphere, as brute force does
+//   (the sphere tests then see NaN: closest misses, any hit reports occlusion, on both sides).
+// Exact zeros, subnormals and finite components with an overflowing 1/d all come out as unconstrained axes. Once per ray, not per node.
+constexpr float kSlabReach = 18446744073709551616.0f;  // 2^64
+constexpr float kSlabRange = 8.50705917302346159e37f;  // 2^126, a factor 4 below FLT_MAX
+B2R_HD void slab_setup(float ox, float oy, float oz, float dx, float dy, float dz, float* ix, float* iy, float* iz, float* nx, float* ny, float* nz,
+                       float* ax, float* ay, float* az) {
+	const float sx = 1.0f / dx, sy = 1.0f / dy, sz = 1.0f / dz;
+	const float reach = ((fabsf(ox) + fabsf(oy)) + fabsf(oz)) + kSlabReach;   // NaN or inf for a non-finite origin
+	const float nan = from_bits(0x7fc00000u);
+	*ix = sx; *iy = sy; *iz = sz;
+	*nx = fabsf(sx) * reach <= kSlabRange ? -(ox * sx) : nan;
+	*ny = fabsf(sy) * reach <= kSlabRange ? -(oy * sy) : nan;
+	*nz = fabsf(sz) * reach <= kSlabRange ? -(oz * sz) : nan;
+	*ax = fabsf(sx); *ay = fabsf(sy); *az = fabsf(sz);
+}
 B2R_HD void slab(const float4 a, const float4 b, float ix, float iy, float iz, float nx, float ny, float nz, float ax, float ay, float az,
                  float limit, float* tnear, bool* hit) {
 	// box tests never decide a result (they are conservative), so FMA is used freely; a NaN (0 * inf on an axis the ray is parallel
@@ -297,9 +324,7 @@ struct TravBase {
 	uint32_t node;
 	B2R_HD void arm(const Ray& r) {
 		ox = r.ox; oy = r.oy; oz = r.oz; dx = r.dx; dy = r.dy; dz = r.dz;
-		ix = 1.0f / r.dx; iy = 1.0f / r.dy; iz = 1.0f / r.dz;
-		nx = -(r.ox * ix); ny = -(r.oy * iy); nz = -(r.oz * iz);
-		ax = fabsf(ix); ay = fabsf(iy); az = fabsf(iz);
+		slab_setup(r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, &ix, &iy, &iz, &nx, &ny, &nz, &ax, &ay, &az);
 		node = 0u;
 	}
 };
@@ -335,7 +360,7 @@ struct TravClosestT : TravBase {
 			float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, ax, ay, az, best, &tn, &h);
 			if (COUNT && l != kEmptyLink) (*c_box)++;
 			key[k] = (h && l >= 0) ? bits(tn) : 0xffffffffu; link[k] = static_cast<uint32_t>(l);
-			leaves |= (h && l < 0) ? (1u << k) : 0u;  // an empty slot's box (h = -1e30) is never hit
+			leaves |= (h && l < 0) ? (1u << k) : 0u;  // an empty slot's box (h = -1e30) fails every constrained axis: never hit by a ray that keeps one (slab_setup)
 		}
 		while (leaves) {
 			const int k = first_bit(leaves);

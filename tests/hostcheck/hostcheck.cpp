@@ -193,6 +193,25 @@ void hc_closest_brute(const b2r_sphere* prims, uint32_t n, const float* rays, ui
 	}
 }
 
+// brute-force any hit over spheres in order along [0, tfar) (Traverse_shadow without a tree, BVH.hpp:290-305): occ_out[i] = 0 / 1
+void hc_any_brute(const b2r_sphere* prims, uint32_t n, const float* rays, const float* tfar, uint32_t n_rays, uint8_t* occ_out) {
+	for (uint32_t i = 0; i < n_rays; i++) {
+		const float* r = rays + 6 * static_cast<size_t>(i);
+		bool occ = false;
+		for (uint32_t j = 0; j < n && !occ; j++) occ = sphere_hit_any(prims[j].position[0], prims[j].position[1], prims[j].position[2], prims[j].radius_sq, r[0], r[1], r[2], r[3], r[4], r[5], tfar[i]);
+		occ_out[i] = occ ? 1 : 0;
+	}
+}
+// the same with the scalar-tail formula of the closest-hit loop (BVH.hpp:270-286), spheres in order: what B2R_FLAG_REFERENCE_EXACT's tail rays get
+void hc_closest_brute_scalar(const b2r_sphere* prims, uint32_t n, const float* rays, uint32_t n_rays, float* tfar_out, int32_t* prim_out) {
+	for (uint32_t i = 0; i < n_rays; i++) {
+		const float* r = rays + 6 * static_cast<size_t>(i);
+		float best = FLT_MAX; int32_t prim = -1;
+		for (uint32_t j = 0; j < n; j++) sphere_closest_scalar_update(prims[j].position[0], prims[j].position[1], prims[j].position[2], prims[j].radius_sq, static_cast<int32_t>(j), r[0], r[1], r[2], r[3], r[4], r[5], &best, &prim);
+		tfar_out[i] = best; prim_out[i] = prim;
+	}
+}
+
 // scalar taps of csrc/b2r_math.h for function-level comparison with the oracle
 uint32_t hc_hash_2d(uint32_t x, uint32_t y) { return hash_2d(x, y); }
 uint32_t hc_hash_u32(uint32_t x) { return hash_u32(x); }
@@ -222,6 +241,141 @@ void hc_closest_scalar(const float* spheres4, uint32_t n, const float ray[6], fl
 	for (uint32_t j = 0; j < n; j++) sphere_closest_scalar_update(spheres4[4 * j], spheres4[4 * j + 1], spheres4[4 * j + 2], spheres4[4 * j + 3], static_cast<int32_t>(j), ray[0], ray[1], ray[2], ray[3], ray[4], ray[5], best, prim);
 }
 int hc_sphere_any(const float s[4], const float ray[6], float tfar) { return sphere_hit_any(s[0], s[1], s[2], s[3], ray[0], ray[1], ray[2], ray[3], ray[4], ray[5], tfar) ? 1 : 0; }
+
+}  // extern "C"
+
+// ---- deterministic traversal taps: every tree the library can trace, the walks the kernels run, and no environment variables.
+// Tree kinds of the taps below (the spheres `prims` are in BVH order, as uploaded):
+enum HcTree { HC_REFERENCE = 0,  // the caller's reference topology (nodes) flattened: B2R_FLAG_REFERENCE_TREE
+              HC_SAH = 1,        // the traversal SAH tree libb2r builds by default
+              HC_PACKED = 2,     // the packed tree (B2R_FLAG_GPU_TREE), host twin
+              HC_SWEEP = 3,      // the curve sweep tree (B2R_FLAG_GPU_TREE | B2R_FLAG_GPU_SAH), host twin
+              HC_SWEEP3 = 4,     // the three-axis sweep tree (B2R_FLAG_GPU_TREE | B2R_FLAG_GPU_SAH3), host twin
+              HC_REFIT = 5 };    // the traversal SAH tree of `prims`, refitted to `moved` (same order): b2r_refit_scene's host twin
+// Builds tree `kind` for the spheres the rays are traced against (prims, or moved for HC_REFIT). The origin box: box6 when given, else the
+// library's rule over the spheres plus the finite ray origins (what b2r_trace_* grows the box to). Returns 0, 1 when a sweep tree would be
+// too deep, or B2R_ERR_ARG / B2R_ERR_BVH.
+static int hc_tree(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n,
+                   const float* box6, const float* rays, uint32_t n_rays, WideBvh& w) {
+	float pts[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
+	for (uint32_t i = 0; i < n_rays; i++) for (int k = 0; k < 3; k++) { const float v = rays[6 * static_cast<size_t>(i) + k]; if (v == v && fabsf(v) <= FLT_MAX) { pts[k] = fminf(pts[k], v); pts[3 + k] = fmaxf(pts[3 + k], v); } }
+	const bool have_pts = pts[0] <= pts[3];
+	const b2r_sphere* target = kind == HC_REFIT ? moved : prims;
+	if (!target) return B2R_ERR_ARG;
+	const OriginBox ob = origin_box_of(target, n, box6, have_pts ? pts : nullptr, have_pts ? 2u : 0u);
+	switch (kind) {
+	case HC_REFERENCE: if (!nodes) return B2R_ERR_ARG; flatten_bvh(nodes, n_nodes, prims, n, w, &ob); break;
+	case HC_SAH: case HC_REFIT: { std::vector<b2r_bvh_node> t; build_traversal_tree(prims, n, t); flatten_bvh(t.data(), static_cast<uint32_t>(t.size()), prims, n, w, &ob); break; }
+	case HC_PACKED: build_packed_tree(prims, n, w, &ob); break;
+	case HC_SWEEP: if (!build_sweep_tree(prims, n, w, &ob)) return 1; break;
+	case HC_SWEEP3: if (!build_sweep3_tree(prims, n, w, &ob)) return 1; break;
+	default: return B2R_ERR_ARG;
+	}
+	if (kind == HC_REFIT) {
+		std::vector<float4> packed(n);
+		for (uint32_t i = 0; i < n; i++) packed[i] = make_float4(moved[i].position[0], moved[i].position[1], moved[i].position[2], moved[i].radius_sq);
+		refit_wide(w, packed.data(), nullptr, ob);
+	}
+	if (w.max_stack + 3u > static_cast<uint32_t>(kTraversalStack)) return B2R_ERR_BVH;
+	return 0;
+}
+// the tables k_link_tables writes: the wide node that links to node i (the root's entry is 0) and the node holding sphere i's leaf slot
+static void hc_link_tables(const WideBvh& w, uint32_t n_prims, std::vector<uint32_t>& parent, std::vector<uint32_t>& leaf_node) {
+	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
+	const uint32_t nn = static_cast<uint32_t>(w.nodes.size());
+	parent.assign(nn, 0u); leaf_node.assign(n_prims, 0u);
+	for (uint32_t nd = 0; nd < nn; nd++) for (int k = 0; k < 4; k++) {
+		const int32_t l = as_int(wide[static_cast<size_t>(nd) * 8 + 2 * k + 1].z);
+		if (l == kEmptyLink) continue;
+		if (l < 0) leaf_node[~l] = nd; else parent[l] = nd;
+	}
+}
+
+extern "C" {
+
+// closest hit through traverse_closest (tail = 1: TravClosestT with the scalar-tail sphere formula, B2R_FLAG_REFERENCE_EXACT's tail rays).
+// Compare with hc_closest_brute / hc_closest_brute_scalar over the same spheres (moved for HC_REFIT).
+int hc_trace_closest(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
+                     const float* rays, uint32_t n_rays, int tail, float* tfar_out, int32_t* prim_out) {
+	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
+	uint32_t cs = 0, cb = 0;
+	for (uint32_t i = 0; i < n_rays; i++) {
+		const float* r = rays + 6 * static_cast<size_t>(i);
+		TravClosest t; t.begin(Ray{r[0], r[1], r[2], r[3], r[4], r[5]}, tail != 0);
+		while (t.step<false>(w.nodes.data(), w.tn_bits, &cs, &cb)) {}
+		tfar_out[i] = t.best; prim_out[i] = t.prim;
+	}
+	return 0;
+}
+// any hit along [0, tfar) through traverse_any, from the root. Compare with hc_any_brute.
+int hc_trace_any(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
+                 const float* rays, const float* tfar, uint32_t n_rays, uint8_t* occ_out) {
+	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
+	uint32_t cs = 0, cb = 0;
+	for (uint32_t i = 0; i < n_rays; i++) {
+		const float* r = rays + 6 * static_cast<size_t>(i);
+		occ_out[i] = traverse_any<false>(w.nodes.data(), Ray{r[0], r[1], r[2], r[3], r[4], r[5]}, tfar[i], &cs, &cb) ? 1 : 0;
+	}
+	return 0;
+}
+// k_intersect_shadow's walk restated on the host: it starts at the node holding sphere origin_prim[i]'s leaf slot, visits the nearest hit child
+// next and pushes the others, and when the subtree below `root` holds no occluder climbs to the parent, skipping the child already searched.
+int hc_trace_shadow_climb(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
+                          const float* rays, const float* tfar, const int32_t* origin_prim, uint32_t n_rays, uint8_t* occ_out) {
+	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
+	std::vector<uint32_t> parent, leaf_node; hc_link_tables(w, n, parent, leaf_node);
+	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
+	constexpr uint32_t kNone = 0xffffffffu;
+	for (uint32_t i = 0; i < n_rays; i++) {
+		const float* r = rays + 6 * static_cast<size_t>(i);
+		if (origin_prim[i] < 0 || static_cast<uint32_t>(origin_prim[i]) >= n) return B2R_ERR_ARG;
+		TravBase t; t.arm(Ray{r[0], r[1], r[2], r[3], r[4], r[5]});
+		ArrayStack stack; stack.reset();
+		uint32_t root = leaf_node[origin_prim[i]], up = parent[root], skip = kNone, node = root;
+		bool occ = false;
+		while (node != kNone) {
+			const float4* nd = wide + static_cast<size_t>(node) * 8;
+			uint32_t next = kNone, leaves = 0u; float next_tn = FLT_MAX;
+			for (int k = 0; k < 4; k++) {
+				const float4 a = nd[2 * k], b = nd[2 * k + 1]; const int32_t l = as_int(b.z);
+				float tn; bool h; slab(a, b, t.ix, t.iy, t.iz, t.nx, t.ny, t.nz, t.ax, t.ay, t.az, tfar[i], &tn, &h);
+				if (h && l >= 0 && static_cast<uint32_t>(l) != skip) {
+					const bool nearer = tn < next_tn;
+					const uint32_t later = nearer ? next : static_cast<uint32_t>(l);
+					if (later != kNone) stack.push(later);
+					if (nearer) { next = static_cast<uint32_t>(l); next_tn = tn; }
+				}
+				leaves |= (h && l < 0) ? (1u << k) : 0u;
+			}
+			while (leaves && !occ) {
+				const int k = first_bit(leaves); leaves &= leaves - 1u;
+				const float4 s4 = nd[2 * k];
+				occ = sphere_hit_any(s4.x, s4.y, s4.z, s4.w, t.ox, t.oy, t.oz, t.dx, t.dy, t.dz, tfar[i]);
+			}
+			if (occ) break;
+			if (next == kNone && !stack.empty()) next = stack.pop();
+			if (next == kNone && root != 0u) { skip = root; root = up; next = up; up = parent[up]; }
+			node = next;
+		}
+		occ_out[i] = occ ? 1 : 0;
+	}
+	return 0;
+}
+// the slot boxes of tree `kind` as {lo.xyz, hi.xyz, link} per non-empty slot (7 floats, link as int bits); out may be null to count
+int hc_tree_boxes(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
+                  const float* rays, uint32_t n_rays, float* out, uint32_t* n_out) {
+	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
+	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
+	uint32_t m = 0;
+	for (size_t nd = 0; nd < w.nodes.size(); nd++) for (int k = 0; k < 4; k++) {
+		const float4 a = wide[nd * 8 + 2 * k], b = wide[nd * 8 + 2 * k + 1];
+		if (as_int(b.z) == kEmptyLink) continue;
+		if (out) { float* o = out + 7 * static_cast<size_t>(m); o[0] = a.x - b.x; o[1] = a.y - b.y; o[2] = a.z - b.w; o[3] = a.x + b.x; o[4] = a.y + b.y; o[5] = a.z + b.w; o[6] = b.z; }
+		m++;
+	}
+	*n_out = m;
+	return 0;
+}
 
 }  // extern "C"
 
