@@ -28,6 +28,7 @@ FLAG_FORCE_BRUTE, FLAG_FORCE_BVH, FLAG_NO_MIS, FLAG_COUNT_TESTS, FLAG_NO_GRAPH, 
 FLAG_GPU_SAH = 1024  # with FLAG_GPU_TREE: the sweep tree (SAH cuts along the curve order) instead of the packed one
 FLAG_GPU_SAH3 = 2048  # with FLAG_GPU_TREE: the three-axis sweep tree (full-sweep SAH over the x, y, z orders)
 FLAG_GGX = 512  # the reference's `#define BRDF 1` closure (Closure<GGX>, DataStreams.hpp:184-219)
+TAP_CLOSEST, TAP_SHADOW, TAP_PACKET = 0, 1, 2  # b2r_trace_kernel: which traversal kernel of a frame runs
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_NO_LIGHTS, ERR_BVH, NOT_READY = 0, -1, -2, -3, -4, -5, 1
 KERNEL_KINDS = ["generate", "bounce_brute", "intersect_closest", "shade", "intersect_shadow", "accumulate", "resolve"]
 COUNTER_NAMES = ["extension_rays", "shadow_rays", "shaded_hits", "terminated", "dropped", "sphere_tests", "box_tests", "launches", "radiance_events", "reserved"]
@@ -37,7 +38,7 @@ ABI_SYMBOLS = [
     "b2r_bvh_build", "b2r_bvh_build_ex", "b2r_find_lights", "b2r_camera_lookat", "b2r_camera_ray", "b2r_create", "b2r_destroy", "b2r_resize", "b2r_reset", "b2r_set_stream",
     "b2r_sync", "b2r_upload_scene", "b2r_refit_scene", "b2r_set_camera", "b2r_accumulate", "b2r_resolve", "b2r_resolve_async", "b2r_resolve_device", "b2r_frame_wait", "b2r_resolve_from", "b2r_ipc_export_buckets", "b2r_ipc_open_peers", "b2r_ipc_close", "b2r_resolve_peers", "b2r_team_export", "b2r_team_open", "b2r_team_resolve", "b2r_team_error", "b2r_team_close", "b2r_host_register", "b2r_host_unregister", "b2r_get_accumulations", "b2r_set_accumulations",
     "b2r_read_buckets", "b2r_write_buckets", "b2r_save_checkpoint", "b2r_load_checkpoint", "b2r_device_buckets", "b2r_device_framebuffer", "b2r_read_counters", "b2r_reset_counters", "b2r_read_bounce_counts",
-    "b2r_read_kernel_times", "b2r_set_flags", "b2r_generate_rays", "b2r_trace_closest", "b2r_trace_shadow", "b2r_read_wide_nodes", "b2r_get_origin_box",
+    "b2r_read_kernel_times", "b2r_set_flags", "b2r_generate_rays", "b2r_trace_closest", "b2r_trace_shadow", "b2r_trace_kernel", "b2r_read_wide_nodes", "b2r_read_link_tables", "b2r_get_origin_box",
     "b2r_write_hdr", "b2r_read_hdr", "b2r_last_error", "b2r_abi_version",
 ]
 
@@ -74,7 +75,7 @@ def lib():
             "b2r_host_register": [vp, C.c_size_t], "b2r_host_unregister": [vp], "b2r_get_accumulations": [vp, vp], "b2r_set_accumulations": [vp, u32], "b2r_read_buckets": [vp, vp], "b2r_write_buckets": [vp, vp],
             "b2r_device_buckets": [vp, vp, vp], "b2r_device_framebuffer": [vp, vp, vp], "b2r_read_counters": [vp, vp], "b2r_reset_counters": [vp], "b2r_read_bounce_counts": [vp, vp, vp, u32],
             "b2r_read_kernel_times": [vp, vp, vp, C.c_int], "b2r_set_flags": [vp, u32], "b2r_generate_rays": [vp, u32, vp],
-            "b2r_save_checkpoint": [vp, C.c_char_p], "b2r_load_checkpoint": [vp, C.c_char_p], "b2r_write_hdr": [C.c_char_p, vp, u32, u32], "b2r_read_hdr": [C.c_char_p, vp, vp, vp], "b2r_trace_closest": [vp, vp, u32, vp, vp], "b2r_trace_shadow": [vp, vp, vp, u32, vp], "b2r_read_wide_nodes": [vp, vp, vp, vp], "b2r_get_origin_box": [vp, vp],
+            "b2r_save_checkpoint": [vp, C.c_char_p], "b2r_load_checkpoint": [vp, C.c_char_p], "b2r_write_hdr": [C.c_char_p, vp, u32, u32], "b2r_read_hdr": [C.c_char_p, vp, vp, vp], "b2r_trace_closest": [vp, vp, u32, vp, vp], "b2r_trace_shadow": [vp, vp, vp, u32, vp], "b2r_trace_kernel": [vp, C.c_int, vp, vp, vp, vp, u32, u32, vp, vp, vp], "b2r_read_wide_nodes": [vp, vp, vp, vp], "b2r_read_link_tables": [vp, vp, vp], "b2r_get_origin_box": [vp, vp],
         }
         for name, args in sig.items():
             fn = getattr(L, name); fn.argtypes = args; fn.restype = C.c_int
@@ -344,6 +345,32 @@ class Renderer:
     def trace_shadow(self, rays, tfar):
         r = np.ascontiguousarray(rays, np.float32); tf = np.ascontiguousarray(tfar, np.float32); n = len(r); o = np.empty(n, np.uint8)
         _check(lib().b2r_trace_shadow(self._h, _ptr(r), _ptr(tf), n, _ptr(o))); return o
+
+    def trace_kernel_closest(self, rays, tail=None):
+        """k_intersect_closest, the per-lane closest-hit kernel of bounces >= 1, on caller rays (b2r_trace_kernel). tail (n bools, with
+        FLAG_REFERENCE_EXACT): rays that take the scalar-tail sphere formula. Returns (tfar, prim) as trace_closest."""
+        r = np.ascontiguousarray(rays, np.float32); n = len(r); t = np.empty(n, np.float32); p = np.empty(n, np.int32)
+        tl = None if tail is None else np.ascontiguousarray(tail, np.uint8)
+        _check(lib().b2r_trace_kernel(self._h, TAP_CLOSEST, _ptr(r), None, None, _ptr(tl), n, 0, _ptr(t), _ptr(p), None)); return t, p
+
+    def trace_kernel_shadow(self, rays, tfar, origin_prim):
+        """k_intersect_shadow, the climbing any-hit kernel, on caller rays: ray i's walk starts at the node holding sphere origin_prim[i]
+        (BVH order; -1 = the root). Returns occlusion flags as trace_shadow."""
+        r = np.ascontiguousarray(rays, np.float32); tf = np.ascontiguousarray(tfar, np.float32); op = np.ascontiguousarray(origin_prim, np.int32)
+        n = len(r); o = np.empty(n, np.uint8)
+        _check(lib().b2r_trace_kernel(self._h, TAP_SHADOW, _ptr(r), _ptr(tf), _ptr(op), None, n, 0, None, None, _ptr(o))); return o
+
+    def trace_kernel_packet(self, acc):
+        """k_intersect_packet, the camera-ray kernel, on the camera rays of sample index acc: (tfar, prim) per pixel in tile order, entry t
+        for ray t of generate_rays(acc)."""
+        n = self.width * self.height; t = np.empty(n, np.float32); p = np.empty(n, np.int32)
+        _check(lib().b2r_trace_kernel(self._h, TAP_PACKET, None, None, None, None, n, acc, _ptr(t), _ptr(p), None)); return t, p
+
+    def link_tables(self):
+        """(parent, leaf_node) of the device tree as k_link_tables wrote them (b2r_read_link_tables)."""
+        n = C.c_uint32(0); _check(lib().b2r_read_wide_nodes(self._h, None, C.byref(n), None))
+        parent = np.empty(n.value, np.uint32); leaf = np.empty(len(self.scene.prims), np.uint32)
+        _check(lib().b2r_read_link_tables(self._h, _ptr(parent), _ptr(leaf))); return parent, leaf
 
     def wide_nodes(self):
         n = C.c_uint32(0); ms = C.c_uint32(0)

@@ -88,6 +88,7 @@ struct b2r_ctx {
 	std::vector<uint32_t> cur_geom_of_prim;  // after a refit into a new BVH order: that order's index -> geometry index (empty: wide_host's)
 	uint32_t* d_remap = nullptr; size_t cap_remap = 0;
 	uint8_t* d_trace = nullptr; size_t cap_trace = 0;  // b2r_trace_* staging (rays in, results out)
+	uint8_t* d_tap = nullptr; size_t cap_tap = 0;      // b2r_trace_kernel: the queue planes, counters and batch descriptor of its launches
 	bool wide_refit = false; double* d_cost = nullptr;  // b2r_refit_scene: the device tree no longer equals wide_host
 	// where ray origins may lie (leaf_half_extent, b2r_shade.h): bounds of the current spheres + camera + caller-supplied ray origins
 	OriginBox obox{}; bool obox_valid = false; float sph_lo[3] = {0, 0, 0}, sph_hi[3] = {0, 0, 0}; float cam_pos[3] = {0, 0, 0};
@@ -751,7 +752,7 @@ void b2r_destroy(b2r_ctx* c) {
 	drop_graph(c);
 	for (auto& t : c->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
 	dev_free(&c->d_prims); dev_free(&c->d_mat_albedo); dev_free(&c->d_mat_emission); dev_free(&c->d_mat_f0); dev_free(&c->d_light_sphere); dev_free(&c->d_light_emit);
-	dev_free(&c->d_hdri); dev_free(&c->d_prim_mat); dev_free(&c->d_wide); dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep);
+	dev_free(&c->d_hdri); dev_free(&c->d_prim_mat); dev_free(&c->d_wide); dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_tap); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep);
 	for (int k = 0; k < 2; k++) { dev_free(&c->d_mkey[k]); dev_free(&c->d_midx[k]); }
 	for (int s = 0; s < 2; s++) { dev_free(&c->d_A[s]); dev_free(&c->d_B[s]); dev_free(&c->d_T[s]); }
 	dev_free(&c->d_H); dev_free(&c->d_SA); dev_free(&c->d_SB); dev_free(&c->d_SL); dev_free(&c->d_SS); dev_free(&c->d_parent); dev_free(&c->d_leaf_node); dev_free(&c->d_rad); dev_free(&c->d_acc); dev_free(&c->d_fb);
@@ -1486,16 +1487,18 @@ int b2r_generate_rays(b2r_ctx* c, uint32_t acc, float* out_host) {
 	return B2R_OK;
 }
 
+// the leaf extents of the traversal tree must cover the finite origins of caller rays (rays[6 * i + 0..2])
+static int cover_ray_origins(b2r_ctx* c, const float* rays, uint32_t n) {
+	float pts[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
+	for (uint32_t i = 0; i < n; i++) for (int k = 0; k < 3; k++) { const float v = rays[6 * static_cast<size_t>(i) + k]; if (v == v && fabsf(v) <= FLT_MAX) { pts[k] = fminf(pts[k], v); pts[3 + k] = fmaxf(pts[3 + k], v); } }
+	return pts[0] <= pts[3] ? ensure_origin_box(c, pts, 2) : B2R_OK;
+}
 static int trace_common(b2r_ctx* c, const float* rays, const float* tfar_in, uint32_t n, int shadow, float* tfar_out, int32_t* prim_out, uint8_t* occ_out) {
 	if (!c || !rays) return fail(B2R_ERR_ARG, "null argument");
 	if (!c->have_scene) return fail(B2R_ERR_STATE, "upload_scene first");
 	if (n == 0) return B2R_OK;
 	int rc = ensure_device(c); if (rc) return rc;
-	if (c->use_bvh) {  // the leaf extents of the traversal tree must cover these ray origins
-		float pts[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
-		for (uint32_t i = 0; i < n; i++) for (int k = 0; k < 3; k++) { const float v = rays[6 * static_cast<size_t>(i) + k]; if (v == v && fabsf(v) <= FLT_MAX) { pts[k] = fminf(pts[k], v); pts[3 + k] = fmaxf(pts[3 + k], v); } }
-		if (pts[0] <= pts[3] && (rc = ensure_origin_box(c, pts, 2))) return rc;
-	}
+	if (c->use_bvh && (rc = cover_ray_origins(c, rays, n))) return rc;
 	c->main_reads_scene = true;  // (k_tap_trace reads the primary scene arrays on the caller's stream)
 	// one grow-only device block per context, carved into the five arrays (focus picking calls this per mouse click, Application.cpp:282-298)
 	const size_t n6 = (static_cast<size_t>(n) * 6 * sizeof(float) + 255) & ~static_cast<size_t>(255), n4 = (static_cast<size_t>(n) * 4 + 255) & ~static_cast<size_t>(255), n1 = (static_cast<size_t>(n) + 255) & ~static_cast<size_t>(255);
@@ -1521,6 +1524,116 @@ int b2r_trace_closest(b2r_ctx* c, const float* rays_host, uint32_t n, float* tfa
 int b2r_trace_shadow(b2r_ctx* c, const float* rays_host, const float* tfar_host, uint32_t n, uint8_t* occluded_out) {
 	if (!tfar_host || !occluded_out) return fail(B2R_ERR_ARG, "null argument");
 	return trace_common(c, rays_host, tfar_host, n, 1, nullptr, nullptr, occluded_out);
+}
+// The per-lane kernels take caller rays in chunks of this many: a chunk is one frame of `cap` pixels (the chunk rounded up to whole
+// tiles) and one sample, so ray i of a chunk has pid i.
+constexpr uint32_t kTapChunk = 1u << 16;
+int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfar, const int32_t* origin_prim, const uint8_t* tail,
+                     uint32_t n, uint32_t acc, float* tfar_out, int32_t* prim_out, uint8_t* occluded_out) {
+	if (!c) return fail(B2R_ERR_ARG, "null context");
+	const bool closest = kernel == B2R_TAP_CLOSEST, shadow = kernel == B2R_TAP_SHADOW, packet = kernel == B2R_TAP_PACKET;
+	if (!closest && !shadow && !packet) return fail(B2R_ERR_ARG, "unknown traversal kernel");
+	if ((!packet && !rays) || (shadow ? (!tfar || !origin_prim || !occluded_out) : (!tfar_out || !prim_out))) return fail(B2R_ERR_ARG, "null argument");
+	if (!c->have_scene) return fail(B2R_ERR_STATE, "upload_scene first");
+	if (!c->use_bvh) return fail(B2R_ERR_STATE, "the traversal kernels run on BVH contexts only");
+	if (packet && !c->have_camera) return fail(B2R_ERR_STATE, "set_camera first");
+	if (packet && n != c->params.frame.npix) return fail(B2R_ERR_ARG, "packet kernel: n must be width * height");
+	const uint32_t n_prims = c->params.scene.n_prims;
+	if (shadow) for (uint32_t i = 0; i < n; i++) if (origin_prim[i] >= static_cast<int32_t>(n_prims)) return fail(B2R_ERR_ARG, "origin_prim out of range");
+	if (n == 0) return B2R_OK;
+	int rc = ensure_device(c); if (rc) return rc;
+	if (!packet && (rc = cover_ray_origins(c, rays, n))) return rc;
+	cudaStream_t st = c->stream;
+	std::vector<uint32_t> leaf_node;  // where the shadow walks start, as k_shade takes it for a hit on that sphere
+	if (shadow) { leaf_node.resize(n_prims); CU(cudaMemcpyAsync(leaf_node.data(), c->d_leaf_node, n_prims * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)); CU(sync_main(c)); }
+	c->main_reads_scene = true;  // (the kernels read the primary scene arrays on the caller's stream)
+	// one grow-only block: the queue planes, RAD, the B2R_FLAG_REFERENCE_EXACT tables, counters and batch descriptors of these launches
+	// (never the context's own: its RAD may hold samples traced ahead, its queues may belong to a side in flight)
+	const uint32_t chunk = packet ? n : std::min(n, kTapChunk), cap = (chunk + 255u) & ~255u;
+	size_t off = 0; auto take = [&](size_t bytes) { const size_t at = off; off += (bytes + 255u) & ~static_cast<size_t>(255u); return at; };
+	const size_t o_a = take(cap * sizeof(float4)), o_b = take(cap * sizeof(float4)), o_t = take(3u * cap * sizeof(float)), o_h = take(cap * sizeof(float2)),
+	             o_sa = take(cap * sizeof(float4)), o_sb = take(cap * sizeof(float4)), o_sl = take(3u * cap * sizeof(float)), o_ss = take(cap * sizeof(uint32_t)),
+	             o_rad = take(3u * cap * sizeof(float)), o_slot = take(cap), o_act = take(cap / 256u * sizeof(uint16_t)), o_cnt = take(16u * sizeof(uint32_t)),
+	             o_stats = take(ST_COUNT * sizeof(unsigned long long)), o_batch = take((1u + kMaxLanes) * sizeof(BatchDev));
+	if ((rc = dev_reserve(&c->d_tap, &c->cap_tap, off))) return rc;
+	uint8_t* base = c->d_tap;
+	Params p = c->params;
+	p.q.A[0] = p.q.A[1] = reinterpret_cast<float4*>(base + o_a); p.q.B[0] = p.q.B[1] = reinterpret_cast<float4*>(base + o_b); p.q.T[0] = p.q.T[1] = reinterpret_cast<float*>(base + o_t);
+	p.q.H = reinterpret_cast<float2*>(base + o_h); p.q.SA = reinterpret_cast<float4*>(base + o_sa); p.q.SB = reinterpret_cast<float4*>(base + o_sb);
+	p.q.SL = reinterpret_cast<float*>(base + o_sl); p.q.SS = reinterpret_cast<uint32_t*>(base + o_ss); p.q.cap = cap;
+	p.rad = reinterpret_cast<float*>(base + o_rad);
+	p.ex.slot[0] = p.ex.slot[1] = base + o_slot; p.ex.act[0] = p.ex.act[1] = reinterpret_cast<uint16_t*>(base + o_act);
+	uint32_t* cnt = reinterpret_cast<uint32_t*>(base + o_cnt);   // paths, shadow, work_a, work_b: four bounces each
+	p.cnt.paths = cnt; p.cnt.shadow = cnt + 4; p.cnt.work_a = cnt + 8; p.cnt.work_b = cnt + 12;
+	p.cnt.stats = reinterpret_cast<unsigned long long*>(base + o_stats);
+	BatchDev* batch = reinterpret_cast<BatchDev*>(base + o_batch); p.batch = batch;
+	const KernelSet k = pick_kernels(c);
+	std::vector<float2> h(chunk);
+	if (packet) {  // one sample of the context's own frame, camera and sample index acc
+		BatchArgs a; a.n = 1u; a.acc[0] = acc; a.cam = c->params.frame.cam;
+		k_set_batch<<<1, kMaxSlots, 0, st>>>(batch, a);
+		CU(cudaMemsetAsync(cnt, 0, 16u * sizeof(uint32_t), st));
+		k.packet<<<c->grid_packet, kTravBlock, 0, st>>>(p, 0u);
+		CU(cudaGetLastError()); c->launches += 2;
+		CU(cudaMemcpyAsync(h.data(), p.q.H, n * sizeof(float2), cudaMemcpyDeviceToHost, st));
+		CU(sync_main(c));
+		for (uint32_t i = 0; i < n; i++) { tfar_out[i] = h[i].x; std::memcpy(&prim_out[i], &h[i].y, sizeof(int32_t)); }
+		return B2R_OK;
+	}
+	p.frame.npix = cap; p.frame.npix_magic = magic_for(cap);
+	std::vector<float4> ha(chunk), hb(chunk);
+	std::vector<uint32_t> hs(chunk);
+	std::vector<uint8_t> hslot(chunk);
+	std::vector<float> hrad(chunk);
+	if (shadow) { const std::vector<float> ones(3u * static_cast<size_t>(cap), 1.0f); CU(cudaMemcpyAsync(p.q.SL, ones.data(), ones.size() * sizeof(float), cudaMemcpyHostToDevice, st)); CU(sync_main(c)); }
+	else {  // with B2R_FLAG_REFERENCE_EXACT a ray takes the scalar tail when its slot >= (act & ~7) = 8: exactly the rays marked 255 below
+		const std::vector<uint16_t> act(cap / 256u, static_cast<uint16_t>(8u));
+		CU(cudaMemcpyAsync(p.ex.act[1], act.data(), act.size() * sizeof(uint16_t), cudaMemcpyHostToDevice, st)); CU(sync_main(c));
+	}
+	for (uint32_t first = 0; first < n; first += chunk) {
+		const uint32_t m = std::min(chunk, n - first);
+		for (uint32_t i = 0; i < m; i++) {
+			const float* r = rays + 6 * static_cast<size_t>(first + i);
+			float pid; const uint32_t pid_i = i; std::memcpy(&pid, &pid_i, sizeof pid);  // slot 0, pixel i
+			ha[i] = make_float4(r[0], r[1], r[2], r[3]);
+			hb[i] = make_float4(r[4], r[5], shadow ? tfar[first + i] : 0.0f, pid);
+			if (shadow) { const int32_t o = origin_prim[first + i]; hs[i] = o < 0 ? 0u : leaf_node[o]; }
+			else hslot[i] = tail && tail[first + i] ? 255u : 0u;
+		}
+		uint32_t counts[16] = {0};
+		if (shadow) counts[4] = m; else counts[1] = m;   // shadow rays of bounce 0 / paths entering bounce 1 (queue side 1)
+		CU(cudaMemcpyAsync(cnt, counts, sizeof counts, cudaMemcpyHostToDevice, st));
+		CU(cudaMemcpyAsync(shadow ? p.q.SA : p.q.A[1], ha.data(), m * sizeof(float4), cudaMemcpyHostToDevice, st));
+		CU(cudaMemcpyAsync(shadow ? p.q.SB : p.q.B[1], hb.data(), m * sizeof(float4), cudaMemcpyHostToDevice, st));
+		if (shadow) {
+			CU(cudaMemcpyAsync(p.q.SS, hs.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+			CU(cudaMemsetAsync(p.rad, 0, 3u * static_cast<size_t>(cap) * sizeof(float), st));
+			k.shadow<<<c->grid_shadow, kTravBlock, 0, st>>>(p, 0u);
+			CU(cudaGetLastError()); c->launches++;
+			CU(cudaMemcpyAsync(hrad.data(), p.rad, m * sizeof(float), cudaMemcpyDeviceToHost, st));   // a lit ray adds its L = 1 to RAD
+			CU(sync_main(c));
+			for (uint32_t i = 0; i < m; i++) occluded_out[first + i] = hrad[i] == 0.0f ? 1u : 0u;
+		} else {
+			CU(cudaMemcpyAsync(p.ex.slot[1], hslot.data(), m, cudaMemcpyHostToDevice, st));
+			k.closest<<<c->grid_closest, kTravBlock, 0, st>>>(p, 1u);
+			CU(cudaGetLastError()); c->launches++;
+			CU(cudaMemcpyAsync(h.data(), p.q.H, m * sizeof(float2), cudaMemcpyDeviceToHost, st));
+			CU(sync_main(c));
+			for (uint32_t i = 0; i < m; i++) { tfar_out[first + i] = h[i].x; std::memcpy(&prim_out[first + i], &h[i].y, sizeof(int32_t)); }
+		}
+	}
+	return B2R_OK;
+}
+int b2r_read_link_tables(b2r_ctx* c, uint32_t* parent_out, uint32_t* leaf_node_out) {
+	if (!c || !parent_out || !leaf_node_out) return fail(B2R_ERR_ARG, "null argument");
+	if (!c->have_scene) return fail(B2R_ERR_STATE, "upload_scene first");
+	if (!c->use_bvh) return fail(B2R_ERR_STATE, "a brute-force context has no traversal tree");
+	int rc = ensure_device(c); if (rc) return rc;
+	c->main_reads_scene = true;
+	CU(cudaMemcpyAsync(parent_out, c->d_parent, static_cast<size_t>(c->n_wide) * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaMemcpyAsync(leaf_node_out, c->d_leaf_node, static_cast<size_t>(c->params.scene.n_prims) * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(sync_main(c));
+	return B2R_OK;
 }
 int b2r_get_origin_box(b2r_ctx* c, float out[6]) {
 	if (!c || !out) return fail(B2R_ERR_ARG, "null argument");

@@ -250,8 +250,23 @@ int  b2r_generate_rays(b2r_ctx* ctx, uint32_t acc, float* out_host);
  * rays_host[n*6] = origin, dir. closest: tfar_out[n] (FLT_MAX on miss), prim_out[n] (BVH-order index or -1). */
 int  b2r_trace_closest(b2r_ctx* ctx, const float* rays_host, uint32_t n, float* tfar_out, int32_t* prim_out);
 int  b2r_trace_shadow(b2r_ctx* ctx, const float* rays_host, const float* tfar_host, uint32_t n, uint8_t* occluded_out);
+/* The traversal kernels a frame uses, on caller input (tests): the instantiation and grid the context's flags and scene select for a
+ * frame, run on queue buffers of the call's own, so nothing of the renderer's state (queues, samples traced ahead, counters) is touched.
+ * B2R_ERR_STATE before an upload or on a brute-force context; B2R_ERR_ARG for a null pointer the kernel needs or an unknown kernel.
+ *  B2R_TAP_CLOSEST  k_intersect_closest: rays[n*6] -> tfar_out[n], prim_out[n] (as b2r_trace_closest). tail: NULL or n bytes; with
+ *                   B2R_FLAG_REFERENCE_EXACT, nonzero = this ray takes the scalar-tail sphere formula (BVH.hpp:270-286).
+ *  B2R_TAP_SHADOW   k_intersect_shadow: rays, tfar[n] -> occluded_out[n]; ray i's walk starts at the wide node holding sphere
+ *                   origin_prim[i] (BVH order), or at the root for -1, and climbs (B2R_ERR_ARG for an index >= the sphere count).
+ *  B2R_TAP_PACKET   k_intersect_packet on the camera rays of sample index acc (rays unused): n == width*height (else B2R_ERR_ARG),
+ *                   tfar_out / prim_out in tile order, entry t being ray t of b2r_generate_rays(acc). */
+enum { B2R_TAP_CLOSEST = 0, B2R_TAP_SHADOW = 1, B2R_TAP_PACKET = 2 };
+int  b2r_trace_kernel(b2r_ctx* ctx, int kernel, const float* rays, const float* tfar, const int32_t* origin_prim, const uint8_t* tail,
+                      uint32_t n, uint32_t acc, float* tfar_out, int32_t* prim_out, uint8_t* occluded_out);
 /* the flattened 128-byte node array (for the layout round-trip test): out may be NULL to size */
 int  b2r_read_wide_nodes(b2r_ctx* ctx, void* out_host, uint32_t* n_wide_nodes, uint32_t* max_stack);
+/* the link tables k_link_tables derives from the device tree: parent_out[n_wide_nodes] (the node that links to node i, 0 for the root)
+ * and leaf_node_out[n_prims] (the node whose leaf slot holds sphere i, BVH order). Synchronises. */
+int  b2r_read_link_tables(b2r_ctx* ctx, uint32_t* parent_out, uint32_t* leaf_node_out);
 /* the box ray origins are assumed to lie in ({lo.xyz, hi.xyz}: sphere bounds, camera, origins passed to b2r_trace_*): the leaf slots of the
  * traversal tree are sized for it, so a host twin of the tree needs the same box (tests) */
 int  b2r_get_origin_box(b2r_ctx* ctx, float lo_hi_out[6]);
