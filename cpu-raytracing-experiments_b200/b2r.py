@@ -36,7 +36,7 @@ COUNTER_NAMES = ["extension_rays", "shadow_rays", "shaded_hits", "terminated", "
 # every symbol include/b2r.h declares (tests/test_abi.py checks the header against this list and the library against both)
 ABI_SYMBOLS = [
     "b2r_bvh_build", "b2r_bvh_build_ex", "b2r_find_lights", "b2r_camera_lookat", "b2r_camera_ray", "b2r_create", "b2r_destroy", "b2r_resize", "b2r_reset", "b2r_set_stream",
-    "b2r_sync", "b2r_upload_scene", "b2r_refit_scene", "b2r_set_camera", "b2r_accumulate", "b2r_resolve", "b2r_resolve_async", "b2r_resolve_device", "b2r_frame_wait", "b2r_resolve_from", "b2r_ipc_export_buckets", "b2r_ipc_open_peers", "b2r_ipc_close", "b2r_resolve_peers", "b2r_team_export", "b2r_team_open", "b2r_team_resolve", "b2r_team_error", "b2r_team_close", "b2r_host_register", "b2r_host_unregister", "b2r_get_accumulations", "b2r_set_accumulations",
+    "b2r_sync", "b2r_upload_scene", "b2r_refit_scene", "b2r_set_camera", "b2r_set_lens", "b2r_accumulate", "b2r_resolve", "b2r_resolve_async", "b2r_resolve_device", "b2r_frame_wait", "b2r_resolve_from", "b2r_ipc_export_buckets", "b2r_ipc_open_peers", "b2r_ipc_close", "b2r_resolve_peers", "b2r_team_export", "b2r_team_open", "b2r_team_resolve", "b2r_team_error", "b2r_team_close", "b2r_host_register", "b2r_host_unregister", "b2r_get_accumulations", "b2r_set_accumulations",
     "b2r_read_buckets", "b2r_write_buckets", "b2r_save_checkpoint", "b2r_load_checkpoint", "b2r_device_buckets", "b2r_device_framebuffer", "b2r_read_counters", "b2r_reset_counters", "b2r_read_bounce_counts",
     "b2r_read_kernel_times", "b2r_set_flags", "b2r_generate_rays", "b2r_trace_closest", "b2r_trace_shadow", "b2r_trace_kernel", "b2r_read_wide_nodes", "b2r_read_link_tables", "b2r_get_origin_box",
     "b2r_write_hdr", "b2r_read_hdr", "b2r_last_error", "b2r_abi_version",
@@ -71,7 +71,7 @@ def lib():
             "b2r_set_stream": [vp, vp], "b2r_sync": [vp],
             "b2r_upload_scene": [vp, vp, vp, u32, u32, vp, u32, vp, u32, vp, u32, vp, vp, i32, i32],
             "b2r_refit_scene": [vp, vp, u32, vp, u32, vp, u32, vp, u32, vp],
-            "b2r_set_camera": [vp, vp, vp, f32, f32, f32, f32], "b2r_accumulate": [vp, u32], "b2r_resolve": [vp, vp, C.c_int], "b2r_resolve_async": [vp, vp, C.c_int], "b2r_resolve_device": [vp, C.c_int], "b2r_frame_wait": [vp], "b2r_resolve_from": [vp, vp, vp, C.c_int], "b2r_ipc_export_buckets": [vp, vp], "b2r_ipc_open_peers": [vp, vp, u32, u32], "b2r_ipc_close": [vp], "b2r_resolve_peers": [vp, vp, C.c_int], "b2r_team_export": [vp, vp], "b2r_team_open": [vp, vp, u32, u32], "b2r_team_resolve": [vp, vp, C.c_int, C.c_int], "b2r_team_error": [vp, vp], "b2r_team_close": [vp],
+            "b2r_set_camera": [vp, vp, vp, f32, f32, f32, f32], "b2r_set_lens": [vp, f32, f32], "b2r_accumulate": [vp, u32], "b2r_resolve": [vp, vp, C.c_int], "b2r_resolve_async": [vp, vp, C.c_int], "b2r_resolve_device": [vp, C.c_int], "b2r_frame_wait": [vp], "b2r_resolve_from": [vp, vp, vp, C.c_int], "b2r_ipc_export_buckets": [vp, vp], "b2r_ipc_open_peers": [vp, vp, u32, u32], "b2r_ipc_close": [vp], "b2r_resolve_peers": [vp, vp, C.c_int], "b2r_team_export": [vp, vp], "b2r_team_open": [vp, vp, u32, u32], "b2r_team_resolve": [vp, vp, C.c_int, C.c_int], "b2r_team_error": [vp, vp], "b2r_team_close": [vp],
             "b2r_host_register": [vp, C.c_size_t], "b2r_host_unregister": [vp], "b2r_get_accumulations": [vp, vp], "b2r_set_accumulations": [vp, u32], "b2r_read_buckets": [vp, vp], "b2r_write_buckets": [vp, vp],
             "b2r_device_buckets": [vp, vp, vp], "b2r_device_framebuffer": [vp, vp, vp], "b2r_read_counters": [vp, vp], "b2r_reset_counters": [vp], "b2r_read_bounce_counts": [vp, vp, vp, u32],
             "b2r_read_kernel_times": [vp, vp, vp, C.c_int], "b2r_set_flags": [vp, u32], "b2r_generate_rays": [vp, u32, vp],
@@ -207,6 +207,12 @@ class Renderer:
         cam = np.ascontiguousarray(cam11, np.float32)
         self._cam = cam
         _check(lib().b2r_set_camera(self._h, _ptr(cam[0:3]), _ptr(cam[3:7]), float(cam[7]), float(cam[8]), float(cam[9]), float(cam[10])))
+
+    def SetLens(self, radius, focus_distance):
+        """Thin-lens depth of field (b2r_set_lens): lens radius and focus distance in scene units (the caller converts the app's
+        Projection::aperture_radius, which is in mm); the plane at focus_distance along the view direction is sharp. radius 0 = the
+        pinhole camera, bit for bit. Takes effect from the next Accumulate, like SetCamera."""
+        _check(lib().b2r_set_lens(self._h, float(radius), float(focus_distance)))
 
     # -- Renderer.hpp:53-67
     def Resize(self, width, height):

@@ -24,7 +24,7 @@ enum KernelKind { KK_GENERATE = 0, KK_BRUTE, KK_CLOSEST, KK_SHADE, KK_SHADOW, KK
 
 constexpr uint32_t kMaxLanes = 4;
 struct BatchArgs {
-	uint32_t n; uint32_t acc[kMaxSlots]; unsigned long long fold = ~0ull; CameraParams cam;
+	uint32_t n; uint32_t acc[kMaxSlots]; unsigned long long fold = ~0ull; CameraParams cam; LensParams lens{0.0f, 0.0f};
 	// lanes (run_batch): lane j holds n_lane[j] consecutive samples of the batch in slots [j * lane_slots, j * lane_slots + n_lane[j]); the slots
 	// between the lanes hold nothing. lanes == 0: one lane, slots 0..n-1.
 	uint32_t lanes = 0, lane_slots = 0, n_lane[kMaxLanes] = {0, 0, 0, 0};
@@ -36,11 +36,11 @@ struct BatchArgs {
 };
 // dst[0] describes the whole batch (k_accumulate), dst[1 + j] lane j's part of it (slot numbers local to the lane)
 __global__ void k_set_batch(BatchDev* dst, const BatchArgs a) {
-	if (threadIdx.x == 0) { dst[0].n_slots = a.n; dst[0].fold = a.fold; dst[0].cam = a.cam; }
+	if (threadIdx.x == 0) { dst[0].n_slots = a.n; dst[0].fold = a.fold; dst[0].cam = a.cam; dst[0].lens = a.lens; }
 	if (threadIdx.x < a.n) dst[0].acc[threadIdx.x] = a.acc[threadIdx.x];
 	for (uint32_t j = 0; j < kMaxLanes; j++) {
 		const uint32_t nj = j < a.lanes ? a.n_lane[j] : 0u;
-		if (threadIdx.x == 0) { dst[1 + j].n_slots = nj; dst[1 + j].fold = 0ull; dst[1 + j].cam = a.cam; }
+		if (threadIdx.x == 0) { dst[1 + j].n_slots = nj; dst[1 + j].fold = 0ull; dst[1 + j].cam = a.cam; dst[1 + j].lens = a.lens; }
 		if (threadIdx.x < nj) dst[1 + j].acc[threadIdx.x] = a.acc[j * a.lane_slots + threadIdx.x];
 	}
 }
@@ -92,6 +92,7 @@ struct b2r_ctx {
 	bool wide_refit = false; double* d_cost = nullptr;  // b2r_refit_scene: the device tree no longer equals wide_host
 	// where ray origins may lie (leaf_half_extent, b2r_shade.h): bounds of the current spheres + camera + caller-supplied ray origins
 	OriginBox obox{}; bool obox_valid = false; float sph_lo[3] = {0, 0, 0}, sph_hi[3] = {0, 0, 0}; float cam_pos[3] = {0, 0, 0};
+	LensParams lens{0.0f, 0.0f};  // b2r_set_lens: radius 0 = pinhole (the instantiations without LENS)
 	// frame
 	float4 *d_A[2] = {nullptr, nullptr}, *d_B[2] = {nullptr, nullptr}, *d_SA = nullptr, *d_SB = nullptr, *d_fb = nullptr;
 	float *d_T[2] = {nullptr, nullptr}, *d_SL = nullptr, *d_rad = nullptr, *d_acc = nullptr;
@@ -106,6 +107,7 @@ struct b2r_ctx {
 	int grid_brute_first_exact = 0, grid_brute_exact = 0;
 	int grid_brute_first_ggx = 0, grid_brute_ggx = 0, grid_brute_finish_ggx = 0, grid_shade_ggx = 0;
 	int grid_brute_first = 0, grid_brute = 0, grid_closest = 0, grid_shade = 0, grid_shadow = 0, grid_stream = 0, grid_packet = 0, grid_brute_finish = 0; bool packet_primary = true;
+	int grid_brute_first_lens = 0, grid_brute_first_ggx_lens = 0, grid_packet_lens = 0;  // thin-lens bounce-0 instantiations
 	cudaGraphExec_t graph_exec = nullptr; bool graph_valid = false;
 	// twin lanes: a batch of two or more samples is traced as two independent half batches on two streams (own queues, counters and batch
 	// descriptors) inside one graph, so that the drained end of every launch of one half is filled by the other half's kernels
@@ -249,6 +251,9 @@ int compute_grids(b2r_ctx* c) {
 	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, true>), kBruteBlock, &c->grid_brute_ggx))) return rc;
 	if ((rc = occ(reinterpret_cast<const void*>(&k_brute_finish<false, true>), kBruteBlock, &c->grid_brute_finish_ggx))) return rc;
 	if ((rc = occ(reinterpret_cast<const void*>(&k_shade<false, true>), kBruteBlock, &c->grid_shade_ggx))) return rc;
+	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, true>), kBruteBlock, &c->grid_brute_first_lens))) return rc;
+	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, true>), kBruteBlock, &c->grid_brute_first_ggx_lens))) return rc;
+	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_packet<false, B2R_PACKET_RPL_LENS, true>), kTravBlock, &c->grid_packet_lens))) return rc;
 	c->packet_primary = std::getenv("B2R_NO_PACKET") == nullptr;  // A/B switch for measurements: per-lane walks for the camera rays too
 	c->lanes_max = std::getenv("B2R_NO_TWIN") ? 1u : 2u;          // A/B switches for measurements: every batch as one lane / B2R_LANES = 1, 2 or 4
 	if (const char* e = std::getenv("B2R_SIDES")) { c->sides = std::atoi(e) == 1 ? 1u : 2u; }   // A/B switch: 1 = every batch on the caller's stream, one after the other
@@ -273,20 +278,27 @@ template <typename F> int launch(b2r_ctx* c, int kind, bool profile, F&& f) {
 using BounceKernel = void (*)(const Params, const uint32_t);
 struct KernelSet {
 	BounceKernel brute_first, brute, brute_finish, packet, closest, shade, shadow;
-	int g_brute_first, g_brute, g_brute_finish;
+	void (*generate)(const Params);
+	int g_brute_first, g_brute, g_brute_finish, g_packet;
 };
 KernelSet pick_kernels(const b2r_ctx* c) {
 	const bool count = (c->cfg.flags & B2R_FLAG_COUNT_TESTS) != 0, exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0, ggx = (c->cfg.flags & B2R_FLAG_GGX) != 0;
 	const bool tn16 = c->params.scene.stack_tn_bits == 16u;  // stack entries split 16/16 (up to 65536 wide nodes: C3) get immediate shifts; other sizes read the split from the scene
+	const bool lens = c->lens.radius > 0.0f && !exact;  // (b2r_set_lens refuses a reference-exact context)
 	KernelSet k{};
 	// brute-force pipeline: <FIRST, COUNT, EXACT, GGX> (the GGX closure's kernels are built without the sphere-test counters)
 	if (ggx)        { k.brute_first = k_bounce_brute<true, false, false, true>; k.brute = k_bounce_brute<false, false, false, true>; k.g_brute_first = c->grid_brute_first_ggx; k.g_brute = c->grid_brute_ggx; }
 	else if (exact) { k.brute_first = count ? k_bounce_brute<true, true, true> : k_bounce_brute<true, false, true>; k.brute = count ? k_bounce_brute<false, true, true> : k_bounce_brute<false, false, true>; k.g_brute_first = c->grid_brute_first_exact; k.g_brute = c->grid_brute_exact; }
 	else            { k.brute_first = count ? k_bounce_brute<true, true, false> : k_bounce_brute<true, false, false>; k.brute = count ? k_bounce_brute<false, true, false> : k_bounce_brute<false, false, false>; k.g_brute_first = c->grid_brute_first; k.g_brute = c->grid_brute; }
+	// thin lens: only bounce 0 changes (later bounces read their origins from the path records)
+	if (lens && ggx) { k.brute_first = k_bounce_brute<true, false, false, true, true>; k.g_brute_first = c->grid_brute_first_ggx_lens; }
+	else if (lens)   { k.brute_first = count ? k_bounce_brute<true, true, false, false, true> : k_bounce_brute<true, false, false, false, true>; k.g_brute_first = c->grid_brute_first_lens; }
 	k.brute_finish = ggx ? k_brute_finish<false, true> : count ? k_brute_finish<true> : k_brute_finish<false>;
 	k.g_brute_finish = ggx ? c->grid_brute_finish_ggx : c->grid_brute_finish;
 	// BVH pipeline
-	k.packet = count ? k_intersect_packet<true, B2R_PACKET_RPL> : k_intersect_packet<false, B2R_PACKET_RPL>;
+	if (lens) { k.packet = count ? k_intersect_packet<true, B2R_PACKET_RPL_LENS, true> : k_intersect_packet<false, B2R_PACKET_RPL_LENS, true>; k.g_packet = c->grid_packet_lens; }
+	else      { k.packet = count ? k_intersect_packet<true, B2R_PACKET_RPL> : k_intersect_packet<false, B2R_PACKET_RPL>; k.g_packet = c->grid_packet; }
+	k.generate = lens ? k_generate<true> : k_generate<false>;
 	if (exact) k.closest = count ? (tn16 ? k_intersect_closest<true, true, 16u> : k_intersect_closest<true, true, 0u>) : (tn16 ? k_intersect_closest<false, true, 16u> : k_intersect_closest<false, true, 0u>);
 	else       k.closest = count ? (tn16 ? k_intersect_closest<true, false, 16u> : k_intersect_closest<true, false, 0u>) : (tn16 ? k_intersect_closest<false, false, 16u> : k_intersect_closest<false, false, 0u>);
 	k.shade = ggx ? k_shade<false, true> : exact ? k_shade<true> : k_shade<false>;
@@ -319,10 +331,10 @@ int enqueue_rounds(b2r_ctx* c, const Params& p_in, cudaStream_t st, bool profile
 		}
 		return B2R_OK;
 	}
-	if (!c->packet_primary && (rc = launch(c, KK_GENERATE, profile, [&] { k_generate<<<c->grid_stream, kBlock, 0, st>>>(p); }))) return rc;  // (the packet kernel generates the camera rays itself)
+	if (!c->packet_primary && (rc = launch(c, KK_GENERATE, profile, [&] { k.generate<<<c->grid_stream, kBlock, 0, st>>>(p); }))) return rc;  // (the packet kernel generates the camera rays itself)
 	const bool mis = !(c->cfg.flags & B2R_FLAG_NO_MIS);
 	for (uint32_t b = 0; b < mb; b++) {
-		if (b == 0 && c->packet_primary) { if ((rc = run(KK_CLOSEST, k.packet, G(c->grid_packet), kTravBlock, b))) return rc; }  // camera rays: one walk per warp
+		if (b == 0 && c->packet_primary) { if ((rc = run(KK_CLOSEST, k.packet, G(k.g_packet), kTravBlock, b))) return rc; }  // camera rays: one walk per warp
 		else if ((rc = run(KK_CLOSEST, k.closest, G(c->grid_closest), kTravBlock, b))) return rc;
 		if ((rc = run(KK_SHADE, k.shade, G(ggx ? c->grid_shade_ggx : c->grid_shade), kBruteBlock, b))) return rc;
 		if (exact && b + 1 < mb && (rc = run(KK_SHADE, k_stream_rank, c->grid_stream, 256, b))) return rc;
@@ -424,7 +436,7 @@ int run_batch(b2r_ctx* c, BatchArgs& args) {
 		}
 		args.lanes = lanes; args.lane_slots = ls; args.n = span; args.fold = fold;
 	} else { args.lanes = 0; args.lane_slots = 0; if (args.n < 64u) args.fold &= (1ull << args.n) - 1ull; }
-	args.cam = c->params.frame.cam;  // the camera travels with the batch descriptor: a camera move leaves the captured graph alone
+	args.cam = c->params.frame.cam; args.lens = c->lens;  // the camera and lens travel with the batch descriptor: a camera move leaves the captured graph alone
 	if (use_sides(c)) {
 		const uint32_t sidx = c->next_side; c->next_side ^= 1u;
 		b2r_ctx::Side& S = c->side[sidx];
@@ -689,13 +701,26 @@ int launch_link_tables(b2r_ctx* c) {
 	CU(cudaGetLastError()); c->launches++;
 	return B2R_OK;
 }
+// The points the camera's rays leave from, for the origin box (out: up to two points, returns how many): none before b2r_set_camera, the
+// eye without a lens, and with a lens of radius R the corners pos - R and pos + R of the cube that holds the lens disk in any orientation.
+// A lens origin pos + orient * L can round a few ulp beyond that cube; the origin box's slack (origin_box_rule: an eighth of the extent, which
+// is at least 2R, plus 1 on every side) absorbs that whenever ulp(|pos| + R) < R / 4 + 1, i.e. unless the eye lies more than ~2^24 lens radii
+// (and units) from the origin. DESIGN §2's domain (origins below 2^61) holds for lens origins as for any other.
+uint32_t camera_origins(const b2r_ctx* c, float out[6]) {
+	if (!c->have_camera) return 0u;
+	const float r = c->lens.radius;
+	if (r == 0.0f) { for (int k = 0; k < 3; k++) out[k] = c->cam_pos[k]; return 1u; }
+	for (int k = 0; k < 3; k++) { out[k] = c->cam_pos[k] - r; out[3 + k] = c->cam_pos[k] + r; }
+	return 2u;
+}
 // Ray origins about to be used (camera position, caller-supplied rays) must lie in the origin box the leaf extents were computed for;
 // if they do not, the box grows and the device tree's boxes are recomputed for it (tens of microseconds; the box has an eighth of
 // slack on every side, so an interactive camera move does not get here every frame).
 int ensure_origin_box(b2r_ctx* c, const float* points, uint32_t n_points) {
 	if (c->obox_valid && origin_box_holds(c->obox, points, n_points)) return B2R_OK;
 	std::vector<float> extra(points, points + 3 * static_cast<size_t>(n_points));
-	if (c->have_camera) extra.insert(extra.end(), c->cam_pos, c->cam_pos + 3);
+	float cam[6]; const uint32_t n_cam = camera_origins(c, cam);
+	extra.insert(extra.end(), cam, cam + 3 * n_cam);
 	if (c->obox_valid) { extra.insert(extra.end(), c->obox.lo, c->obox.lo + 3); extra.insert(extra.end(), c->obox.hi, c->obox.hi + 3); }  // never shrinks between uploads
 	c->obox = origin_box_rule(c->sph_lo, c->sph_hi, extra.data(), static_cast<uint32_t>(extra.size() / 3)); c->obox_valid = true;
 	if (c->have_wide && !c->gpu_tree) wide_fill_boxes(c->wide_host, c->wide_host.prims.data(), c->obox);  // the host copy (and its reference cost) follows: same routine, same result
@@ -880,8 +905,9 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 		// the tree is built on the device below (after the spheres have been copied): only its shape is worked out here
 		float lo[3], hi[3]; sphere_bounds(prims, n_prims, lo, hi);
 		const float corners[6] = {lo[0], lo[1], lo[2], hi[0], hi[1], hi[2]};
-		if (!c->obox_valid || !origin_box_holds(c->obox, corners, 2) || (c->have_camera && !origin_box_holds(c->obox, c->cam_pos, 1)))
-			{ c->obox = origin_box_rule(lo, hi, c->have_camera ? c->cam_pos : nullptr, c->have_camera ? 1u : 0u); c->obox_valid = true; }
+		float cam[6]; const uint32_t n_cam = camera_origins(c, cam);
+		if (!c->obox_valid || !origin_box_holds(c->obox, corners, 2) || !origin_box_holds(c->obox, cam, n_cam))
+			{ c->obox = origin_box_rule(lo, hi, cam, n_cam); c->obox_valid = true; }
 		for (int k = 0; k < 3; k++) { c->sph_lo[k] = lo[k]; c->sph_hi[k] = hi[k]; c->wide_host.sphere_lo[k] = lo[k]; c->wide_host.sphere_hi[k] = hi[k]; }
 		WideBvh& w = c->wide_host;
 		w.nodes.clear(); w.prims.clear(); w.geom_of_prim.clear(); w.cost = 0.0; w.ob = c->obox;
@@ -907,8 +933,9 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 			float lo[3], hi[3]; sphere_bounds(prims, n_prims, lo, hi);
 			// the origin box is kept while it still holds the spheres and the camera; a different scene starts from a fresh one
 			const float corners[6] = {lo[0], lo[1], lo[2], hi[0], hi[1], hi[2]};
-			if (!same_tree || !c->obox_valid || !origin_box_holds(c->obox, corners, 2) || (c->have_camera && !origin_box_holds(c->obox, c->cam_pos, 1)))
-				{ c->obox = origin_box_rule(lo, hi, c->have_camera ? c->cam_pos : nullptr, c->have_camera ? 1u : 0u); c->obox_valid = true; }
+			float cam[6]; const uint32_t n_cam = camera_origins(c, cam);
+			if (!same_tree || !c->obox_valid || !origin_box_holds(c->obox, corners, 2) || !origin_box_holds(c->obox, cam, n_cam))
+				{ c->obox = origin_box_rule(lo, hi, cam, n_cam); c->obox_valid = true; }
 			for (int k = 0; k < 3; k++) { c->sph_lo[k] = lo[k]; c->sph_hi[k] = hi[k]; }
 			if (!same_tree) {
 				if (ref_tree) flatten_bvh(nodes, n_nodes, prims, n_prims, c->wide_host, &c->obox);
@@ -1056,8 +1083,9 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 		float lo[3], hi[3]; sphere_bounds(prims, n_prims, lo, hi);
 		for (int k = 0; k < 3; k++) { c->sph_lo[k] = lo[k]; c->sph_hi[k] = hi[k]; }
 		const float corners[6] = {lo[0], lo[1], lo[2], hi[0], hi[1], hi[2]};
+		float cam[6]; const uint32_t n_cam = camera_origins(c, cam);
 		if (!c->obox_valid || !origin_box_holds(c->obox, corners, 2)) {
-			c->obox = origin_box_rule(lo, hi, c->have_camera ? c->cam_pos : nullptr, c->have_camera ? 1u : 0u); c->obox_valid = true;
+			c->obox = origin_box_rule(lo, hi, cam, n_cam); c->obox_valid = true;
 			if (!c->gpu_tree) wide_fill_boxes(c->wide_host, c->wide_host.prims.data(), c->obox);  // the as-built tree (reference cost) for the same origin box
 		}
 	}
@@ -1095,7 +1123,27 @@ int b2r_set_camera(b2r_ctx* c, const float pos[3], const float q[4], float half_
 	if (!c->have_camera || std::memcmp(&cam, &c->params.frame.cam, sizeof cam) != 0) { c->params.frame.cam = cam; drop_speculation(c); }  // samples traced ahead saw the old camera
 	c->have_camera = true;
 	c->cam_pos[0] = pos[0]; c->cam_pos[1] = pos[1]; c->cam_pos[2] = pos[2];
-	if (c->have_scene) return ensure_origin_box(c, c->cam_pos, 1);
+	float pts[6]; const uint32_t n_pts = camera_origins(c, pts);
+	if (c->have_scene) return ensure_origin_box(c, pts, n_pts);
+	return B2R_OK;
+}
+
+int b2r_set_lens(b2r_ctx* c, float lens_radius, float focus_distance) {
+	if (!c) return fail(B2R_ERR_ARG, "null context");
+	if (!(lens_radius >= 0.0f && lens_radius <= FLT_MAX)) return fail(B2R_ERR_ARG, "lens_radius must be finite and >= 0");
+	if (!(focus_distance > 0.0f && focus_distance <= FLT_MAX)) return fail(B2R_ERR_ARG, "focus_distance must be finite and > 0");
+	if (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) return fail(B2R_ERR_STATE, "B2R_FLAG_REFERENCE_EXACT reproduces the reference's pinhole camera: no lens");
+	int rc = ensure_device(c); if (rc) return rc;
+	// the lens travels with every batch's descriptor as the camera does; switching between pinhole and lens switches the bounce-0 kernels,
+	// which are part of the captured graph
+	const LensParams lens{lens_radius, focus_distance};
+	if (std::memcmp(&lens, &c->lens, sizeof lens) != 0) {
+		const bool switched = (lens_radius > 0.0f) != (c->lens.radius > 0.0f);
+		c->lens = lens;
+		if (switched) drop_graph(c); else drop_speculation(c);  // samples traced ahead saw the old lens
+	}
+	float cam[6]; const uint32_t n_cam = camera_origins(c, cam);
+	if (c->have_scene) return ensure_origin_box(c, cam, n_cam);
 	return B2R_OK;
 }
 
@@ -1478,7 +1526,8 @@ int b2r_generate_rays(b2r_ctx* c, uint32_t acc, float* out_host) {
 	int rc = ensure_device(c); if (rc) return rc;
 	float* d = nullptr; const size_t n = static_cast<size_t>(c->params.frame.npix) * 6;
 	if ((rc = dev_alloc(&d, n))) return rc;
-	k_tap_generate<<<c->grid_stream, kBlock, 0, c->stream>>>(c->params, acc, d);
+	if (c->lens.radius > 0.0f) k_tap_generate<true><<<c->grid_stream, kBlock, 0, c->stream>>>(c->params, acc, c->lens, d);
+	else k_tap_generate<false><<<c->grid_stream, kBlock, 0, c->stream>>>(c->params, acc, c->lens, d);
 	cudaError_t e = cudaGetLastError();
 	if (e == cudaSuccess) e = cudaMemcpyAsync(out_host, d, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
 	if (e == cudaSuccess) e = sync_main(c);
@@ -1570,10 +1619,10 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 	const KernelSet k = pick_kernels(c);
 	std::vector<float2> h(chunk);
 	if (packet) {  // one sample of the context's own frame, camera and sample index acc
-		BatchArgs a; a.n = 1u; a.acc[0] = acc; a.cam = c->params.frame.cam;
+		BatchArgs a; a.n = 1u; a.acc[0] = acc; a.cam = c->params.frame.cam; a.lens = c->lens;
 		k_set_batch<<<1, kMaxSlots, 0, st>>>(batch, a);
 		CU(cudaMemsetAsync(cnt, 0, 16u * sizeof(uint32_t), st));
-		k.packet<<<c->grid_packet, kTravBlock, 0, st>>>(p, 0u);
+		k.packet<<<k.g_packet, kTravBlock, 0, st>>>(p, 0u);
 		CU(cudaGetLastError()); c->launches += 2;
 		CU(cudaMemcpyAsync(h.data(), p.q.H, n * sizeof(float2), cudaMemcpyDeviceToHost, st));
 		CU(sync_main(c));

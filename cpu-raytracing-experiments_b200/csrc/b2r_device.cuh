@@ -111,15 +111,18 @@ __device__ __forceinline__ bool finished_elsewhere(const Params& p, uint32_t bou
 // EXACT (B2R_FLAG_REFERENCE_EXACT): rays that sit in the last `active % 8` slots of their tile's stream take the reference's
 // scalar-tail sphere formula (BVH.hpp:270-286) instead of the AVX2+FMA one (:250-268), and survivors leave (material, slot) behind
 // for k_stream_rank, which computes the slots of the next bounce (the reference's stable counting sort by material).
-template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false>
+// LENS (bounce 0 with a thin lens): every camera ray has its own origin, so there is no shared-origin sphere precompute (s_pre); phase 1
+// runs sphere_hit_closest per ray, and phase 2 regenerates a hit's camera ray from its path id instead of queueing its origin.
+template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false, bool LENS = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_brute(const Params p, const uint32_t bounce) {
 	constexpr int kQ = 2 * kBruteBlock;  // hit queue: up to kBruteBlock-1 waiting + kBruteBlock new
 	__shared__ float4 s_prim[kBruteTile];
-	__shared__ float4 s_pre[FIRST ? kBruteTile : 1];  // bounce 0: {c - o, r^2 - |c - o|^2} per sphere for the shared camera origin
+	constexpr bool PRE = FIRST && !LENS;
+	__shared__ float4 s_pre[PRE ? kBruteTile : 1];  // bounce 0: {c - o, r^2 - |c - o|^2} per sphere for the shared camera origin
 	__shared__ int32_t s_prim_mat[kBruteTile];
 	__shared__ float4 s_table[4][kSmemTable];  // mat_albedo, mat_emission, light_sphere, light_emit
 	__shared__ uint32_t s_hit_i[kQ]; __shared__ float s_hit_t[kQ]; __shared__ int32_t s_hit_prim[kQ];
-	__shared__ float s_hit_d[FIRST ? 3 : 1][FIRST ? kQ : 1];
+	__shared__ float s_hit_d[PRE ? 3 : 1][PRE ? kQ : 1];
 	__shared__ float s_shadow[11][kQ];         // shadow-ray queue: o.xyz, d.xyz, tfar, L.rgb, pid
 	__shared__ uint32_t s_cnt_a[kBruteWarps], s_cnt_b[kBruteWarps], s_cnt_c[kBruteWarps], s_base;
 	SceneDev sc = p.scene;
@@ -136,7 +139,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 	if (n_tiles == 1) {
 		for (uint32_t j = threadIdx.x; j < sc.n_prims; j += blockDim.x) {
 			const float4 sp = sc.prims[j]; s_prim[j] = sp; s_prim_mat[j] = sc.prim_mat[j];
-			if (FIRST) { const SpherePre q = sphere_prepare(sp.x, sp.y, sp.z, sp.w, p.batch->cam.px, p.batch->cam.py, p.batch->cam.pz); s_pre[j] = make_float4(q.tx, q.ty, q.tz, q.disc0); }
+			if (PRE) { const SpherePre q = sphere_prepare(sp.x, sp.y, sp.z, sp.w, p.batch->cam.px, p.batch->cam.py, p.batch->cam.pz); s_pre[j] = make_float4(q.tx, q.ty, q.tz, q.disc0); }
 		}
 		sc.prim_mat = s_prim_mat; sc.prims = s_prim;
 	}
@@ -163,7 +166,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 			if (live) {
 				if (FIRST) {
 					const uint32_t sl0 = div_by(i, p.frame.npix, p.frame.npix_magic);
-					const PathState s0 = primary_path(p.frame, p.batch->cam, p.batch->acc[sl0], sl0, i - sl0 * p.frame.npix);
+					const PathState s0 = primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[sl0], sl0, i - sl0 * p.frame.npix, p.batch->lens);
 					ox = s0.ox; oy = s0.oy; oz = s0.oz; dx = s0.dx; dy = s0.dy; dz = s0.dz;
 					pid0 = s0.pid; rad_zero(p.rad, p.frame.npix, s0.pid);  // a path's radiance starts at 0 here (coalesced stores); contributions are added after a CTA barrier
 				} else {
@@ -182,7 +185,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 					__syncthreads();
 					for (uint32_t j = threadIdx.x; j < cnt; j += blockDim.x) {
 						const float4 sp = p.scene.prims[first + j]; s_prim[j] = sp;
-						if (FIRST) { const SpherePre q = sphere_prepare(sp.x, sp.y, sp.z, sp.w, p.batch->cam.px, p.batch->cam.py, p.batch->cam.pz); s_pre[j] = make_float4(q.tx, q.ty, q.tz, q.disc0); }
+						if (PRE) { const SpherePre q = sphere_prepare(sp.x, sp.y, sp.z, sp.w, p.batch->cam.px, p.batch->cam.py, p.batch->cam.pz); s_pre[j] = make_float4(q.tx, q.ty, q.tz, q.disc0); }
 					}
 					__syncthreads();
 				}
@@ -193,7 +196,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 				#pragma unroll 3
 					for (uint32_t j = 0; j < cnt; j++) {
 						float d; bool h;
-						if (FIRST) { const float4 q = lds_f4(a_pre + j * 16u); h = sphere_hit_prepared(SpherePre{q.x, q.y, q.z, q.w}, dx, dy, dz, &d); }
+						if (PRE) { const float4 q = lds_f4(a_pre + j * 16u); h = sphere_hit_prepared(SpherePre{q.x, q.y, q.z, q.w}, dx, dy, dz, &d); }
 						else { const float4 sp = lds_f4(a_prim + j * 16u); h = sphere_hit_closest(sp.x, sp.y, sp.z, sp.w, ox, oy, oz, dx, dy, dz, &d); }
 						if (h && d < best) { best = d; prim = static_cast<int32_t>(first + j); }
 					}
@@ -205,7 +208,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 				c_term++;
 				if (sc.has_ambient) {
 					const uint32_t slm = FIRST ? div_by(i, p.frame.npix, p.frame.npix_magic) : 0u;
-					const PathState sm = FIRST ? primary_path(p.frame, p.batch->cam, p.batch->acc[slm], slm, i - slm * p.frame.npix) : load_path(p.q, side, i);
+					const PathState sm = FIRST ? primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[slm], slm, i - slm * p.frame.npix, p.batch->lens) : load_path(p.q, side, i);
 					rad_add(p.rad, p.frame.npix, sm.pid, shade_sky(sc, sm), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++;
 				}
 			}
@@ -214,7 +217,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 			const uint32_t slot = queued + block_rank(is_hit, s_cnt_a, &n_hits);
 			if (is_hit) {
 				s_hit_i[slot] = FIRST ? pid0 : i; s_hit_t[slot] = best; s_hit_prim[slot] = prim;  // bounce 0 queues the path id itself (no queue record to index)
-				if (FIRST) { s_hit_d[0][slot] = dx; s_hit_d[FIRST ? 1 : 0][slot] = dy; s_hit_d[FIRST ? 2 : 0][slot] = dz; }
+				if (PRE) { s_hit_d[0][slot] = dx; s_hit_d[PRE ? 1 : 0][slot] = dy; s_hit_d[PRE ? 2 : 0][slot] = dz; }
 			}
 			queued += n_hits;
 			base += gridDim.x * kBruteBlock;
@@ -231,11 +234,12 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 			if (shade) {
 				const uint32_t hi = s_hit_i[qi]; const float depth = s_hit_t[qi]; const int32_t hprim = s_hit_prim[qi];
 				if (EXACT) ex_slot = FIRST ? (hi & 255u) : static_cast<uint32_t>(p.ex.slot[side][hi]);  // bounce 0: hi is the path id, slot = pixel ID
-				if (FIRST) {
+				if (PRE) {
 					s.ox = p.batch->cam.px; s.oy = p.batch->cam.py; s.oz = p.batch->cam.pz;
-					s.dx = s_hit_d[0][FIRST ? qi : 0]; s.dy = s_hit_d[FIRST ? 1 : 0][FIRST ? qi : 0]; s.dz = s_hit_d[FIRST ? 2 : 0][FIRST ? qi : 0];
+					s.dx = s_hit_d[0][PRE ? qi : 0]; s.dy = s_hit_d[PRE ? 1 : 0][PRE ? qi : 0]; s.dz = s_hit_d[PRE ? 2 : 0][PRE ? qi : 0];
 					s.tr = s.tg = s.tb = 1.0f; s.pdf = 0.0f; s.pid = hi;
-				} else s = load_path(p.q, side, hi);
+				} else if (FIRST) s = primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[hi >> 26], hi >> 26, hi & kPixMask, p.batch->lens);  // the same bits phase 1 traced
+				else s = load_path(p.q, side, hi);
 				pid = s.pid;
 				const uint32_t acc = p.batch->acc[s.pid >> 26], seed = pixel_seed(s.pid & kPixMask, p.frame.max_bounces);
 				const Surface sf = shade_surface<GGX>(sc, s, depth, hprim);
@@ -501,10 +505,11 @@ __global__ void __launch_bounds__(256) k_stream_rank(const Params p, const uint3
 }
 
 // camera rays of a batch -> queue side 0 (Renderer.hpp:97-127)
+template <bool LENS = false>
 __global__ void __launch_bounds__(kBlock) k_generate(const Params p) {
 	const uint32_t n = p.batch->n_slots * p.frame.npix;
 	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-		{ const uint32_t sl = div_by(i, p.frame.npix, p.frame.npix_magic); const PathState s = primary_path(p.frame, p.batch->cam, p.batch->acc[sl], sl, i - sl * p.frame.npix); store_path(p.q, 0, i, s); rad_zero(p.rad, p.frame.npix, s.pid); }
+		{ const uint32_t sl = div_by(i, p.frame.npix, p.frame.npix_magic); const PathState s = primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[sl], sl, i - sl * p.frame.npix, p.batch->lens); store_path(p.q, 0, i, s); rad_zero(p.rad, p.frame.npix, s.pid); }
 	if (blockIdx.x == 0 && threadIdx.x == 0) p.cnt.paths[0] = n;
 }
 // Work distribution of the traversal kernels: every warp owns a pool of ray indices claimed kTravChunk at a time from the
@@ -635,7 +640,14 @@ constexpr int kPacketStack = 64;
 #ifndef B2R_PACKET_RPL
 #define B2R_PACKET_RPL 4
 #endif
-template <bool COUNT, int RPL = 1>
+// LENS: thin-lens camera rays leave different points of the lens disk, so each ray keeps its own origin (3 more registers per ray). The walk
+// stays exact for any rays (each lane keeps its own best and tests only boxes its own ray passes); only coherence changes. RPL 4 with a lens:
+// 118 registers, no spills; measured on C3 against RPL 2 (79 registers), A/B in one run: bounce 0 2.92 / 3.03 / 6.58 ms against 3.03 / 3.17 /
+// 6.93 ms for circles of confusion of 4, 7.5 and 75 pixels at twice the focus distance (DESIGN §6).
+#ifndef B2R_PACKET_RPL_LENS
+#define B2R_PACKET_RPL_LENS 4
+#endif
+template <bool COUNT, int RPL = 1, bool LENS = false>
 __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p, const uint32_t bounce) {
 	// The camera rays are GENERATED here (Renderer.hpp:97-127: hash_2d -> PCG -> Camera::generate_ray, in registers) and their path
 	// records and zeroed radiance entries written behind the walk (plain coalesced stores that nobody waits for) for k_shade to read:
@@ -656,15 +668,17 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p,
 			next = b; end = min(b + kClaim, n_in);
 		}
 		const uint32_t idx0 = next + lane_id(); next += 32u * RPL;
-		float ox = 0, oy = 0, oz = 0, dx[RPL], dy[RPL], dz[RPL], ix[RPL], iy[RPL], iz[RPL], nx[RPL], ny[RPL], nz[RPL], ax[RPL], ay[RPL], az[RPL], best[RPL]; int32_t prim[RPL];
+		constexpr int NO = LENS ? RPL : 1;   // origins kept: one per ray with a lens, one shared by the packet's camera rays without
+		float ox[NO], oy[NO], oz[NO], dx[RPL], dy[RPL], dz[RPL], ix[RPL], iy[RPL], iz[RPL], nx[RPL], ny[RPL], nz[RPL], ax[RPL], ay[RPL], az[RPL], best[RPL]; int32_t prim[RPL];
 #pragma unroll
 		for (int r = 0; r < RPL; r++) {
 			const uint32_t idx = idx0 + 32u * r;
 			const uint32_t sl = div_by(idx, p.frame.npix, p.frame.npix_magic);
-			const PathState s0 = primary_path(p.frame, p.batch->cam, p.batch->acc[sl], sl, idx - sl * p.frame.npix);
+			const PathState s0 = primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[sl], sl, idx - sl * p.frame.npix, p.batch->lens);
 			store_path(p.q, 0, idx, s0); rad_zero(p.rad, p.frame.npix, s0.pid);
-			ox = s0.ox; oy = s0.oy; oz = s0.oz; dx[r] = s0.dx; dy[r] = s0.dy; dz[r] = s0.dz;   // (all camera rays leave the same point)
-			slab_setup(ox, oy, oz, dx[r], dy[r], dz[r], &ix[r], &iy[r], &iz[r], &nx[r], &ny[r], &nz[r], &ax[r], &ay[r], &az[r]);
+			const int ro = LENS ? r : 0;
+			ox[ro] = s0.ox; oy[ro] = s0.oy; oz[ro] = s0.oz; dx[r] = s0.dx; dy[r] = s0.dy; dz[r] = s0.dz;   // (without a lens all camera rays leave the same point)
+			slab_setup(ox[ro], oy[ro], oz[ro], dx[r], dy[r], dz[r], &ix[r], &iy[r], &iz[r], &nx[r], &ny[r], &nz[r], &ax[r], &ay[r], &az[r]);
 			best[r] = FLT_MAX; prim[r] = -1;
 		}
 		uint32_t node = 0u, sp = 0u;
@@ -691,7 +705,8 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p,
 #pragma unroll
 					for (int r = 0; r < RPL; r++) if (h[r]) {
 						float d; if (COUNT) c_sphere++;
-						if (sphere_hit_closest(a.x, a.y, a.z, a.w, ox, oy, oz, dx[r], dy[r], dz[r], &d) && (d < best[r] || (d == best[r] && ~l < prim[r]))) { best[r] = d; prim[r] = ~l; }
+						const int ro = LENS ? r : 0;
+						if (sphere_hit_closest(a.x, a.y, a.z, a.w, ox[ro], oy[ro], oz[ro], dx[r], dy[r], dz[r], &d) && (d < best[r] || (d == best[r] && ~l < prim[r]))) { best[r] = d; prim[r] = ~l; }
 					}
 				} else key[k] = __reduce_min_sync(0xffffffffu, tmin);  // the packet's entry distance
 			}
@@ -1305,14 +1320,12 @@ __global__ void __launch_bounds__(kBlock) k_tree_cost(const float4* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------- taps
-__global__ void k_tap_generate(const Params p, const uint32_t acc, float* __restrict__ out) {
+template <bool LENS>
+__global__ void k_tap_generate(const Params p, const uint32_t acc, const LensParams lens, float* __restrict__ out) {
 	for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < p.frame.npix; t += gridDim.x * blockDim.x) {
-		Pcg rng{hash_2d(acc, pixel_seed(t, p.frame.max_bounces))};
-		const float s0 = rng.next_unit(), s1 = rng.next_unit();
-		int32_t x, y; pixel_xy(t, p.frame, &x, &y);
-		const f3 d = camera_dir(p.frame.cam, x, y, s0, s1);
+		const PathState s = primary_path<LENS>(p.frame, p.frame.cam, acc, 0u, t, lens);
 		float* o = out + static_cast<size_t>(t) * 6u;
-		o[0] = p.frame.cam.px; o[1] = p.frame.cam.py; o[2] = p.frame.cam.pz; o[3] = d.x; o[4] = d.y; o[5] = d.z;
+		o[0] = s.ox; o[1] = s.oy; o[2] = s.oz; o[3] = s.dx; o[4] = s.dy; o[5] = s.dz;
 	}
 }
 // Traverse / Traverse_shadow on caller-supplied rays (Application.cpp:282-298)

@@ -113,6 +113,13 @@ B2R_HD f3 camera_dir(const CameraParams& c, int32_t x, int32_t y, float s0, floa
 	f3 v{static_cast<float>(x) + s0 - c.half_width, static_cast<float>(y) + s1 - c.half_height, c.z};
 	return unit3(quat_rotate(c.qw, c.qx, c.qy, c.qz, v));
 }
+// Thin lens (not in the reference: Camera.hpp computes an aperture it never uses, Q22). radius R and focus distance F in scene units; F is
+// measured along the forward axis, so the plane in focus is camera-space z = -F. radius 0 = pinhole: callers take camera_dir instead (this
+// routine at R = 0 rounds differently: v is scaled by -F/z).
+struct LensParams { float radius, focus; };
+// pinhole part v as camera_dir; focus point P = v * (-F / z); lens point L = (r cos phi, r sin phi, 0), r = R sqrt(u0), phi = 2 pi u1;
+// origin = pos + orient * L, dir = normalize(orient * (P - L)). Same order of operations in the test oracle's generate_ray_lens (tests/lenscheck/lens_oracle.cpp).
+B2R_HD void camera_lens_ray(const CameraParams& c, int32_t x, int32_t y, float s0, float s1, const LensParams& lens, float u0, float u1, f3* origin, f3* dir);
 // glm::quatLookAt(normalize(forward), {0,1,0}) (Camera.hpp:47-50): RH basis {right, up', -dir} -> quat_cast
 B2R_HD void look_at_quat(f3 forward, float out_wxyz[4]) {
 	f3 d = unit3(forward);
@@ -161,6 +168,16 @@ B2R_HD void sincos_poly(float x, float* s_out, float* c_out) {  // fast_sincos, 
 	if (from_bits(bits(s) & 0x7fffffffu) > 1.0f) s = 0.0f;
 	if (from_bits(bits(c) & 0x7fffffffu) > 1.0f) c = 0.0f;
 	*s_out = s; *c_out = c;
+}
+B2R_HD void camera_lens_ray(const CameraParams& c, int32_t x, int32_t y, float s0, float s1, const LensParams& lens, float u0, float u1, f3* origin, f3* dir) {
+	const f3 v{static_cast<float>(x) + s0 - c.half_width, static_cast<float>(y) + s1 - c.half_height, c.z};
+	const f3 P = scale3(v, -lens.focus / c.z);
+	float sn, cs; sincos_poly(u1 * B2R_TWO_PI, &sn, &cs);
+	const float r = lens.radius * sqrtf(u0);
+	const f3 L{r * cs, r * sn, 0.0f};
+	const f3 lw = quat_rotate(c.qw, c.qx, c.qy, c.qz, L);
+	*origin = f3{c.px + lw.x, c.py + lw.y, c.pz + lw.z};
+	*dir = unit3(quat_rotate(c.qw, c.qx, c.qy, c.qz, f3{P.x - L.x, P.y - L.y, P.z - L.z}));
 }
 B2R_HD float asin_poly(float x) {  // fast_asin, VectorMath.hpp:625-630
 	float f = from_bits(bits(x) & 0x7fffffffu);

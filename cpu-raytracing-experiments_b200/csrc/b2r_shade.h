@@ -71,6 +71,7 @@ struct BatchDev {  // one wavefront batch: n_slots samples traced together
 	uint32_t acc[kMaxSlots];  // sample index (the reference's `accumulations` value, Q1) of each slot
 	CameraParams cam;         // the camera this batch is traced with: it travels with the batch descriptor (written by k_set_batch in front of every batch),
 	                          // not with the kernels' parameter block, so a camera move neither re-captures the batch graph nor waits for the stream
+	LensParams lens;          // likewise (read by the LENS instantiations only; a pinhole <-> lens switch changes the instantiation and re-captures)
 	unsigned long long fold;  // slots k_accumulate folds into the buckets now (the others were traced ahead of the caller's Accumulate() calls)
 };
 struct QueueDev {
@@ -113,14 +114,24 @@ B2R_HD void pixel_xy(uint32_t t, const FrameDev& fr, int32_t* x, int32_t* y) {
 
 struct PathState { float ox, oy, oz, dx, dy, dz, tr, tg, tb, pdf; uint32_t pid; };
 
-// primary ray of (slot, pixel t): Renderer.hpp:97-127
-B2R_HD PathState primary_path(const FrameDev& fr, const CameraParams& cam, uint32_t acc, uint32_t slot, uint32_t t) {
+// primary ray of (slot, pixel t): Renderer.hpp:97-127. LENS: the thin-lens ray (camera_lens_ray, lens.radius > 0). Its lens sample is drawn
+// from branch 2 * max_bounces of the pixel's seed range [seed, seed + 2 mb + 1): branches 2b (light sample) and 2b + 1 (BRDF continuation)
+// of bounces b < mb use at most 2 mb - 1, so that stream is used by nothing else, and the camera jitter keeps its stream (branch 0).
+template <bool LENS = false>
+B2R_HD PathState primary_path(const FrameDev& fr, const CameraParams& cam, uint32_t acc, uint32_t slot, uint32_t t, const LensParams& lens = LensParams{0.0f, 0.0f}) {
 	Pcg rng{hash_2d(acc, pixel_seed(t, fr.max_bounces))};
 	const float s0 = rng.next_unit(), s1 = rng.next_unit();
 	int32_t x, y; pixel_xy(t, fr, &x, &y);
-	const f3 d = camera_dir(cam, x, y, s0, s1);
 	PathState s;
-	s.ox = cam.px; s.oy = cam.py; s.oz = cam.pz; s.dx = d.x; s.dy = d.y; s.dz = d.z;
+	if constexpr (LENS) {
+		Pcg lr{hash_2d(acc, pixel_seed(t, fr.max_bounces) + 2u * fr.max_bounces)};
+		const float u0 = lr.next_unit(), u1 = lr.next_unit();
+		f3 o, d; camera_lens_ray(cam, x, y, s0, s1, lens, u0, u1, &o, &d);
+		s.ox = o.x; s.oy = o.y; s.oz = o.z; s.dx = d.x; s.dy = d.y; s.dz = d.z;
+	} else {
+		const f3 d = camera_dir(cam, x, y, s0, s1);
+		s.ox = cam.px; s.oy = cam.py; s.oz = cam.pz; s.dx = d.x; s.dy = d.y; s.dz = d.z;
+	}
 	s.tr = s.tg = s.tb = 1.0f; s.pdf = 0.0f; s.pid = (slot << 26) | t;
 	return s;
 }

@@ -113,6 +113,9 @@ struct Renderer {
 		const float pos[3] = {c.view.pos.x, c.view.pos.y, c.view.pos.z}, q[4] = {c.view.orient.w, c.view.orient.x, c.view.orient.y, c.view.orient.z};
 		check(b2r_set_camera(ctx, pos, q, c.projection.half_width, c.projection.half_height, c.projection.z, c.exp));
 	}
+	// Thin-lens depth of field (b2r_set_lens), in scene units: the app's focus pick gives the distance; Projection::aperture_radius is in mm and
+	// the caller scales it to scene units. lens_radius 0 = the pinhole camera.
+	void SetLens(float lens_radius, float focus_distance) { check(b2r_set_lens(ctx, lens_radius, focus_distance)); }
 
 	void Accumulate() { ++accumulations; check(b2r_accumulate(ctx, 1)); }             // Renderer.hpp:73-434
 	void Accumulate(uint32_t n) { accumulations += n; check(b2r_accumulate(ctx, n)); } // n calls in one submission

@@ -162,6 +162,14 @@ int  b2r_refit_scene(b2r_ctx* ctx, const b2r_sphere* prims_bvh_order, uint32_t n
 /* Camera (Camera.hpp:61-88): view.pos, view.orient (w,x,y,z), projection.half_width/half_height/z, exp */
 int  b2r_set_camera(b2r_ctx* ctx, const float pos[3], const float orient_wxyz[4], float half_width, float half_height,
                     float z, float exposure);
+/* Thin-lens depth of field (opt-in; the reference computes Projection::aperture_radius but renders a pinhole, Camera.hpp:80-88).
+ * lens_radius R and focus_distance F are in SCENE UNITS: the library does not guess a millimetre-to-scene scale, the caller converts
+ * (aperture_radius = focal_length / (2 f_number) is in mm). F is measured along the camera's forward axis: the plane camera-space
+ * z = -F is in focus. Camera ray = from pos + orient * L, L a point of the lens disk of radius R, through the point where the pinhole ray
+ * of the same pixel sample meets that plane. R = 0 (the default) is the pinhole camera, bit for bit. Takes effect like b2r_set_camera
+ * (batches already enqueued keep their lens). b2r_camera_ray stays the pinhole ray through the lens centre (focus picking).
+ * B2R_ERR_ARG: R negative or not finite, F not finite or <= 0. B2R_ERR_STATE: a B2R_FLAG_REFERENCE_EXACT context. */
+int  b2r_set_lens(b2r_ctx* ctx, float lens_radius, float focus_distance);
 
 /* ---- the hot path ---------------------------------------------------------------------------------- */
 /* Renderer::Accumulate() n_samples times (Renderer.hpp:73-434): accumulations += n_samples; each new sample index
