@@ -582,7 +582,6 @@ __device__ __forceinline__ void warp_stage_nodes(const WideNode* __restrict__ wi
 #define B2R_SMEM_STACK 16
 #endif
 constexpr int kSmemStack = B2R_SMEM_STACK, kEvict = 8;
-constexpr uint32_t kNoNode = 0xffffffffu;
 static_assert(kSmemStack >= kEvict + 3 && kTraversalStack % kEvict == 0, "stack geometry");
 constexpr uint32_t kStackStride = kTravBlock * 4u;  // bytes between consecutive entries of one thread
 __device__ __forceinline__ void sts_u32(uint32_t addr, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v)); }
@@ -622,6 +621,30 @@ struct SmemStack {
 // ordering the children with the slot index in the low key bits and min/max pairs — same SASS size as the compare-and-swap
 // network (the compiler already emits VIMNMX), 5 % slower; refill thresholds 16/20/28 and 12/20 stack entries in shared memory —
 // flat; full-sweep SAH and a cost-optimal 2->4 collapse of the traversal tree — 12.3 instead of 12.4 node visits per ray.
+// The loop itself, for a Walk (TravClosestT / TravAnyT over SmemStack) and the kernel's three pieces: read(t, idx) arms the walk with
+// claimed ray idx, step(t, row) visits the staged node row and returns false once the ray is finished, write(t, idx) stores its result.
+template <class Walk, class Read, class Step, class Write>
+__device__ __forceinline__ void lane_walks(const WideNode* __restrict__ wide, uint32_t* cursor, const uint32_t n_in, Read read, Step step, Write write) {
+	__shared__ __align__(128) float4 s_nodes[kTravBlock / 32][32 * kNodeRowF4];
+	__shared__ uint32_t s_stack[kSmemStack][kTravBlock];
+	float4* rows = s_nodes[threadIdx.x >> 5];
+	uint32_t backing[kTraversalStack];
+	WarpPool pool; Walk t; bool active = false, unsent = false; uint32_t idx = 0;
+	t.node = 0u; t.stack.bind(&s_stack[0][threadIdx.x], backing);
+	for (;;) {
+		// rays that finished since the last refill hand their results over together (dense stores instead of one per finish)
+		if (unsent) { write(t, idx); unsent = false; }
+		const uint32_t got = pool.take(!active, cursor, n_in);
+		if (got != 0xffffffffu) { idx = got; active = true; read(t, idx); }
+		uint32_t live = __ballot_sync(0xffffffffu, active);
+		if (live == 0u) break;
+		do {
+			warp_stage_nodes(wide, rows, active ? t.node : 0u);
+			if (active && !step(t, rows + lane_id() * kNodeRowF4)) { active = false; unsent = true; }
+			live = __ballot_sync(0xffffffffu, active);
+		} while (live != 0u && (pool.dry || __popc(live) >= kRefillBelow));
+	}
+}
 
 // ---- bounce 0: packet traversal ------------------------------------------------------------------------------------------------
 // Camera rays are coherent: the 32 consecutive tile-order pixels of a warp (two rows of 16 in one 16x16 tile) walk almost the same
@@ -743,20 +766,10 @@ template <bool COUNT, bool EXACT, uint32_t TNB>
 __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p, const uint32_t bounce) {
 	const uint32_t n_in = p.cnt.paths[bounce];
 	const int side = bounce & 1;
-	const WideNode* __restrict__ wide = p.scene.wide;
 	uint32_t c_sphere = 0, c_box = 0;
-	__shared__ __align__(128) float4 s_nodes[kTravBlock / 32][32 * kNodeRowF4];
-	__shared__ uint32_t s_stack[kSmemStack][kTravBlock];
-	float4* rows = s_nodes[threadIdx.x >> 5];
-	WarpPool pool; TravClosestT<SmemStack> t; bool active = false, unsent = false; uint32_t idx = 0;
-	uint32_t backing[kTraversalStack];
-	t.node = 0u; t.stack.bind(&s_stack[0][threadIdx.x], backing);
-	for (;;) {
-		// rays that finished since the last refill hand their hit records over together (one dense store instead of one per finish)
-		if (unsent) { p.q.H[idx] = make_float2(t.best, __int_as_float(t.prim)); unsent = false; }
-		const uint32_t got = pool.take(!active, p.cnt.work_a + bounce, n_in);
-		if (got != 0xffffffffu) {
-			idx = got; active = true;
+	using Walk = TravClosestT<SmemStack>;
+	lane_walks<Walk>(p.scene.wide, p.cnt.work_a + bounce, n_in,
+		[&](Walk& t, uint32_t idx) {
 			const float4 a = p.q.A[side][idx], b = p.q.B[side][idx];
 			bool tail = false;
 			if (EXACT && bounce > 0u) {  // B2R_FLAG_REFERENCE_EXACT: scalar-tail formula for the last `active % 8` slots of the ray's stream
@@ -764,15 +777,9 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p
 				tail = static_cast<uint32_t>(p.ex.slot[side][idx]) >= (static_cast<uint32_t>(p.ex.act[side][stream]) & ~7u);
 			}
 			t.begin(Ray{a.x, a.y, a.z, a.w, b.x, b.y}, tail);
-		}
-		uint32_t live = __ballot_sync(0xffffffffu, active);
-		if (live == 0u) break;
-		do {
-			warp_stage_nodes(wide, rows, active ? t.node : 0u);
-			if (active && !t.template step_staged<COUNT, TNB>(rows + lane_id() * kNodeRowF4, p.scene.stack_tn_bits, &c_sphere, &c_box)) { active = false; unsent = true; }
-			live = __ballot_sync(0xffffffffu, active);
-		} while (live != 0u && (pool.dry || __popc(live) >= kRefillBelow));
-	}
+		},
+		[&](Walk& t, const float4* row) { return t.template step_staged<COUNT, TNB>(row, p.scene.stack_tn_bits, &c_sphere, &c_box); },
+		[&](const Walk& t, uint32_t idx) { p.q.H[idx] = make_float2(t.best, __int_as_float(t.prim)); });
 	if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(p.cnt.stats + ST_EXT, static_cast<unsigned long long>(n_in));
 	if (COUNT) { stat_add(p.cnt.stats, ST_SPHERE, c_sphere); stat_add(p.cnt.stats, ST_BOX, c_box); }
 }
@@ -845,7 +852,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 					const f3 emit = shade_emission(sc, sf, s, depth, bounce, mis);
 					if (want_shadow) {
 						uint32_t cs = 0, cb = 0;
-						const bool occluded = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb);
+						const bool occluded = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb, sc.parent, 0u);
 						rad_add(p.rad, p.frame.npix, s.pid, sr.L, emit, !occluded, true);
 						want_shadow = false; c_inline_shadow++;
 					} else rad_add(p.rad, p.frame.npix, s.pid, emit, f3{0.0f, 0.0f, 0.0f}, true, false);
@@ -880,88 +887,26 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 	stat_add(p.cnt.stats, ST_HITS, c_hits); stat_add(p.cnt.stats, ST_TERM, c_term);
 	stat_add(p.cnt.stats, ST_DROPPED, c_drop); stat_add(p.cnt.stats, ST_EVENTS, c_events); stat_add(p.cnt.stats, ST_SHADOW, c_inline_shadow);
 }
-// shadow rays of this bounce: any-hit traversal (same per-lane walk as above: the nearest hit child is visited next, the others are
-// pushed; the first occluding leaf sphere ends the ray), unoccluded light samples are added to the pixel's radiance.
-// The walk starts at the BOTTOM of the tree and climbs. A shadow ray leaves a point on a sphere, and in a dense scene its occluder is
-// usually a neighbour of that sphere (C3: every shadow ray is occluded): a walk from the root spends ~8 of its 12-13 node visits descending
-// to the origin's neighbourhood before it tests the first sphere. So the ray starts at the wide node that holds its origin sphere's leaf
-// slot (SS, written by k_shade from scene.leaf_node); when that subtree holds no occluder the walk moves up to its parent, searches the
-// parent's other children (the child it came from is skipped), and so on up to the root. Any-hit is an order-independent boolean over the
-// same sphere tests, and a ray that reaches the root has visited exactly the nodes a root walk would have, so results are unchanged;
-// measured on C3's shadow rays (tests/hostcheck hc_anyhit_local_stats): 12.3 -> 6.5 node visits per ray for the shadow rays of camera-ray
-// hits, 13.1 -> 8.5 for those of later bounces. The parent index a climb needs is fetched one climb ahead (`up`), so no step waits for it.
+// shadow rays of this bounce: the climbing any-hit walk (TravAnyT) from the node that holds each ray's origin sphere; unoccluded light
+// samples are added to the pixel's radiance.
 template <bool COUNT>
 __global__ void __launch_bounds__(kTravBlock, 8) k_intersect_shadow(const Params p, const uint32_t bounce) {
 	const uint32_t n_in = p.cnt.shadow[bounce];
-	const WideNode* __restrict__ wide = p.scene.wide;
-	uint32_t c_sphere = 0, c_box = 0, c_events = 0;
-	__shared__ __align__(128) float4 s_nodes[kTravBlock / 32][32 * kNodeRowF4];
-	__shared__ uint32_t s_stack[kSmemStack][kTravBlock];
-	float4* rows = s_nodes[threadIdx.x >> 5];
-	const float4* row = rows + lane_id() * kNodeRowF4;
-	uint32_t backing[kTraversalStack];
-	SmemStack stack; stack.bind(&s_stack[0][threadIdx.x], backing);
-	WarpPool pool;
-	float ox = 0, oy = 0, oz = 0, dx = 0, dy = 0, dz = 0, ix = 0, iy = 0, iz = 0, nx = 0, ny = 0, nz = 0, ax = 0, ay = 0, az = 0, tfar = 0;
-	uint32_t node = 0u, idx = 0, pid = 0; bool active = false, lit = false;
-	uint32_t root = 0u, up = 0u, skip = kNoNode;   // top of the subtree searched so far, its parent, and the child of `root` already searched
 	const uint32_t* __restrict__ parent = p.scene.parent;
-	for (;;) {
-		// light samples found unoccluded since the last refill are added together (dense loads and reductions)
-		if (lit) {
-			const f3 L{p.q.SL[idx], p.q.SL[p.q.cap + idx], p.q.SL[2u * p.q.cap + idx]};
-			rad_add(p.rad, p.frame.npix, pid, L, f3{0.0f, 0.0f, 0.0f}, true, false); c_events++; lit = false;
-		}
-		const uint32_t got = pool.take(!active, p.cnt.work_b + bounce, n_in);
-		if (got != 0xffffffffu) {
-			idx = got; active = true;
+	uint32_t c_sphere = 0, c_box = 0, c_events = 0, pid = 0;
+	using Walk = TravAnyT<SmemStack>;
+	lane_walks<Walk>(p.scene.wide, p.cnt.work_b + bounce, n_in,
+		[&](Walk& t, uint32_t idx) {
 			const float4 a = p.q.SA[idx], b = p.q.SB[idx];
-			ox = a.x; oy = a.y; oz = a.z; dx = a.w; dy = b.x; dz = b.y; tfar = b.z; pid = __float_as_uint(b.w);
-			slab_setup(ox, oy, oz, dx, dy, dz, &ix, &iy, &iz, &nx, &ny, &nz, &ax, &ay, &az);
-			node = root = p.q.SS[idx]; up = __ldg(parent + root); skip = kNoNode; stack.reset();
-		}
-		uint32_t live = __ballot_sync(0xffffffffu, active);
-		if (live == 0u) break;
-		do {
-			warp_stage_nodes(wide, rows, active ? node : 0u);
-			if (active) {
-				uint32_t next = kNoNode, leaves = 0u; float next_tn = FLT_MAX;
-				stack.room();
-#pragma unroll
-				for (int k = 0; k < 4; k++) {
-					const float4 a = row[2 * k], b = row[2 * k + 1];
-					const int32_t l = __float_as_int(b.z);
-					float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, ax, ay, az, tfar, &tn, &h);
-					if (COUNT && l != kEmptyLink) c_box++;
-					if (h && l >= 0 && static_cast<uint32_t>(l) != skip) {
-						// the NEAREST hit child is visited next, the others are pushed: the result is an order-independent boolean, but in a
-						// dense scene the occluder is usually close to the origin (C3: every shadow ray is occluded; 12.4 -> 10.2 node visits per ray)
-						const bool nearer = tn < next_tn;
-						const uint32_t later = nearer ? next : static_cast<uint32_t>(l);
-						if (later != kNoNode) stack.push(later);
-						if (nearer) { next = static_cast<uint32_t>(l); next_tn = tn; }
-					}
-					leaves |= (h && l < 0) ? (1u << k) : 0u;  // leaf slots whose (inflated) box the ray passes within [0, tfar]
-				}
-				bool occluded = false;
-				while (leaves) {
-					const uint32_t k = static_cast<uint32_t>(__ffs(static_cast<int>(leaves)) - 1);
-					leaves &= leaves - 1u;
-					const float4 s4 = row[2u * k];
-					if (COUNT) c_sphere++;
-					if (sphere_hit_any(s4.x, s4.y, s4.z, s4.w, ox, oy, oz, dx, dy, dz, tfar)) { occluded = true; break; }
-				}
-				if (occluded) active = false;  // the light sample is dropped
-				else {
-					if (next == kNoNode && (!stack.empty() || stack.refill())) next = stack.pop();
-					if (next == kNoNode && root != 0u) { skip = root; root = up; next = up; up = __ldg(parent + up); }  // nothing below `root`: climb
-					node = next;
-					if (next == kNoNode) { active = false; lit = true; }  // walked the whole tree without an occluder
-				}
-			}
-			live = __ballot_sync(0xffffffffu, active);
-		} while (live != 0u && (pool.dry || __popc(live) >= kRefillBelow));
-	}
+			pid = __float_as_uint(b.w);
+			t.begin(Ray{a.x, a.y, a.z, a.w, b.x, b.y}, b.z, p.q.SS[idx], parent);
+		},
+		[&](Walk& t, const float4* row) { return t.template step_staged<COUNT>(row, parent, &c_sphere, &c_box); },
+		[&](const Walk& t, uint32_t idx) {
+			if (t.occluded) return;  // the light sample is dropped
+			const f3 L{p.q.SL[idx], p.q.SL[p.q.cap + idx], p.q.SL[2u * p.q.cap + idx]};
+			rad_add(p.rad, p.frame.npix, pid, L, f3{0.0f, 0.0f, 0.0f}, true, false); c_events++;
+		});
 	if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(p.cnt.stats + ST_SHADOW, static_cast<unsigned long long>(n_in));
 	stat_add(p.cnt.stats, ST_EVENTS, c_events);
 	if (COUNT) { stat_add(p.cnt.stats, ST_SPHERE, c_sphere); stat_add(p.cnt.stats, ST_BOX, c_box); }
@@ -1345,7 +1290,7 @@ __global__ void k_tap_trace(const SceneDev sc, const float* __restrict__ rays, c
 			tfar_out[i] = best; prim_out[i] = prim;
 		} else {
 			bool occ = false;
-			if (use_bvh) occ = traverse_any<false>(sc.wide, r, tfar_in[i], &cs, &cb);
+			if (use_bvh) occ = traverse_any<false>(sc.wide, r, tfar_in[i], &cs, &cb, sc.parent, 0u);
 			else for (uint32_t j = 0; j < sc.n_prims && !occ; j++) {
 				const float4 sp = ldg4(sc.prims + j);
 				occ = sphere_hit_any(sp.x, sp.y, sp.z, sp.w, r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, tfar_in[i]);

@@ -33,6 +33,18 @@ static void ray_origin_bounds(const float* rays, uint32_t n, float out[6]) {
 	for (uint32_t i = 0; i < n; i++) for (int k = 0; k < 3; k++) { out[k] = fminf(out[k], rays[6 * static_cast<size_t>(i) + k]); out[3 + k] = fmaxf(out[3 + k], rays[6 * static_cast<size_t>(i) + k]); }
 }
 
+// the tables k_link_tables writes: the wide node that links to node i (the root's entry is 0) and the node holding sphere i's leaf slot
+static void hc_link_tables(const WideBvh& w, uint32_t n_prims, std::vector<uint32_t>& parent, std::vector<uint32_t>& leaf_node) {
+	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
+	const uint32_t nn = static_cast<uint32_t>(w.nodes.size());
+	parent.assign(nn, 0u); leaf_node.assign(n_prims, 0u);
+	for (uint32_t nd = 0; nd < nn; nd++) for (int k = 0; k < 4; k++) {
+		const int32_t l = as_int(wide[static_cast<size_t>(nd) * 8 + 2 * k + 1].z);
+		if (l == kEmptyLink) continue;
+		if (l < 0) leaf_node[~l] = nd; else parent[l] = nd;
+	}
+}
+
 extern "C" {
 
 // One sample (`acc`) for every pixel: rad_out[3][npix] (tile order). counters: ext rays, shadow rays, hits, term, dropped.
@@ -48,7 +60,9 @@ int hc_render_sample(const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_
 	if (use_bvh == 2) { std::vector<b2r_bvh_node> tree; build_traversal_tree(prims, n_prims, tree); flatten_bvh(tree.data(), static_cast<uint32_t>(tree.size()), prims, n_prims, wide, &ob); }  // what libb2r uploads by default
 	else flatten_bvh(nodes, n_nodes, prims, n_prims, wide, &ob);  // B2R_FLAG_REFERENCE_TREE
 	if (wide.max_stack + 3u > static_cast<uint32_t>(kTraversalStack)) return B2R_ERR_BVH;
+	std::vector<uint32_t> parent, leaf_node; hc_link_tables(wide, n_prims, parent, leaf_node);
 	SceneDev sc{};
+	sc.parent = parent.data();
 	sc.prims = ps.prims.data(); sc.prim_mat = ps.prim_mat.data(); sc.mat_albedo = ps.mat_albedo.data(); sc.mat_emission = ps.mat_emission.data(); sc.mat_f0 = ps.mat_f0.data();
 	sc.light_sphere = ps.light_sphere.data(); sc.light_emit = ps.light_emit.data(); sc.wide = wide.nodes.data(); sc.hdri = nullptr;
 	sc.n_prims = n_prims; sc.n_mat = n_mat; sc.n_lights = n_lights; sc.light_sel_pdf = 1.0f / static_cast<float>(n_lights);
@@ -91,7 +105,7 @@ int hc_render_sample(const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_
 			if (want_shadow) {
 				counters[1]++;
 				bool occ = false;
-				if (use_bvh) occ = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb);
+				if (use_bvh) occ = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb, sc.parent, 0u);
 				else for (uint32_t j = 0; j < n_prims && !occ; j++) {
 					const float4 sp = sc.prims[j];
 					occ = sphere_hit_any(sp.x, sp.y, sp.z, sp.w, sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z, sr.tfar);
@@ -279,18 +293,6 @@ static int hc_tree(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes,
 	if (w.max_stack + 3u > static_cast<uint32_t>(kTraversalStack)) return B2R_ERR_BVH;
 	return 0;
 }
-// the tables k_link_tables writes: the wide node that links to node i (the root's entry is 0) and the node holding sphere i's leaf slot
-static void hc_link_tables(const WideBvh& w, uint32_t n_prims, std::vector<uint32_t>& parent, std::vector<uint32_t>& leaf_node) {
-	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
-	const uint32_t nn = static_cast<uint32_t>(w.nodes.size());
-	parent.assign(nn, 0u); leaf_node.assign(n_prims, 0u);
-	for (uint32_t nd = 0; nd < nn; nd++) for (int k = 0; k < 4; k++) {
-		const int32_t l = as_int(wide[static_cast<size_t>(nd) * 8 + 2 * k + 1].z);
-		if (l == kEmptyLink) continue;
-		if (l < 0) leaf_node[~l] = nd; else parent[l] = nd;
-	}
-}
-
 extern "C" {
 
 // closest hit through traverse_closest (tail = 1: TravClosestT with the scalar-tail sphere formula, B2R_FLAG_REFERENCE_EXACT's tail rays).
@@ -307,57 +309,18 @@ int hc_trace_closest(int kind, const b2r_sphere* prims, const b2r_bvh_node* node
 	}
 	return 0;
 }
-// any hit along [0, tfar) through traverse_any, from the root. Compare with hc_any_brute.
+// any hit along [0, tfar) through traverse_any. origin_prim null: every walk starts at the root; else walk i starts, as k_intersect_shadow's
+// does, at the node holding sphere origin_prim[i]'s leaf slot and climbs. Compare with hc_any_brute.
 int hc_trace_any(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
-                 const float* rays, const float* tfar, uint32_t n_rays, uint8_t* occ_out) {
+                 const float* rays, const float* tfar, const int32_t* origin_prim, uint32_t n_rays, uint8_t* occ_out) {
 	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
+	std::vector<uint32_t> parent, leaf_node; hc_link_tables(w, n, parent, leaf_node);
 	uint32_t cs = 0, cb = 0;
 	for (uint32_t i = 0; i < n_rays; i++) {
 		const float* r = rays + 6 * static_cast<size_t>(i);
-		occ_out[i] = traverse_any<false>(w.nodes.data(), Ray{r[0], r[1], r[2], r[3], r[4], r[5]}, tfar[i], &cs, &cb) ? 1 : 0;
-	}
-	return 0;
-}
-// k_intersect_shadow's walk restated on the host: it starts at the node holding sphere origin_prim[i]'s leaf slot, visits the nearest hit child
-// next and pushes the others, and when the subtree below `root` holds no occluder climbs to the parent, skipping the child already searched.
-int hc_trace_shadow_climb(int kind, const b2r_sphere* prims, const b2r_bvh_node* nodes, uint32_t n_nodes, const b2r_sphere* moved, uint32_t n, const float* box6,
-                          const float* rays, const float* tfar, const int32_t* origin_prim, uint32_t n_rays, uint8_t* occ_out) {
-	WideBvh w; const int rc = hc_tree(kind, prims, nodes, n_nodes, moved, n, box6, rays, n_rays, w); if (rc) return rc;
-	std::vector<uint32_t> parent, leaf_node; hc_link_tables(w, n, parent, leaf_node);
-	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
-	constexpr uint32_t kNone = 0xffffffffu;
-	for (uint32_t i = 0; i < n_rays; i++) {
-		const float* r = rays + 6 * static_cast<size_t>(i);
-		if (origin_prim[i] < 0 || static_cast<uint32_t>(origin_prim[i]) >= n) return B2R_ERR_ARG;
-		TravBase t; t.arm(Ray{r[0], r[1], r[2], r[3], r[4], r[5]});
-		ArrayStack stack; stack.reset();
-		uint32_t root = leaf_node[origin_prim[i]], up = parent[root], skip = kNone, node = root;
-		bool occ = false;
-		while (node != kNone) {
-			const float4* nd = wide + static_cast<size_t>(node) * 8;
-			uint32_t next = kNone, leaves = 0u; float next_tn = FLT_MAX;
-			for (int k = 0; k < 4; k++) {
-				const float4 a = nd[2 * k], b = nd[2 * k + 1]; const int32_t l = as_int(b.z);
-				float tn; bool h; slab(a, b, t.ix, t.iy, t.iz, t.nx, t.ny, t.nz, t.ax, t.ay, t.az, tfar[i], &tn, &h);
-				if (h && l >= 0 && static_cast<uint32_t>(l) != skip) {
-					const bool nearer = tn < next_tn;
-					const uint32_t later = nearer ? next : static_cast<uint32_t>(l);
-					if (later != kNone) stack.push(later);
-					if (nearer) { next = static_cast<uint32_t>(l); next_tn = tn; }
-				}
-				leaves |= (h && l < 0) ? (1u << k) : 0u;
-			}
-			while (leaves && !occ) {
-				const int k = first_bit(leaves); leaves &= leaves - 1u;
-				const float4 s4 = nd[2 * k];
-				occ = sphere_hit_any(s4.x, s4.y, s4.z, s4.w, t.ox, t.oy, t.oz, t.dx, t.dy, t.dz, tfar[i]);
-			}
-			if (occ) break;
-			if (next == kNone && !stack.empty()) next = stack.pop();
-			if (next == kNone && root != 0u) { skip = root; root = up; next = up; up = parent[up]; }
-			node = next;
-		}
-		occ_out[i] = occ ? 1 : 0;
+		if (origin_prim && (origin_prim[i] < 0 || static_cast<uint32_t>(origin_prim[i]) >= n)) return B2R_ERR_ARG;
+		const uint32_t start = origin_prim ? leaf_node[origin_prim[i]] : 0u;
+		occ_out[i] = traverse_any<false>(w.nodes.data(), Ray{r[0], r[1], r[2], r[3], r[4], r[5]}, tfar[i], &cs, &cb, parent.data(), start) ? 1 : 0;
 	}
 	return 0;
 }
@@ -513,9 +476,7 @@ extern "C" int hc_anyhit_local_stats(const b2r_sphere* prims, uint32_t n_prims, 
 	std::vector<b2r_bvh_node> tn; build_traversal_tree(prims, n_prims, tn);
 	WideBvh w; flatten_bvh(tn.data(), static_cast<uint32_t>(tn.size()), prims, n_prims, w, &ob);
 	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
-	const uint32_t nn = static_cast<uint32_t>(w.nodes.size());
-	std::vector<uint32_t> parent(nn, 0u), leaf_node(n_prims, 0u);
-	for (uint32_t nd = 0; nd < nn; nd++) for (int k = 0; k < 4; k++) { const int32_t l = as_int(wide[static_cast<size_t>(nd) * 8 + 2 * k + 1].z); if (l == kEmptyLink) continue; if (l < 0) leaf_node[~l] = nd; else parent[l] = nd; }
+	std::vector<uint32_t> parent, leaf_node; hc_link_tables(w, n_prims, parent, leaf_node);
 	int bad = 0;
 	for (uint32_t i = 0; i < n; i++) {
 		const float* r = rays + 6 * static_cast<size_t>(i);
@@ -564,9 +525,7 @@ extern "C" int hc_closest_climb_stats(const b2r_sphere* prims, uint32_t n_prims,
 	std::vector<b2r_bvh_node> tn; build_traversal_tree(prims, n_prims, tn);
 	WideBvh w; flatten_bvh(tn.data(), static_cast<uint32_t>(tn.size()), prims, n_prims, w, &ob);
 	const float4* wide = reinterpret_cast<const float4*>(w.nodes.data());
-	const uint32_t nn = static_cast<uint32_t>(w.nodes.size());
-	std::vector<uint32_t> parent(nn, 0u), leaf_node(n_prims, 0u);
-	for (uint32_t nd = 0; nd < nn; nd++) for (int k = 0; k < 4; k++) { const int32_t l = as_int(wide[static_cast<size_t>(nd) * 8 + 2 * k + 1].z); if (l == kEmptyLink) continue; if (l < 0) leaf_node[~l] = nd; else parent[l] = nd; }
+	std::vector<uint32_t> parent, leaf_node; hc_link_tables(w, n_prims, parent, leaf_node);
 	int bad = 0;
 	for (uint32_t i = 0; i < n; i++) {
 		const float* r = rays + 6 * static_cast<size_t>(i);

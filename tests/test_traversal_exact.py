@@ -5,7 +5,8 @@ the tie rule and [0, tfar) (duplicate, touching and nested spheres, tfar at a hi
 spheres, far away, non-finite).
 
 CPU tier: every family through every tree kind of tests/hostcheck (the product's own B2R_HD traversal compiled with g++), through
-the any-hit walk from the root and through k_intersect_shadow's climbing walk, against brute force over all spheres. GPU tier: the
+the closest-hit walk k_intersect_closest runs and the any-hit walk k_intersect_shadow runs (TravAnyT), once from the root and once
+climbing from each ray's origin sphere as the kernel does, against brute force over all spheres. GPU tier: the
 same families through b2r_trace_closest / b2r_trace_shadow for every tree flag, and the frame kernels (BVH vs brute force on the GPU)
 on scenes aimed at the same mechanisms. Every comparison is exact: prim ids and tfar bits, occlusion, bucket sums bit for bit."""
 import ctypes as C
@@ -25,8 +26,7 @@ def _declare(hc):
     vp, u32, i32 = C.c_void_p, C.c_uint32, C.c_int
     tree = [i32, vp, vp, u32, vp, u32, vp]
     hc.hc_trace_closest.argtypes = tree + [vp, u32, i32, vp, vp]; hc.hc_trace_closest.restype = i32
-    hc.hc_trace_any.argtypes = tree + [vp, vp, u32, vp]; hc.hc_trace_any.restype = i32
-    hc.hc_trace_shadow_climb.argtypes = tree + [vp, vp, vp, u32, vp]; hc.hc_trace_shadow_climb.restype = i32
+    hc.hc_trace_any.argtypes = tree + [vp, vp, vp, u32, vp]; hc.hc_trace_any.restype = i32
     hc.hc_tree_boxes.argtypes = tree + [vp, u32, vp, C.POINTER(u32)]; hc.hc_tree_boxes.restype = i32
     hc.hc_closest_brute.argtypes = [vp, u32, vp, u32, vp, vp]; hc.hc_closest_brute.restype = None
     hc.hc_closest_brute_scalar.argtypes = [vp, u32, vp, u32, vp, vp]; hc.hc_closest_brute_scalar.restype = None
@@ -80,7 +80,7 @@ def host_any(hc, case, kind, climb=False):
     n = len(case.rays); o = np.empty(n, np.uint8)
     prims, moved = (_moved_copy(case.prims), case.prims) if kind == KINDS["refit"] else (case.prims, None)
     args = (kind, _p(prims), _p(case.nodes), len(case.nodes), _p(moved), len(case.prims), _p(case.box6), _p(case.rays), _p(case.tfar))
-    rc = hc.hc_trace_shadow_climb(*args, _p(case.origin_prim), n, _p(o)) if climb else hc.hc_trace_any(*args, n, _p(o))
+    rc = hc.hc_trace_any(*args, _p(case.origin_prim) if climb else None, n, _p(o))
     return rc, o
 
 
