@@ -28,6 +28,7 @@ FLAG_FORCE_BRUTE, FLAG_FORCE_BVH, FLAG_NO_MIS, FLAG_COUNT_TESTS, FLAG_NO_GRAPH, 
 FLAG_GPU_SAH = 1024  # with FLAG_GPU_TREE: the sweep tree (SAH cuts along the curve order) instead of the packed one
 FLAG_GPU_SAH3 = 2048  # with FLAG_GPU_TREE: the three-axis sweep tree (full-sweep SAH over the x, y, z orders)
 FLAG_GGX = 512  # the reference's `#define BRDF 1` closure (Closure<GGX>, DataStreams.hpp:184-219)
+FLAG_DIELECTRIC = 4096  # materials with max(transmission) > 0 render as smooth dielectrics of IOR 1 + IOR_minus_one (DESIGN.md §2)
 TAP_CLOSEST, TAP_SHADOW, TAP_PACKET = 0, 1, 2  # b2r_trace_kernel: which traversal kernel of a frame runs
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_NO_LIGHTS, ERR_BVH, NOT_READY = 0, -1, -2, -3, -4, -5, 1
 KERNEL_KINDS = ["generate", "bounce_brute", "intersect_closest", "shade", "intersect_shadow", "accumulate", "resolve"]

@@ -18,6 +18,7 @@ namespace {
 
 thread_local std::string g_error;
 int fail(int code, const std::string& what) { g_error = what; return code; }
+constexpr const char* kDielInvalid = "B2R_FLAG_DIELECTRIC: a material has a non-finite transmission, or is dielectric (max(transmission) > 0) with a transmission outside [0, 1] or 1 + IOR_minus_one not finite or < 1";
 #define CU(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) return fail(B2R_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e_)); } while (0)
 
 enum KernelKind { KK_GENERATE = 0, KK_BRUTE, KK_CLOSEST, KK_SHADE, KK_SHADOW, KK_ACCUMULATE, KK_RESOLVE, KK_COUNT };
@@ -76,10 +77,11 @@ struct b2r_ctx {
 	uint32_t slots = 8;
 	int sm_count = 0;
 	// scene
-	float4 *d_prims = nullptr, *d_mat_albedo = nullptr, *d_mat_emission = nullptr, *d_mat_f0 = nullptr, *d_light_sphere = nullptr, *d_light_emit = nullptr, *d_hdri = nullptr;
+	float4 *d_prims = nullptr, *d_mat_albedo = nullptr, *d_mat_emission = nullptr, *d_mat_f0 = nullptr, *d_mat_diel = nullptr, *d_light_sphere = nullptr, *d_light_emit = nullptr, *d_hdri = nullptr;
 	int32_t* d_prim_mat = nullptr;
+	bool scene_diel_valid = true;  // the current scene's materials pass dielectric_materials_valid (checked when B2R_FLAG_DIELECTRIC is turned on)
 	WideNode* d_wide = nullptr;
-	size_t cap_prims = 0, cap_prim_mat = 0, cap_mat_albedo = 0, cap_mat_emission = 0, cap_mat_f0 = 0, cap_light_sphere = 0, cap_light_emit = 0, cap_wide = 0, cap_hdri = 0;
+	size_t cap_prims = 0, cap_prim_mat = 0, cap_mat_albedo = 0, cap_mat_emission = 0, cap_mat_f0 = 0, cap_mat_diel = 0, cap_light_sphere = 0, cap_light_emit = 0, cap_wide = 0, cap_hdri = 0;
 	WideBvh wide_host; uint64_t wide_key = 0; std::vector<unsigned char> wide_blob; bool have_wide = false;
 	uint32_t n_wide = 0;  // wide nodes of the current tree
 	// B2R_FLAG_GPU_TREE: the tree was built on the device (no host copy of its nodes); sort scratch; the arrays a later refit needs to match
@@ -108,6 +110,7 @@ struct b2r_ctx {
 	int grid_brute_first_ggx = 0, grid_brute_ggx = 0, grid_brute_finish_ggx = 0, grid_shade_ggx = 0;
 	int grid_brute_first = 0, grid_brute = 0, grid_closest = 0, grid_shade = 0, grid_shadow = 0, grid_stream = 0, grid_packet = 0, grid_brute_finish = 0; bool packet_primary = true;
 	int grid_brute_first_lens = 0, grid_brute_first_ggx_lens = 0, grid_packet_lens = 0;  // thin-lens bounce-0 instantiations
+	int grid_diel_brute_first[2][2] = {{0, 0}, {0, 0}}, grid_diel_brute[2] = {0, 0}, grid_diel_finish[2] = {0, 0}, grid_diel_shade[2] = {0, 0};  // B2R_FLAG_DIELECTRIC, [ggx][lens]
 	cudaGraphExec_t graph_exec = nullptr; bool graph_valid = false;
 	// twin lanes: a batch of two or more samples is traced as two independent half batches on two streams (own queues, counters and batch
 	// descriptors) inside one graph, so that the drained end of every launch of one half is filled by the other half's kernels
@@ -127,7 +130,7 @@ struct b2r_ctx {
 		bool folded_valid = false; uint64_t epoch = ~0ull;
 		// the side's own copy of the scene arrays (refreshed from the primary ones, device to device, on the side's stream when scene_version has
 		// moved on): tracing never reads the primary arrays, so a scene upload does not have to wait for the batch in flight
-		float4 *prims = nullptr, *mat_albedo = nullptr, *mat_emission = nullptr, *mat_f0 = nullptr, *light_sphere = nullptr, *light_emit = nullptr, *hdri = nullptr;
+		float4 *prims = nullptr, *mat_albedo = nullptr, *mat_emission = nullptr, *mat_f0 = nullptr, *mat_diel = nullptr, *light_sphere = nullptr, *light_emit = nullptr, *hdri = nullptr;
 		int32_t* prim_mat = nullptr; WideNode* wide = nullptr; uint32_t *parent = nullptr, *leaf_node = nullptr;
 		bool have_copy = false, refreshed_valid = false; uint64_t scene_version = ~0ull; cudaEvent_t ev_refreshed = nullptr;
 		cudaGraphExec_t exec[kMaxLanes + 1] = {nullptr, nullptr, nullptr, nullptr, nullptr}; bool valid[kMaxLanes + 1] = {false, false, false, false, false}; uint64_t launches[kMaxLanes + 1] = {0, 0, 0, 0, 0};
@@ -254,6 +257,15 @@ int compute_grids(b2r_ctx* c) {
 	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, true>), kBruteBlock, &c->grid_brute_first_lens))) return rc;
 	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, true>), kBruteBlock, &c->grid_brute_first_ggx_lens))) return rc;
 	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_packet<false, B2R_PACKET_RPL_LENS, true>), kTravBlock, &c->grid_packet_lens))) return rc;
+	const void* diel_first[2][2] = {{reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, true, true>)},
+	                                {reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, true, true>)}};
+	const void* diel_brute[2] = {reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, false, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, true, false, true>)};
+	const void* diel_finish[2] = {reinterpret_cast<const void*>(&k_brute_finish<false, false, true>), reinterpret_cast<const void*>(&k_brute_finish<false, true, true>)};
+	const void* diel_shade[2] = {reinterpret_cast<const void*>(&k_shade<false, false, true>), reinterpret_cast<const void*>(&k_shade<false, true, true>)};
+	for (int g = 0; g < 2; g++) {
+		for (int l = 0; l < 2; l++) if ((rc = occ(diel_first[g][l], kBruteBlock, &c->grid_diel_brute_first[g][l]))) return rc;
+		if ((rc = occ(diel_brute[g], kBruteBlock, &c->grid_diel_brute[g])) || (rc = occ(diel_finish[g], kBruteBlock, &c->grid_diel_finish[g])) || (rc = occ(diel_shade[g], kBruteBlock, &c->grid_diel_shade[g]))) return rc;
+	}
 	c->packet_primary = std::getenv("B2R_NO_PACKET") == nullptr;  // A/B switch for measurements: per-lane walks for the camera rays too
 	c->lanes_max = std::getenv("B2R_NO_TWIN") ? 1u : 2u;          // A/B switches for measurements: every batch as one lane / B2R_LANES = 1, 2 or 4
 	if (const char* e = std::getenv("B2R_SIDES")) { c->sides = std::atoi(e) == 1 ? 1u : 2u; }   // A/B switch: 1 = every batch on the caller's stream, one after the other
@@ -279,12 +291,13 @@ using BounceKernel = void (*)(const Params, const uint32_t);
 struct KernelSet {
 	BounceKernel brute_first, brute, brute_finish, packet, closest, shade, shadow;
 	void (*generate)(const Params);
-	int g_brute_first, g_brute, g_brute_finish, g_packet;
+	int g_brute_first, g_brute, g_brute_finish, g_packet, g_shade;
 };
 KernelSet pick_kernels(const b2r_ctx* c) {
 	const bool count = (c->cfg.flags & B2R_FLAG_COUNT_TESTS) != 0, exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0, ggx = (c->cfg.flags & B2R_FLAG_GGX) != 0;
 	const bool tn16 = c->params.scene.stack_tn_bits == 16u;  // stack entries split 16/16 (up to 65536 wide nodes: C3) get immediate shifts; other sizes read the split from the scene
 	const bool lens = c->lens.radius > 0.0f && !exact;  // (b2r_set_lens refuses a reference-exact context)
+	const bool diel = (c->cfg.flags & B2R_FLAG_DIELECTRIC) != 0;  // (never with exact: refused at b2r_create / b2r_set_flags)
 	KernelSet k{};
 	// brute-force pipeline: <FIRST, COUNT, EXACT, GGX> (the GGX closure's kernels are built without the sphere-test counters)
 	if (ggx)        { k.brute_first = k_bounce_brute<true, false, false, true>; k.brute = k_bounce_brute<false, false, false, true>; k.g_brute_first = c->grid_brute_first_ggx; k.g_brute = c->grid_brute_ggx; }
@@ -302,6 +315,19 @@ KernelSet pick_kernels(const b2r_ctx* c) {
 	if (exact) k.closest = count ? (tn16 ? k_intersect_closest<true, true, 16u> : k_intersect_closest<true, true, 0u>) : (tn16 ? k_intersect_closest<false, true, 16u> : k_intersect_closest<false, true, 0u>);
 	else       k.closest = count ? (tn16 ? k_intersect_closest<true, false, 16u> : k_intersect_closest<true, false, 0u>) : (tn16 ? k_intersect_closest<false, false, 16u> : k_intersect_closest<false, false, 0u>);
 	k.shade = ggx ? k_shade<false, true> : exact ? k_shade<true> : k_shade<false>;
+	k.g_shade = ggx ? c->grid_shade_ggx : c->grid_shade;
+	// smooth dielectric: its own shading instantiations, built without the sphere-test counters like GGX's; the traversal kernels are shared
+	if (diel) {
+		const int g = ggx ? 1 : 0, l = lens ? 1 : 0;
+		if (ggx) {
+			k.brute_first = lens ? k_bounce_brute<true, false, false, true, true, true> : k_bounce_brute<true, false, false, true, false, true>;
+			k.brute = k_bounce_brute<false, false, false, true, false, true>; k.brute_finish = k_brute_finish<false, true, true>; k.shade = k_shade<false, true, true>;
+		} else {
+			k.brute_first = lens ? k_bounce_brute<true, false, false, false, true, true> : k_bounce_brute<true, false, false, false, false, true>;
+			k.brute = k_bounce_brute<false, false, false, false, false, true>; k.brute_finish = k_brute_finish<false, false, true>; k.shade = k_shade<false, false, true>;
+		}
+		k.g_brute_first = c->grid_diel_brute_first[g][l]; k.g_brute = c->grid_diel_brute[g]; k.g_brute_finish = c->grid_diel_finish[g]; k.g_shade = c->grid_diel_shade[g];
+	}
 	k.shadow = count ? k_intersect_shadow<true> : k_intersect_shadow<false>;
 	return k;
 }
@@ -311,7 +337,7 @@ int enqueue_rounds(b2r_ctx* c, const Params& p_in, cudaStream_t st, bool profile
 	// (measurement tap, B2R_LANE_GRID: the lanes of a twin batch may be given a fraction of the resident-CTA grid each, so that the two lanes'
 	// kernels sit on every SM side by side instead of taking turns)
 	auto G = [&](int g) { const int per_sm = g / c->sm_count; int k = static_cast<int>(per_sm * grid_frac + 0.5f); if (k < 1) k = 1; return k * c->sm_count; };
-	const bool exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0, ggx = (c->cfg.flags & B2R_FLAG_GGX) != 0;
+	const bool exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0;
 	if (exact && c->params.scene.n_mat > 64) return fail(B2R_ERR_STATE, "B2R_FLAG_REFERENCE_EXACT: at most 64 materials (RendererPolicy::max_materialID, Renderer.hpp:23)");
 	const KernelSet k = pick_kernels(c);
 	const uint32_t mb = c->cfg.max_bounces;
@@ -336,7 +362,7 @@ int enqueue_rounds(b2r_ctx* c, const Params& p_in, cudaStream_t st, bool profile
 	for (uint32_t b = 0; b < mb; b++) {
 		if (b == 0 && c->packet_primary) { if ((rc = run(KK_CLOSEST, k.packet, G(k.g_packet), kTravBlock, b))) return rc; }  // camera rays: one walk per warp
 		else if ((rc = run(KK_CLOSEST, k.closest, G(c->grid_closest), kTravBlock, b))) return rc;
-		if ((rc = run(KK_SHADE, k.shade, G(ggx ? c->grid_shade_ggx : c->grid_shade), kBruteBlock, b))) return rc;
+		if ((rc = run(KK_SHADE, k.shade, G(k.g_shade), kBruteBlock, b))) return rc;
 		if (exact && b + 1 < mb && (rc = run(KK_SHADE, k_stream_rank, c->grid_stream, 256, b))) return rc;
 		if (mis && b + 1 < mb && (rc = run(KK_SHADOW, k.shadow, G(c->grid_shadow), kTravBlock, b))) return rc;
 	}
@@ -368,6 +394,7 @@ Params lane_params(const b2r_ctx* c, uint32_t which, uint32_t lanes, uint32_t si
 		sc.prims = S.prims; sc.prim_mat = S.prim_mat; sc.mat_albedo = S.mat_albedo; sc.mat_emission = S.mat_emission; sc.mat_f0 = S.mat_f0;
 		sc.light_sphere = S.light_sphere; sc.light_emit = S.light_emit; sc.wide = S.wide; sc.parent = S.parent; sc.leaf_node = S.leaf_node;
 		if (sc.hdri) sc.hdri = S.hdri;
+		p.mat_diel = S.mat_diel;
 	}
 	return p;
 }
@@ -533,7 +560,7 @@ bool owns_sample(const b2r_ctx* c, uint32_t acc) {
 // earlier waits), and the sides learn that their copies are stale.
 void free_side_scenes(b2r_ctx* c) {
 	for (auto& S : c->side) {
-		dev_free(&S.prims); dev_free(&S.mat_albedo); dev_free(&S.mat_emission); dev_free(&S.mat_f0); dev_free(&S.light_sphere); dev_free(&S.light_emit); dev_free(&S.hdri);
+		dev_free(&S.prims); dev_free(&S.mat_albedo); dev_free(&S.mat_emission); dev_free(&S.mat_f0); dev_free(&S.mat_diel); dev_free(&S.light_sphere); dev_free(&S.light_emit); dev_free(&S.hdri);
 		dev_free(&S.prim_mat); dev_free(&S.wide); dev_free(&S.parent); dev_free(&S.leaf_node);
 		S.have_copy = false; S.scene_version = ~0ull;
 		for (uint32_t l = 0; l <= kMaxLanes; l++) S.valid[l] = false;  // the captured graphs hold the old addresses
@@ -567,7 +594,7 @@ int refresh_side_scene(b2r_ctx* c, uint32_t sidx) {
 	if (!S.have_copy) {
 		int rc;
 		if ((rc = dev_alloc(&S.prims, c->cap_prims)) || (rc = dev_alloc(&S.prim_mat, c->cap_prim_mat)) || (rc = dev_alloc(&S.mat_albedo, c->cap_mat_albedo)) ||
-		    (rc = dev_alloc(&S.mat_emission, c->cap_mat_emission)) || (rc = dev_alloc(&S.mat_f0, c->cap_mat_f0)) || (rc = dev_alloc(&S.light_sphere, c->cap_light_sphere)) ||
+		    (rc = dev_alloc(&S.mat_emission, c->cap_mat_emission)) || (rc = dev_alloc(&S.mat_f0, c->cap_mat_f0)) || (rc = dev_alloc(&S.mat_diel, c->cap_mat_diel)) || (rc = dev_alloc(&S.light_sphere, c->cap_light_sphere)) ||
 		    (rc = dev_alloc(&S.light_emit, c->cap_light_emit)) || (rc = dev_alloc(&S.wide, c->cap_wide)) || (rc = dev_alloc(&S.parent, c->cap_parent)) ||
 		    (rc = dev_alloc(&S.leaf_node, c->cap_leaf_node)) || (rc = dev_alloc(&S.hdri, c->cap_hdri))) return rc;
 		if (!S.ev_refreshed) CU(cudaEventCreateWithFlags(&S.ev_refreshed, cudaEventDisableTiming));
@@ -579,6 +606,7 @@ int refresh_side_scene(b2r_ctx* c, uint32_t sidx) {
 	const size_t n_l = sc.n_lights ? sc.n_lights : 1u;
 	CU(copy(S.prims, c->d_prims, sc.n_prims * sizeof(float4))); CU(copy(S.prim_mat, c->d_prim_mat, sc.n_prims * sizeof(int32_t)));
 	CU(copy(S.mat_albedo, c->d_mat_albedo, sc.n_mat * sizeof(float4))); CU(copy(S.mat_emission, c->d_mat_emission, sc.n_mat * sizeof(float4))); CU(copy(S.mat_f0, c->d_mat_f0, sc.n_mat * sizeof(float4)));
+	CU(copy(S.mat_diel, c->d_mat_diel, sc.n_mat * sizeof(float4)));
 	CU(copy(S.light_sphere, c->d_light_sphere, n_l * sizeof(float4))); CU(copy(S.light_emit, c->d_light_emit, n_l * sizeof(float4)));
 	CU(copy(S.wide, c->d_wide, static_cast<size_t>(c->n_wide) * sizeof(WideNode))); CU(copy(S.parent, c->d_parent, static_cast<size_t>(c->n_wide) * sizeof(uint32_t)));
 	CU(copy(S.leaf_node, c->d_leaf_node, sc.n_prims * sizeof(uint32_t)));
@@ -751,6 +779,7 @@ int b2r_create(b2r_ctx** out, const b2r_config* cfg) {
 	if (cfg->bucket_stride > 1 && cfg->bucket_first >= cfg->bucket_stride) return fail(B2R_ERR_ARG, "bucket_first must be < bucket_stride");
 	if (cfg->samples_in_flight > static_cast<uint32_t>(kMaxSlots)) return fail(B2R_ERR_ARG, "samples_in_flight must be <= 64");
 	if ((cfg->flags & B2R_FLAG_GGX) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_GGX cannot be combined with B2R_FLAG_REFERENCE_EXACT");
+	if ((cfg->flags & B2R_FLAG_DIELECTRIC) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	int n_dev = 0;
 	cudaError_t e = cudaGetDeviceCount(&n_dev);
 	if (e != cudaSuccess || n_dev == 0) return fail(B2R_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(e) + " (libb2r has no CPU fallback)");
@@ -776,7 +805,7 @@ void b2r_destroy(b2r_ctx* c) {
 	b2r_team_close(c); if (c->d_team) { cudaFree(c->d_team); c->d_team = nullptr; }
 	drop_graph(c);
 	for (auto& t : c->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
-	dev_free(&c->d_prims); dev_free(&c->d_mat_albedo); dev_free(&c->d_mat_emission); dev_free(&c->d_mat_f0); dev_free(&c->d_light_sphere); dev_free(&c->d_light_emit);
+	dev_free(&c->d_prims); dev_free(&c->d_mat_albedo); dev_free(&c->d_mat_emission); dev_free(&c->d_mat_f0); dev_free(&c->d_mat_diel); dev_free(&c->d_light_sphere); dev_free(&c->d_light_emit);
 	dev_free(&c->d_hdri); dev_free(&c->d_prim_mat); dev_free(&c->d_wide); dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_tap); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep);
 	for (int k = 0; k < 2; k++) { dev_free(&c->d_mkey[k]); dev_free(&c->d_midx[k]); }
 	for (int s = 0; s < 2; s++) { dev_free(&c->d_A[s]); dev_free(&c->d_B[s]); dev_free(&c->d_T[s]); }
@@ -847,6 +876,8 @@ int b2r_set_flags(b2r_ctx* c, uint32_t flags) {
 	if ((c->cfg.flags ^ flags) & B2R_FLAG_REFERENCE_TREE) return fail(B2R_ERR_STATE, "B2R_FLAG_REFERENCE_TREE can only be chosen at b2r_create");
 	if ((c->cfg.flags ^ flags) & B2R_FLAG_REFERENCE_EXACT) return fail(B2R_ERR_STATE, "B2R_FLAG_REFERENCE_EXACT can only be chosen at b2r_create");
 	if ((flags & B2R_FLAG_GGX) && (flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_GGX cannot be combined with B2R_FLAG_REFERENCE_EXACT");
+	if ((flags & B2R_FLAG_DIELECTRIC) && (flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
+	if ((flags & B2R_FLAG_DIELECTRIC) && c->have_scene && !c->scene_diel_valid) return fail(B2R_ERR_ARG, kDielInvalid);
 	c->cfg.flags = flags; c->params.frame.flags = flags;
 	if (c->have_scene) {
 		const uint32_t n = c->params.scene.n_prims;
@@ -895,6 +926,8 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	if (has_ambient && (!hdri_rgba || hdri_w <= 0 || hdri_h <= 0)) return fail(B2R_ERR_ARG, "ambient > 0 needs an HDRI (the reference terminates without one, Application.cpp:225-229)");
 	for (uint32_t i = 0; i < n_prims; i++) if (prims[i].material_ID < 0 || static_cast<uint32_t>(prims[i].material_ID) >= n_mat || geometry[i].material_ID < 0 || static_cast<uint32_t>(geometry[i].material_ID) >= n_mat) return fail(B2R_ERR_ARG, "material_ID out of range");
 	for (uint32_t i = 0; i < n_lights; i++) if (light_geom_idx[i] < 0 || static_cast<uint32_t>(light_geom_idx[i]) >= n_geom) return fail(B2R_ERR_ARG, "light index out of range");
+	const bool diel_valid = dielectric_materials_valid(materials, n_mat);
+	if (!diel_valid && (c->cfg.flags & B2R_FLAG_DIELECTRIC)) return fail(B2R_ERR_ARG, kDielInvalid);
 	int rc = ensure_device(c); if (rc) return rc;
 	// No stream synchronisation from here on: the copies below are ordered after the kernels already enqueued on the stream (which
 	// may still read the old scene) and before the ones enqueued next. The host side is staged in one page-locked block that is only
@@ -950,8 +983,8 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	if (c->n_wide >= kMaxWideNodes) { c->have_wide = false; return fail(B2R_ERR_BVH, "more than 2^22 traversal nodes (stack entries keep 22 node bits)"); }
 
 	PackedScene ps; pack_scene(prims, n_prims, materials, n_mat, light_geom_idx, n_lights, geometry, ps);
-	auto &h_prims = ps.prims, &h_alb = ps.mat_albedo, &h_em = ps.mat_emission, &h_f0 = ps.mat_f0, &h_ls = ps.light_sphere, &h_le = ps.light_emit; auto& h_pm = ps.prim_mat;
-	const bool grow = h_prims.size() > c->cap_prims || h_pm.size() > c->cap_prim_mat || h_alb.size() > c->cap_mat_albedo || h_em.size() > c->cap_mat_emission || h_f0.size() > c->cap_mat_f0 ||
+	auto &h_prims = ps.prims, &h_alb = ps.mat_albedo, &h_em = ps.mat_emission, &h_f0 = ps.mat_f0, &h_diel = ps.mat_diel, &h_ls = ps.light_sphere, &h_le = ps.light_emit; auto& h_pm = ps.prim_mat;
+	const bool grow = h_prims.size() > c->cap_prims || h_pm.size() > c->cap_prim_mat || h_alb.size() > c->cap_mat_albedo || h_em.size() > c->cap_mat_emission || h_f0.size() > c->cap_mat_f0 || h_diel.size() > c->cap_mat_diel ||
 	                  h_ls.size() > c->cap_light_sphere || h_le.size() > c->cap_light_emit || c->n_wide > c->cap_wide || c->n_wide > c->cap_parent || n_prims > c->cap_leaf_node ||
 	                  (has_ambient && static_cast<size_t>(hdri_w) * hdri_h > c->cap_hdri);
 	if (grow) {  // device arrays in use are about to be replaced (first upload, or a larger scene): nothing may be running, and the sides' copies go too
@@ -964,6 +997,7 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	if ((rc = dev_reserve(&c->d_mat_albedo, &c->cap_mat_albedo, h_alb.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_mat_emission, &c->cap_mat_emission, h_em.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_mat_f0, &c->cap_mat_f0, h_f0.size()))) return rc;
+	if ((rc = dev_reserve(&c->d_mat_diel, &c->cap_mat_diel, h_diel.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_light_sphere, &c->cap_light_sphere, h_ls.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_light_emit, &c->cap_light_emit, h_le.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_wide, &c->cap_wide, static_cast<size_t>(c->n_wide)))) return rc;
@@ -974,6 +1008,7 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	const UploadPart parts[] = {
 		{c->d_prims, h_prims.data(), h_prims.size() * sizeof(float4)}, {c->d_prim_mat, h_pm.data(), h_pm.size() * sizeof(int32_t)},
 		{c->d_mat_albedo, h_alb.data(), h_alb.size() * sizeof(float4)}, {c->d_mat_emission, h_em.data(), h_em.size() * sizeof(float4)}, {c->d_mat_f0, h_f0.data(), h_f0.size() * sizeof(float4)},
+		{c->d_mat_diel, h_diel.data(), h_diel.size() * sizeof(float4)},
 		{c->d_light_sphere, h_ls.data(), h_ls.size() * sizeof(float4)}, {c->d_light_emit, h_le.data(), h_le.size() * sizeof(float4)},
 		{c->d_wide, c->wide_host.nodes.data(), gpu_tree ? 0 : c->wide_host.nodes.size() * sizeof(WideNode)}, {c->d_hdri, hdri_rgba, texels * sizeof(float4)},
 	};
@@ -1010,9 +1045,9 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	}
 	if ((rc = launch_link_tables(c))) return rc;
 	if ((rc = end_scene_write(c))) return rc;
-	const SceneDev before = c->params.scene; const bool bvh_before = c->use_bvh;
+	const SceneDev before = c->params.scene; const bool bvh_before = c->use_bvh; const float4* diel_before = c->params.mat_diel;
 	SceneDev& s = c->params.scene;
-	s.prims = c->d_prims; s.prim_mat = c->d_prim_mat; s.mat_albedo = c->d_mat_albedo; s.mat_emission = c->d_mat_emission; s.mat_f0 = c->d_mat_f0;
+	s.prims = c->d_prims; s.prim_mat = c->d_prim_mat; s.mat_albedo = c->d_mat_albedo; s.mat_emission = c->d_mat_emission; s.mat_f0 = c->d_mat_f0; c->params.mat_diel = c->d_mat_diel;
 	s.light_sphere = c->d_light_sphere; s.light_emit = c->d_light_emit; s.wide = c->d_wide; s.hdri = has_ambient ? c->d_hdri : nullptr;
 	s.parent = c->d_parent; s.leaf_node = c->d_leaf_node;
 	s.n_prims = n_prims; s.n_mat = n_mat; s.n_lights = n_lights; s.stack_tn_bits = c->wide_host.tn_bits;
@@ -1021,8 +1056,8 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	s.hdri_w = hdri_w; s.hdri_h = hdri_h; s.hdri_fw = static_cast<float>(hdri_w - 1); s.hdri_fh = static_cast<float>(hdri_h - 1);  // Application.cpp:230-231
 	c->use_bvh = (c->cfg.flags & B2R_FLAG_FORCE_BVH) ? true : (c->cfg.flags & B2R_FLAG_FORCE_BRUTE) ? false : n_prims > 32;
 	// the scene's pointers and scalars travel in the kernels' parameter block: the captured graph stays valid unless they changed
-	if (!c->have_scene || bvh_before != c->use_bvh || std::memcmp(&before, &s, sizeof s) != 0) drop_graph(c);
-	c->have_scene = true;
+	if (!c->have_scene || bvh_before != c->use_bvh || diel_before != c->params.mat_diel || std::memcmp(&before, &s, sizeof s) != 0) drop_graph(c);
+	c->have_scene = true; c->scene_diel_valid = diel_valid;
 	return B2R_OK;
 }
 
@@ -1034,6 +1069,8 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	if (n_lights && !light_geom_idx) return fail(B2R_ERR_ARG, "null light list");
 	for (uint32_t i = 0; i < n_prims; i++) if (prims[i].material_ID < 0 || static_cast<uint32_t>(prims[i].material_ID) >= n_mat || geometry[i].material_ID < 0 || static_cast<uint32_t>(geometry[i].material_ID) >= n_mat) return fail(B2R_ERR_ARG, "material_ID out of range");
 	for (uint32_t i = 0; i < n_lights; i++) if (light_geom_idx[i] < 0 || static_cast<uint32_t>(light_geom_idx[i]) >= n_geom) return fail(B2R_ERR_ARG, "light index out of range");
+	const bool diel_valid = dielectric_materials_valid(materials, n_mat);
+	if (!diel_valid && (c->cfg.flags & B2R_FLAG_DIELECTRIC)) return fail(B2R_ERR_ARG, kDielInvalid);
 	int rc = ensure_device(c); if (rc) return rc;
 	// The caller may have re-sorted its prims (the reference's constructor does on every rebuild, BVH.hpp:201-205): leaf links become
 	// indices into the NEW order. old index -> geometry index (known from the last upload / refit) -> new index (matched by value).
@@ -1056,7 +1093,7 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	}
 	PackedScene ps; pack_scene(prims, n_prims, materials, n_mat, light_geom_idx, n_lights, geometry, ps);
 	if ((rc = dev_reserve(&c->d_remap, &c->cap_remap, remap.size()))) return rc;
-	const bool grow = ps.mat_albedo.size() > c->cap_mat_albedo || ps.mat_emission.size() > c->cap_mat_emission || ps.mat_f0.size() > c->cap_mat_f0 ||
+	const bool grow = ps.mat_albedo.size() > c->cap_mat_albedo || ps.mat_emission.size() > c->cap_mat_emission || ps.mat_f0.size() > c->cap_mat_f0 || ps.mat_diel.size() > c->cap_mat_diel ||
 	                  ps.light_sphere.size() > c->cap_light_sphere || ps.light_emit.size() > c->cap_light_emit;
 	if (grow) {  // more materials or lights than before: those (small) arrays are replaced
 		CU(sync_main(c)); if (c->up_stream) CU(cudaStreamSynchronize(c->up_stream));
@@ -1066,12 +1103,14 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	if ((rc = dev_reserve(&c->d_mat_albedo, &c->cap_mat_albedo, ps.mat_albedo.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_mat_emission, &c->cap_mat_emission, ps.mat_emission.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_mat_f0, &c->cap_mat_f0, ps.mat_f0.size()))) return rc;
+	if ((rc = dev_reserve(&c->d_mat_diel, &c->cap_mat_diel, ps.mat_diel.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_light_sphere, &c->cap_light_sphere, ps.light_sphere.size()))) return rc;
 	if ((rc = dev_reserve(&c->d_light_emit, &c->cap_light_emit, ps.light_emit.size()))) return rc;
 	if (!c->d_cost) { size_t cap = 0; if ((rc = dev_reserve(&c->d_cost, &cap, 1))) return rc; }
 	const UploadPart parts[] = {
 		{c->d_prims, ps.prims.data(), ps.prims.size() * sizeof(float4)}, {c->d_prim_mat, ps.prim_mat.data(), ps.prim_mat.size() * sizeof(int32_t)},
 		{c->d_mat_albedo, ps.mat_albedo.data(), ps.mat_albedo.size() * sizeof(float4)}, {c->d_mat_emission, ps.mat_emission.data(), ps.mat_emission.size() * sizeof(float4)}, {c->d_mat_f0, ps.mat_f0.data(), ps.mat_f0.size() * sizeof(float4)},
+		{c->d_mat_diel, ps.mat_diel.data(), ps.mat_diel.size() * sizeof(float4)},
 		{c->d_light_sphere, ps.light_sphere.data(), ps.light_sphere.size() * sizeof(float4)}, {c->d_light_emit, ps.light_emit.data(), ps.light_emit.size() * sizeof(float4)},
 		{c->d_remap, remap.data(), remap.size() * sizeof(uint32_t)},
 	};
@@ -1092,12 +1131,12 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	if ((rc = launch_refit_levels(c, same_order ? nullptr : c->d_remap))) return rc;
 	if (!same_order && (rc = launch_link_tables(c))) return rc;  // leaves were re-linked into the new BVH order
 	if ((rc = end_scene_write(c))) return rc;
-	c->wide_refit = true; drop_speculation(c);
-	const SceneDev before = c->params.scene;
+	c->wide_refit = true; drop_speculation(c); c->scene_diel_valid = diel_valid;
+	const SceneDev before = c->params.scene; const float4* diel_before = c->params.mat_diel;
 	SceneDev& s = c->params.scene;
-	s.mat_albedo = c->d_mat_albedo; s.mat_emission = c->d_mat_emission; s.mat_f0 = c->d_mat_f0; s.light_sphere = c->d_light_sphere; s.light_emit = c->d_light_emit;
+	s.mat_albedo = c->d_mat_albedo; s.mat_emission = c->d_mat_emission; s.mat_f0 = c->d_mat_f0; c->params.mat_diel = c->d_mat_diel; s.light_sphere = c->d_light_sphere; s.light_emit = c->d_light_emit;
 	s.n_mat = n_mat; s.n_lights = n_lights; s.light_sel_pdf = n_lights ? 1.0f / static_cast<float>(n_lights) : 0.0f;  // Renderer.hpp:78
-	if (std::memcmp(&before, &s, sizeof s) != 0) drop_graph(c);
+	if (diel_before != c->params.mat_diel || std::memcmp(&before, &s, sizeof s) != 0) drop_graph(c);
 	if (quality_out) {  // optional: costs one launch and a stream synchronisation
 		c->main_reads_scene = true;
 		CU(cudaMemsetAsync(c->d_cost, 0, sizeof(double), c->stream));
@@ -1435,7 +1474,7 @@ int b2r_write_buckets(b2r_ctx* c, const float* in_host) {
 namespace {
 struct CheckpointHeader { char magic[8]; uint32_t width, height, buckets, max_bounces, accumulations, result_flags; uint64_t payload_hash; uint64_t payload_bytes; uint32_t reserved[4]; };
 static_assert(sizeof(CheckpointHeader) == 64, "checkpoint header");
-constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT;  // flags that change which image is being accumulated
+constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT | B2R_FLAG_DIELECTRIC;  // flags that change which image is being accumulated
 uint64_t fnv1a64(const void* data, size_t bytes) { const unsigned char* b = static_cast<const unsigned char*>(data); uint64_t h = 1469598103934665603ull; for (size_t i = 0; i < bytes; i++) h = (h ^ b[i]) * 1099511628211ull; return h; }
 }  // namespace
 int b2r_save_checkpoint(b2r_ctx* c, const char* path) {

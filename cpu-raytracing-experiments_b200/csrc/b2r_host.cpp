@@ -579,13 +579,16 @@ void pack_scene(const b2r_sphere* prims, uint32_t n_prims, const b2r_material* m
 		out.prims[i] = f4(prims[i].position[0], prims[i].position[1], prims[i].position[2], prims[i].radius_sq);
 		out.prim_mat[i] = prims[i].material_ID;
 	}
-	out.mat_albedo.resize(n_mat); out.mat_emission.resize(n_mat); out.mat_f0.resize(n_mat);
+	out.mat_albedo.resize(n_mat); out.mat_emission.resize(n_mat); out.mat_f0.resize(n_mat); out.mat_diel.resize(n_mat);
 	for (uint32_t i = 0; i < n_mat; i++) {
 		const float* e = materials[i].emission;
 		const bool emissive = sel_max(e[0], sel_max(e[1], e[2])) > FLT_EPSILON;  // is_emissive, Renderer.hpp:201
 		out.mat_albedo[i] = f4(materials[i].albedo[0], materials[i].albedo[1], materials[i].albedo[2], emissive ? 1.0f : 0.0f);
 		out.mat_emission[i] = f4(e[0], e[1], e[2], 0.0f);
 		out.mat_f0[i] = f4(materials[i].F0[0], materials[i].F0[1], materials[i].F0[2], materials[i].roughness);  // Closure<GGX>, Renderer.hpp:210-211
+		const float* t = materials[i].transmission;
+		const bool diel = sel_max(t[0], sel_max(t[1], t[2])) > 0.0f;  // B2R_FLAG_DIELECTRIC: eta = 0 marks a material that is not dielectric
+		out.mat_diel[i] = diel ? f4(t[0], t[1], t[2], 1.0f + materials[i].IOR_minus_one) : f4(0.0f, 0.0f, 0.0f, 0.0f);
 	}
 	out.light_sphere.resize(n_lights ? n_lights : 1, f4(0, 0, 0, 0)); out.light_emit.resize(n_lights ? n_lights : 1, f4(0, 0, 0, 0));
 	for (uint32_t i = 0; i < n_lights; i++) {  // NEE reads the light from scene.geometry, original order (Renderer.hpp:261-262,277)
@@ -594,6 +597,18 @@ void pack_scene(const b2r_sphere* prims, uint32_t n_prims, const b2r_material* m
 		out.light_sphere[i] = f4(g.position[0], g.position[1], g.position[2], g.radius_sq);
 		out.light_emit[i] = f4(e[0], e[1], e[2], int_as_float(light_geom_idx[i]));
 	}
+}
+
+bool dielectric_materials_valid(const b2r_material* materials, uint32_t n_mat) {
+	for (uint32_t i = 0; i < n_mat; i++) {
+		const float* t = materials[i].transmission;
+		if (!std::isfinite(t[0]) || !std::isfinite(t[1]) || !std::isfinite(t[2])) return false;
+		if (!(sel_max(t[0], sel_max(t[1], t[2])) > 0.0f)) continue;
+		const float eta = 1.0f + materials[i].IOR_minus_one;
+		for (int k = 0; k < 3; k++) if (!(t[k] >= 0.0f && t[k] <= 1.0f)) return false;
+		if (!std::isfinite(eta) || !(eta >= 1.0f)) return false;
+	}
+	return true;
 }
 
 }  // namespace b2r

@@ -80,10 +80,13 @@ bool match_prims_to_geometry(const b2r_sphere* prims, const b2r_sphere* geometry
 // Scene arrays in the packed form the kernels read (SceneDev): spheres {c.xyz, r^2} in BVH leaf order, per-material
 // {albedo, emissive flag} and {emission}, per-light {sphere of scene.geometry[light]} and {emission, light_primID}.
 struct PackedScene {
-	std::vector<float4> prims, mat_albedo, mat_emission, mat_f0, light_sphere, light_emit;
+	std::vector<float4> prims, mat_albedo, mat_emission, mat_f0, mat_diel, light_sphere, light_emit;
 	std::vector<int32_t> prim_mat;
 };
 void pack_scene(const b2r_sphere* prims, uint32_t n_prims, const b2r_material* materials, uint32_t n_mat,
                 const int32_t* light_geom_idx, uint32_t n_lights, const b2r_sphere* geometry, PackedScene& out);
+// B2R_FLAG_DIELECTRIC input rule: every transmission component is finite, and a dielectric material (max(transmission) > 0) has every
+// component in [0, 1] and eta = 1 + IOR_minus_one finite and >= 1. Returns false when some material breaks it.
+bool dielectric_materials_valid(const b2r_material* materials, uint32_t n_mat);
 
 }  // namespace b2r

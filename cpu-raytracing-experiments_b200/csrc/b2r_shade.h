@@ -108,6 +108,9 @@ struct Params {
 	const BatchDev* batch;
 	float* rad;   // RAD
 	float* acc;   // ACC
+	// [n_mat] {transmission.rgb, eta}, eta = 0 when max(transmission) == 0: read by the DIELECTRIC shading routines only (B2R_FLAG_DIELECTRIC).
+	// A scene table, but kept here at the end rather than in SceneDev, so the parameter block of every other instantiation keeps its layout.
+	const float4* mat_diel;
 };
 
 // ---------------------------------------------------------------------------------------------- small helpers
@@ -145,19 +148,41 @@ B2R_HD PathState primary_path(const FrameDev& fr, const CameraParams& cam, uint3
 
 
 // ---------------------------------------------------------------------------------------------- shading
-struct Surface { f3 P; TangentQuat T; float n_dot_v; f3 albedo; bool emissive; int32_t mat; float r2; f3 v_local; float alpha; };  // GGX: albedo holds F0; v_local / alpha are only set (and read) by the GGX closure
+struct Surface {
+	f3 P; TangentQuat T; float n_dot_v; f3 albedo; bool emissive; int32_t mat; float r2; f3 v_local; float alpha;  // GGX: albedo holds F0; v_local / alpha are only set (and read) by the GGX closure
+	bool inside; float4 diel; f3 P_in;  // DIELECTRIC only: N was flipped (the ray leaves the sphere), {transmission.rgb, eta} (eta = 0: not dielectric), hit - 1e-4 N
+};
 struct ShadowRay { f3 o, d; float tfar; f3 L; };
+
+// Smooth dielectric (B2R_FLAG_DIELECTRIC, DESIGN §2): v = the direction towards the viewer in the local frame (N = +z, flipped against
+// the ray), r = the ratio of the indices of refraction (1 / eta entering, eta leaving). With c = clamp(v.z, 0, 1) and s2 = r^2 (1 - c^2),
+// s2 >= 1 is total internal reflection (F = 1, reflected whatever u0 is: next_unit can return 1.0, Q4); otherwise ct = sqrt(1 - s2) and F is
+// the unpolarised Fresnel reflectance. u0 < F reflects into (-v.x, -v.y, c), else the ray refracts into (-r v.x, -r v.y, -ct). Only + - * / and
+// sqrt, so host (-ffp-contract=off) and device (-fmad=false) agree bit for bit. Returns true for a reflection.
+B2R_HD bool dielectric_scatter(f3 v, float r, float u0, f3* dir, float* F) {
+	const float c = sel_min(sel_max(v.z, 0.0f), 1.0f);
+	const float s2 = r * r * (1.0f - c * c);
+	if (s2 >= 1.0f) { *F = 1.0f; *dir = f3{-v.x, -v.y, c}; return true; }
+	const float ct = sqrtf(1.0f - s2);
+	const float rs = (r * c - ct) / (r * c + ct), rp = (r * ct - c) / (r * ct + c);
+	*F = (rs * rs + rp * rp) * 0.5f;
+	const bool refl = u0 < *F;
+	*dir = refl ? f3{-v.x, -v.y, c} : f3{-r * v.x, -r * v.y, -ct};
+	return refl;
+}
 
 // closest-hit shader, Renderer.hpp:169-214. GGX = the reference's `#define BRDF 1` build (Renderer.hpp:70,207-213): the closure takes F0 and
 // alpha = roughness^2 + (1 - roughness^2) * gloss_decay_table[bounce]; the reference never declares that table, it is all zeros here as in
-// oracle/ref_renderer_build.sh's build of the reference itself.
-template <bool GGX = false>
-B2R_HD Surface shade_surface(const SceneDev& sc, const PathState& s, float depth, int32_t prim) {
+// oracle/ref_renderer_build.sh's build of the reference itself. DIELECTRIC (B2R_FLAG_DIELECTRIC): also the material's dielectric data, whether
+// the ray leaves the sphere, and the refracted ray's origin, 1e-4 behind the surface.
+template <bool GGX = false, bool DIELECTRIC = false>
+B2R_HD Surface shade_surface(const SceneDev& sc, const PathState& s, float depth, int32_t prim, const float4* mat_diel = nullptr) {
 	const float4 sp = ld4(sc.prims + prim);
 	const f3 D{s.dx, s.dy, s.dz};
 	const f3 hp{s.ox + D.x * depth, s.oy + D.y * depth, s.oz + D.z * depth};
 	f3 N = unit3(f3{hp.x - sp.x, hp.y - sp.y, hp.z - sp.z});
-	if (dot3(N, D) >= 0.0f) N = f3{-N.x, -N.y, -N.z};  // backface
+	const bool flip = dot3(N, D) >= 0.0f;
+	if (flip) N = f3{-N.x, -N.y, -N.z};  // backface
 	Surface sf;
 	sf.T = tangent_frame(N);
 	const f3 vl = frame_to_local(sf.T, f3{-D.x, -D.y, -D.z});
@@ -171,12 +196,18 @@ B2R_HD Surface shade_surface(const SceneDev& sc, const PathState& s, float depth
 		float alpha = fr.w; alpha *= alpha;
 		sf.albedo = f3{fr.x, fr.y, fr.z}; sf.alpha = alpha + (1.0f - alpha) * 0.0f; sf.v_local = vl;  // Renderer.hpp:210-212
 	}
+	if (DIELECTRIC) {
+		sf.diel = ld4(mat_diel + sf.mat); sf.inside = flip; sf.v_local = vl;
+		sf.P_in = f3{hp.x - N.x * 1e-4f, hp.y - N.y * 1e-4f, hp.z - N.z * 1e-4f};
+	}
 	return sf;
 }
-// next-event estimation, Renderer.hpp:249-298. Returns false when no shadow ray is produced.
-template <bool GGX = false>
+template <bool DIELECTRIC> B2R_HD bool is_dielectric(const Surface& sf) { return DIELECTRIC && sf.diel.w != 0.0f; }
+// next-event estimation, Renderer.hpp:249-298. Returns false when no shadow ray is produced; a dielectric surface (delta BSDF) never makes one.
+template <bool GGX = false, bool DIELECTRIC = false>
 B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const PathState& s, int32_t hit_prim,
                                                    uint32_t acc, uint32_t seed, uint32_t bounce, ShadowRay* out) {
+	if (is_dielectric<DIELECTRIC>(sf)) return false;
 	if (sc.n_lights == 0u) return false;  // undefined in the reference (Q15); defined here as "no light sampling"
 	Pcg rng{hash_2d(acc, seed + bounce * 2u)};  // Q3
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
@@ -209,31 +240,42 @@ B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const Path
 	out->o = sf.P; out->d = L; out->tfar = ldist; out->L = rad;
 	return true;
 }
-// emissive-hit contribution, Renderer.hpp:319-353
+// emissive-hit contribution, Renderer.hpp:319-353. DIELECTRIC: a path continued from a dielectric surface carries pdf = -1 (no light sample
+// competes with a delta BSDF), and its MIS weight is 1.
+template <bool DIELECTRIC = false>
 B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState& s, float depth, uint32_t bounce, bool mis) {
 	const float4 em = ld4(sc.mat_emission + sf.mat);
 	if (!mis) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};  // this repo's MIS-off (Q23)
 	if (bounce == 0) return f3{em.x, em.y, em.z};
+	if (DIELECTRIC && s.pdf < 0.0f) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};
 	const float d2 = depth * (depth + sf.n_dot_v * (2.0f * sqrtf(sf.r2))) + sf.r2;  // law of cosines, Renderer.hpp:331
 	const float w = power_heuristic(s.pdf, sc.light_sel_pdf * sphere_light_pdf(sf.r2, d2));
 	return f3{(s.tr * w) * em.x, (s.tg * w) * em.y, (s.tb * w) * em.z};
 }
-// BRDF sampling + Russian roulette, Renderer.hpp:359-403. Returns false when the path is terminated by roulette.
-template <bool GGX = false>
+// BRDF sampling + Russian roulette, Renderer.hpp:359-403. Returns false when the path is terminated by roulette. A dielectric surface
+// (DIELECTRIC) reflects or refracts by the stream's first float (dielectric_scatter; the second is unused, roulette keeps the third), a
+// refraction scales the throughput by the transmission and leaves from P_in, and the path stores pdf = -1 (specular predecessor).
+template <bool GGX = false, bool DIELECTRIC = false>
 B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32_t seed, uint32_t bounce) {
 	Pcg rng{hash_2d(acc, seed + bounce * 2u + 1u)};
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
-	f3 dl, est = sf.albedo;
-	if (GGX) ggx_sample(sf.albedo, sf.alpha, sf.v_local, u0, u1, &dl, &est);  // Closure<GGX>::sample, DataStreams.hpp:199-218
+	f3 dl, est = sf.albedo, o = sf.P;
+	const bool delta = is_dielectric<DIELECTRIC>(sf);
+	if (delta) {
+		float F;
+		if (dielectric_scatter(sf.v_local, sf.inside ? sf.diel.w : 1.0f / sf.diel.w, u0, &dl, &F)) est = f3{1.0f, 1.0f, 1.0f};
+		else { est = f3{sf.diel.x, sf.diel.y, sf.diel.z}; o = sf.P_in; }
+	}
+	else if (GGX) ggx_sample(sf.albedo, sf.alpha, sf.v_local, u0, u1, &dl, &est);  // Closure<GGX>::sample, DataStreams.hpp:199-218
 	else dl = cosine_hemisphere(u0, u1);
 	f3 thr{s->tr * est.x, s->tg * est.y, s->tb * est.z};
 	const float q = 1.0f - sel_max(thr.x, sel_max(thr.y, thr.z));
 	if (rng.next_unit() < q) return false;
 	thr = scale3(thr, 1.0f / sel_max(FLT_EPSILON, 1.0f - q));
 	const f3 dw = frame_to_world(sf.T, dl);
-	s->ox = sf.P.x; s->oy = sf.P.y; s->oz = sf.P.z; s->dx = dw.x; s->dy = dw.y; s->dz = dw.z;
+	s->ox = o.x; s->oy = o.y; s->oz = o.z; s->dx = dw.x; s->dy = dw.y; s->dz = dw.z;
 	s->tr = thr.x; s->tg = thr.y; s->tb = thr.z;
-	s->pdf = GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
+	s->pdf = delta ? -1.0f : GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
 	return true;
 }
 // miss shader with ambient sky, Renderer.hpp:411-420 + Sky::operator(), Primitives.hpp:35-46

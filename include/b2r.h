@@ -74,6 +74,13 @@ enum {
 	                                    * Closure<GGX>::pdf returns 0 as it does there. Not combinable with B2R_FLAG_REFERENCE_EXACT. */
 	B2R_FLAG_NO_SPECULATION = 1u << 7, /* b2r_accumulate(ctx, 1) traces exactly one sample (default: a caller that asks for one sample per frame gets
 	                                    * batches of 2, 4, ... 16 samples traced ahead while nothing changes; results are identical either way) */
+	B2R_FLAG_DIELECTRIC = 1u << 12,    /* renders the materials' transmission and IOR, which the reference carries but never reads: a material with
+	                                    * max(transmission) > 0 is a smooth dielectric of eta = 1 + IOR_minus_one (its albedo, F0, F80 and roughness are
+	                                    * ignored). Each hit reflects with the Fresnel reflectance or refracts (throughput *= transmission), makes no light
+	                                    * sample, and the emitter it reaches next gets MIS weight 1 (DESIGN.md §2). Other materials keep their closure; combines
+	                                    * with B2R_FLAG_GGX, not with B2R_FLAG_REFERENCE_EXACT. With the flag, b2r_upload_scene, b2r_refit_scene and
+	                                    * b2r_set_flags refuse (B2R_ERR_ARG) a non-finite transmission, and a dielectric with a transmission outside [0, 1]
+	                                    * or an eta that is not finite or is < 1. A checkpoint does not load across the flag (b2r_load_checkpoint: B2R_ERR_STATE). */
 };
 
 typedef struct b2r_config {
