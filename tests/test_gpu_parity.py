@@ -696,24 +696,34 @@ def test_frames_enqueued_back_to_back_equal_frames_waited_for(n, flags):
 def test_a_scene_upload_every_frame_does_not_wait_for_the_frame_in_flight():
     """The e2e pattern, stressed: a DIFFERENT scene is uploaded (or refitted) before every frame and nothing waits for the device. Scene writes
     go to the library's upload stream while the previous frame still traces from its side's own copy of the scene arrays; every frame must
-    still see exactly the scene uploaded before it."""
+    still see exactly the scene uploaded before it. Two of the writes outgrow every scene before them (the upload of sc_e: more spheres,
+    materials and lights; the refit to mat_f: more materials and lights), so the library's tables and the sides' copies are replaced while
+    the previous frame may still be tracing."""
     w, h, mb, K = 192, 128, 6, 2
     sc_a = scenes.random_scene(2500, light_every=40); rs = np.random.RandomState(11)
     sc_b = scenes.Scene(sc_a); sc_b["geometry"] = _moved_geometry(sc_a["geometry"], rs, jitter=0.4)
     sc_c = scenes.random_scene(1800, light_every=25, seed=0x1234567)           # another sphere count: other array sizes, other tree
     geo_d = _moved_geometry(sc_a["geometry"], rs, jitter=0.2)                  # reached by a refit of sc_a
-    plan = ["a", "b", "a", "c", "a", "refit_d", "b", "c"]
+    sc_e = scenes.random_scene(3200, light_every=20, seed=0x2468ace)           # 3200 spheres, 160 lights
+    extra = sc_e["material"][:4].copy(); extra["albedo"] *= 0.5
+    sc_e["material"] = np.concatenate([sc_e["material"], extra])               # 13 materials, the last four on every seventh non-emissive sphere
+    geo_e = sc_e["geometry"].copy(); pick = (np.arange(len(geo_e)) % 7 == 3) & (geo_e["material_ID"] < 8)
+    geo_e["material_ID"][pick] = 9 + geo_e["material_ID"][pick] % 4; sc_e["geometry"] = geo_e
+    geo_f = _moved_geometry(geo_e, rs, jitter=0.2)                             # reached by a refit of sc_e with mat_f:
+    mat_f = np.concatenate([sc_e["material"], extra[:3]]); mat_f["emission"][0] = 2.0   # 16 materials, material 0's spheres become lights too
+    plan = ["a", "b", "a", "c", "a", "refit_d", "b", "c", "e", "refit_f", "a"]
     def drive(r, wait):
         out = []
         for step in plan:
             if step == "refit_d": r.RefitScene(geo_d, want_quality=False)
-            else: r.SetScene(b2r.PreparedScene({"a": sc_a, "b": sc_b, "c": sc_c}[step], w, h))
+            elif step == "refit_f": r.RefitScene(geo_f, material=mat_f, want_quality=False)
+            else: r.SetScene(b2r.PreparedScene({"a": sc_a, "b": sc_b, "c": sc_c, "e": sc_e}[step], w, h))
             r.ResetAccumulator(); r.Accumulate(2 * K)
             if wait: assert r.Render(); out.append(r.buckets_host().copy())
             else: assert r.RenderDevice()
         return out
     a = b2r.Renderer(sc_a, w, h, max_bounces=mb, buckets=K); want = drive(a, True)
-    for upto in (len(plan), 5, 6):   # drain after the whole plan, and after prefixes that end on other sides / other kinds of write
+    for upto in (len(plan), 5, 6, 9, 10):   # drain after the whole plan, and after prefixes that end on other sides / other kinds of write
         b = b2r.Renderer(sc_a, w, h, max_bounces=mb, buckets=K)
         full = plan[:]; del plan[upto:]
         drive(b, False); b.sync()
