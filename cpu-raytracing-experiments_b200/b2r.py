@@ -353,12 +353,14 @@ class Renderer:
         r = np.ascontiguousarray(rays, np.float32); tf = np.ascontiguousarray(tfar, np.float32); n = len(r); o = np.empty(n, np.uint8)
         _check(lib().b2r_trace_shadow(self._h, _ptr(r), _ptr(tf), n, _ptr(o))); return o
 
-    def trace_kernel_closest(self, rays, tail=None):
+    def trace_kernel_closest(self, rays, tail=None, origin_prim=None):
         """k_intersect_closest, the per-lane closest-hit kernel of bounces >= 1, on caller rays (b2r_trace_kernel). tail (n bools, with
-        FLAG_REFERENCE_EXACT): rays that take the scalar-tail sphere formula. Returns (tfar, prim) as trace_closest."""
+        FLAG_REFERENCE_EXACT): rays that take the scalar-tail sphere formula. origin_prim (n ints, BVH order; -1 = the root; None = all
+        from the root): ray i's walk starts at the node holding that sphere and climbs. Returns (tfar, prim) as trace_closest."""
         r = np.ascontiguousarray(rays, np.float32); n = len(r); t = np.empty(n, np.float32); p = np.empty(n, np.int32)
         tl = None if tail is None else np.ascontiguousarray(tail, np.uint8)
-        _check(lib().b2r_trace_kernel(self._h, TAP_CLOSEST, _ptr(r), None, None, _ptr(tl), n, 0, _ptr(t), _ptr(p), None)); return t, p
+        op = None if origin_prim is None else np.ascontiguousarray(origin_prim, np.int32)
+        _check(lib().b2r_trace_kernel(self._h, TAP_CLOSEST, _ptr(r), None, _ptr(op), _ptr(tl), n, 0, _ptr(t), _ptr(p), None)); return t, p
 
     def trace_kernel_shadow(self, rays, tfar, origin_prim):
         """k_intersect_shadow, the climbing any-hit kernel, on caller rays: ray i's walk starts at the node holding sphere origin_prim[i]

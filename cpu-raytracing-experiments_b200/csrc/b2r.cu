@@ -126,6 +126,7 @@ struct b2r_ctx {
 	// frame
 	float4 *d_A[2] = {nullptr, nullptr}, *d_B[2] = {nullptr, nullptr}, *d_SA = nullptr, *d_SB = nullptr, *d_fb = nullptr;
 	float *d_T[2] = {nullptr, nullptr}, *d_SL = nullptr, *d_rad = nullptr, *d_acc = nullptr;
+	uint32_t* d_N[2] = {nullptr, nullptr};  // start nodes of the paths' closest-hit walks (QueueDev::N)
 	uint8_t *d_ex_slot[2] = {nullptr, nullptr}, *d_ex_key = nullptr; uint16_t* d_ex_act[2] = {nullptr, nullptr}; uint32_t* d_ex_next = nullptr;  // B2R_FLAG_REFERENCE_EXACT
 	float2* d_H = nullptr; uint32_t* d_SS = nullptr;
 	uint32_t* d_counts = nullptr; size_t counts_bytes = 0;
@@ -218,6 +219,7 @@ int alloc_frame(b2r_ctx* c) {
 		if ((rc = dev_alloc(&c->d_A[s], cap))) return rc;
 		if ((rc = dev_alloc(&c->d_B[s], cap))) return rc;
 		if ((rc = dev_alloc(&c->d_T[s], 3 * cap))) return rc;
+		if ((rc = dev_alloc(&c->d_N[s], cap))) return rc;
 	}
 	if ((rc = dev_alloc(&c->d_H, cap))) return rc;
 	if ((rc = dev_alloc(&c->d_SA, cap))) return rc;
@@ -249,7 +251,7 @@ int alloc_frame(b2r_ctx* c) {
 		p.frame.finish_below = e ? static_cast<uint32_t>(std::strtoul(e, nullptr, 10)) : kFinishBelow;
 		p.frame.finish_first = f ? static_cast<uint32_t>(std::strtoul(f, nullptr, 10)) : 2u;
 	}
-	for (int s = 0; s < 2; s++) { p.q.A[s] = c->d_A[s]; p.q.B[s] = c->d_B[s]; p.q.T[s] = c->d_T[s]; }
+	for (int s = 0; s < 2; s++) { p.q.A[s] = c->d_A[s]; p.q.B[s] = c->d_B[s]; p.q.T[s] = c->d_T[s]; p.q.N[s] = c->d_N[s]; }
 	p.q.H = c->d_H; p.q.SA = c->d_SA; p.q.SB = c->d_SB; p.q.SL = c->d_SL; p.q.SS = c->d_SS; p.q.cap = static_cast<uint32_t>(cap);
 	p.cnt.paths = c->d_counts; p.cnt.shadow = c->d_counts + (mb + 1); p.cnt.work_a = c->d_counts + 2 * (mb + 1); p.cnt.work_b = c->d_counts + 3 * (mb + 1);
 	p.cnt.stats = c->d_stats;
@@ -409,7 +411,7 @@ Params lane_params(const b2r_ctx* c, uint32_t which, uint32_t lanes, uint32_t si
 	Params p = c->params;
 	const uint32_t cap_slots = batch_cap(c), ls = lane_slots_of(c, lanes), rel = which * ls, mine = rel >= cap_slots ? 0u : (cap_slots - rel < ls ? cap_slots - rel : ls);
 	const size_t npix = p.frame.npix, off = static_cast<size_t>(side * cap_slots + rel) * npix, cap = static_cast<size_t>(mine) * npix;
-	for (int s = 0; s < 2; s++) { p.q.A[s] += off; p.q.B[s] += off; p.q.T[s] += 3 * off; }
+	for (int s = 0; s < 2; s++) { p.q.A[s] += off; p.q.B[s] += off; p.q.T[s] += 3 * off; p.q.N[s] += off; }
 	p.q.H += off; p.q.SA += off; p.q.SB += off; p.q.SL += 3 * off; p.q.SS += off; p.q.cap = static_cast<uint32_t>(cap);
 	const uint32_t block = (c->cfg.max_bounces + 1u) * 4u, blk = side * kMaxLanes + which;
 	p.cnt.paths += blk * block; p.cnt.shadow += blk * block; p.cnt.work_a += blk * block; p.cnt.work_b += blk * block;
@@ -834,7 +836,7 @@ void b2r_destroy(b2r_ctx* c) {
 	free_tables(c->tables);
 	dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_tap); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep);
 	for (int k = 0; k < 2; k++) { dev_free(&c->d_mkey[k]); dev_free(&c->d_midx[k]); }
-	for (int s = 0; s < 2; s++) { dev_free(&c->d_A[s]); dev_free(&c->d_B[s]); dev_free(&c->d_T[s]); }
+	for (int s = 0; s < 2; s++) { dev_free(&c->d_A[s]); dev_free(&c->d_B[s]); dev_free(&c->d_T[s]); dev_free(&c->d_N[s]); }
 	dev_free(&c->d_H); dev_free(&c->d_SA); dev_free(&c->d_SB); dev_free(&c->d_SL); dev_free(&c->d_SS); dev_free(&c->d_rad); dev_free(&c->d_acc); dev_free(&c->d_fb);
 	for (int s = 0; s < 2; s++) { dev_free(&c->d_ex_slot[s]); dev_free(&c->d_ex_act[s]); }
 	dev_free(&c->d_ex_key); dev_free(&c->d_ex_next);
@@ -1624,13 +1626,14 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 	if (packet && !c->have_camera) return fail(B2R_ERR_STATE, "set_camera first");
 	if (packet && n != c->params.frame.npix) return fail(B2R_ERR_ARG, "packet kernel: n must be width * height");
 	const uint32_t n_prims = c->params.scene.n_prims;
-	if (shadow) for (uint32_t i = 0; i < n; i++) if (origin_prim[i] >= static_cast<int32_t>(n_prims)) return fail(B2R_ERR_ARG, "origin_prim out of range");
+	const bool starts = shadow || (closest && origin_prim);  // walks that start at the node holding their origin sphere (-1: the root)
+	if (starts) for (uint32_t i = 0; i < n; i++) if (origin_prim[i] >= static_cast<int32_t>(n_prims)) return fail(B2R_ERR_ARG, "origin_prim out of range");
 	if (n == 0) return B2R_OK;
 	int rc = ensure_device(c); if (rc) return rc;
 	if (!packet && (rc = cover_ray_origins(c, rays, n))) return rc;
 	cudaStream_t st = c->stream;
-	std::vector<uint32_t> leaf_node;  // where the shadow walks start, as k_shade takes it for a hit on that sphere
-	if (shadow) { leaf_node.resize(n_prims); CU(cudaMemcpyAsync(leaf_node.data(), c->tables.leaf_node.p, n_prims * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)); CU(sync_main(c)); }
+	std::vector<uint32_t> leaf_node;  // where the walks start, as k_shade takes it for a hit on that sphere
+	if (starts) { leaf_node.resize(n_prims); CU(cudaMemcpyAsync(leaf_node.data(), c->tables.leaf_node.p, n_prims * sizeof(uint32_t), cudaMemcpyDeviceToHost, st)); CU(sync_main(c)); }
 	c->main_reads_scene = true;  // (the kernels read the primary scene arrays on the caller's stream)
 	// one grow-only block: the queue planes, RAD, the B2R_FLAG_REFERENCE_EXACT tables, counters and batch descriptors of these launches
 	// (never the context's own: its RAD may hold samples traced ahead, its queues may belong to a side in flight)
@@ -1644,6 +1647,7 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 	uint8_t* base = c->d_tap;
 	Params p = c->params;
 	p.q.A[0] = p.q.A[1] = reinterpret_cast<float4*>(base + o_a); p.q.B[0] = p.q.B[1] = reinterpret_cast<float4*>(base + o_b); p.q.T[0] = p.q.T[1] = reinterpret_cast<float*>(base + o_t);
+	p.q.N[0] = p.q.N[1] = reinterpret_cast<uint32_t*>(base + o_ss);   // (a launch reads either the shadow walks' or the paths' start nodes)
 	p.q.H = reinterpret_cast<float2*>(base + o_h); p.q.SA = reinterpret_cast<float4*>(base + o_sa); p.q.SB = reinterpret_cast<float4*>(base + o_sb);
 	p.q.SL = reinterpret_cast<float*>(base + o_sl); p.q.SS = reinterpret_cast<uint32_t*>(base + o_ss); p.q.cap = cap;
 	p.rad = reinterpret_cast<float*>(base + o_rad);
@@ -1682,8 +1686,8 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 			float pid; const uint32_t pid_i = i; std::memcpy(&pid, &pid_i, sizeof pid);  // slot 0, pixel i
 			ha[i] = make_float4(r[0], r[1], r[2], r[3]);
 			hb[i] = make_float4(r[4], r[5], shadow ? tfar[first + i] : 0.0f, pid);
-			if (shadow) { const int32_t o = origin_prim[first + i]; hs[i] = o < 0 ? 0u : leaf_node[o]; }
-			else hslot[i] = tail && tail[first + i] ? 255u : 0u;
+			if (starts) { const int32_t o = origin_prim[first + i]; hs[i] = o < 0 ? 0u : leaf_node[o]; } else hs[i] = 0u;
+			if (!shadow) hslot[i] = tail && tail[first + i] ? 255u : 0u;
 		}
 		uint32_t counts[16] = {0};
 		if (shadow) counts[4] = m; else counts[1] = m;   // shadow rays of bounce 0 / paths entering bounce 1 (queue side 1)
@@ -1700,6 +1704,7 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 			for (uint32_t i = 0; i < m; i++) occluded_out[first + i] = hrad[i] == 0.0f ? 1u : 0u;
 		} else {
 			CU(cudaMemcpyAsync(p.ex.slot[1], hslot.data(), m, cudaMemcpyHostToDevice, st));
+			CU(cudaMemcpyAsync(p.q.N[1], hs.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
 			k.closest<<<c->grid_closest, kTravBlock, 0, st>>>(p, 1u);
 			CU(cudaGetLastError()); c->launches++;
 			CU(cudaMemcpyAsync(h.data(), p.q.H, m * sizeof(float2), cudaMemcpyDeviceToHost, st));

@@ -5,6 +5,7 @@
 //       A[i] = {o.x, o.y, o.z, d.x}   B[i] = {d.y, d.z, pdf, as_float(pid)}   T[c*cap + i] = throughput channel c
 //     = 44 B per path (RayStream<>::Buffer, DataStreams.hpp:75-88, minus radiance). pid = slot << 26 | t with t the
 //     pixel's tile-order index (tile*256 + ID) and slot the sample-in-flight index inside the batch.
+//     BVH pipeline: + N[i] = the wide node the path's closest-hit walk starts at (4 B, written by k_shade).
 //   radiance RAD[(slot*3 + c)*npix + t]: a path's running radiance lives at its pixel (one path per pixel per sample)
 //     and is touched only when a contribution arrives (unoccluded light sample, emissive hit, sky).
 //   hit queue H[i] = {tfar, as_float(prim)} and shadow queue SA/SB/SL (ray, light-sample radiance): BVH pipeline only.
@@ -761,13 +762,19 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_packet(const Params p,
 	if (COUNT) { stat_add(p.cnt.stats, ST_SPHERE, c_sphere); stat_add(p.cnt.stats, ST_BOX, c_box); }
 }
 
-// closest-hit traversal of queue side (bounce & 1)
+// closest-hit traversal of queue side (bounce & 1). After bounce 0 every path leaves the surface of a sphere, and its walk starts at the
+// node holding that sphere (q.N, written by k_shade) and climbs (TravClosestT); camera rays (bounce 0 without the packet kernel) start at
+// the root. The walk is exact from any node of the tree it walks, so what a start node must be is an index into that tree: k_shade wrote it
+// from the leaf_node table of the same table set, in the same batch — a batch's launches all read one set (the side's own copy, refreshed
+// on the side's stream only between its batches, or the primary arrays, which a scene write reaches only in stream order behind the
+// batch), and no path outlives its batch.
 // (63 registers without a minimum-blocks bound = 8 resident CTAs. Measured: bounding it to 8 costs 4 %; 71/79/96 registers with
 // 7/6/5 CTAs cost 3/5/16 %; 56/48 registers with 9/10 CTAs and a shorter shared-memory stack cost 5/8 %.)
 template <bool COUNT, bool EXACT, uint32_t TNB>
 __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p, const uint32_t bounce) {
 	const uint32_t n_in = p.cnt.paths[bounce];
 	const int side = bounce & 1;
+	const uint32_t* __restrict__ parent = p.scene.parent;
 	uint32_t c_sphere = 0, c_box = 0;
 	using Walk = TravClosestT<SmemStack>;
 	lane_walks<Walk>(p.scene.wide, p.cnt.work_a + bounce, n_in,
@@ -778,9 +785,9 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p
 				const uint32_t pid_i = __float_as_uint(b.w), stream = (pid_i >> 26) * (p.frame.npix >> 8) + ((pid_i & kPixMask) >> 8);
 				tail = static_cast<uint32_t>(p.ex.slot[side][idx]) >= (static_cast<uint32_t>(p.ex.act[side][stream]) & ~7u);
 			}
-			t.begin(Ray{a.x, a.y, a.z, a.w, b.x, b.y}, tail);
+			t.begin(Ray{a.x, a.y, a.z, a.w, b.x, b.y}, tail, bounce == 0u ? 0u : p.q.N[side][idx], parent);
 		},
-		[&](Walk& t, const float4* row) { return t.template step_staged<COUNT, TNB>(row, p.scene.stack_tn_bits, &c_sphere, &c_box); },
+		[&](Walk& t, const float4* row) { return t.template step_staged<COUNT, TNB>(row, p.scene.stack_tn_bits, parent, &c_sphere, &c_box); },
 		[&](const Walk& t, uint32_t idx) { p.q.H[idx] = make_float2(t.best, __int_as_float(t.prim)); });
 	if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(p.cnt.stats + ST_EXT, static_cast<unsigned long long>(n_in));
 	if (COUNT) { stat_add(p.cnt.stats, ST_SPHERE, c_sphere); stat_add(p.cnt.stats, ST_BOX, c_box); }
@@ -837,7 +844,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 		bool keep = false, want_shadow = false; ShadowRay sr; PathState s; uint32_t pid = 0, ex_slot = 0, ex_mat = 0, start = 0;
 		if (shade) {
 			const uint32_t hi = s_hit_i[qi]; const float depth = s_hit_t[qi]; const int32_t prim = s_hit_prim[qi];
-			start = __ldg(sc.leaf_node + prim);  // where this hit's shadow ray will start its walk (asked for early: nothing waits for it before the queue write)
+			start = __ldg(sc.leaf_node + prim);  // where this hit's shadow ray and continued path will start their walks (asked for early: nothing waits for it before the queue writes)
 			s = load_path(p.q, side, hi); pid = s.pid;
 			if (EXACT) ex_slot = bounce == 0u ? (pid & 255u) : static_cast<uint32_t>(p.ex.slot[side][hi]);  // bounce 0: slot = pixel ID
 			const uint32_t acc = p.batch->acc[s.pid >> 26], seed = pixel_seed(s.pid & kPixMask, p.frame.max_bounces);
@@ -880,6 +887,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 		}
 		if (keep) {
 			store_path(p.q, side ^ 1, s_base + rank, s);
+			p.q.N[side ^ 1][s_base + rank] = start;
 			if (EXACT) {  // (stream, slot) -> material and next-queue index, for k_stream_rank
 				const uint32_t e = (pid >> 26) * p.frame.npix + ((pid & kPixMask) & ~255u) + ex_slot;
 				p.ex.key[e] = static_cast<uint8_t>(ex_mat + 1u); p.ex.next_idx[e] = s_base + rank;

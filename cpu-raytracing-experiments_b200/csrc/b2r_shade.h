@@ -46,8 +46,8 @@ struct SceneDev {
 	const float4* light_sphere; // [n_lights] scene.geometry[light] {c.xyz, r^2}   (Renderer.hpp:261-262)
 	const float4* light_emit;   // [n_lights] {emission.rgb of its material, as_float(light_primID)}
 	const WideNode* wide;       // flattened BVH
-	const uint32_t* parent;     // [n_wide] the wide node that links to node i (the root's entry is 0)      } written by k_link_tables from the device tree itself;
-	const uint32_t* leaf_node;  // [n_prims] the wide node that holds sphere i (BVH order) in a leaf slot       } k_intersect_shadow starts its walks there
+	const uint32_t* parent;     // [n_wide] the wide node that links to node i (the root's entry is 0)      } written by k_link_tables from the device tree itself; the walks
+	const uint32_t* leaf_node;  // [n_prims] the wide node that holds sphere i (BVH order) in a leaf slot       } of k_intersect_shadow and k_intersect_closest start there
 	const float4* hdri;         // equirect RGBA32F or null
 	uint32_t n_prims, n_mat, n_lights;
 	uint32_t stack_tn_bits;     // traversal stack entry split (WideBvh::tn_bits)
@@ -83,6 +83,7 @@ struct BatchDev {  // one wavefront batch: n_slots samples traced together
 };
 struct QueueDev {
 	float4* A[2]; float4* B[2]; float* T[2];
+	uint32_t* N[2];          // [cap] the wide node a path's closest-hit walk starts at (the node holding the sphere it leaves from; written by k_shade, not read at bounce 0)
 	float2* H;
 	float4* SA; float4* SB; float* SL;
 	uint32_t* SS;            // [cap] the wide node a shadow ray's walk starts at (the node holding the sphere it leaves from)
@@ -377,15 +378,33 @@ B2R_HD uint32_t pack_entry(uint32_t node, uint32_t tnear_bits, uint32_t tn_bits)
 B2R_HD float entry_tnear(uint32_t e, uint32_t tn_bits) { return from_bits((e & ((1u << tn_bits) - 1u)) << (31u - tn_bits)); }
 B2R_HD uint32_t entry_node(uint32_t e, uint32_t tn_bits) { return e >> tn_bits; }
 
+// Both per-lane walks can start at the BOTTOM of the tree and climb: a ray that leaves a point on a sphere starts at the wide node that
+// holds that sphere's leaf slot (scene.leaf_node), searches that subtree, and once it has nothing left there moves up to the parent, searches
+// the parent's other children (the child it came from, `skip`, is not entered again), and so on up to the root. The parent index a climb needs
+// is fetched one climb ahead (`up`), so no step waits for it. A walk started at node 0 never climbs (`root != 0` guards it) and never reads
+// parent[]: it is the plain walk from the root. Which boxes a climbing walk tests differs from a root walk only in the ancestors of the start
+// node, whose own boxes it never tests: boxes are conservative and never decide a result, so a skipped box test can only lose culling, never a
+// sphere test the result depends on (each walk's comment says why its result is unchanged).
+constexpr uint32_t kNoNode = 0xffffffffu;
 struct TravBase {
 	float ox, oy, oz, dx, dy, dz;   // ray
 	float ix, iy, iz, nx, ny, nz;   // 1/d and -o/d
-	float ax, ay, az;               // |1/d|
+	float ax, ay, az;               // |1/d| (the per-lane walks pass fabsf(i) to slab() instead: FFMA takes |R| as a free operand modifier, so these are not live in a walk)
 	uint32_t node;
+	uint32_t root, up, skip;        // climbing walks: top of the subtree searched so far, its parent, and the child of `root` already searched
 	B2R_HD void arm(const Ray& r) {
 		ox = r.ox; oy = r.oy; oz = r.oz; dx = r.dx; dy = r.dy; dz = r.dz;
 		slab_setup(r.ox, r.oy, r.oz, r.dx, r.dy, r.dz, &ix, &iy, &iz, &nx, &ny, &nz, &ax, &ay, &az);
 		node = 0u;
+	}
+	B2R_HD void start_at(uint32_t start, const uint32_t* __restrict__ parent) {
+		node = root = start; up = start != 0u ? ldg_u32(parent + start) : 0u; skip = kNoNode;  // (the root's parent entry is 0)
+	}
+	// nothing is left below `root`: move up one level (node = the parent, to be visited next). False once the root has been searched.
+	B2R_HD bool climb(const uint32_t* __restrict__ parent) {
+		if (root == 0u) return false;
+		skip = root; root = up; node = up; up = ldg_u32(parent + up);
+		return true;
 	}
 };
 // node access: STAGED = the node's eight float4 were copied to shared memory by the warp (kernels); otherwise read-only LDG
@@ -403,23 +422,34 @@ B2R_HD int first_bit(uint32_t m) {
 // when its box is entered beyond the best distance. All four slots are slab-tested in one uniform pass; the leaf slots that passed
 // are sphere-tested right away from the staged row (they can only shorten `best`), then the inner slots that passed are ordered by
 // entry distance and re-checked against the possibly shorter `best` before they are pushed.
+// Secondary rays climb (TravBase): k_shade queues, with every path it continues, the node that holds the sphere the path leaves from, and
+// k_intersect_closest starts there; the walk climbs when its stack and backing store are empty. The result is still exact: the closest hit
+// is the lexicographic minimum of (d, id) over the sphere tests made, which does not depend on the order they are made in; a sphere that
+// holds the minimum lies inside every box on its path from the root (boxes are conservative) and entered no later than d <= best, so no
+// cull rejects it wherever the walk starts; and a climbing walk only tests fewer boxes (the start node's ancestors'), never fewer spheres
+// that could hold the minimum. A walk that climbs to the root has searched every subtree a root walk searches. Measured on C3's bounce-1
+// rays (tests/hostcheck hc_closest_climb_stats, DESIGN §4): the node visits stay (13.0 -> 12.8: every ancestor is still searched), the
+// pushes and pops of entries that the first nearby hit makes useless drop from 3.4 to 0.9 per ray.
 template <class Stack>
 struct TravClosestT : TravBase {
 	float best; int32_t prim;
 	bool tail = false;  // B2R_FLAG_REFERENCE_EXACT: this ray sits in the scalar tail of its tile's stream (BVH.hpp:270-286)
 	Stack stack;
-	B2R_HD void begin(const Ray& r, bool scalar_tail = false) { arm(r); best = FLT_MAX; prim = -1; tail = scalar_tail; stack.reset(); }
+	// start: the node the walk begins at and climbs from; a walk from the root (start = 0) never reads `parent`, which may then be null
+	B2R_HD void begin(const Ray& r, bool scalar_tail = false, uint32_t start = 0u, const uint32_t* __restrict__ parent = nullptr) {
+		arm(r); start_at(start, parent); best = FLT_MAX; prim = -1; tail = scalar_tail; stack.reset();
+	}
 	template <bool COUNT, bool STAGED, uint32_t TNB = 0u>  // TNB != 0: the stack-entry split is a compile-time constant (immediate shifts)
-	B2R_HD bool visit(const float4* n, uint32_t tn_bits_rt, uint32_t* c_sphere, uint32_t* c_box) {
+	B2R_HD bool visit(const float4* n, uint32_t tn_bits_rt, const uint32_t* __restrict__ parent, uint32_t* c_sphere, uint32_t* c_box) {
 		const uint32_t tn_bits = TNB ? TNB : tn_bits_rt;
 		uint32_t key[4], link[4]; uint32_t leaves = 0u;
 #pragma unroll
 		for (int k = 0; k < 4; k++) {
 			const float4 a = node_f4<STAGED>(n, 2 * k), b = node_f4<STAGED>(n, 2 * k + 1);
 			const int32_t l = as_int(b.z);
-			float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, ax, ay, az, best, &tn, &h);
+			float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, fabsf(ix), fabsf(iy), fabsf(iz), best, &tn, &h);
 			if (COUNT && l != kEmptyLink) (*c_box)++;
-			key[k] = (h && l >= 0) ? bits(tn) : 0xffffffffu; link[k] = static_cast<uint32_t>(l);
+			key[k] = (h && l >= 0 && static_cast<uint32_t>(l) != skip) ? bits(tn) : 0xffffffffu; link[k] = static_cast<uint32_t>(l);
 			leaves |= (h && l < 0) ? (1u << k) : 0u;  // an empty slot's box (h = -1e30) fails every constrained axis: never hit by a ray that keeps one (slab_setup)
 		}
 		while (leaves) {
@@ -449,35 +479,30 @@ struct TravClosestT : TravBase {
 				const uint32_t e = stack.pop();
 				if (entry_tnear(e, tn_bits) <= best) { node = entry_node(e, tn_bits); return true; }
 			}
-			if (!stack.refill()) return false;
+			if (!stack.refill()) return climb(parent);  // false: walked the whole tree
 		}
 	}
+	// (parent last and defaulted: a walk from the root never reads it)
 	template <bool COUNT>
-	B2R_HD bool step(const WideNode* __restrict__ wide, uint32_t tn_bits, uint32_t* c_sphere, uint32_t* c_box) { return visit<COUNT, false>(reinterpret_cast<const float4*>(wide + node), tn_bits, c_sphere, c_box); }
+	B2R_HD bool step(const WideNode* __restrict__ wide, uint32_t tn_bits, uint32_t* c_sphere, uint32_t* c_box, const uint32_t* __restrict__ parent = nullptr) { return visit<COUNT, false>(reinterpret_cast<const float4*>(wide + node), tn_bits, parent, c_sphere, c_box); }
 	template <bool COUNT, uint32_t TNB = 0u>
-	B2R_HD bool step_staged(const float4* n, uint32_t tn_bits, uint32_t* c_sphere, uint32_t* c_box) { return visit<COUNT, true, TNB>(n, tn_bits, c_sphere, c_box); }
+	B2R_HD bool step_staged(const float4* n, uint32_t tn_bits, const uint32_t* __restrict__ parent, uint32_t* c_sphere, uint32_t* c_box) { return visit<COUNT, true, TNB>(n, tn_bits, parent, c_sphere, c_box); }
 };
 // Any hit along [0, tfar) — Traverse_shadow semantics (BVH.hpp:290-305): an order-independent boolean. The nearest hit child is visited
 // next, the others are pushed (in a dense scene the occluder is usually close to the origin — C3: every shadow ray is occluded; 12.4 -> 10.2
 // node visits per ray); the first occluding leaf sphere ends the walk.
-// The walk can start at the BOTTOM of the tree and climb. A shadow ray leaves a point on a sphere, and in a dense scene its occluder is
-// usually a neighbour of that sphere: a walk from the root spends ~8 of its 12-13 node visits descending to the origin's neighbourhood
-// before it tests the first sphere. So k_intersect_shadow starts each ray at the wide node that holds its origin sphere's leaf slot (SS,
-// written by k_shade from scene.leaf_node); when that subtree holds no occluder the walk moves up to its parent, searches the parent's
-// other children (the child it came from is skipped), and so on up to the root. Any-hit is an order-independent boolean over the same
-// sphere tests, and a ray that reaches the root has visited exactly the nodes a root walk would have, so results are unchanged; measured
-// on C3's shadow rays (tests/hostcheck hc_anyhit_local_stats): 12.3 -> 6.5 node visits per ray for the shadow rays of camera-ray hits,
-// 13.1 -> 8.5 for those of later bounces. The parent index a climb needs is fetched one climb ahead (`up`), so no step waits for it.
-// A walk started at node 0 never climbs (`root != 0` guards the climb) and never reads parent[]: it is the plain walk from the root.
-constexpr uint32_t kNoNode = 0xffffffffu;
+// The walk climbs (TravBase). A shadow ray leaves a point on a sphere, and in a dense scene its occluder is usually a neighbour of that
+// sphere: a walk from the root spends ~8 of its 12-13 node visits descending to the origin's neighbourhood before it tests the first
+// sphere. So k_intersect_shadow starts each ray at the wide node that holds its origin sphere's leaf slot (SS, written by k_shade from
+// scene.leaf_node). Any-hit is an order-independent boolean over the same sphere tests, and a ray that reaches the root has visited
+// exactly the nodes a root walk would have, so results are unchanged; measured on C3's shadow rays (tests/hostcheck hc_anyhit_local_stats):
+// 12.3 -> 6.5 node visits per ray for the shadow rays of camera-ray hits, 13.1 -> 8.5 for those of later bounces.
 template <class Stack>
 struct TravAnyT : TravBase {
 	float tfar; bool occluded;
-	uint32_t root, up, skip;   // top of the subtree searched so far, its parent, and the child of `root` already searched
 	Stack stack;
 	B2R_HD void begin(const Ray& r, float limit, uint32_t start, const uint32_t* __restrict__ parent) {
-		arm(r); tfar = limit; occluded = false; stack.reset();
-		node = root = start; up = start != 0u ? ldg_u32(parent + start) : 0u; skip = kNoNode;  // (the root's parent entry is 0)
+		arm(r); start_at(start, parent); tfar = limit; occluded = false; stack.reset();
 	}
 	template <bool COUNT, bool STAGED>
 	B2R_HD bool visit(const float4* n, const uint32_t* __restrict__ parent, uint32_t* c_sphere, uint32_t* c_box) {
@@ -487,7 +512,7 @@ struct TravAnyT : TravBase {
 		for (int k = 0; k < 4; k++) {
 			const float4 a = node_f4<STAGED>(n, 2 * k), b = node_f4<STAGED>(n, 2 * k + 1);
 			const int32_t l = as_int(b.z);
-			float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, ax, ay, az, tfar, &tn, &h);
+			float tn; bool h; slab(a, b, ix, iy, iz, nx, ny, nz, fabsf(ix), fabsf(iy), fabsf(iz), tfar, &tn, &h);
 			if (COUNT && l != kEmptyLink) (*c_box)++;
 			if (h && l >= 0 && static_cast<uint32_t>(l) != skip) {
 				const bool nearer = tn < next_tn;
@@ -505,9 +530,8 @@ struct TravAnyT : TravBase {
 			if (sphere_hit_any(sp.x, sp.y, sp.z, sp.w, ox, oy, oz, dx, dy, dz, tfar)) { occluded = true; return false; }
 		}
 		if (next == kNoNode && (!stack.empty() || stack.refill())) next = stack.pop();
-		if (next == kNoNode && root != 0u) { skip = root; root = up; next = up; up = ldg_u32(parent + up); }  // nothing below `root`: climb
-		node = next;
-		return next != kNoNode;  // false: walked the whole tree without an occluder
+		if (next != kNoNode) { node = next; return true; }
+		return climb(parent);  // false: walked the whole tree without an occluder
 	}
 	template <bool COUNT>
 	B2R_HD bool step(const WideNode* __restrict__ wide, const uint32_t* __restrict__ parent, uint32_t* c_sphere, uint32_t* c_box) { return visit<COUNT, false>(reinterpret_cast<const float4*>(wide + node), parent, c_sphere, c_box); }
@@ -516,14 +540,15 @@ struct TravAnyT : TravBase {
 };
 using TravClosest = TravClosestT<ArrayStack>;
 using TravAny = TravAnyT<ArrayStack>;
-// whole-ray wrappers (trace taps, host check)
+// whole-ray wrappers (trace taps, host check). start: the node the walk begins at and climbs from; a walk from the root (start = 0) never
+// reads `parent`, which may then be null
 template <bool COUNT>
-B2R_HD void traverse_closest(const WideNode* __restrict__ wide, uint32_t tn_bits, const Ray& r, float* best_out, int32_t* prim_out, uint32_t* c_sphere, uint32_t* c_box) {
-	TravClosest t; t.begin(r);
-	while (t.template step<COUNT>(wide, tn_bits, c_sphere, c_box)) {}
+B2R_HD void traverse_closest(const WideNode* __restrict__ wide, uint32_t tn_bits, const Ray& r, float* best_out, int32_t* prim_out, uint32_t* c_sphere, uint32_t* c_box,
+                             const uint32_t* __restrict__ parent = nullptr, uint32_t start = 0u, bool scalar_tail = false) {
+	TravClosest t; t.begin(r, scalar_tail, start, parent);
+	while (t.template step<COUNT>(wide, tn_bits, c_sphere, c_box, parent)) {}
 	*best_out = t.best; *prim_out = t.prim;
 }
-// start: the node the walk begins at and climbs from; a walk from the root (start = 0) never reads `parent`, which may then be null
 template <bool COUNT>
 B2R_HD bool traverse_any(const WideNode* __restrict__ wide, const Ray& r, float tfar, uint32_t* c_sphere, uint32_t* c_box, const uint32_t* __restrict__ parent = nullptr, uint32_t start = 0u) {
 	TravAny t; t.begin(r, tfar, start, parent);

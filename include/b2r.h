@@ -270,6 +270,8 @@ int  b2r_trace_shadow(b2r_ctx* ctx, const float* rays_host, const float* tfar_ho
  * B2R_ERR_STATE before an upload or on a brute-force context; B2R_ERR_ARG for a null pointer the kernel needs or an unknown kernel.
  *  B2R_TAP_CLOSEST  k_intersect_closest: rays[n*6] -> tfar_out[n], prim_out[n] (as b2r_trace_closest). tail: NULL or n bytes; with
  *                   B2R_FLAG_REFERENCE_EXACT, nonzero = this ray takes the scalar-tail sphere formula (BVH.hpp:270-286).
+ *                   origin_prim: NULL (every walk starts at the root) or n entries, as for B2R_TAP_SHADOW: ray i's walk starts at the
+ *                   wide node holding sphere origin_prim[i], or at the root for -1, and climbs (B2R_ERR_ARG for an index >= the sphere count).
  *  B2R_TAP_SHADOW   k_intersect_shadow: rays, tfar[n] -> occluded_out[n]; ray i's walk starts at the wide node holding sphere
  *                   origin_prim[i] (BVH order), or at the root for -1, and climbs (B2R_ERR_ARG for an index >= the sphere count).
  *  B2R_TAP_PACKET   k_intersect_packet on the camera rays of sample index acc (rays unused): n == width*height (else B2R_ERR_ARG),
