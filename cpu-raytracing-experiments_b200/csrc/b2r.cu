@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 using namespace b2r;
@@ -95,6 +96,28 @@ void bind_tables(Params& p, const SceneTables& t, bool sky) {
 	p.mat_diel = t.mat_diel.p;
 }
 
+// One launch of a batch's rounds: the kernel instantiation, its block size and its grid (kernels_of).
+template <typename F> struct Role { F fn = nullptr; int block = 0, grid = 0; };
+using BounceKernel = void (*)(const Params, const uint32_t);
+struct KernelSet { Role<BounceKernel> brute_first, brute, brute_finish, packet, closest, shade, shadow; Role<void (*)(const Params)> generate; };
+// The bits of the key that selects a KernelSet (kernels_of).
+enum : uint32_t { KEY_COUNT = 1, KEY_EXACT = 2, KEY_GGX = 4, KEY_LENS = 8, KEY_DIEL = 16, KEY_TN16 = 32, KEYS = 64 };
+
+// A stream the batches are traced on (the caller's, or a side's) and what a batch's lanes add to it: lane j > 0 runs on lane_stream[j],
+// forked from the stream by ev_fork and joined back by ev_join[j]; one captured graph per lane count (index = lanes).
+struct Track {
+	cudaStream_t lane_stream[kMaxLanes] = {}; cudaEvent_t ev_fork = nullptr, ev_join[kMaxLanes] = {};
+	cudaGraphExec_t exec[kMaxLanes + 1] = {}; bool valid[kMaxLanes + 1] = {};
+	uint64_t launches[kMaxLanes + 1] = {};  // kernels one replay of each graph launches (counted while capturing)
+	void invalidate() { for (bool& v : valid) v = false; }
+	void drop_graphs() { for (cudaGraphExec_t& e : exec) if (e) { cudaGraphExecDestroy(e); e = nullptr; } invalidate(); }  // (nothing of them may still run)
+	void destroy() {
+		drop_graphs();
+		for (uint32_t j = 1; j < kMaxLanes; j++) if (lane_stream[j]) { cudaStreamDestroy(lane_stream[j]); cudaEventDestroy(ev_join[j]); }
+		if (ev_fork) cudaEventDestroy(ev_fork);
+	}
+};
+
 }  // namespace
 
 struct b2r_ctx {
@@ -134,33 +157,26 @@ struct b2r_ctx {
 	BatchDev* d_batch = nullptr;
 	Params params{};
 	// launch
-	int grid_brute_first_exact = 0, grid_brute_exact = 0;
-	int grid_brute_first_ggx = 0, grid_brute_ggx = 0, grid_brute_finish_ggx = 0, grid_shade_ggx = 0;
-	int grid_brute_first = 0, grid_brute = 0, grid_closest = 0, grid_shade = 0, grid_shadow = 0, grid_stream = 0, grid_packet = 0, grid_brute_finish = 0; bool packet_primary = true;
-	int grid_brute_first_lens = 0, grid_brute_first_ggx_lens = 0, grid_packet_lens = 0;  // thin-lens bounce-0 instantiations
-	int grid_diel_brute_first[2][2] = {{0, 0}, {0, 0}}, grid_diel_brute[2] = {0, 0}, grid_diel_finish[2] = {0, 0}, grid_diel_shade[2] = {0, 0};  // B2R_FLAG_DIELECTRIC, [ggx][lens]
-	cudaGraphExec_t graph_exec = nullptr; bool graph_valid = false;
+	KernelSet kernels[KEYS];  // the kernel set of every key this context has used, with its grids (kernels_of)
+	int grid_stream = 0; bool packet_primary = true;
 	// twin lanes: a batch of two or more samples is traced as two independent half batches on two streams (own queues, counters and batch
 	// descriptors) inside one graph, so that the drained end of every launch of one half is filled by the other half's kernels
-	cudaGraphExec_t lane_exec[kMaxLanes + 1] = {nullptr, nullptr, nullptr, nullptr, nullptr}; bool lane_valid[kMaxLanes + 1] = {false, false, false, false, false};  // index = lanes (2, 4)
+	Track main;  // the batches traced on the caller's stream (sides off)
 	bool idle = true;  // nothing of this context is running on the device (set by sync_main, cleared by run_batch)
 	uint32_t lanes_max = 2; bool lanes_forced = false;  // B2R_LANES given: no per-batch choice
-	cudaStream_t lane_stream[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr}; cudaEvent_t ev_fork = nullptr, ev_join[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr};
 	float lane_grid_frac = 1.0f;
-	uint64_t graph_launches = 0, lane_launches[kMaxLanes + 1] = {0, 0, 0, 0, 0};  // kernels one replay of each graph launches (counted while capturing)
 	// sides: consecutive batches alternate between two halves of the queue memory and are TRACED on two library-owned streams, so that the thin
 	// late bounces of one batch (and its fold and the frame's resolve) run under the first, fat bounces of the next; only k_accumulate stays on
 	// the caller's stream, behind an event, so buckets are still folded in sample order and everything the caller enqueues later (reset,
 	// resolve, a scene upload) is ordered behind all tracing enqueued so far
 	struct Side {
-		cudaStream_t stream = nullptr, lane_stream[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr};
-		cudaEvent_t ev_traced = nullptr, ev_folded = nullptr, ev_sync = nullptr, ev_fork = nullptr, ev_join[kMaxLanes] = {nullptr, nullptr, nullptr, nullptr};
+		cudaStream_t stream = nullptr; Track track;
+		cudaEvent_t ev_traced = nullptr, ev_folded = nullptr, ev_sync = nullptr;
 		bool folded_valid = false; uint64_t epoch = ~0ull;
 		// the side's own copy of the scene arrays (refreshed from the primary ones, device to device, on the side's stream when scene_version has
 		// moved on): tracing never reads the primary arrays, so a scene upload does not have to wait for the batch in flight
 		SceneTables tables;  // (allocated at the primary tables' capacities)
 		bool have_copy = false, refreshed_valid = false; uint64_t scene_version = ~0ull; cudaEvent_t ev_refreshed = nullptr;
-		cudaGraphExec_t exec[kMaxLanes + 1] = {nullptr, nullptr, nullptr, nullptr, nullptr}; bool valid[kMaxLanes + 1] = {false, false, false, false, false}; uint64_t launches[kMaxLanes + 1] = {0, 0, 0, 0, 0};
 	} side[2];
 	uint32_t sides = 2, next_side = 0, last_side = 0, spec_side = 0, counts_first = 0;  // counts_first: first counter block of the last batch
 	uint64_t scene_epoch = 0;  // bumped by what the side streams must not run ahead of on the caller's stream (counter resets)
@@ -198,13 +214,11 @@ void drop_speculation(b2r_ctx* c) { c->spec_count = 0; c->spec_used = 0; c->spec
 void drop_graph(b2r_ctx* c) {
 	drop_speculation(c);  // everything that invalidates the captured graph (camera, scene pointers, flags, frame size) invalidates them too
 	if (c->stream) sync_main(c);  // (a launch of a graph may still be running)
-	if (c->graph_exec) { cudaGraphExecDestroy(c->graph_exec); c->graph_exec = nullptr; }
-	for (uint32_t l = 0; l <= kMaxLanes; l++) { if (c->lane_exec[l]) { cudaGraphExecDestroy(c->lane_exec[l]); c->lane_exec[l] = nullptr; } c->lane_valid[l] = false; }
+	c->main.drop_graphs();
 	for (auto& S : c->side) {
 		if (S.stream) cudaStreamSynchronize(S.stream);
-		for (uint32_t l = 0; l <= kMaxLanes; l++) { if (S.exec[l]) { cudaGraphExecDestroy(S.exec[l]); S.exec[l] = nullptr; } S.valid[l] = false; }
+		S.track.drop_graphs();
 	}
-	c->graph_valid = false;
 }
 
 int alloc_frame(b2r_ctx* c) {
@@ -263,46 +277,6 @@ int alloc_frame(b2r_ctx* c) {
 	return B2R_OK;
 }
 
-int compute_grids(b2r_ctx* c) {
-	auto occ = [&](const void* fn, int block, int* out) -> int {
-		int n = 0; CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fn, block, 0));
-		*out = (n < 1 ? 1 : n) * c->sm_count; return B2R_OK;
-	};
-	int rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false>), kBruteBlock, &c->grid_brute_first))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<false, false, false>), kBruteBlock, &c->grid_brute))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, true>), kBruteBlock, &c->grid_brute_first_exact))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<false, false, true>), kBruteBlock, &c->grid_brute_exact))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_closest<false, false, 16u>), kTravBlock, &c->grid_closest))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_shade<false>), kBruteBlock, &c->grid_shade))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_shadow<false>), kTravBlock, &c->grid_shadow))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_packet<false, B2R_PACKET_RPL>), kTravBlock, &c->grid_packet))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_brute_finish<false>), kBruteBlock, &c->grid_brute_finish))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true>), kBruteBlock, &c->grid_brute_first_ggx))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, true>), kBruteBlock, &c->grid_brute_ggx))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_brute_finish<false, true>), kBruteBlock, &c->grid_brute_finish_ggx))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_shade<false, true>), kBruteBlock, &c->grid_shade_ggx))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, true>), kBruteBlock, &c->grid_brute_first_lens))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, true>), kBruteBlock, &c->grid_brute_first_ggx_lens))) return rc;
-	if ((rc = occ(reinterpret_cast<const void*>(&k_intersect_packet<false, B2R_PACKET_RPL_LENS, true>), kTravBlock, &c->grid_packet_lens))) return rc;
-	const void* diel_first[2][2] = {{reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, false, true, true>)},
-	                                {reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<true, false, false, true, true, true>)}};
-	const void* diel_brute[2] = {reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, false, false, true>), reinterpret_cast<const void*>(&k_bounce_brute<false, false, false, true, false, true>)};
-	const void* diel_finish[2] = {reinterpret_cast<const void*>(&k_brute_finish<false, false, true>), reinterpret_cast<const void*>(&k_brute_finish<false, true, true>)};
-	const void* diel_shade[2] = {reinterpret_cast<const void*>(&k_shade<false, false, true>), reinterpret_cast<const void*>(&k_shade<false, true, true>)};
-	for (int g = 0; g < 2; g++) {
-		for (int l = 0; l < 2; l++) if ((rc = occ(diel_first[g][l], kBruteBlock, &c->grid_diel_brute_first[g][l]))) return rc;
-		if ((rc = occ(diel_brute[g], kBruteBlock, &c->grid_diel_brute[g])) || (rc = occ(diel_finish[g], kBruteBlock, &c->grid_diel_finish[g])) || (rc = occ(diel_shade[g], kBruteBlock, &c->grid_diel_shade[g]))) return rc;
-	}
-	c->packet_primary = std::getenv("B2R_NO_PACKET") == nullptr;  // A/B switch for measurements: per-lane walks for the camera rays too
-	c->lanes_max = std::getenv("B2R_NO_TWIN") ? 1u : 2u;          // A/B switches for measurements: every batch as one lane / B2R_LANES = 1, 2 or 4
-	if (const char* e = std::getenv("B2R_SIDES")) { c->sides = std::atoi(e) == 1 ? 1u : 2u; }   // A/B switch: 1 = every batch on the caller's stream, one after the other
-	if (const char* e = std::getenv("B2R_LANES")) { const int v = std::atoi(e); if (v == 1 || v == 2 || v == 4) { c->lanes_max = static_cast<uint32_t>(v); c->lanes_forced = true; } }
-	if (const char* e = std::getenv("B2R_LANE_GRID")) { c->lane_grid_frac = static_cast<float>(std::atof(e)); if (!(c->lane_grid_frac > 0.0f && c->lane_grid_frac <= 1.0f)) c->lane_grid_frac = 1.0f; }
-	c->grid_stream = c->sm_count * 8;
-	return B2R_OK;
-}
-
 // One launch; in profiling mode bracketed by events.
 template <typename F> int launch(b2r_ctx* c, int kind, bool profile, F&& f) {
 	b2r_ctx::Timed t{kind, nullptr, nullptr};
@@ -314,85 +288,87 @@ template <typename F> int launch(b2r_ctx* c, int kind, bool profile, F&& f) {
 	return B2R_OK;
 }
 
-// The kernel variants a context's flags select (template instantiations of b2r_device.cuh), chosen once per enqueue instead of at every launch.
-using BounceKernel = void (*)(const Params, const uint32_t);
-struct KernelSet {
-	BounceKernel brute_first, brute, brute_finish, packet, closest, shade, shadow;
-	void (*generate)(const Params);
-	int g_brute_first, g_brute, g_brute_finish, g_packet, g_shade;
-};
-KernelSet pick_kernels(const b2r_ctx* c) {
-	const bool count = (c->cfg.flags & B2R_FLAG_COUNT_TESTS) != 0, exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0, ggx = (c->cfg.flags & B2R_FLAG_GGX) != 0;
-	const bool tn16 = c->params.scene.stack_tn_bits == 16u;  // stack entries split 16/16 (up to 65536 wide nodes: C3) get immediate shifts; other sizes read the split from the scene
-	const bool lens = c->lens.radius > 0.0f && !exact;  // (b2r_set_lens refuses a reference-exact context)
-	const bool diel = (c->cfg.flags & B2R_FLAG_DIELECTRIC) != 0;  // (never with exact: refused at b2r_create / b2r_set_flags)
-	KernelSet k{};
-	// brute-force pipeline: <FIRST, COUNT, EXACT, GGX> (the GGX closure's kernels are built without the sphere-test counters)
-	if (ggx)        { k.brute_first = k_bounce_brute<true, false, false, true>; k.brute = k_bounce_brute<false, false, false, true>; k.g_brute_first = c->grid_brute_first_ggx; k.g_brute = c->grid_brute_ggx; }
-	else if (exact) { k.brute_first = count ? k_bounce_brute<true, true, true> : k_bounce_brute<true, false, true>; k.brute = count ? k_bounce_brute<false, true, true> : k_bounce_brute<false, false, true>; k.g_brute_first = c->grid_brute_first_exact; k.g_brute = c->grid_brute_exact; }
-	else            { k.brute_first = count ? k_bounce_brute<true, true, false> : k_bounce_brute<true, false, false>; k.brute = count ? k_bounce_brute<false, true, false> : k_bounce_brute<false, false, false>; k.g_brute_first = c->grid_brute_first; k.g_brute = c->grid_brute; }
-	// thin lens: only bounce 0 changes (later bounces read their origins from the path records)
-	if (lens && ggx) { k.brute_first = k_bounce_brute<true, false, false, true, true>; k.g_brute_first = c->grid_brute_first_ggx_lens; }
-	else if (lens)   { k.brute_first = count ? k_bounce_brute<true, true, false, false, true> : k_bounce_brute<true, false, false, false, true>; k.g_brute_first = c->grid_brute_first_lens; }
-	k.brute_finish = ggx ? k_brute_finish<false, true> : count ? k_brute_finish<true> : k_brute_finish<false>;
-	k.g_brute_finish = ggx ? c->grid_brute_finish_ggx : c->grid_brute_finish;
-	// BVH pipeline
-	if (lens) { k.packet = count ? k_intersect_packet<true, B2R_PACKET_RPL_LENS, true> : k_intersect_packet<false, B2R_PACKET_RPL_LENS, true>; k.g_packet = c->grid_packet_lens; }
-	else      { k.packet = count ? k_intersect_packet<true, B2R_PACKET_RPL> : k_intersect_packet<false, B2R_PACKET_RPL>; k.g_packet = c->grid_packet; }
-	k.generate = lens ? k_generate<true> : k_generate<false>;
-	if (exact) k.closest = count ? (tn16 ? k_intersect_closest<true, true, 16u> : k_intersect_closest<true, true, 0u>) : (tn16 ? k_intersect_closest<false, true, 16u> : k_intersect_closest<false, true, 0u>);
-	else       k.closest = count ? (tn16 ? k_intersect_closest<true, false, 16u> : k_intersect_closest<true, false, 0u>) : (tn16 ? k_intersect_closest<false, false, 16u> : k_intersect_closest<false, false, 0u>);
-	k.shade = ggx ? k_shade<false, true> : exact ? k_shade<true> : k_shade<false>;
-	k.g_shade = ggx ? c->grid_shade_ggx : c->grid_shade;
-	// smooth dielectric: its own shading instantiations, built without the sphere-test counters like GGX's; the traversal kernels are shared
-	if (diel) {
-		const int g = ggx ? 1 : 0, l = lens ? 1 : 0;
-		if (ggx) {
-			k.brute_first = lens ? k_bounce_brute<true, false, false, true, true, true> : k_bounce_brute<true, false, false, true, false, true>;
-			k.brute = k_bounce_brute<false, false, false, true, false, true>; k.brute_finish = k_brute_finish<false, true, true>; k.shade = k_shade<false, true, true>;
-		} else {
-			k.brute_first = lens ? k_bounce_brute<true, false, false, false, true, true> : k_bounce_brute<true, false, false, false, false, true>;
-			k.brute = k_bounce_brute<false, false, false, false, false, true>; k.brute_finish = k_brute_finish<false, false, true>; k.shade = k_shade<false, false, true>;
-		}
-		k.g_brute_first = c->grid_diel_brute_first[g][l]; k.g_brute = c->grid_diel_brute[g]; k.g_brute_finish = c->grid_diel_finish[g]; k.g_shade = c->grid_diel_shade[g];
+// The kernel variant (template instantiation of b2r_device.cuh) of every role for one key. The sphere-test counters (COUNT) are built into
+// the traversal kernels always, and into the shading kernels only without GGX and without DIELECTRIC. A lens changes bounce 0 only (later
+// bounces read their origins from the path records). TN16: stack entries split 16/16 (up to 65536 wide nodes: C3) get immediate shifts;
+// other trees read the split from the scene.
+template <uint32_t KEY> KernelSet kernel_set() {
+	constexpr bool COUNT = KEY & KEY_COUNT, EXACT = KEY & KEY_EXACT, GGX = KEY & KEY_GGX, LENS = KEY & KEY_LENS, DIEL = KEY & KEY_DIEL, TN16 = KEY & KEY_TN16;
+	if constexpr (EXACT && (GGX || LENS || DIEL)) return {};  // refused by b2r_create, b2r_set_flags and b2r_set_lens: nothing instantiated
+	else {
+		constexpr bool SHADE_COUNT = COUNT && !GGX && !DIEL;
+		KernelSet k;
+		k.brute_first = {k_bounce_brute<true, SHADE_COUNT, EXACT, GGX, LENS, DIEL>, kBruteBlock};
+		k.brute = {k_bounce_brute<false, SHADE_COUNT, EXACT, GGX, false, DIEL>, kBruteBlock};
+		k.brute_finish = {k_brute_finish<SHADE_COUNT, GGX, DIEL>, kBruteBlock};
+		k.packet = {k_intersect_packet<COUNT, LENS ? B2R_PACKET_RPL_LENS : B2R_PACKET_RPL, LENS>, kTravBlock};
+		k.closest = {k_intersect_closest<COUNT, EXACT, TN16 ? 16u : 0u>, kTravBlock};
+		k.shade = {k_shade<EXACT, GGX, DIEL>, kBruteBlock};
+		k.shadow = {k_intersect_shadow<COUNT>, kTravBlock};
+		k.generate = {k_generate<LENS>, kBlock};
+		return k;
 	}
-	k.shadow = count ? k_intersect_shadow<true> : k_intersect_shadow<false>;
-	return k;
+}
+template <uint32_t... KEY> KernelSet kernel_set(uint32_t key, std::integer_sequence<uint32_t, KEY...>) {
+	static const KernelSet sets[] = {kernel_set<KEY>()...};
+	return sets[key];
+}
+// The kernel set of the context's flags, lens and tree. Every role's grid is SM count x the resident CTAs of its instantiation at its block
+// size, queried once per context and key: run_batch and b2r_trace_kernel look the set up before they enqueue (no query inside a capture).
+int kernels_of(b2r_ctx* c, const KernelSet** out) {
+	const uint32_t f = c->cfg.flags;
+	const bool exact = (f & B2R_FLAG_REFERENCE_EXACT) != 0;
+	const uint32_t key = ((f & B2R_FLAG_COUNT_TESTS) ? KEY_COUNT : 0u) | (exact ? KEY_EXACT : 0u) | ((f & B2R_FLAG_GGX) ? KEY_GGX : 0u) |
+	                     (c->lens.radius > 0.0f && !exact ? KEY_LENS : 0u) | ((f & B2R_FLAG_DIELECTRIC) ? KEY_DIEL : 0u) | (c->params.scene.stack_tn_bits == 16u ? KEY_TN16 : 0u);
+	KernelSet& k = c->kernels[key];
+	if (!k.shade.fn) {
+		KernelSet s = kernel_set(key, std::make_integer_sequence<uint32_t, KEYS>());
+		auto occ = [&](auto& r) -> int {
+			int n = 0; CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, reinterpret_cast<const void*>(r.fn), r.block, 0));
+			r.grid = (n < 1 ? 1 : n) * c->sm_count; return B2R_OK;
+		};
+		int rc;
+		if ((rc = occ(s.brute_first)) || (rc = occ(s.brute)) || (rc = occ(s.brute_finish)) || (rc = occ(s.packet)) || (rc = occ(s.closest)) || (rc = occ(s.shade)) ||
+		    (rc = occ(s.shadow)) || (rc = occ(s.generate))) return rc;
+		k = s;
+	}
+	*out = &k;
+	return B2R_OK;
 }
 
 // The max_bounces rounds of one batch — or of one lane's half of it — on stream st; p carries that batch's queues, counters and descriptor.
-int enqueue_rounds(b2r_ctx* c, const Params& p_in, cudaStream_t st, bool profile, float grid_frac = 1.0f, uint32_t lanes = 1) {
+int enqueue_rounds(b2r_ctx* c, const KernelSet& k, const Params& p_in, cudaStream_t st, bool profile, float grid_frac = 1.0f, uint32_t lanes = 1) {
 	// (measurement tap, B2R_LANE_GRID: the lanes of a twin batch may be given a fraction of the resident-CTA grid each, so that the two lanes'
 	// kernels sit on every SM side by side instead of taking turns)
 	auto G = [&](int g) { const int per_sm = g / c->sm_count; int k = static_cast<int>(per_sm * grid_frac + 0.5f); if (k < 1) k = 1; return k * c->sm_count; };
 	const bool exact = (c->cfg.flags & B2R_FLAG_REFERENCE_EXACT) != 0;
 	if (exact && c->params.scene.n_mat > 64) return fail(B2R_ERR_STATE, "B2R_FLAG_REFERENCE_EXACT: at most 64 materials (RendererPolicy::max_materialID, Renderer.hpp:23)");
-	const KernelSet k = pick_kernels(c);
 	const uint32_t mb = c->cfg.max_bounces;
 	Params p = p_in;
 	int rc;
-	auto run = [&](int kind, BounceKernel fn, int grid, int block, uint32_t b) { return launch(c, kind, profile, [&] { fn<<<grid, block, 0, st>>>(p, b); }); };
+	auto run = [&](int kind, const Role<BounceKernel>& r, int grid, uint32_t b) { return launch(c, kind, profile, [&] { r.fn<<<grid, r.block, 0, st>>>(p, b); }); };
+	const Role<BounceKernel> rank{k_stream_rank, 256, c->grid_stream};
 	if (!c->use_bvh) {
 		const bool finish = !exact && p.frame.finish_below != 0u && p.scene.n_prims <= static_cast<uint32_t>(kBruteTile);
 		if (!finish) p.frame.finish_below = 0u;  // the hand-over threshold only reaches the kernels when k_brute_finish is launched too
 		else if (lanes > 1u) p.frame.finish_below /= lanes;  // the threshold is a batch's; a lane sees 1 / lanes of its paths (C2, two lanes: 13.15 -> 12.80 ms per frame)
 		for (uint32_t b = 0; b < mb; b++) {
 			// k_brute_finish takes the remaining paths over once few enough are left (a no-op launch otherwise)
-			if (finish && b >= p.frame.finish_first && b + 1 < mb && (rc = run(KK_BRUTE, k.brute_finish, k.g_brute_finish, kBruteBlock, b))) return rc;
-			if ((rc = b == 0 ? run(KK_BRUTE, k.brute_first, k.g_brute_first, kBruteBlock, b) : run(KK_BRUTE, k.brute, k.g_brute, kBruteBlock, b))) return rc;
+			if (finish && b >= p.frame.finish_first && b + 1 < mb && (rc = run(KK_BRUTE, k.brute_finish, k.brute_finish.grid, b))) return rc;
+			if ((rc = b == 0 ? run(KK_BRUTE, k.brute_first, k.brute_first.grid, b) : run(KK_BRUTE, k.brute, k.brute.grid, b))) return rc;
 			// the reference's stream order for the next bounce (the ranking kernel's time is booked under the brute kind)
-			if (exact && b + 1 < mb && (rc = run(KK_BRUTE, k_stream_rank, c->grid_stream, 256, b))) return rc;
+			if (exact && b + 1 < mb && (rc = run(KK_BRUTE, rank, rank.grid, b))) return rc;
 		}
 		return B2R_OK;
 	}
-	if (!c->packet_primary && (rc = launch(c, KK_GENERATE, profile, [&] { k.generate<<<c->grid_stream, kBlock, 0, st>>>(p); }))) return rc;  // (the packet kernel generates the camera rays itself)
+	if (!c->packet_primary && (rc = launch(c, KK_GENERATE, profile, [&] { k.generate.fn<<<k.generate.grid, k.generate.block, 0, st>>>(p); }))) return rc;  // (the packet kernel generates the camera rays itself)
 	const bool mis = !(c->cfg.flags & B2R_FLAG_NO_MIS);
 	for (uint32_t b = 0; b < mb; b++) {
-		if (b == 0 && c->packet_primary) { if ((rc = run(KK_CLOSEST, k.packet, G(k.g_packet), kTravBlock, b))) return rc; }  // camera rays: one walk per warp
-		else if ((rc = run(KK_CLOSEST, k.closest, G(c->grid_closest), kTravBlock, b))) return rc;
-		if ((rc = run(KK_SHADE, k.shade, G(k.g_shade), kBruteBlock, b))) return rc;
-		if (exact && b + 1 < mb && (rc = run(KK_SHADE, k_stream_rank, c->grid_stream, 256, b))) return rc;
-		if (mis && b + 1 < mb && (rc = run(KK_SHADOW, k.shadow, G(c->grid_shadow), kTravBlock, b))) return rc;
+		if (b == 0 && c->packet_primary) { if ((rc = run(KK_CLOSEST, k.packet, G(k.packet.grid), b))) return rc; }  // camera rays: one walk per warp
+		else if ((rc = run(KK_CLOSEST, k.closest, G(k.closest.grid), b))) return rc;
+		if ((rc = run(KK_SHADE, k.shade, G(k.shade.grid), b))) return rc;
+		if (exact && b + 1 < mb && (rc = run(KK_SHADE, rank, rank.grid, b))) return rc;
+		if (mis && b + 1 < mb && (rc = run(KK_SHADOW, k.shadow, G(k.shadow.grid), b))) return rc;
 	}
 	return B2R_OK;
 }
@@ -427,34 +403,49 @@ Params side_params(const b2r_ctx* c, uint32_t side) {
 	p.rad += 3 * static_cast<size_t>(side * batch_cap(c)) * p.frame.npix;
 	return p;
 }
-// The tracing of one batch on a side's streams: counters reset, max_bounces rounds per lane (fork / join), no fold.
-int enqueue_trace(b2r_ctx* c, uint32_t sidx, uint32_t lanes) {
-	b2r_ctx::Side& S = c->side[sidx];
-	cudaStream_t st = S.stream;
-	CU(cudaMemsetAsync(c->d_counts + static_cast<size_t>(sidx) * kMaxLanes * (c->counts_bytes / sizeof(uint32_t)), 0, kMaxLanes * c->counts_bytes, st));
+// One batch (everything after k_set_batch) on track t, whose own stream st runs lane 0, in side `side`'s part of the queue memory (the
+// caller's stream: side 0's): the side's counter blocks reset, then max_bounces rounds per lane, forked from st and joined back before
+// anything that follows. fold: the batch's k_accumulate follows on st (which adds in sample order over all lanes).
+int enqueue_batch(b2r_ctx* c, const KernelSet& k, Track& t, cudaStream_t st, uint32_t side, uint32_t lanes, bool fold, bool profile) {
+	CU(cudaMemsetAsync(c->d_counts + static_cast<size_t>(side) * kMaxLanes * (c->counts_bytes / sizeof(uint32_t)), 0, kMaxLanes * c->counts_bytes, st));
 	int rc;
-	if (lanes <= 1u) { Params p = lane_params(c, 0, 1, sidx); p.batch = c->d_batch + sidx * (1u + kMaxLanes); return enqueue_rounds(c, p, st, false); }  // one lane: the whole-batch descriptor is the lane's
-	CU(cudaEventRecord(S.ev_fork, st));
-	for (uint32_t j = 1; j < lanes; j++) CU(cudaStreamWaitEvent(S.lane_stream[j], S.ev_fork, 0));
-	for (uint32_t j = 0; j < lanes; j++) if ((rc = enqueue_rounds(c, lane_params(c, j, lanes, sidx), j ? S.lane_stream[j] : st, false, c->lane_grid_frac, lanes))) return rc;
-	for (uint32_t j = 1; j < lanes; j++) { CU(cudaEventRecord(S.ev_join[j], S.lane_stream[j])); CU(cudaStreamWaitEvent(st, S.ev_join[j], 0)); }
-	return B2R_OK;
-}
-
-// Enqueue one wavefront batch (everything after k_set_batch): counters reset, max_bounces rounds, fold into buckets.
-int enqueue_batch(b2r_ctx* c, bool profile, uint32_t lanes) {
-	cudaStream_t st = c->stream;
-	CU(cudaMemsetAsync(c->d_counts, 0, kMaxLanes * c->counts_bytes, st));
-	int rc;
-	if (lanes <= 1u) { if ((rc = enqueue_rounds(c, c->params, st, profile))) return rc; }
-	else {
-		// fork: lane 0's rounds on the main stream, the others' on their own; join before the fold (which adds in sample order over all lanes)
-		CU(cudaEventRecord(c->ev_fork, st));
-		for (uint32_t j = 1; j < lanes; j++) CU(cudaStreamWaitEvent(c->lane_stream[j], c->ev_fork, 0));
-		for (uint32_t j = 0; j < lanes; j++) if ((rc = enqueue_rounds(c, lane_params(c, j, lanes), j ? c->lane_stream[j] : st, false, c->lane_grid_frac, lanes))) return rc;
-		for (uint32_t j = 1; j < lanes; j++) { CU(cudaEventRecord(c->ev_join[j], c->lane_stream[j])); CU(cudaStreamWaitEvent(st, c->ev_join[j], 0)); }
+	if (lanes <= 1u) {  // one lane: the whole-batch descriptor is the lane's
+		Params p = lane_params(c, 0, 1, side); p.batch = c->d_batch + side * (1u + kMaxLanes);
+		if ((rc = enqueue_rounds(c, k, p, st, profile))) return rc;
+	} else {
+		CU(cudaEventRecord(t.ev_fork, st));
+		for (uint32_t j = 1; j < lanes; j++) CU(cudaStreamWaitEvent(t.lane_stream[j], t.ev_fork, 0));
+		for (uint32_t j = 0; j < lanes; j++) if ((rc = enqueue_rounds(c, k, lane_params(c, j, lanes, side), j ? t.lane_stream[j] : st, false, c->lane_grid_frac, lanes))) return rc;
+		for (uint32_t j = 1; j < lanes; j++) { CU(cudaEventRecord(t.ev_join[j], t.lane_stream[j])); CU(cudaStreamWaitEvent(st, t.ev_join[j], 0)); }
 	}
+	if (!fold) return B2R_OK;
 	return launch(c, KK_ACCUMULATE, profile, [&] { k_accumulate<<<c->grid_stream, kBlock, 0, st>>>(c->params); });
+}
+// The same batch as a replay of track t's graph for this lane count, captured on first use. An invalidated graph is destroyed once st has
+// drained.
+int replay_batch(b2r_ctx* c, const KernelSet& k, Track& t, cudaStream_t st, uint32_t side, uint32_t lanes, bool fold) {
+	if (!t.valid[lanes]) {
+		if (t.exec[lanes]) { CU(st == c->stream ? sync_main(c) : cudaStreamSynchronize(st)); cudaGraphExecDestroy(t.exec[lanes]); t.exec[lanes] = nullptr; }
+		if (lanes > 1u && !t.ev_fork) CU(cudaEventCreateWithFlags(&t.ev_fork, cudaEventDisableTiming));
+		for (uint32_t j = 1; j < lanes; j++) if (!t.lane_stream[j]) {
+			CU(cudaStreamCreateWithFlags(&t.lane_stream[j], cudaStreamNonBlocking)); CU(cudaEventCreateWithFlags(&t.ev_join[j], cudaEventDisableTiming));
+		}
+		cudaGraph_t graph = nullptr;
+		const uint64_t before = c->launches;
+		CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+		int rc = enqueue_batch(c, k, t, st, side, lanes, fold, false);
+		cudaError_t e = cudaStreamEndCapture(st, &graph);
+		t.launches[lanes] = c->launches - before; c->launches = before;
+		if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
+		if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e));
+		e = cudaGraphInstantiate(&t.exec[lanes], graph, 0);
+		cudaGraphDestroy(graph);
+		if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e));
+		t.valid[lanes] = true;
+	}
+	CU(cudaGraphLaunch(t.exec[lanes], st));
+	c->launches += t.launches[lanes];
+	return B2R_OK;
 }
 
 int refresh_side_scene(b2r_ctx* c, uint32_t sidx);
@@ -486,14 +477,15 @@ int run_batch(b2r_ctx* c, BatchArgs& args) {
 		args.lanes = lanes; args.lane_slots = ls; args.n = span; args.fold = fold;
 	} else { args.lanes = 0; args.lane_slots = 0; if (args.n < 64u) args.fold &= (1ull << args.n) - 1ull; }
 	args.cam = c->params.frame.cam; args.lens = c->lens;  // the camera and lens travel with the batch descriptor: a camera move leaves the captured graph alone
+	const KernelSet* k = nullptr;
+	{ const int rc = kernels_of(c, &k); if (rc) return rc; }
 	if (use_sides(c)) {
 		const uint32_t sidx = c->next_side; c->next_side ^= 1u;
 		b2r_ctx::Side& S = c->side[sidx];
 		if (!S.stream) {
 			CU(cudaStreamCreateWithFlags(&S.stream, cudaStreamNonBlocking));
-			for (cudaEvent_t* e : {&S.ev_traced, &S.ev_folded, &S.ev_sync, &S.ev_fork}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+			for (cudaEvent_t* e : {&S.ev_traced, &S.ev_folded, &S.ev_sync}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
 		}
-		for (uint32_t j = 1; j < lanes; j++) if (!S.lane_stream[j]) { CU(cudaStreamCreateWithFlags(&S.lane_stream[j], cudaStreamNonBlocking)); CU(cudaEventCreateWithFlags(&S.ev_join[j], cudaEventDisableTiming)); }
 		// the side must not run ahead of scene copies / refits enqueued on the caller's stream since it last looked, nor overwrite its part of
 		// RAD before the previous batch it traced has been folded
 		if (S.epoch != c->scene_epoch) { CU(cudaEventRecord(S.ev_sync, c->stream)); CU(cudaStreamWaitEvent(S.stream, S.ev_sync, 0)); S.epoch = c->scene_epoch; }
@@ -501,61 +493,22 @@ int run_batch(b2r_ctx* c, BatchArgs& args) {
 		{ const int rc = refresh_side_scene(c, sidx); if (rc) return rc; }
 		k_set_batch<<<1, kMaxSlots, 0, S.stream>>>(c->d_batch + sidx * (1u + kMaxLanes), args);
 		CU(cudaGetLastError());
-		if (!S.valid[lanes]) {
-			if (S.exec[lanes]) { CU(cudaStreamSynchronize(S.stream)); cudaGraphExecDestroy(S.exec[lanes]); S.exec[lanes] = nullptr; }
-			cudaGraph_t graph = nullptr;
-			const uint64_t before = c->launches;
-			CU(cudaStreamBeginCapture(S.stream, cudaStreamCaptureModeThreadLocal));
-			int rc = enqueue_trace(c, sidx, lanes);
-			cudaError_t e = cudaStreamEndCapture(S.stream, &graph);
-			S.launches[lanes] = c->launches - before; c->launches = before;
-			if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-			if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e));
-			e = cudaGraphInstantiate(&S.exec[lanes], graph, 0);
-			cudaGraphDestroy(graph);
-			if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e));
-			S.valid[lanes] = true;
-		}
-		CU(cudaGraphLaunch(S.exec[lanes], S.stream));
+		{ const int rc = replay_batch(c, *k, S.track, S.stream, sidx, lanes, false); if (rc) return rc; }
 		CU(cudaEventRecord(S.ev_traced, S.stream));
 		// the fold stays on the caller's stream: buckets are added to in sample order, behind whatever the caller enqueued before (reset)
 		CU(cudaStreamWaitEvent(c->stream, S.ev_traced, 0));
 		k_accumulate<<<c->grid_stream, kBlock, 0, c->stream>>>(side_params(c, sidx));
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(S.ev_folded, c->stream)); S.folded_valid = true;
-		c->launches += S.launches[lanes] + 1u;
+		c->launches += 1u;
 		c->last_side = sidx; c->counts_first = sidx * kMaxLanes;
 		return B2R_OK;
 	}
 	c->counts_first = 0; c->main_reads_scene = true;  // (this batch traces from the primary scene arrays, on the caller's stream)
 	k_set_batch<<<1, kMaxSlots, 0, c->stream>>>(c->d_batch, args);
 	CU(cudaGetLastError());
-	if (no_graph) return enqueue_batch(c, true, 1);
-	cudaGraphExec_t& exec = lanes > 1u ? c->lane_exec[lanes] : c->graph_exec;
-	bool& valid = lanes > 1u ? c->lane_valid[lanes] : c->graph_valid;
-	uint64_t& per_replay = lanes > 1u ? c->lane_launches[lanes] : c->graph_launches;
-	if (!valid) {
-		if (exec) { CU(sync_main(c)); cudaGraphExecDestroy(exec); exec = nullptr; }
-		if (lanes > 1u && !c->ev_fork) CU(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-		for (uint32_t j = 1; j < lanes; j++) if (!c->lane_stream[j]) {
-			CU(cudaStreamCreateWithFlags(&c->lane_stream[j], cudaStreamNonBlocking)); CU(cudaEventCreateWithFlags(&c->ev_join[j], cudaEventDisableTiming));
-		}
-		cudaGraph_t graph = nullptr;
-		const uint64_t before = c->launches;
-		CU(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-		int rc = enqueue_batch(c, false, lanes);
-		cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
-		per_replay = c->launches - before; c->launches = before;
-		if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-		if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e));
-		e = cudaGraphInstantiate(&exec, graph, 0);
-		cudaGraphDestroy(graph);
-		if (e != cudaSuccess) return fail(B2R_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e));
-		valid = true;
-	}
-	CU(cudaGraphLaunch(exec, c->stream));
-	c->launches += per_replay;
-	return B2R_OK;
+	if (no_graph) return enqueue_batch(c, *k, c->main, c->stream, 0, 1, true, true);
+	return replay_batch(c, *k, c->main, c->stream, 0, lanes, true);
 }
 
 int collect_timings(b2r_ctx* c) {
@@ -584,7 +537,7 @@ void free_side_scenes(b2r_ctx* c) {
 	for (auto& S : c->side) {
 		free_tables(S.tables);
 		S.have_copy = false; S.scene_version = ~0ull;
-		for (uint32_t l = 0; l <= kMaxLanes; l++) S.valid[l] = false;  // the captured graphs hold the old addresses
+		S.track.invalidate();  // the captured graphs hold the old addresses
 	}
 }
 // Grow-only reserve of the primary tables for a scene write, len[] elements each (a length of 0 leaves its tables alone). A table that has
@@ -629,7 +582,7 @@ int refresh_side_scene(b2r_ctx* c, uint32_t sidx) {
 		if (rc) return rc;
 		if (!S.ev_refreshed) CU(cudaEventCreateWithFlags(&S.ev_refreshed, cudaEventDisableTiming));
 		S.have_copy = true;
-		for (uint32_t l = 0; l <= kMaxLanes; l++) S.valid[l] = false;
+		S.track.invalidate();
 	}
 	if (c->uploaded_valid) CU(cudaStreamWaitEvent(S.stream, c->ev_uploaded, 0));
 	const size_t len[LEN_COUNT] = {sc.n_prims, sc.n_mat, sc.n_lights ? sc.n_lights : 1u, c->n_wide, sc.hdri ? c->hdri_texels : 0u};
@@ -815,10 +768,14 @@ int b2r_create(b2r_ctx** out, const b2r_config* cfg) {
 	b2r_ctx* c = new b2r_ctx();
 	c->cfg = *cfg;
 	c->slots = cfg->samples_in_flight;  // 0 = chosen from the image size in alloc_frame
+	c->packet_primary = std::getenv("B2R_NO_PACKET") == nullptr;  // A/B switch for measurements: per-lane walks for the camera rays too
+	c->lanes_max = std::getenv("B2R_NO_TWIN") ? 1u : 2u;          // A/B switches for measurements: every batch as one lane / B2R_LANES = 1, 2 or 4
+	if (const char* v = std::getenv("B2R_SIDES")) { c->sides = std::atoi(v) == 1 ? 1u : 2u; }   // A/B switch: 1 = every batch on the caller's stream, one after the other
+	if (const char* v = std::getenv("B2R_LANES")) { const int n = std::atoi(v); if (n == 1 || n == 2 || n == 4) { c->lanes_max = static_cast<uint32_t>(n); c->lanes_forced = true; } }
+	if (const char* v = std::getenv("B2R_LANE_GRID")) { c->lane_grid_frac = static_cast<float>(std::atof(v)); if (!(c->lane_grid_frac > 0.0f && c->lane_grid_frac <= 1.0f)) c->lane_grid_frac = 1.0f; }
 	int rc = ensure_device(c);
-	if (!rc) { cudaDeviceProp prop; e = cudaGetDeviceProperties(&prop, cfg->device); if (e != cudaSuccess) rc = fail(B2R_ERR_CUDA, cudaGetErrorString(e)); else c->sm_count = prop.multiProcessorCount; }
+	if (!rc) { cudaDeviceProp prop; e = cudaGetDeviceProperties(&prop, cfg->device); if (e != cudaSuccess) rc = fail(B2R_ERR_CUDA, cudaGetErrorString(e)); else { c->sm_count = prop.multiProcessorCount; c->grid_stream = c->sm_count * 8; } }
 	if (!rc) { e = cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking); if (e != cudaSuccess) rc = fail(B2R_ERR_CUDA, cudaGetErrorString(e)); c->stream = c->own_stream; }
-	if (!rc) rc = compute_grids(c);
 	if (!rc) rc = alloc_frame(c);
 	if (rc) { b2r_destroy(c); return rc; }
 	*out = c;
@@ -849,11 +806,10 @@ void b2r_destroy(b2r_ctx* c) {
 	if (c->ev_uploaded) cudaEventDestroy(c->ev_uploaded);
 	for (auto& S : c->side) {
 		if (S.ev_refreshed) cudaEventDestroy(S.ev_refreshed);
-		for (uint32_t j = 1; j < kMaxLanes; j++) if (S.lane_stream[j]) { cudaStreamDestroy(S.lane_stream[j]); cudaEventDestroy(S.ev_join[j]); }
-		if (S.stream) { cudaStreamDestroy(S.stream); cudaEventDestroy(S.ev_traced); cudaEventDestroy(S.ev_folded); cudaEventDestroy(S.ev_sync); cudaEventDestroy(S.ev_fork); }
+		S.track.destroy();
+		if (S.stream) { cudaStreamDestroy(S.stream); cudaEventDestroy(S.ev_traced); cudaEventDestroy(S.ev_folded); cudaEventDestroy(S.ev_sync); }
 	}
-	for (uint32_t j = 1; j < kMaxLanes; j++) if (c->lane_stream[j]) { cudaStreamDestroy(c->lane_stream[j]); cudaEventDestroy(c->ev_join[j]); }
-	if (c->ev_fork) cudaEventDestroy(c->ev_fork);
+	c->main.destroy();
 	if (c->own_stream) cudaStreamDestroy(c->own_stream);
 	delete c;
 }
@@ -1656,13 +1612,14 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 	p.cnt.paths = cnt; p.cnt.shadow = cnt + 4; p.cnt.work_a = cnt + 8; p.cnt.work_b = cnt + 12;
 	p.cnt.stats = reinterpret_cast<unsigned long long*>(base + o_stats);
 	BatchDev* batch = reinterpret_cast<BatchDev*>(base + o_batch); p.batch = batch;
-	const KernelSet k = pick_kernels(c);
+	const KernelSet* k = nullptr;
+	if ((rc = kernels_of(c, &k))) return rc;
 	std::vector<float2> h(chunk);
 	if (packet) {  // one sample of the context's own frame, camera and sample index acc
 		BatchArgs a; a.n = 1u; a.acc[0] = acc; a.cam = c->params.frame.cam; a.lens = c->lens;
 		k_set_batch<<<1, kMaxSlots, 0, st>>>(batch, a);
 		CU(cudaMemsetAsync(cnt, 0, 16u * sizeof(uint32_t), st));
-		k.packet<<<k.g_packet, kTravBlock, 0, st>>>(p, 0u);
+		k->packet.fn<<<k->packet.grid, k->packet.block, 0, st>>>(p, 0u);
 		CU(cudaGetLastError()); c->launches += 2;
 		CU(cudaMemcpyAsync(h.data(), p.q.H, n * sizeof(float2), cudaMemcpyDeviceToHost, st));
 		CU(sync_main(c));
@@ -1697,7 +1654,7 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 		if (shadow) {
 			CU(cudaMemcpyAsync(p.q.SS, hs.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
 			CU(cudaMemsetAsync(p.rad, 0, 3u * static_cast<size_t>(cap) * sizeof(float), st));
-			k.shadow<<<c->grid_shadow, kTravBlock, 0, st>>>(p, 0u);
+			k->shadow.fn<<<k->shadow.grid, k->shadow.block, 0, st>>>(p, 0u);
 			CU(cudaGetLastError()); c->launches++;
 			CU(cudaMemcpyAsync(hrad.data(), p.rad, m * sizeof(float), cudaMemcpyDeviceToHost, st));   // a lit ray adds its L = 1 to RAD
 			CU(sync_main(c));
@@ -1705,7 +1662,7 @@ int b2r_trace_kernel(b2r_ctx* c, int kernel, const float* rays, const float* tfa
 		} else {
 			CU(cudaMemcpyAsync(p.ex.slot[1], hslot.data(), m, cudaMemcpyHostToDevice, st));
 			CU(cudaMemcpyAsync(p.q.N[1], hs.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-			k.closest<<<c->grid_closest, kTravBlock, 0, st>>>(p, 1u);
+			k->closest.fn<<<k->closest.grid, k->closest.block, 0, st>>>(p, 1u);
 			CU(cudaGetLastError()); c->launches++;
 			CU(cudaMemcpyAsync(h.data(), p.q.H, m * sizeof(float2), cudaMemcpyDeviceToHost, st));
 			CU(sync_main(c));
