@@ -70,8 +70,10 @@ template <typename T> void dev_free(T** p) { if (*p) { cudaFree(*p); *p = nullpt
 // (reserve, free, the side copies, binding into Params) walks this list, so a new table is added here and where it is filled and read.
 #define B2R_PACKED_TABLES(X) X(float4, prims, LEN_PRIMS) X(int32_t, prim_mat, LEN_PRIMS) X(float4, mat_albedo, LEN_MAT) X(float4, mat_emission, LEN_MAT) \
                              X(float4, mat_f0, LEN_MAT) X(float4, mat_diel, LEN_MAT) X(float4, light_sphere, LEN_LIGHTS) X(float4, light_emit, LEN_LIGHTS)
-#define B2R_SCENE_TABLES(X) B2R_PACKED_TABLES(X) X(WideNode, wide, LEN_WIDE) X(uint32_t, parent, LEN_WIDE) X(uint32_t, leaf_node, LEN_PRIMS) X(float4, hdri, LEN_TEXELS)
-enum TableLen { LEN_PRIMS = 0, LEN_MAT, LEN_LIGHTS, LEN_WIDE, LEN_TEXELS, LEN_COUNT };  // 0 lights: one (zero) light row
+#define B2R_SCENE_TABLES(X) B2R_PACKED_TABLES(X) X(WideNode, wide, LEN_WIDE) X(uint32_t, parent, LEN_WIDE) X(uint32_t, leaf_node, LEN_PRIMS) X(float4, hdri, LEN_TEXELS) \
+                            X(float, sky_marg, LEN_SKY_MARG) X(float, sky_cond, LEN_SKY_COND) X(float, sky_pdf, LEN_SKY_PDF)
+// 0 lights: one (zero) light row. LEN_SKY_*: the sky's tables (B2R_FLAG_SKY_LIGHT), 0 while they are not built
+enum TableLen { LEN_PRIMS = 0, LEN_MAT, LEN_LIGHTS, LEN_WIDE, LEN_TEXELS, LEN_SKY_MARG, LEN_SKY_COND, LEN_SKY_PDF, LEN_COUNT };
 struct SceneTables {
 	template <typename T> struct Table { T* p = nullptr; size_t cap = 0; };
 #define X(T, name, len) Table<T> name;
@@ -94,6 +96,7 @@ void bind_tables(Params& p, const SceneTables& t, bool sky) {
 	s.light_sphere = t.light_sphere.p; s.light_emit = t.light_emit.p; s.wide = t.wide.p; s.parent = t.parent.p; s.leaf_node = t.leaf_node.p;
 	s.hdri = sky ? t.hdri.p : nullptr;
 	p.mat_diel = t.mat_diel.p;
+	p.sky.marg = t.sky_marg.p; p.sky.cond = t.sky_cond.p; p.sky.pdf = t.sky_pdf.p;
 }
 
 // One launch of a batch's rounds: the kernel instantiation, its block size and its grid (kernels_of).
@@ -101,7 +104,7 @@ template <typename F> struct Role { F fn = nullptr; int block = 0, grid = 0; };
 using BounceKernel = void (*)(const Params, const uint32_t);
 struct KernelSet { Role<BounceKernel> brute_first, brute, brute_finish, packet, closest, shade, shadow; Role<void (*)(const Params)> generate; };
 // The bits of the key that selects a KernelSet (kernels_of).
-enum : uint32_t { KEY_COUNT = 1, KEY_EXACT = 2, KEY_GGX = 4, KEY_LENS = 8, KEY_DIEL = 16, KEY_TN16 = 32, KEYS = 64 };
+enum : uint32_t { KEY_COUNT = 1, KEY_EXACT = 2, KEY_GGX = 4, KEY_LENS = 8, KEY_DIEL = 16, KEY_TN16 = 32, KEY_SKY = 64, KEYS = 128 };
 
 // A stream the batches are traced on (the caller's, or a side's) and what a batch's lanes add to it: lane j > 0 runs on lane_stream[j],
 // forked from the stream by ev_fork and joined back by ev_join[j]; one captured graph per lane count (index = lanes).
@@ -133,6 +136,9 @@ struct b2r_ctx {
 	// scene
 	SceneTables tables;  // the primary tables, written by the scene writes (grow-only: reserve_tables)
 	bool scene_diel_valid = true;  // the current scene's materials pass dielectric_materials_valid (checked when B2R_FLAG_DIELECTRIC is turned on)
+	// B2R_FLAG_SKY_LIGHT: whether the current sky's texels were checked (sky_texels_valid: only under the flag, or when it is turned on), passed,
+	// and are not zero everywhere; whether the sky's tables in `tables` are built for the current sky; the build's scratch
+	bool sky_checked = false, sky_valid = true, sky_nonzero = false, sky_built = false; double* d_sky_tmp = nullptr; size_t cap_sky_tmp = 0;
 	WideBvh wide_host; uint64_t wide_key = 0; std::vector<unsigned char> wide_blob; bool have_wide = false;
 	uint32_t n_wide = 0;  // wide nodes of the current tree
 	// B2R_FLAG_GPU_TREE: the tree was built on the device (no host copy of its nodes); sort scratch; the arrays a later refit needs to match
@@ -293,17 +299,18 @@ template <typename F> int launch(b2r_ctx* c, int kind, bool profile, F&& f) {
 // bounces read their origins from the path records). TN16: stack entries split 16/16 (up to 65536 wide nodes: C3) get immediate shifts;
 // other trees read the split from the scene.
 template <uint32_t KEY> KernelSet kernel_set() {
-	constexpr bool COUNT = KEY & KEY_COUNT, EXACT = KEY & KEY_EXACT, GGX = KEY & KEY_GGX, LENS = KEY & KEY_LENS, DIEL = KEY & KEY_DIEL, TN16 = KEY & KEY_TN16;
-	if constexpr (EXACT && (GGX || LENS || DIEL)) return {};  // refused by b2r_create, b2r_set_flags and b2r_set_lens: nothing instantiated
+	constexpr bool COUNT = KEY & KEY_COUNT, EXACT = KEY & KEY_EXACT, GGX = KEY & KEY_GGX, LENS = KEY & KEY_LENS, DIEL = KEY & KEY_DIEL, TN16 = KEY & KEY_TN16,
+	               SKY = KEY & KEY_SKY;
+	if constexpr ((EXACT && (GGX || LENS || DIEL)) || (SKY && (EXACT || GGX))) return {};  // refused by b2r_create, b2r_set_flags and b2r_set_lens: nothing instantiated
 	else {
-		constexpr bool SHADE_COUNT = COUNT && !GGX && !DIEL;
+		constexpr bool SHADE_COUNT = COUNT && !GGX && !DIEL && !SKY;
 		KernelSet k;
-		k.brute_first = {k_bounce_brute<true, SHADE_COUNT, EXACT, GGX, LENS, DIEL>, kBruteBlock};
-		k.brute = {k_bounce_brute<false, SHADE_COUNT, EXACT, GGX, false, DIEL>, kBruteBlock};
-		k.brute_finish = {k_brute_finish<SHADE_COUNT, GGX, DIEL>, kBruteBlock};
+		k.brute_first = {k_bounce_brute<true, SHADE_COUNT, EXACT, GGX, LENS, DIEL, SKY>, kBruteBlock};
+		k.brute = {k_bounce_brute<false, SHADE_COUNT, EXACT, GGX, false, DIEL, SKY>, kBruteBlock};
+		k.brute_finish = {k_brute_finish<SHADE_COUNT, GGX, DIEL, SKY>, kBruteBlock};
 		k.packet = {k_intersect_packet<COUNT, LENS ? B2R_PACKET_RPL_LENS : B2R_PACKET_RPL, LENS>, kTravBlock};
 		k.closest = {k_intersect_closest<COUNT, EXACT, TN16 ? 16u : 0u>, kTravBlock};
-		k.shade = {k_shade<EXACT, GGX, DIEL>, kBruteBlock};
+		k.shade = {k_shade<EXACT, GGX, DIEL, SKY>, kBruteBlock};
 		k.shadow = {k_intersect_shadow<COUNT>, kTravBlock};
 		k.generate = {k_generate<LENS>, kBlock};
 		return k;
@@ -319,7 +326,8 @@ int kernels_of(b2r_ctx* c, const KernelSet** out) {
 	const uint32_t f = c->cfg.flags;
 	const bool exact = (f & B2R_FLAG_REFERENCE_EXACT) != 0;
 	const uint32_t key = ((f & B2R_FLAG_COUNT_TESTS) ? KEY_COUNT : 0u) | (exact ? KEY_EXACT : 0u) | ((f & B2R_FLAG_GGX) ? KEY_GGX : 0u) |
-	                     (c->lens.radius > 0.0f && !exact ? KEY_LENS : 0u) | ((f & B2R_FLAG_DIELECTRIC) ? KEY_DIEL : 0u) | (c->params.scene.stack_tn_bits == 16u ? KEY_TN16 : 0u);
+	                     (c->lens.radius > 0.0f && !exact ? KEY_LENS : 0u) | ((f & B2R_FLAG_DIELECTRIC) ? KEY_DIEL : 0u) | (c->params.scene.stack_tn_bits == 16u ? KEY_TN16 : 0u) |
+	                     ((f & B2R_FLAG_SKY_LIGHT) ? KEY_SKY : 0u);
 	KernelSet& k = c->kernels[key];
 	if (!k.shade.fn) {
 		KernelSet s = kernel_set(key, std::make_integer_sequence<uint32_t, KEYS>());
@@ -585,7 +593,8 @@ int refresh_side_scene(b2r_ctx* c, uint32_t sidx) {
 		S.track.invalidate();
 	}
 	if (c->uploaded_valid) CU(cudaStreamWaitEvent(S.stream, c->ev_uploaded, 0));
-	const size_t len[LEN_COUNT] = {sc.n_prims, sc.n_mat, sc.n_lights ? sc.n_lights : 1u, c->n_wide, sc.hdri ? c->hdri_texels : 0u};
+	const size_t len[LEN_COUNT] = {sc.n_prims, sc.n_mat, sc.n_lights ? sc.n_lights : 1u, c->n_wide, sc.hdri ? c->hdri_texels : 0u, c->sky_built ? c->params.sky.rows + 1u : 0u,
+	                               c->sky_built ? static_cast<size_t>(c->params.sky.rows) * (c->params.sky.cols + 1u) : 0u, c->sky_built ? c->hdri_texels : 0u};
 	const int rc = SceneTables::for_each([&](int l, auto& s, const auto& m) -> int {
 		const size_t bytes = len[l] * sizeof(*m.p);
 		if (bytes) CU(cudaMemcpyAsync(s.p, m.p, bytes, cudaMemcpyDeviceToDevice, S.stream));
@@ -741,6 +750,47 @@ int ensure_origin_box(b2r_ctx* c, const float* points, uint32_t n_points) {
 	return B2R_OK;
 }
 
+// B2R_FLAG_SKY_LIGHT (DESIGN §2): the flags it cannot be combined with (null: none)
+const char* sky_flag_conflict(uint32_t flags) {
+	if (!(flags & B2R_FLAG_SKY_LIGHT)) return nullptr;
+	if (flags & B2R_FLAG_REFERENCE_EXACT) return "B2R_FLAG_SKY_LIGHT cannot be combined with B2R_FLAG_REFERENCE_EXACT";
+	if (flags & B2R_FLAG_NO_MIS) return "B2R_FLAG_SKY_LIGHT cannot be combined with B2R_FLAG_NO_MIS (there is no light sampling to add the sky to)";
+	if (flags & B2R_FLAG_GGX) return "B2R_FLAG_SKY_LIGHT cannot be combined with B2R_FLAG_GGX (Closure<GGX>::pdf is 0: the sky's MIS weights need the BSDF's pdf)";
+	return nullptr;
+}
+// whether `flags` sample the current sky: a sky (ambient > 0) whose texels are not zero everywhere
+bool sky_sampled(const b2r_ctx* c, uint32_t flags) { return (flags & B2R_FLAG_SKY_LIGHT) && c->params.scene.has_ambient && c->sky_nonzero; }
+// SkyDev's scalars for the context's flags and scene (the tables' pointers are bound with the others)
+void set_sky_scalars(b2r_ctx* c) {
+	SkyDev& k = c->params.sky; const SceneDev& s = c->params.scene;
+	k.p_sky = !sky_sampled(c, c->cfg.flags) ? 0.0f : s.n_lights == 0u ? 1.0f : 0.5f;
+	k.light_sel_pdf = s.n_lights ? (1.0f - k.p_sky) / static_cast<float>(s.n_lights) : 0.0f;
+	k.cols = s.hdri_w > 1 ? static_cast<uint32_t>(s.hdri_w - 1) : 1u; k.rows = s.hdri_h > 1 ? static_cast<uint32_t>(s.hdri_h - 1) : 1u;
+}
+// lengths of the sky's tables for a w x h texture (reserve_tables)
+void sky_table_lens(int32_t w, int32_t h, size_t (&len)[LEN_COUNT]) {
+	const size_t cols = w > 1 ? static_cast<size_t>(w - 1) : 1u, rows = h > 1 ? static_cast<size_t>(h - 1) : 1u;
+	len[LEN_SKY_MARG] = rows + 1u; len[LEN_SKY_COND] = rows * (cols + 1u); len[LEN_SKY_PDF] = static_cast<size_t>(w) * static_cast<size_t>(h);
+}
+// The sky's tables from the device copy of the texture, on the scene-write stream (k_sky_*, b2r_device.cuh; tables reserved by the caller)
+int launch_sky_build(b2r_ctx* c, int32_t w, int32_t h, const float amb[3]) {
+	const uint32_t cols = w > 1 ? static_cast<uint32_t>(w - 1) : 1u, rows = h > 1 ? static_cast<uint32_t>(h - 1) : 1u;
+	int rc; if ((rc = dev_reserve(&c->d_sky_tmp, &c->cap_sky_tmp, 2u * static_cast<size_t>(rows) + 1u))) return rc;
+	const SkyBuild b{c->tables.hdri.p, w, cols, rows, {amb[0], amb[1], amb[2]}, c->d_sky_tmp, c->d_sky_tmp + rows, c->d_sky_tmp + 2u * rows,
+	                 c->tables.sky_marg.p, c->tables.sky_cond.p, c->tables.sky_pdf.p};
+	const cudaStream_t st = c->scene_st;
+	const uint32_t row_grid = static_cast<uint32_t>((static_cast<size_t>(rows) * 32u + kBlock - 1u) / kBlock);
+	const size_t texels = static_cast<size_t>(w) * static_cast<size_t>(h);
+	k_sky_rows<<<row_grid, kBlock, 0, st>>>(b);
+	k_sky_floor<<<1, 32, 0, st>>>(b);
+	k_sky_cond<<<row_grid, kBlock, 0, st>>>(b);
+	k_sky_marg<<<1, 32, 0, st>>>(b);
+	k_sky_pdf<<<static_cast<uint32_t>((texels + kBlock - 1u) / kBlock), kBlock, 0, st>>>(b, static_cast<uint32_t>(h));
+	CU(cudaGetLastError()); c->launches += 5;
+	return B2R_OK;
+}
+constexpr const char* kSkyInvalid = "B2R_FLAG_SKY_LIGHT: a sky texel is not finite, or negative, in a channel whose ambient is > 0";
+
 }  // namespace
 
 // ================================================================================================ C ABI
@@ -761,6 +811,7 @@ int b2r_create(b2r_ctx** out, const b2r_config* cfg) {
 	if (cfg->samples_in_flight > static_cast<uint32_t>(kMaxSlots)) return fail(B2R_ERR_ARG, "samples_in_flight must be <= 64");
 	if ((cfg->flags & B2R_FLAG_GGX) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_GGX cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if ((cfg->flags & B2R_FLAG_DIELECTRIC) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
+	if (const char* why = sky_flag_conflict(cfg->flags)) return fail(B2R_ERR_ARG, why);
 	int n_dev = 0;
 	cudaError_t e = cudaGetDeviceCount(&n_dev);
 	if (e != cudaSuccess || n_dev == 0) return fail(B2R_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(e) + " (libb2r has no CPU fallback)");
@@ -791,7 +842,7 @@ void b2r_destroy(b2r_ctx* c) {
 	drop_graph(c);
 	for (auto& t : c->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
 	free_tables(c->tables);
-	dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_tap); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep);
+	dev_free(&c->d_cost); dev_free(&c->d_remap); dev_free(&c->d_trace); dev_free(&c->d_tap); dev_free(&c->d_cost_base); dev_free(&c->d_sort_tmp); dev_free(&c->d_sweep); dev_free(&c->d_sky_tmp);
 	for (int k = 0; k < 2; k++) { dev_free(&c->d_mkey[k]); dev_free(&c->d_midx[k]); }
 	for (int s = 0; s < 2; s++) { dev_free(&c->d_A[s]); dev_free(&c->d_B[s]); dev_free(&c->d_T[s]); dev_free(&c->d_N[s]); }
 	dev_free(&c->d_H); dev_free(&c->d_SA); dev_free(&c->d_SB); dev_free(&c->d_SL); dev_free(&c->d_SS); dev_free(&c->d_rad); dev_free(&c->d_acc); dev_free(&c->d_fb);
@@ -862,7 +913,21 @@ int b2r_set_flags(b2r_ctx* c, uint32_t flags) {
 	if ((flags & B2R_FLAG_GGX) && (flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_GGX cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if ((flags & B2R_FLAG_DIELECTRIC) && (flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if ((flags & B2R_FLAG_DIELECTRIC) && c->have_scene && !c->scene_diel_valid) return fail(B2R_ERR_ARG, kDielInvalid);
+	if (const char* why = sky_flag_conflict(flags)) return fail(B2R_ERR_ARG, why);
+	const SceneDev& sc = c->params.scene;
+	if ((flags & B2R_FLAG_SKY_LIGHT) && c->have_scene && sc.has_ambient && !c->sky_checked) {  // uploaded without the flag: the rule is checked on the texels now
+		std::vector<float4> tex(c->hdri_texels);
+		CU(cudaMemcpyAsync(tex.data(), c->tables.hdri.p, tex.size() * sizeof(float4), cudaMemcpyDeviceToHost, c->stream)); CU(sync_main(c));
+		c->sky_valid = sky_texels_valid(tex.data(), tex.size(), sc.ambient, &c->sky_nonzero); c->sky_checked = true;
+	}
+	if ((flags & B2R_FLAG_SKY_LIGHT) && c->have_scene && sc.has_ambient && !c->sky_valid) return fail(B2R_ERR_ARG, kSkyInvalid);
+	if (c->have_scene && sky_sampled(c, flags) && !c->sky_built) {  // turned on over a sky: its tables, from the device copy of the texture
+		size_t len[LEN_COUNT] = {}; sky_table_lens(sc.hdri_w, sc.hdri_h, len);
+		if ((rc = reserve_tables(c, len)) || (rc = begin_scene_write(c, use_sides(c))) || (rc = launch_sky_build(c, sc.hdri_w, sc.hdri_h, sc.ambient)) || (rc = end_scene_write(c))) return rc;
+		c->sky_built = true; bind_tables(c->params, c->tables, sc.hdri != nullptr);
+	}
 	c->cfg.flags = flags; c->params.frame.flags = flags;
+	set_sky_scalars(c);
 	if (c->have_scene) {
 		const uint32_t n = c->params.scene.n_prims;
 		c->use_bvh = (flags & B2R_FLAG_FORCE_BVH) ? true : (flags & B2R_FLAG_FORCE_BRUTE) ? false : n > 32;
@@ -919,6 +984,7 @@ template <typename F> void rebind_scene(b2r_ctx* c, bool sky, F&& set) {
 	const Params before = c->params; const bool bvh_before = c->use_bvh;
 	bind_tables(c->params, c->tables, sky);
 	set(c->params.scene);
+	set_sky_scalars(c);
 	if (!c->have_scene || bvh_before != c->use_bvh || std::memcmp(&before, &c->params, sizeof before) != 0) drop_graph(c);
 }
 }  // namespace
@@ -936,6 +1002,11 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	if (has_ambient && (!hdri_rgba || hdri_w <= 0 || hdri_h <= 0)) return fail(B2R_ERR_ARG, "ambient > 0 needs an HDRI (the reference terminates without one, Application.cpp:225-229)");
 	bool diel_valid = true;
 	int rc = check_scene_refs(c, prims, geometry, n_prims, n_geom, materials, n_mat, light_geom_idx, n_lights, &diel_valid); if (rc) return rc;
+	// B2R_FLAG_SKY_LIGHT: the input rule on the sky's texels, checked here under the flag (otherwise when b2r_set_flags turns it on)
+	const bool sky_checked = (c->cfg.flags & B2R_FLAG_SKY_LIGHT) && has_ambient;
+	bool sky_nonzero = false;
+	if (sky_checked && !sky_texels_valid(reinterpret_cast<const float4*>(hdri_rgba), static_cast<size_t>(hdri_w) * hdri_h, amb, &sky_nonzero)) return fail(B2R_ERR_ARG, kSkyInvalid);
+	const bool sky_build = sky_checked && sky_nonzero;
 	if ((rc = ensure_device(c))) return rc;
 	// No stream synchronisation from here on: the copies below are ordered after the kernels already enqueued on the stream (which
 	// may still read the old scene) and before the ones enqueued next. The host side is staged in one page-locked block that is only
@@ -992,12 +1063,15 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 
 	PackedScene ps; pack_scene(prims, n_prims, materials, n_mat, light_geom_idx, n_lights, geometry, ps);
 	const size_t texels = has_ambient ? static_cast<size_t>(hdri_w) * hdri_h : 0;
-	const size_t len[LEN_COUNT] = {n_prims, n_mat, ps.light_sphere.size(), c->n_wide, texels};  // (no sky: the sky's table is left alone)
+	size_t len[LEN_COUNT] = {n_prims, n_mat, ps.light_sphere.size(), c->n_wide, texels, 0, 0, 0};  // (no sky: the sky's tables are left alone)
+	if (sky_build) sky_table_lens(hdri_w, hdri_h, len);
 	if ((rc = reserve_tables(c, len))) return rc;
 	const bool bvh_next = (c->cfg.flags & B2R_FLAG_FORCE_BVH) ? true : (c->cfg.flags & B2R_FLAG_FORCE_BRUTE) ? false : n_prims > 32;
 	if ((rc = begin_scene_write(c, sides_for(c, bvh_next)))) return rc;
 	if ((rc = stage_packed(c, ps, {{c->tables.wide.p, c->wide_host.nodes.data(), gpu_tree ? 0 : c->wide_host.nodes.size() * sizeof(WideNode)}, {c->tables.hdri.p, hdri_rgba, texels * sizeof(float4)}}))) return rc;
 	c->hdri_texels = texels;
+	if (sky_build && (rc = launch_sky_build(c, hdri_w, hdri_h, amb))) return rc;
+	c->sky_built = sky_build; c->sky_checked = sky_checked; c->sky_valid = true; c->sky_nonzero = sky_nonzero;
 	c->wide_refit = false; c->cur_geom_of_prim.clear(); drop_speculation(c);
 	if (gpu_tree) {  // Morton keys -> stable radix sort -> implicit 4-ary links -> boxes, all on the stream behind the copies above
 		if (n_prims > c->cap_mkey) { for (int k = 0; k < 2; k++) { size_t cap = 0; if ((rc = dev_reserve(&c->d_mkey[k], &cap, n_prims)) || (cap = 0, rc = dev_reserve(&c->d_midx[k], &cap, n_prims))) return rc; } c->cap_mkey = n_prims; }
@@ -1068,7 +1142,7 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	}
 	PackedScene ps; pack_scene(prims, n_prims, materials, n_mat, light_geom_idx, n_lights, geometry, ps);
 	if ((rc = dev_reserve(&c->d_remap, &c->cap_remap, remap.size()))) return rc;
-	const size_t len[LEN_COUNT] = {0, n_mat, ps.light_sphere.size(), 0, 0};  // the sphere count is kept: only the (small) material and light tables can grow
+	const size_t len[LEN_COUNT] = {0, n_mat, ps.light_sphere.size(), 0, 0, 0, 0, 0};  // the sphere count is kept: only the (small) material and light tables can grow
 	if ((rc = reserve_tables(c, len))) return rc;
 	if (!c->d_cost) { size_t cap = 0; if ((rc = dev_reserve(&c->d_cost, &cap, 1))) return rc; }
 	if ((rc = begin_scene_write(c, use_sides(c)))) return rc;
@@ -1429,7 +1503,7 @@ int b2r_write_buckets(b2r_ctx* c, const float* in_host) {
 namespace {
 struct CheckpointHeader { char magic[8]; uint32_t width, height, buckets, max_bounces, accumulations, result_flags; uint64_t payload_hash; uint64_t payload_bytes; uint32_t reserved[4]; };
 static_assert(sizeof(CheckpointHeader) == 64, "checkpoint header");
-constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT | B2R_FLAG_DIELECTRIC;  // flags that change which image is being accumulated
+constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT | B2R_FLAG_DIELECTRIC | B2R_FLAG_SKY_LIGHT;  // flags that change which image is being accumulated
 uint64_t fnv1a64(const void* data, size_t bytes) { const unsigned char* b = static_cast<const unsigned char*>(data); uint64_t h = 1469598103934665603ull; for (size_t i = 0; i < bytes; i++) h = (h ^ b[i]) * 1099511628211ull; return h; }
 }  // namespace
 int b2r_save_checkpoint(b2r_ctx* c, const char* path) {
@@ -1679,6 +1753,20 @@ int b2r_read_link_tables(b2r_ctx* c, uint32_t* parent_out, uint32_t* leaf_node_o
 	c->main_reads_scene = true;
 	CU(cudaMemcpyAsync(parent_out, c->tables.parent.p, static_cast<size_t>(c->n_wide) * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaMemcpyAsync(leaf_node_out, c->tables.leaf_node.p, static_cast<size_t>(c->params.scene.n_prims) * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(sync_main(c));
+	return B2R_OK;
+}
+int b2r_read_sky_tables(b2r_ctx* c, float* marginal_out, float* conditional_out, float* pdf_out, uint32_t* cols_out, uint32_t* rows_out) {
+	if (!c || !cols_out || !rows_out) return fail(B2R_ERR_ARG, "null argument");
+	if (!c->have_scene) return fail(B2R_ERR_STATE, "upload_scene first");
+	if (!c->sky_built) return fail(B2R_ERR_STATE, "no sky tables: B2R_FLAG_SKY_LIGHT over a sky that is not zero everywhere builds them");
+	const SkyDev& k = c->params.sky;
+	*cols_out = k.cols; *rows_out = k.rows;
+	int rc = ensure_device(c); if (rc) return rc;
+	c->main_reads_scene = true;
+	if (marginal_out) CU(cudaMemcpyAsync(marginal_out, c->tables.sky_marg.p, (k.rows + 1u) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+	if (conditional_out) CU(cudaMemcpyAsync(conditional_out, c->tables.sky_cond.p, static_cast<size_t>(k.rows) * (k.cols + 1u) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+	if (pdf_out) CU(cudaMemcpyAsync(pdf_out, c->tables.sky_pdf.p, c->hdri_texels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 	CU(sync_main(c));
 	return B2R_OK;
 }

@@ -115,8 +115,8 @@ __device__ __forceinline__ bool finished_elsewhere(const Params& p, uint32_t bou
 // LENS (bounce 0 with a thin lens): every camera ray has its own origin, so there is no shared-origin sphere precompute (s_pre); phase 1
 // runs sphere_hit_closest per ray, and phase 2 regenerates a hit's camera ray from its path id instead of queueing its origin.
 // DIELECTRIC (B2R_FLAG_DIELECTRIC): the shading routines' smooth-dielectric path (b2r_shade.h dielectric_scatter); the same axis in k_brute_finish
-// and k_shade.
-template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false, bool LENS = false, bool DIELECTRIC = false>
+// and k_shade. SKY (B2R_FLAG_SKY_LIGHT): the sky as a light (b2r_shade.h sky_light_sample, shade_sky<true>); likewise.
+template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false, bool LENS = false, bool DIELECTRIC = false, bool SKY = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_brute(const Params p, const uint32_t bounce) {
 	constexpr int kQ = 2 * kBruteBlock;  // hit queue: up to kBruteBlock-1 waiting + kBruteBlock new
 	__shared__ float4 s_prim[kBruteTile];
@@ -212,7 +212,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 				if (sc.has_ambient) {
 					const uint32_t slm = FIRST ? div_by(i, p.frame.npix, p.frame.npix_magic) : 0u;
 					const PathState sm = FIRST ? primary_path<LENS>(p.frame, p.batch->cam, p.batch->acc[slm], slm, i - slm * p.frame.npix, p.batch->lens) : load_path(p.q, side, i);
-					rad_add(p.rad, p.frame.npix, sm.pid, shade_sky(sc, sm), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++;
+					rad_add(p.rad, p.frame.npix, sm.pid, shade_sky<SKY>(sc, sm, bounce, p.sky), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++;
 				}
 			}
 			// ---------------- the CTA's hits join the shared-memory queue
@@ -250,11 +250,11 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 				c_hits++;
 				if (last) { rad_zero(p.rad, p.frame.npix, s.pid); c_drop++; }  // survivors of the last bounce lose their radiance (Q11)
 				else {
-					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC>(sc, sf, s, hprim, acc, seed, bounce, &sr);
+					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, hprim, acc, seed, bounce, &sr, p.sky);
 					if (sf.emissive) {
 						// light sample first, then emission (Renderer.hpp:304-353). The shadow test of an emissive hit (rare) is done
 						// right here so that order holds; every other shadow ray goes to the queue and is tested by dense warps.
-						const f3 e_add = shade_emission<DIELECTRIC>(sc, sf, s, depth, bounce, mis);
+						const f3 e_add = shade_emission<DIELECTRIC, SKY>(sc, sf, s, depth, bounce, mis, p.sky);
 						if (want_shadow) {
 							c_shadow++;
 							bool occluded = false;
@@ -268,7 +268,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 						} else rad_add(p.rad, p.frame.npix, s.pid, e_add, f3{0.0f, 0.0f, 0.0f}, true, false);
 						c_events++;
 					}
-					keep = shade_continue<GGX, DIELECTRIC>(sf, &s, acc, seed, bounce);
+					keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
 					if (!keep) c_term++;  // roulette: path ends here, radiance stays at the pixel (Renderer.hpp:379-381,424-430)
 				}
 			}
@@ -349,7 +349,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 // lane; both sphere loops are warp-uniform (every lane walks all the spheres of the shared-memory copy), so the only divergence is paths
 // ending, and a lane whose path has ended picks up the next waiting path. Same routines, same RNG streams (a function of sample, pixel and
 // bounce), same order of a path's radiance additions (light sample, then emission) as k_bounce_brute: every path ends with the same bits.
-template <bool COUNT, bool GGX = false, bool DIELECTRIC = false>
+template <bool COUNT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_brute_finish(const Params p, const uint32_t bounce0) {
 	__shared__ float4 s_prim[kBruteTile];
 	__shared__ int32_t s_prim_mat[kBruteTile];
@@ -411,16 +411,16 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_brute_fin
 		if (alive) {
 			if (prim < 0) {  // miss shader (Renderer.hpp:408-420)
 				c_term++;
-				if (sc.has_ambient) { rad_add(p.rad, p.frame.npix, pid, shade_sky(sc, s), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++; }
+				if (sc.has_ambient) { rad_add(p.rad, p.frame.npix, pid, shade_sky<SKY>(sc, s, bounce, p.sky), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++; }
 			} else {
 				const uint32_t acc = p.batch->acc[pid >> 26], seed = pixel_seed(pid & kPixMask, mb);
 				const Surface sf = shade_surface<GGX, DIELECTRIC>(sc, s, best, prim, p.mat_diel);
 				c_hits++;
 				if (bounce + 1u >= mb) { rad_zero(p.rad, p.frame.npix, pid); c_drop++; }  // Q11
 				else {
-					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC>(sc, sf, s, prim, acc, seed, bounce, &sr);
-					if (sf.emissive) { emit = shade_emission<DIELECTRIC>(sc, sf, s, best, bounce, mis); has_emit = true; }
-					keep = shade_continue<GGX, DIELECTRIC>(sf, &s, acc, seed, bounce);
+					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky);
+					if (sf.emissive) { emit = shade_emission<DIELECTRIC, SKY>(sc, sf, s, best, bounce, mis, p.sky); has_emit = true; }
+					keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
 					if (!keep) c_term++;
 				}
 			}
@@ -794,7 +794,7 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p
 }
 // shade the hit records: light sample -> shadow queue, emission, BRDF sample / roulette -> next path queue.
 // Same CTA structure as the brute-force kernel: hits are collected in a shared-memory queue and shaded a full CTA at a time.
-template <bool EXACT, bool GGX = false, bool DIELECTRIC = false>
+template <bool EXACT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(const Params p, const uint32_t bounce) {
 	constexpr int kQ = 2 * kBruteBlock;
 	__shared__ uint32_t s_hit_i[kQ]; __shared__ float s_hit_t[kQ]; __shared__ int32_t s_hit_prim[kQ];
@@ -826,7 +826,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 #endif
 			if (live && !is_hit) {  // miss shader (Renderer.hpp:408-420)
 				c_term++;
-				if (sc.has_ambient) { const PathState sm = load_path(p.q, side, i); rad_add(p.rad, p.frame.npix, sm.pid, shade_sky(sc, sm), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++; }
+				if (sc.has_ambient) { const PathState sm = load_path(p.q, side, i); rad_add(p.rad, p.frame.npix, sm.pid, shade_sky<SKY>(sc, sm, bounce, p.sky), f3{0.0f, 0.0f, 0.0f}, true, false); c_events++; }
 			}
 			uint32_t n_hits;
 			const uint32_t slot = queued + block_rank(is_hit, s_cnt_a, &n_hits);
@@ -853,12 +853,12 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 			c_hits++;
 			if (last) { rad_zero(p.rad, p.frame.npix, s.pid); c_drop++; }  // Q11
 			else {
-				if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC>(sc, sf, s, prim, acc, seed, bounce, &sr);
+				if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky);
 				if (sf.emissive) {
 					// the reference adds the light sample first, then the emission (Renderer.hpp:304-353). For the (rare) emissive hit
 					// that also has a shadow ray the any-hit traversal is done right here so that order holds; every other shadow ray
 					// goes to the shadow queue and is traced by k_intersect_shadow.
-					const f3 emit = shade_emission<DIELECTRIC>(sc, sf, s, depth, bounce, mis);
+					const f3 emit = shade_emission<DIELECTRIC, SKY>(sc, sf, s, depth, bounce, mis, p.sky);
 					if (want_shadow) {
 						uint32_t cs = 0, cb = 0;
 						const bool occluded = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb, sc.parent, 0u);
@@ -867,7 +867,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 					} else rad_add(p.rad, p.frame.npix, s.pid, emit, f3{0.0f, 0.0f, 0.0f}, true, false);
 					c_events++;
 				}
-				keep = shade_continue<GGX, DIELECTRIC>(sf, &s, acc, seed, bounce);
+				keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
 				if (!keep) c_term++;
 			}
 		}
@@ -1043,6 +1043,83 @@ __global__ void __launch_bounds__(kBlock) k_link_tables(const float4* __restrict
 	const int32_t l = __float_as_int(wide[static_cast<size_t>(i) * 2u + 1u].z);
 	if (l == kEmptyLink) return;
 	if (l < 0) leaf_node[~l] = node; else parent[l] = node;
+}
+// ---------------------------------------------------------------------------------------------- sky tables (B2R_FLAG_SKY_LIGHT)
+// Built from the device copy of the texture with fixed-order double sums and no atomics, so the host twin (build_sky_tables, b2r_host.cpp)
+// reproduces them bit for bit (DESIGN §4). A sum is one warp's chunked scan: chunks of 32 in order, a Kogge-Stone inclusive scan inside a
+// chunk (offsets 1, 2, 4, 8, 16; lanes past the end hold 0), then the running carry added; write(k, inclusive prefix); returns the total.
+template <class V, class W>
+__device__ double sky_warp_scan(uint32_t n, V&& value, W&& write) {
+	double carry = 0.0;
+	for (uint32_t b = 0; b < n; b += 32u) {
+		const uint32_t k = b + lane_id();
+		double x = k < n ? value(k) : 0.0;
+#pragma unroll
+		for (uint32_t off = 1; off < 32u; off <<= 1) { const double y = __shfl_up_sync(0xffffffffu, x, off); if (lane_id() >= off) x = y + x; }
+		const double incl = carry + x;
+		if (k < n) write(k, incl);
+		carry = __shfl_sync(0xffffffffu, incl, 31);
+	}
+	return carry;
+}
+// cdf[1..n] strictly increasing with cdf[n] kept: cdf[k] = min over m >= k of (bits(cdf[m]) - (m - k)) — a suffix minimum of bits - index,
+// integer and order-free. A cell whose step rounded to 0 gets one ulp, so every cell keeps a non-zero probability.
+__device__ void sky_warp_strict(float* cdf, uint32_t n) {
+	long long carry = 0x7fffffffffffffffll;
+	for (long long top = n; top >= 1; top -= 32) {
+		const long long k = top - static_cast<long long>(lane_id());
+		long long m = k >= 1 ? static_cast<long long>(__float_as_uint(cdf[k])) - k : 0x7fffffffffffffffll;
+#pragma unroll
+		for (uint32_t off = 1; off < 32u; off <<= 1) { const long long y = __shfl_up_sync(0xffffffffu, m, off); if (lane_id() >= off) m = y < m ? y : m; }
+		m = carry < m ? carry : m;
+		if (k >= 1) cdf[k] = __uint_as_float(static_cast<uint32_t>(m + k));
+		carry = __shfl_sync(0xffffffffu, m, 31);
+	}
+}
+struct SkyBuild { const float4* tex; int32_t w; uint32_t cols, rows; float ambient[3]; double* row_lum; double* row_weight; double* floor; float* marg; float* cond; float* pdf; };
+// one warp per row: the row's summed luminance
+__global__ void __launch_bounds__(kBlock) k_sky_rows(const SkyBuild b) {
+	const uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+	if (j >= b.rows) return;
+	const float4* row = b.tex + static_cast<size_t>(j) * b.w;
+	const double s = sky_warp_scan(b.cols, [&](uint32_t i) { return static_cast<double>(sky_lum(__ldg(row + i), b.ambient)); }, [](uint32_t, double) {});
+	if (lane_id() == 0) b.row_lum[j] = s;
+}
+// one warp: the floor, lum_mean / 64
+__global__ void k_sky_floor(const SkyBuild b) {
+	const double s = sky_warp_scan(b.rows, [&](uint32_t j) { return b.row_lum[j]; }, [](uint32_t, double) {});
+	if (lane_id() == 0) *b.floor = s / (static_cast<double>(b.cols) * static_cast<double>(b.rows)) / 64.0;
+}
+// one warp per row: the row's conditional CDF (scanned twice: the total, then the normalised prefixes) and its weight, solid angle * total
+__global__ void __launch_bounds__(kBlock) k_sky_cond(const SkyBuild b) {
+	const uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+	if (j >= b.rows) return;
+	const float4* row = b.tex + static_cast<size_t>(j) * b.w;
+	float* cdf = b.cond + static_cast<size_t>(j) * (b.cols + 1u);
+	const double fl = *b.floor;
+	auto value = [&](uint32_t i) { return static_cast<double>(sky_lum(__ldg(row + i), b.ambient)) + fl; };
+	const double total = sky_warp_scan(b.cols, value, [](uint32_t, double) {});
+	sky_warp_scan(b.cols, value, [&](uint32_t i, double p) { cdf[i + 1u] = static_cast<float>(p / total); });
+	__syncwarp();
+	if (lane_id() == 0) { cdf[0] = 0.0f; cdf[b.cols] = 1.0f; b.row_weight[j] = sky_cell_omega(j, b.rows, b.cols) * total; }
+	__syncwarp();
+	sky_warp_strict(cdf, b.cols);
+}
+// one warp: the marginal CDF over the row weights
+__global__ void k_sky_marg(const SkyBuild b) {
+	auto value = [&](uint32_t j) { return b.row_weight[j]; };
+	const double total = sky_warp_scan(b.rows, value, [](uint32_t, double) {});
+	sky_warp_scan(b.rows, value, [&](uint32_t j, double p) { b.marg[j + 1u] = static_cast<float>(p / total); });
+	__syncwarp();
+	if (lane_id() == 0) { b.marg[0] = 0.0f; b.marg[b.rows] = 1.0f; }
+	__syncwarp();
+	sky_warp_strict(b.marg, b.rows);
+}
+// one thread per texel: the solid-angle pdf of the cell it shows (sky_texel_pdf)
+__global__ void __launch_bounds__(kBlock) k_sky_pdf(const SkyBuild b, const uint32_t h) {
+	const size_t t = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+	if (t >= static_cast<size_t>(b.w) * h) return;
+	b.pdf[t] = sky_texel_pdf(b.marg, b.cond, b.cols, b.rows, static_cast<uint32_t>(t % static_cast<uint32_t>(b.w)), static_cast<uint32_t>(t / static_cast<uint32_t>(b.w)));
 }
 // ---------------------------------------------------------------------------------------------- GPU tree build (B2R_FLAG_GPU_TREE)
 // The traversal tree built on the device for edits that add or remove spheres (the reference rebuilds its BVH on every edit,

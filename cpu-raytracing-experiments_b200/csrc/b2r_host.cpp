@@ -611,6 +611,68 @@ bool dielectric_materials_valid(const b2r_material* materials, uint32_t n_mat) {
 	return true;
 }
 
+bool sky_texels_valid(const float4* texels, size_t n, const float ambient[3], bool* nonzero) {
+	bool any = false;
+	for (size_t t = 0; t < n; t++) {
+		const float v[3] = {texels[t].x, texels[t].y, texels[t].z};
+		for (int k = 0; k < 3; k++) {
+			if (!(ambient[k] > 0.0f)) continue;
+			if (!std::isfinite(v[k]) || !(v[k] >= 0.0f)) return false;
+			any = any || v[k] > 0.0f;
+		}
+	}
+	*nonzero = any;
+	return true;
+}
+
+namespace {
+// the device's sky_warp_scan: chunks of 32 in order, a Kogge-Stone inclusive scan inside each (lanes past the end hold 0), plus the carry
+template <class V, class W> double sky_chunk_scan(uint32_t n, V&& value, W&& write) {
+	double carry = 0.0;
+	for (uint32_t b = 0; b < n; b += 32u) {
+		double x[32];
+		for (uint32_t l = 0; l < 32u; l++) x[l] = b + l < n ? value(b + l) : 0.0;
+		for (uint32_t off = 1; off < 32u; off <<= 1) for (uint32_t l = 31u; l >= off; l--) x[l] = x[l - off] + x[l];
+		for (uint32_t l = 0; l < 32u && b + l < n; l++) write(b + l, carry + x[l]);
+		carry = carry + x[31];
+	}
+	return carry;
+}
+// the device's sky_warp_strict (a suffix minimum of bits - index)
+void sky_strict(float* cdf, uint32_t n) {
+	long long m = 0x7fffffffffffffffll;
+	for (long long k = n; k >= 1; k--) {
+		m = std::min(m, static_cast<long long>(bits(cdf[k])) - k);
+		cdf[k] = from_bits(static_cast<uint32_t>(m + k));
+	}
+}
+}  // namespace
+
+void build_sky_tables(const float4* texels, int32_t w, int32_t h, const float ambient[3], SkyTables& out) {
+	const uint32_t cols = w > 1 ? static_cast<uint32_t>(w - 1) : 1u, rows = h > 1 ? static_cast<uint32_t>(h - 1) : 1u;
+	out.cols = cols; out.rows = rows;
+	out.marg.assign(rows + 1u, 0.0f); out.cond.assign(static_cast<size_t>(rows) * (cols + 1u), 0.0f); out.pdf.assign(static_cast<size_t>(w) * h, 0.0f);
+	auto lum = [&](uint32_t j, uint32_t i) { return static_cast<double>(sky_lum(texels[static_cast<size_t>(j) * w + i], ambient)); };
+	std::vector<double> row_lum(rows), row_weight(rows);
+	for (uint32_t j = 0; j < rows; j++) row_lum[j] = sky_chunk_scan(cols, [&](uint32_t i) { return lum(j, i); }, [](uint32_t, double) {});
+	const double fl = sky_chunk_scan(rows, [&](uint32_t j) { return row_lum[j]; }, [](uint32_t, double) {}) / (static_cast<double>(cols) * static_cast<double>(rows)) / 64.0;
+	for (uint32_t j = 0; j < rows; j++) {
+		float* cdf = out.cond.data() + static_cast<size_t>(j) * (cols + 1u);
+		auto value = [&](uint32_t i) { return lum(j, i) + fl; };
+		const double total = sky_chunk_scan(cols, value, [](uint32_t, double) {});
+		sky_chunk_scan(cols, value, [&](uint32_t i, double p) { cdf[i + 1u] = static_cast<float>(p / total); });
+		cdf[0] = 0.0f; cdf[cols] = 1.0f; row_weight[j] = sky_cell_omega(j, rows, cols) * total;
+		sky_strict(cdf, cols);
+	}
+	auto value = [&](uint32_t j) { return row_weight[j]; };
+	const double total = sky_chunk_scan(rows, value, [](uint32_t, double) {});
+	sky_chunk_scan(rows, value, [&](uint32_t j, double p) { out.marg[j + 1u] = static_cast<float>(p / total); });
+	out.marg[0] = 0.0f; out.marg[rows] = 1.0f;
+	sky_strict(out.marg.data(), rows);
+	for (uint32_t y = 0; y < static_cast<uint32_t>(h); y++)
+		for (uint32_t x = 0; x < static_cast<uint32_t>(w); x++) out.pdf[static_cast<size_t>(y) * w + x] = sky_texel_pdf(out.marg.data(), out.cond.data(), cols, rows, x, y);
+}
+
 }  // namespace b2r
 
 // ---------------------------------------------------------------------------------------------- C ABI (host-only part)

@@ -88,5 +88,12 @@ void pack_scene(const b2r_sphere* prims, uint32_t n_prims, const b2r_material* m
 // B2R_FLAG_DIELECTRIC input rule: every transmission component is finite, and a dielectric material (max(transmission) > 0) has every
 // component in [0, 1] and eta = 1 + IOR_minus_one finite and >= 1. Returns false when some material breaks it.
 bool dielectric_materials_valid(const b2r_material* materials, uint32_t n_mat);
+// B2R_FLAG_SKY_LIGHT input rule: every texel is finite and >= 0 in each channel whose ambient is > 0. *nonzero: some such value is > 0
+// (a sky that is zero everywhere is not sampled).
+bool sky_texels_valid(const float4* texels, size_t n, const float ambient[3], bool* nonzero);
+// B2R_FLAG_SKY_LIGHT: host twin of the device build of the sky's tables (k_sky_*, b2r_device.cuh), bit for bit; the texture must be valid and
+// not zero everywhere. marg: rows + 1, cond: rows * (cols + 1), pdf: w * h floats (SkyDev).
+struct SkyTables { std::vector<float> marg, cond, pdf; uint32_t cols = 0, rows = 0; };
+void build_sky_tables(const float4* texels, int32_t w, int32_t h, const float ambient[3], SkyTables& out);
 
 }  // namespace b2r

@@ -32,6 +32,13 @@ B2R_HD uint32_t ldg_u32(const uint32_t* p) {
 	return *p;
 #endif
 }
+B2R_HD float ldg_f32(const float* p) {
+#if defined(__CUDA_ARCH__)
+	return __ldg(p);
+#else
+	return *p;
+#endif
+}
 // scene tables (spheres, materials, lights): generic loads, because the brute-force kernels point SceneDev at shared-memory copies
 B2R_HD float4 ld4(const float4* p) { return *p; }
 
@@ -104,6 +111,16 @@ struct ExactDev {
 	uint8_t* key;         // [cap] 1 + material of the survivor that sat in (stream, slot) this bounce, 0 = none; cleared by k_stream_rank
 	uint32_t* next_idx;   // [cap] its index in the next path queue
 };
+// B2R_FLAG_SKY_LIGHT (DESIGN §2): the sky's cell distribution and the light choice. The cells follow the miss shader's lookup: cols x rows
+// = max(w - 1, 1) x max(h - 1, 1) cells, cell (i, j) shows texel (i, j). Tables built on the device by k_sky_* (host twin build_sky_tables).
+struct SkyDev {
+	const float* marg;    // [rows + 1] CDF over the rows (0 first, exactly 1 last, strictly increasing)
+	const float* cond;    // [rows][cols + 1] CDF over the cells of each row (likewise)
+	const float* pdf;     // [hdri_h][hdri_w] solid-angle pdf, without p_sky, of the cell each texel shows (the last column / row: the adjacent cell's)
+	uint32_t cols, rows;
+	float p_sky;          // probability that a light sample goes to the sky: 0 without a sky (nothing below reads the tables), 1 without sphere lights
+	float light_sel_pdf;  // (1 - p_sky) / n_lights: a sphere light's selection probability
+};
 struct Params {
 	SceneDev scene; FrameDev frame; QueueDev q; CountDev cnt; ExactDev ex;
 	const BatchDev* batch;
@@ -112,6 +129,7 @@ struct Params {
 	// [n_mat] {transmission.rgb, eta}, eta = 0 when max(transmission) == 0: read by the DIELECTRIC shading routines only (B2R_FLAG_DIELECTRIC).
 	// A scene table, but kept here at the end rather than in SceneDev, so the parameter block of every other instantiation keeps its layout.
 	const float4* mat_diel;
+	SkyDev sky;  // read by the SKY instantiations only (B2R_FLAG_SKY_LIGHT); at the end for the same reason
 };
 
 // ---------------------------------------------------------------------------------------------- small helpers
@@ -204,15 +222,90 @@ B2R_HD Surface shade_surface(const SceneDev& sc, const PathState& s, float depth
 	return sf;
 }
 template <bool DIELECTRIC> B2R_HD bool is_dielectric(const Surface& sf) { return DIELECTRIC && sf.diel.w != 0.0f; }
+
+// ---------------------------------------------------------------------------------------------- the sky as a light (B2R_FLAG_SKY_LIGHT)
+// The texel the miss shader shows in direction d (Primitives.hpp:35-46): nearest texel of the equirect, truncated.
+B2R_HD int32_t sky_texel(const SceneDev& sc, float dx, float dy, float dz) {
+	const float u = sc.hdri_fw * (0.5f + B2R_INV_TWO_PI * atan2_poly(dz, dx));
+	const float v = sc.hdri_fh * (0.5f - B2R_INV_PI * asin_poly(dy));
+	return static_cast<int32_t>(v) * sc.hdri_w + static_cast<int32_t>(u);
+}
+// dy at the border above cell row j (row j spans dy in [z(j + 1), z(j)]): cos(pi j / rows), exactly 1 and -1 at the poles. The sampler and the
+// tables' solid angles use this one function, so a cell's solid angle is exactly the set of directions the sampler draws in it.
+B2R_HD float sky_row_z(uint32_t j, uint32_t rows) {
+	if (j == 0u) return 1.0f;
+	if (j >= rows) return -1.0f;
+	float sn, cs; sincos_poly(B2R_PI * (static_cast<float>(j) / static_cast<float>(rows)), &sn, &cs);
+	return cs;
+}
+// solid angle of a cell of row j: (2 pi / cols) (z(j) - z(j + 1)), in double from the float borders
+B2R_HD double sky_cell_omega(uint32_t j, uint32_t rows, uint32_t cols) {
+	return (6.283185307179586 / static_cast<double>(cols)) * (static_cast<double>(sky_row_z(j, rows)) - static_cast<double>(sky_row_z(j + 1u, rows)));
+}
+// the cell's importance before the floor: mean of the channels of texel * ambient, counting only channels with ambient > 0, clamped at 0
+B2R_HD float sky_lum(const float4 t, const float ambient[3]) {
+	const float r = ambient[0] > 0.0f ? t.x * ambient[0] : 0.0f, g = ambient[1] > 0.0f ? t.y * ambient[1] : 0.0f, b = ambient[2] > 0.0f ? t.z * ambient[2] : 0.0f;
+	return sel_max(((r + g) + b) / 3.0f, 0.0f);
+}
+// SkyDev::pdf of texel (x, y): the probability of its cell as the CDFs give it (steps taken in double, exact) over the cell's solid angle.
+// The last column and row (x >= cols, y >= rows, reached by the lookup only on a set of measure zero) take the adjacent cell's.
+B2R_HD float sky_texel_pdf(const float* marg, const float* cond, uint32_t cols, uint32_t rows, uint32_t x, uint32_t y) {
+	const uint32_t i = x < cols ? x : cols - 1u, j = y < rows ? y : rows - 1u;
+	const float* c = cond + static_cast<size_t>(j) * (cols + 1u);
+	const double pm = static_cast<double>(marg[j + 1u]) - static_cast<double>(marg[j]), pc = static_cast<double>(c[i + 1u]) - static_cast<double>(c[i]);
+	return static_cast<float>(pm * pc / sky_cell_omega(j, rows, cols));
+}
+// the largest k < n with cdf[k] <= u (cdf[0] = 0)
+B2R_HD uint32_t sky_search(const float* cdf, uint32_t n, float u) {
+	uint32_t lo = 0u, hi = n;
+	while (hi - lo > 1u) { const uint32_t mid = (lo + hi) >> 1; if (ldg_f32(cdf + mid) <= u) lo = mid; else hi = mid; }
+	return lo;
+}
+// A direction drawn from the cell distribution: row by um, cell by uc, then uniform in solid angle inside the cell (dy by uy between the row's
+// borders, the longitude by ux across the column). *cell = the drawn cell's texel index (row * hdri_w + column).
+B2R_HD f3 sky_sample_dir(const SkyDev& sky, int32_t hdri_w, float um, float uc, float uy, float ux, int32_t* cell) {
+	const uint32_t j = sky_search(sky.marg, sky.rows, um);
+	const uint32_t i = sky_search(sky.cond + static_cast<size_t>(j) * (sky.cols + 1u), sky.cols, uc);
+	const float z0 = sky_row_z(j, sky.rows), z1 = sky_row_z(j + 1u, sky.rows);
+	const float dy = z0 + uy * (z1 - z0);
+	float sn, cs; sincos_poly(B2R_TWO_PI * ((static_cast<float>(i) + ux) / static_cast<float>(sky.cols)) - B2R_PI, &sn, &cs);
+	const float r = sqrtf(sel_max(0.0f, 1.0f - dy * dy));
+	*cell = static_cast<int32_t>(j) * hdri_w + static_cast<int32_t>(i);
+	return f3{r * cs, dy, r * sn};
+}
+// a^2 / (a^2 + b^2), 0 when both are 0. Unlike power_heuristic there is no floor under the sum, so the sky's two weights of one direction sum to 1.
+B2R_HD float sky_mis(float a, float b) { const float a2 = a * a, d = a2 + b * b; return d > 0.0f ? a2 / d : 0.0f; }
+// The sky light sample of a Lambertian surface, from the light-sample stream after its light choice (four more draws). q = p_sky * the pdf of
+// the cell the LOOKUP maps L to (the function both MIS weights use); the estimate divides by the density of the cell the sample was drawn in.
+B2R_HD bool sky_light_sample(const SceneDev& sc, const SkyDev& sky, const Surface& sf, const PathState& s, Pcg* rng, ShadowRay* out) {
+	const float um = rng->next_unit(), uc = rng->next_unit(), uy = rng->next_unit(), ux = rng->next_unit();
+	int32_t cell; const f3 L = sky_sample_dir(sky, sc.hdri_w, um, uc, uy, ux, &cell);
+	const f3 ll = frame_to_local(sf.T, L);
+	if (ll.z < 0.0f) return false;
+	const int32_t t = sky_texel(sc, L.x, L.y, L.z);
+	const float4 tx = ldg4(sc.hdri + t);
+	const float q = sky.p_sky * ldg_f32(sky.pdf + t), lpdf = sky.p_sky * ldg_f32(sky.pdf + cell);
+	const float f = B2R_INV_PI * sel_max(0.0f, ll.z);  // Closure<Lambertian>::eval and ::pdf
+	f3 rad{(tx.x * sc.ambient[0]) * s.tr, (tx.y * sc.ambient[1]) * s.tg, (tx.z * sc.ambient[2]) * s.tb};
+	rad = f3{rad.x * (sf.albedo.x * f), rad.y * (sf.albedo.y * f), rad.z * (sf.albedo.z * f)};
+	rad = scale3(rad, sky_mis(q, f) / lpdf);
+	if (sel_max(sel_max(rad.x, rad.y), rad.z) <= 0.0f) return false;
+	out->o = sf.P; out->d = L; out->tfar = FLT_MAX; out->L = rad;
+	return true;
+}
+
 // next-event estimation, Renderer.hpp:249-298. Returns false when no shadow ray is produced; a dielectric surface (delta BSDF) never makes one.
-template <bool GGX = false, bool DIELECTRIC = false>
+// SKY (B2R_FLAG_SKY_LIGHT): after u0, u1 and the sphere pick (drawn only when there are sphere lights), one draw chooses the sky when 0 < p_sky < 1
+// (sky when it is < p_sky); the sphere lights keep their estimator with selection pdf (1 - p_sky) / n_lights.
+template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
 B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const PathState& s, int32_t hit_prim,
-                                                   uint32_t acc, uint32_t seed, uint32_t bounce, ShadowRay* out) {
+                                                   uint32_t acc, uint32_t seed, uint32_t bounce, ShadowRay* out, const SkyDev& sky = SkyDev{}) {
 	if (is_dielectric<DIELECTRIC>(sf)) return false;
-	if (sc.n_lights == 0u) return false;  // undefined in the reference (Q15); defined here as "no light sampling"
+	if (sc.n_lights == 0u && !(SKY && sky.p_sky > 0.0f)) return false;  // undefined in the reference (Q15); defined here as "no light sampling"
 	Pcg rng{hash_2d(acc, seed + bounce * 2u)};  // Q3
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
-	const uint32_t pick = rng.next_below(sc.n_lights);
+	const uint32_t pick = (!SKY || sc.n_lights != 0u) ? rng.next_below(sc.n_lights) : 0u;
+	if (SKY && (sky.p_sky >= 1.0f || (sky.p_sky > 0.0f && rng.next_unit() < sky.p_sky))) return sky_light_sample(sc, sky, sf, s, &rng, out);
 	const float4 ls = ld4(sc.light_sphere + pick), le = ld4(sc.light_emit + pick);
 	if (as_int(le.w) == hit_prim) return false;  // Q9: geometry index vs BVH-order index, as in the reference
 	f3 wc{ls.x - sf.P.x, ls.y - sf.P.y, ls.z - sf.P.z};
@@ -233,7 +326,7 @@ B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const Path
 		const float f = B2R_INV_PI * sel_max(0.0f, ll.z);  // Closure<Lambertian>::eval, DataStreams.hpp:169-172
 		rad = f3{rad.x * (sf.albedo.x * f), rad.y * (sf.albedo.y * f), rad.z * (sf.albedo.z * f)};
 	}
-	lpdf *= sc.light_sel_pdf;
+	lpdf *= SKY ? sky.light_sel_pdf : sc.light_sel_pdf;
 	const float bpdf = GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, ll.z);  // Closure<GGX>::pdf is `return 0.0f; //TODO` in the reference (:196-198)
 	const float w = power_heuristic_over_f(lpdf, bpdf);
 	rad = scale3(rad, w);
@@ -242,22 +335,24 @@ B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const Path
 	return true;
 }
 // emissive-hit contribution, Renderer.hpp:319-353. DIELECTRIC: a path continued from a dielectric surface carries pdf = -1 (no light sample
-// competes with a delta BSDF), and its MIS weight is 1.
-template <bool DIELECTRIC = false>
-B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState& s, float depth, uint32_t bounce, bool mis) {
+// competes with a delta BSDF), and its MIS weight is 1. SKY: the sphere's selection pdf is SkyDev::light_sel_pdf.
+template <bool DIELECTRIC = false, bool SKY = false>
+B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState& s, float depth, uint32_t bounce, bool mis, const SkyDev& sky = SkyDev{}) {
 	const float4 em = ld4(sc.mat_emission + sf.mat);
 	if (!mis) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};  // this repo's MIS-off (Q23)
 	if (bounce == 0) return f3{em.x, em.y, em.z};
 	if (DIELECTRIC && s.pdf < 0.0f) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};
 	const float d2 = depth * (depth + sf.n_dot_v * (2.0f * sqrtf(sf.r2))) + sf.r2;  // law of cosines, Renderer.hpp:331
-	const float w = power_heuristic(s.pdf, sc.light_sel_pdf * sphere_light_pdf(sf.r2, d2));
+	const float w = power_heuristic(s.pdf, (SKY ? sky.light_sel_pdf : sc.light_sel_pdf) * sphere_light_pdf(sf.r2, d2));
 	return f3{(s.tr * w) * em.x, (s.tg * w) * em.y, (s.tb * w) * em.z};
 }
 // BRDF sampling + Russian roulette, Renderer.hpp:359-403. Returns false when the path is terminated by roulette. A dielectric surface
 // (DIELECTRIC) reflects or refracts by the stream's first float (dielectric_scatter; the second is unused, roulette keeps the third), a
 // refraction scales the throughput by the transmission and leaves from P_in, and the path stores pdf = -1 (specular predecessor).
-template <bool GGX = false, bool DIELECTRIC = false>
-B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32_t seed, uint32_t bounce) {
+// SKY with p_sky > 0 (the sky is sampled): the path stores the true pdf of the sampled direction, 1/pi times its LOCAL cosine, instead of Q10's
+// world-space one: the sky's MIS weights need the density the direction was drawn with, and the emissive-hit weight then reads it too.
+template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
+B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32_t seed, uint32_t bounce, const SkyDev& sky = SkyDev{}) {
 	Pcg rng{hash_2d(acc, seed + bounce * 2u + 1u)};
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
 	f3 dl, est = sf.albedo, o = sf.P;
@@ -276,14 +371,19 @@ B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32
 	const f3 dw = frame_to_world(sf.T, dl);
 	s->ox = o.x; s->oy = o.y; s->oz = o.z; s->dx = dw.x; s->dy = dw.y; s->dz = dw.z;
 	s->tr = thr.x; s->tg = thr.y; s->tb = thr.z;
-	s->pdf = delta ? -1.0f : GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
+	s->pdf = delta ? -1.0f : GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, (SKY && sky.p_sky > 0.0f) ? dl.z : dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
 	return true;
 }
-// miss shader with ambient sky, Renderer.hpp:411-420 + Sky::operator(), Primitives.hpp:35-46
-B2R_HD f3 shade_sky(const SceneDev& sc, const PathState& s) {
-	const float u = sc.hdri_fw * (0.5f + B2R_INV_TWO_PI * atan2_poly(s.dz, s.dx));
-	const float v = sc.hdri_fh * (0.5f - B2R_INV_PI * asin_poly(s.dy));
-	const float4 tx = ldg4(sc.hdri + (static_cast<int32_t>(v) * sc.hdri_w + static_cast<int32_t>(u)));
+// miss shader with ambient sky, Renderer.hpp:411-420 + Sky::operator(), Primitives.hpp:35-46. SKY (B2R_FLAG_SKY_LIGHT): per channel, tr * L(d) * w
+// with w = sky_mis(pdf, q(d)) against the sky's light samples, and w = 1 for a camera ray and behind a dielectric (pdf < 0) or without sky sampling.
+template <bool SKY = false>
+B2R_HD f3 shade_sky(const SceneDev& sc, const PathState& s, uint32_t bounce = 0u, const SkyDev& sky = SkyDev{}) {
+	const int32_t t = sky_texel(sc, s.dx, s.dy, s.dz);
+	const float4 tx = ldg4(sc.hdri + t);
+	if (SKY) {
+		const float w = (bounce == 0u || s.pdf < 0.0f || sky.p_sky <= 0.0f) ? 1.0f : sky_mis(s.pdf, sky.p_sky * ldg_f32(sky.pdf + t));
+		return f3{(s.tr * (tx.x * sc.ambient[0])) * w, (s.tg * (tx.y * sc.ambient[1])) * w, (s.tb * (tx.z * sc.ambient[2])) * w};
+	}
 	// Q14: all three channels are scaled by throughput.r
 	return f3{s.tr * (tx.x * sc.ambient[0]), s.tr * (tx.y * sc.ambient[1]), s.tr * (tx.z * sc.ambient[2])};
 }

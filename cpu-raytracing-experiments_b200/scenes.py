@@ -172,3 +172,23 @@ def bvh_test_scene(n=255, hdri=None):
     sc["ambient"] = (1.0, 1.0, 1.0)
     sc["hdri"] = synthetic_hdri() if hdri is None else hdri
     return sc
+
+
+def sun_hdri(width=2048, height=1024, sun_dir=(0.35, 0.8, -0.48), sun_radius_deg=1.0, sun_radiance=1.0e4):
+    """Deterministic equirect RGBA32F sky with a sun: a disk of `sun_radiance` (warm white) of angular radius `sun_radius_deg` around `sun_dir`
+    over a dim coloured sky (horizon about 0.3, zenith a deeper blue, ground 0.05). Texel (i, j) is evaluated in the direction the miss
+    shader's lookup shows it at (longitude 2 pi ((i + 0.5) / (w - 1) - 0.5), latitude pi (0.5 - (j + 0.5) / (h - 1))), so almost all of the
+    energy sits in a few dozen texels: the case a cosine-sampled bounce finds rarely (B2R_FLAG_SKY_LIGHT)."""
+    i = (np.arange(width, dtype=np.float64) + 0.5) / max(width - 1, 1)
+    j = (np.arange(height, dtype=np.float64) + 0.5) / max(height - 1, 1)
+    phi = 2.0 * np.pi * (i - 0.5); lat = np.pi * (0.5 - j)
+    dy = np.sin(lat)[:, None] * np.ones((1, width)); r = np.cos(lat)[:, None]
+    dx = r * np.cos(phi)[None, :]; dz = r * np.sin(phi)[None, :]
+    up = np.clip(dy, 0.0, 1.0)[..., None]
+    sky = (1.0 - up) * np.array([0.30, 0.32, 0.36]) + up * np.array([0.06, 0.10, 0.24])
+    sky = np.where((dy < 0.0)[..., None], np.array([0.05, 0.045, 0.04]), sky)
+    s = np.asarray(sun_dir, np.float64); s = s / np.linalg.norm(s)
+    in_sun = dx * s[0] + dy * s[1] + dz * s[2] >= np.cos(np.radians(sun_radius_deg))
+    sky = np.where(in_sun[..., None], sun_radiance * np.array([1.0, 0.95, 0.85]), sky)
+    img = np.ones((height, width, 4), np.float32); img[..., :3] = sky
+    return np.ascontiguousarray(img, np.float32)

@@ -81,6 +81,21 @@ enum {
 	                                    * with B2R_FLAG_GGX, not with B2R_FLAG_REFERENCE_EXACT. With the flag, b2r_upload_scene, b2r_refit_scene and
 	                                    * b2r_set_flags refuse (B2R_ERR_ARG) a non-finite transmission, and a dielectric with a transmission outside [0, 1]
 	                                    * or an eta that is not finite or is < 1. A checkpoint does not load across the flag (b2r_load_checkpoint: B2R_ERR_STATE). */
+	B2R_FLAG_SKY_LIGHT = 1u << 13,     /* samples the HDRI sky as a light (next-event estimation), combined with the BSDF-sampled misses by the power
+	                                    * heuristic, in both pipelines (DESIGN.md §2). The sky is cut into the miss shader's cells, max(w-1,1) x max(h-1,1),
+	                                    * drawn with probability ~ solid angle * (luminance of texel * ambient + its mean / 64) and uniformly in solid angle
+	                                    * inside a cell; a light sample goes to the sky with probability 1 without sphere lights, 1/2 with them (a sphere
+	                                    * light then has selection pdf 1 / (2 n_lights)). Lambertian surfaces only; a sample below the surface's horizon
+	                                    * is dropped. The miss shader's contribution is per channel (quirk Q14 does not apply), and the path record then
+	                                    * carries the local-cosine pdf of its direction (quirk Q10 does not apply). Quirk Q11 (a path that still hits at the
+	                                    * last bounce loses its radiance) then also drops the sky's light samples of its earlier bounces, which without the
+	                                    * flag never happens to sky light (it arrives only at a miss): at a finite max_bounces the flag-on image is lower in
+	                                    * expectation by the energy those paths had gathered from the sky (DESIGN.md §2). Without a sky (ambient 0, or a texture
+	                                    * that is zero everywhere) frames equal those without the flag. The sky's tables are built on the device at
+	                                    * b2r_upload_scene, or when b2r_set_flags turns the flag on (b2r_read_sky_tables reads them). Combines with a lens
+	                                    * and B2R_FLAG_DIELECTRIC; B2R_ERR_ARG with B2R_FLAG_REFERENCE_EXACT, B2R_FLAG_NO_MIS or B2R_FLAG_GGX, at b2r_create
+	                                    * and b2r_set_flags. With the flag, b2r_upload_scene and b2r_set_flags refuse (B2R_ERR_ARG) a sky texel that is not
+	                                    * finite, or negative, in a channel whose ambient is > 0. A checkpoint does not load across the flag. */
 };
 
 typedef struct b2r_config {
@@ -284,6 +299,10 @@ int  b2r_read_wide_nodes(b2r_ctx* ctx, void* out_host, uint32_t* n_wide_nodes, u
 /* the link tables k_link_tables derives from the device tree: parent_out[n_wide_nodes] (the node that links to node i, 0 for the root)
  * and leaf_node_out[n_prims] (the node whose leaf slot holds sphere i, BVH order). Synchronises. */
 int  b2r_read_link_tables(b2r_ctx* ctx, uint32_t* parent_out, uint32_t* leaf_node_out);
+/* B2R_FLAG_SKY_LIGHT: the sky's tables as the device built them. *cols_out = W' = max(w-1,1), *rows_out = H' = max(h-1,1); marginal_out[H'+1]
+ * (CDF over the rows), conditional_out[H'][W'+1] (CDF over the cells of each row), pdf_out[h][w] (solid-angle pdf of the cell each texel shows,
+ * without the sky's selection probability). A null table pointer skips that table. B2R_ERR_STATE when no tables are built. Synchronises. */
+int  b2r_read_sky_tables(b2r_ctx* ctx, float* marginal_out, float* conditional_out, float* pdf_out, uint32_t* cols_out, uint32_t* rows_out);
 /* the box ray origins are assumed to lie in ({lo.xyz, hi.xyz}: sphere bounds, camera, origins passed to b2r_trace_*): the leaf slots of the
  * traversal tree are sized for it, so a host twin of the tree needs the same box (tests) */
 int  b2r_get_origin_box(b2r_ctx* ctx, float lo_hi_out[6]);
