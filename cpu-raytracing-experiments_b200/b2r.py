@@ -30,6 +30,7 @@ FLAG_GPU_SAH3 = 2048  # with FLAG_GPU_TREE: the three-axis sweep tree (full-swee
 FLAG_GGX = 512  # the reference's `#define BRDF 1` closure (Closure<GGX>, DataStreams.hpp:184-219)
 FLAG_DIELECTRIC = 4096  # materials with max(transmission) > 0 render as smooth dielectrics of IOR 1 + IOR_minus_one (DESIGN.md §2)
 FLAG_SKY_LIGHT = 8192  # the HDRI sky sampled as a light, MIS-combined with the BSDF-sampled misses (DESIGN.md §2)
+FLAG_LIGHT_TREE = 16384  # sphere lights picked by importance from a light tree instead of uniformly (DESIGN.md §2)
 TAP_CLOSEST, TAP_SHADOW, TAP_PACKET = 0, 1, 2  # b2r_trace_kernel: which traversal kernel of a frame runs
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_NO_LIGHTS, ERR_BVH, NOT_READY = 0, -1, -2, -3, -4, -5, 1
 KERNEL_KINDS = ["generate", "bounce_brute", "intersect_closest", "shade", "intersect_shadow", "accumulate", "resolve"]
@@ -40,7 +41,7 @@ ABI_SYMBOLS = [
     "b2r_bvh_build", "b2r_bvh_build_ex", "b2r_find_lights", "b2r_camera_lookat", "b2r_camera_ray", "b2r_create", "b2r_destroy", "b2r_resize", "b2r_reset", "b2r_set_stream",
     "b2r_sync", "b2r_upload_scene", "b2r_refit_scene", "b2r_set_camera", "b2r_set_lens", "b2r_accumulate", "b2r_resolve", "b2r_resolve_async", "b2r_resolve_device", "b2r_frame_wait", "b2r_resolve_from", "b2r_ipc_export_buckets", "b2r_ipc_open_peers", "b2r_ipc_close", "b2r_resolve_peers", "b2r_team_export", "b2r_team_open", "b2r_team_resolve", "b2r_team_error", "b2r_team_close", "b2r_host_register", "b2r_host_unregister", "b2r_get_accumulations", "b2r_set_accumulations",
     "b2r_read_buckets", "b2r_write_buckets", "b2r_save_checkpoint", "b2r_load_checkpoint", "b2r_device_buckets", "b2r_device_framebuffer", "b2r_read_counters", "b2r_reset_counters", "b2r_read_bounce_counts",
-    "b2r_read_kernel_times", "b2r_set_flags", "b2r_generate_rays", "b2r_trace_closest", "b2r_trace_shadow", "b2r_trace_kernel", "b2r_read_wide_nodes", "b2r_read_link_tables", "b2r_read_sky_tables", "b2r_get_origin_box",
+    "b2r_read_kernel_times", "b2r_set_flags", "b2r_generate_rays", "b2r_trace_closest", "b2r_trace_shadow", "b2r_trace_kernel", "b2r_read_wide_nodes", "b2r_read_link_tables", "b2r_read_sky_tables", "b2r_read_light_tree", "b2r_get_origin_box",
     "b2r_write_hdr", "b2r_read_hdr", "b2r_last_error", "b2r_abi_version",
 ]
 
@@ -77,7 +78,7 @@ def lib():
             "b2r_host_register": [vp, C.c_size_t], "b2r_host_unregister": [vp], "b2r_get_accumulations": [vp, vp], "b2r_set_accumulations": [vp, u32], "b2r_read_buckets": [vp, vp], "b2r_write_buckets": [vp, vp],
             "b2r_device_buckets": [vp, vp, vp], "b2r_device_framebuffer": [vp, vp, vp], "b2r_read_counters": [vp, vp], "b2r_reset_counters": [vp], "b2r_read_bounce_counts": [vp, vp, vp, u32],
             "b2r_read_kernel_times": [vp, vp, vp, C.c_int], "b2r_set_flags": [vp, u32], "b2r_generate_rays": [vp, u32, vp],
-            "b2r_save_checkpoint": [vp, C.c_char_p], "b2r_load_checkpoint": [vp, C.c_char_p], "b2r_write_hdr": [C.c_char_p, vp, u32, u32], "b2r_read_hdr": [C.c_char_p, vp, vp, vp], "b2r_trace_closest": [vp, vp, u32, vp, vp], "b2r_trace_shadow": [vp, vp, vp, u32, vp], "b2r_trace_kernel": [vp, C.c_int, vp, vp, vp, vp, u32, u32, vp, vp, vp], "b2r_read_wide_nodes": [vp, vp, vp, vp], "b2r_read_link_tables": [vp, vp, vp], "b2r_read_sky_tables": [vp, vp, vp, vp, vp, vp], "b2r_get_origin_box": [vp, vp],
+            "b2r_save_checkpoint": [vp, C.c_char_p], "b2r_load_checkpoint": [vp, C.c_char_p], "b2r_write_hdr": [C.c_char_p, vp, u32, u32], "b2r_read_hdr": [C.c_char_p, vp, vp, vp], "b2r_trace_closest": [vp, vp, u32, vp, vp], "b2r_trace_shadow": [vp, vp, vp, u32, vp], "b2r_trace_kernel": [vp, C.c_int, vp, vp, vp, vp, u32, u32, vp, vp, vp], "b2r_read_wide_nodes": [vp, vp, vp, vp], "b2r_read_link_tables": [vp, vp, vp], "b2r_read_sky_tables": [vp, vp, vp, vp, vp, vp], "b2r_read_light_tree": [vp, vp, vp, vp], "b2r_get_origin_box": [vp, vp],
         }
         for name, args in sig.items():
             fn = getattr(L, name); fn.argtypes = args; fn.restype = C.c_int
@@ -391,6 +392,15 @@ class Renderer:
         marg = np.empty(rows.value + 1, np.float32); cond = np.empty((rows.value, cols.value + 1), np.float32); pdf = np.empty((h, w), np.float32)
         _check(lib().b2r_read_sky_tables(self._h, _ptr(marg), _ptr(cond), _ptr(pdf), C.byref(cols), C.byref(rows)))
         return marg, cond, pdf
+
+    def read_light_tree(self):
+        """B2R_FLAG_LIGHT_TREE: the light tree as the device holds it (b2r_read_light_tree): (nodes[N][8] float32 = {c.xyz, R^2, E, link, 0, 0}
+        with link an int32 in the float's bits, light_prim[n_lights] int32 = each light's BVH-order sphere)."""
+        n = C.c_uint32(0)
+        _check(lib().b2r_read_light_tree(self._h, None, None, C.byref(n)))
+        nodes = np.empty((n.value, 8), np.float32); light_prim = np.empty(len(self.scene.lights), np.int32)
+        _check(lib().b2r_read_light_tree(self._h, _ptr(nodes), _ptr(light_prim), C.byref(n)))
+        return nodes, light_prim
 
     def wide_nodes(self):
         n = C.c_uint32(0); ms = C.c_uint32(0)

@@ -71,9 +71,12 @@ template <typename T> void dev_free(T** p) { if (*p) { cudaFree(*p); *p = nullpt
 #define B2R_PACKED_TABLES(X) X(float4, prims, LEN_PRIMS) X(int32_t, prim_mat, LEN_PRIMS) X(float4, mat_albedo, LEN_MAT) X(float4, mat_emission, LEN_MAT) \
                              X(float4, mat_f0, LEN_MAT) X(float4, mat_diel, LEN_MAT) X(float4, light_sphere, LEN_LIGHTS) X(float4, light_emit, LEN_LIGHTS)
 #define B2R_SCENE_TABLES(X) B2R_PACKED_TABLES(X) X(WideNode, wide, LEN_WIDE) X(uint32_t, parent, LEN_WIDE) X(uint32_t, leaf_node, LEN_PRIMS) X(float4, hdri, LEN_TEXELS) \
-                            X(float, sky_marg, LEN_SKY_MARG) X(float, sky_cond, LEN_SKY_COND) X(float, sky_pdf, LEN_SKY_PDF)
-// 0 lights: one (zero) light row. LEN_SKY_*: the sky's tables (B2R_FLAG_SKY_LIGHT), 0 while they are not built
-enum TableLen { LEN_PRIMS = 0, LEN_MAT, LEN_LIGHTS, LEN_WIDE, LEN_TEXELS, LEN_SKY_MARG, LEN_SKY_COND, LEN_SKY_PDF, LEN_COUNT };
+                            X(float, sky_marg, LEN_SKY_MARG) X(float, sky_cond, LEN_SKY_COND) X(float, sky_pdf, LEN_SKY_PDF) \
+                            X(float4, ltree_nodes, LEN_LTREE_NODES) X(int4, ltree_light, LEN_LTREE_LIGHTS) X(int32_t, ltree_prim_light, LEN_LTREE_PRIMS)
+// 0 lights: one (zero) light row. LEN_SKY_*: the sky's tables (B2R_FLAG_SKY_LIGHT), LEN_LTREE_*: the light tree's (B2R_FLAG_LIGHT_TREE), 0 while
+// they are not built
+enum TableLen { LEN_PRIMS = 0, LEN_MAT, LEN_LIGHTS, LEN_WIDE, LEN_TEXELS, LEN_SKY_MARG, LEN_SKY_COND, LEN_SKY_PDF, LEN_LTREE_NODES, LEN_LTREE_LIGHTS, LEN_LTREE_PRIMS,
+                LEN_COUNT };
 struct SceneTables {
 	template <typename T> struct Table { T* p = nullptr; size_t cap = 0; };
 #define X(T, name, len) Table<T> name;
@@ -97,6 +100,7 @@ void bind_tables(Params& p, const SceneTables& t, bool sky) {
 	s.hdri = sky ? t.hdri.p : nullptr;
 	p.mat_diel = t.mat_diel.p;
 	p.sky.marg = t.sky_marg.p; p.sky.cond = t.sky_cond.p; p.sky.pdf = t.sky_pdf.p;
+	p.ltree.nodes = t.ltree_nodes.p; p.ltree.light = t.ltree_light.p; p.ltree.prim_light = t.ltree_prim_light.p;
 }
 
 // One launch of a batch's rounds: the kernel instantiation, its block size and its grid (kernels_of).
@@ -104,7 +108,7 @@ template <typename F> struct Role { F fn = nullptr; int block = 0, grid = 0; };
 using BounceKernel = void (*)(const Params, const uint32_t);
 struct KernelSet { Role<BounceKernel> brute_first, brute, brute_finish, packet, closest, shade, shadow; Role<void (*)(const Params)> generate; };
 // The bits of the key that selects a KernelSet (kernels_of).
-enum : uint32_t { KEY_COUNT = 1, KEY_EXACT = 2, KEY_GGX = 4, KEY_LENS = 8, KEY_DIEL = 16, KEY_TN16 = 32, KEY_SKY = 64, KEYS = 128 };
+enum : uint32_t { KEY_COUNT = 1, KEY_EXACT = 2, KEY_GGX = 4, KEY_LENS = 8, KEY_DIEL = 16, KEY_TN16 = 32, KEY_SKY = 64, KEY_LTREE = 128, KEYS = 256 };
 
 // A stream the batches are traced on (the caller's, or a side's) and what a batch's lanes add to it: lane j > 0 runs on lane_stream[j],
 // forked from the stream by ev_fork and joined back by ev_join[j]; one captured graph per lane count (index = lanes).
@@ -139,6 +143,9 @@ struct b2r_ctx {
 	// B2R_FLAG_SKY_LIGHT: whether the current sky's texels were checked (sky_texels_valid: only under the flag, or when it is turned on), passed,
 	// and are not zero everywhere; whether the sky's tables in `tables` are built for the current sky; the build's scratch
 	bool sky_checked = false, sky_valid = true, sky_nonzero = false, sky_built = false; double* d_sky_tmp = nullptr; size_t cap_sky_tmp = 0;
+	// B2R_FLAG_LIGHT_TREE: the current light list (geometry[light_geom_idx[i]] and its mean emission, kept so that b2r_set_flags can build the
+	// tree later), whether it follows the input rule (light_list_valid), and whether the tree's tables in `tables` are built for the current scene
+	std::vector<b2r_sphere> lt_lights; std::vector<float> lt_lum; bool lt_valid = true, lt_built = false; uint32_t lt_nodes = 0;
 	WideBvh wide_host; uint64_t wide_key = 0; std::vector<unsigned char> wide_blob; bool have_wide = false;
 	uint32_t n_wide = 0;  // wide nodes of the current tree
 	// B2R_FLAG_GPU_TREE: the tree was built on the device (no host copy of its nodes); sort scratch; the arrays a later refit needs to match
@@ -300,17 +307,17 @@ template <typename F> int launch(b2r_ctx* c, int kind, bool profile, F&& f) {
 // other trees read the split from the scene.
 template <uint32_t KEY> KernelSet kernel_set() {
 	constexpr bool COUNT = KEY & KEY_COUNT, EXACT = KEY & KEY_EXACT, GGX = KEY & KEY_GGX, LENS = KEY & KEY_LENS, DIEL = KEY & KEY_DIEL, TN16 = KEY & KEY_TN16,
-	               SKY = KEY & KEY_SKY;
-	if constexpr ((EXACT && (GGX || LENS || DIEL)) || (SKY && (EXACT || GGX))) return {};  // refused by b2r_create, b2r_set_flags and b2r_set_lens: nothing instantiated
+	               SKY = KEY & KEY_SKY, LTREE = KEY & KEY_LTREE;
+	if constexpr ((EXACT && (GGX || LENS || DIEL)) || (SKY && (EXACT || GGX)) || (LTREE && EXACT)) return {};  // refused by b2r_create, b2r_set_flags and b2r_set_lens: nothing instantiated
 	else {
-		constexpr bool SHADE_COUNT = COUNT && !GGX && !DIEL && !SKY;
+		constexpr bool SHADE_COUNT = COUNT && !GGX && !DIEL && !SKY && !LTREE;
 		KernelSet k;
-		k.brute_first = {k_bounce_brute<true, SHADE_COUNT, EXACT, GGX, LENS, DIEL, SKY>, kBruteBlock};
-		k.brute = {k_bounce_brute<false, SHADE_COUNT, EXACT, GGX, false, DIEL, SKY>, kBruteBlock};
-		k.brute_finish = {k_brute_finish<SHADE_COUNT, GGX, DIEL, SKY>, kBruteBlock};
+		k.brute_first = {k_bounce_brute<true, SHADE_COUNT, EXACT, GGX, LENS, DIEL, SKY, LTREE>, kBruteBlock};
+		k.brute = {k_bounce_brute<false, SHADE_COUNT, EXACT, GGX, false, DIEL, SKY, LTREE>, kBruteBlock};
+		k.brute_finish = {k_brute_finish<SHADE_COUNT, GGX, DIEL, SKY, LTREE>, kBruteBlock};
 		k.packet = {k_intersect_packet<COUNT, LENS ? B2R_PACKET_RPL_LENS : B2R_PACKET_RPL, LENS>, kTravBlock};
 		k.closest = {k_intersect_closest<COUNT, EXACT, TN16 ? 16u : 0u>, kTravBlock};
-		k.shade = {k_shade<EXACT, GGX, DIEL, SKY>, kBruteBlock};
+		k.shade = {k_shade<EXACT, GGX, DIEL, SKY, LTREE>, kBruteBlock};
 		k.shadow = {k_intersect_shadow<COUNT>, kTravBlock};
 		k.generate = {k_generate<LENS>, kBlock};
 		return k;
@@ -327,7 +334,7 @@ int kernels_of(b2r_ctx* c, const KernelSet** out) {
 	const bool exact = (f & B2R_FLAG_REFERENCE_EXACT) != 0;
 	const uint32_t key = ((f & B2R_FLAG_COUNT_TESTS) ? KEY_COUNT : 0u) | (exact ? KEY_EXACT : 0u) | ((f & B2R_FLAG_GGX) ? KEY_GGX : 0u) |
 	                     (c->lens.radius > 0.0f && !exact ? KEY_LENS : 0u) | ((f & B2R_FLAG_DIELECTRIC) ? KEY_DIEL : 0u) | (c->params.scene.stack_tn_bits == 16u ? KEY_TN16 : 0u) |
-	                     ((f & B2R_FLAG_SKY_LIGHT) ? KEY_SKY : 0u);
+	                     ((f & B2R_FLAG_SKY_LIGHT) ? KEY_SKY : 0u) | ((f & B2R_FLAG_LIGHT_TREE) ? KEY_LTREE : 0u);
 	KernelSet& k = c->kernels[key];
 	if (!k.shade.fn) {
 		KernelSet s = kernel_set(key, std::make_integer_sequence<uint32_t, KEYS>());
@@ -594,7 +601,8 @@ int refresh_side_scene(b2r_ctx* c, uint32_t sidx) {
 	}
 	if (c->uploaded_valid) CU(cudaStreamWaitEvent(S.stream, c->ev_uploaded, 0));
 	const size_t len[LEN_COUNT] = {sc.n_prims, sc.n_mat, sc.n_lights ? sc.n_lights : 1u, c->n_wide, sc.hdri ? c->hdri_texels : 0u, c->sky_built ? c->params.sky.rows + 1u : 0u,
-	                               c->sky_built ? static_cast<size_t>(c->params.sky.rows) * (c->params.sky.cols + 1u) : 0u, c->sky_built ? c->hdri_texels : 0u};
+	                               c->sky_built ? static_cast<size_t>(c->params.sky.rows) * (c->params.sky.cols + 1u) : 0u, c->sky_built ? c->hdri_texels : 0u,
+	                               c->lt_built ? 2u * static_cast<size_t>(c->lt_nodes) : 0u, c->lt_built ? sc.n_lights : 0u, c->lt_built ? sc.n_prims : 0u};
 	const int rc = SceneTables::for_each([&](int l, auto& s, const auto& m) -> int {
 		const size_t bytes = len[l] * sizeof(*m.p);
 		if (bytes) CU(cudaMemcpyAsync(s.p, m.p, bytes, cudaMemcpyDeviceToDevice, S.stream));
@@ -760,12 +768,13 @@ const char* sky_flag_conflict(uint32_t flags) {
 }
 // whether `flags` sample the current sky: a sky (ambient > 0) whose texels are not zero everywhere
 bool sky_sampled(const b2r_ctx* c, uint32_t flags) { return (flags & B2R_FLAG_SKY_LIGHT) && c->params.scene.has_ambient && c->sky_nonzero; }
-// SkyDev's scalars for the context's flags and scene (the tables' pointers are bound with the others)
+// SkyDev's scalars and LightTreeDev::sel_scale for the context's flags and scene (the tables' pointers are bound with the others)
 void set_sky_scalars(b2r_ctx* c) {
 	SkyDev& k = c->params.sky; const SceneDev& s = c->params.scene;
 	k.p_sky = !sky_sampled(c, c->cfg.flags) ? 0.0f : s.n_lights == 0u ? 1.0f : 0.5f;
 	k.light_sel_pdf = s.n_lights ? (1.0f - k.p_sky) / static_cast<float>(s.n_lights) : 0.0f;
 	k.cols = s.hdri_w > 1 ? static_cast<uint32_t>(s.hdri_w - 1) : 1u; k.rows = s.hdri_h > 1 ? static_cast<uint32_t>(s.hdri_h - 1) : 1u;
+	c->params.ltree.sel_scale = s.n_lights ? 1.0f - k.p_sky : 0.0f;  // (B2R_FLAG_LIGHT_TREE)
 }
 // lengths of the sky's tables for a w x h texture (reserve_tables)
 void sky_table_lens(int32_t w, int32_t h, size_t (&len)[LEN_COUNT]) {
@@ -791,6 +800,32 @@ int launch_sky_build(b2r_ctx* c, int32_t w, int32_t h, const float amb[3]) {
 }
 constexpr const char* kSkyInvalid = "B2R_FLAG_SKY_LIGHT: a sky texel is not finite, or negative, in a channel whose ambient is > 0";
 
+struct UploadPart { void* dst; const void* src; size_t bytes; };
+int stage_upload(b2r_ctx* c, const UploadPart* parts, size_t n_parts);
+
+// B2R_FLAG_LIGHT_TREE (DESIGN §2): the flags it cannot be combined with (null: none)
+const char* light_tree_flag_conflict(uint32_t flags) {
+	if (!(flags & B2R_FLAG_LIGHT_TREE)) return nullptr;
+	if (flags & B2R_FLAG_REFERENCE_EXACT) return "B2R_FLAG_LIGHT_TREE cannot be combined with B2R_FLAG_REFERENCE_EXACT";
+	if (flags & B2R_FLAG_NO_MIS) return "B2R_FLAG_LIGHT_TREE cannot be combined with B2R_FLAG_NO_MIS (there is no light sampling to pick lights for)";
+	return nullptr;
+}
+constexpr const char* kLightsInvalid = "B2R_FLAG_LIGHT_TREE: a light index appears twice, two lights are equal spheres, or a light's emission is not finite or is negative";
+// The light list of a scene write, kept for a tree build by a later b2r_set_flags: geometry[light_geom_idx[i]] and its material's mean emission
+void keep_light_list(b2r_ctx* c, const b2r_material* materials, const int32_t* light_geom_idx, uint32_t n_lights, const b2r_sphere* geometry, bool valid) {
+	c->lt_lights.resize(n_lights); c->lt_lum.resize(n_lights); c->lt_valid = valid;
+	for (uint32_t i = 0; i < n_lights; i++) {
+		c->lt_lights[i] = geometry[light_geom_idx[i]];
+		const float* e = materials[c->lt_lights[i].material_ID].emission;
+		c->lt_lum[i] = ((e[0] + e[1]) + e[2]) / 3.0f;
+	}
+}
+// The light tree of the kept light list over the BVH-order spheres, and the lengths of its tables (reserve_tables)
+void build_kept_light_tree(const b2r_ctx* c, const float4* prims, const int32_t* prim_mat, uint32_t n_prims, LightTree& lt, size_t (&len)[LEN_COUNT]) {
+	build_light_tree(c->lt_lights.data(), c->lt_lum.data(), static_cast<uint32_t>(c->lt_lights.size()), prims, prim_mat, n_prims, lt);
+	len[LEN_LTREE_NODES] = lt.nodes.size(); len[LEN_LTREE_LIGHTS] = lt.light.size(); len[LEN_LTREE_PRIMS] = lt.prim_light.size();
+}
+
 }  // namespace
 
 // ================================================================================================ C ABI
@@ -812,6 +847,7 @@ int b2r_create(b2r_ctx** out, const b2r_config* cfg) {
 	if ((cfg->flags & B2R_FLAG_GGX) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_GGX cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if ((cfg->flags & B2R_FLAG_DIELECTRIC) && (cfg->flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if (const char* why = sky_flag_conflict(cfg->flags)) return fail(B2R_ERR_ARG, why);
+	if (const char* why = light_tree_flag_conflict(cfg->flags)) return fail(B2R_ERR_ARG, why);
 	int n_dev = 0;
 	cudaError_t e = cudaGetDeviceCount(&n_dev);
 	if (e != cudaSuccess || n_dev == 0) return fail(B2R_ERR_CUDA, std::string("no CUDA device: ") + cudaGetErrorString(e) + " (libb2r has no CPU fallback)");
@@ -914,6 +950,8 @@ int b2r_set_flags(b2r_ctx* c, uint32_t flags) {
 	if ((flags & B2R_FLAG_DIELECTRIC) && (flags & B2R_FLAG_REFERENCE_EXACT)) return fail(B2R_ERR_ARG, "B2R_FLAG_DIELECTRIC cannot be combined with B2R_FLAG_REFERENCE_EXACT");
 	if ((flags & B2R_FLAG_DIELECTRIC) && c->have_scene && !c->scene_diel_valid) return fail(B2R_ERR_ARG, kDielInvalid);
 	if (const char* why = sky_flag_conflict(flags)) return fail(B2R_ERR_ARG, why);
+	if (const char* why = light_tree_flag_conflict(flags)) return fail(B2R_ERR_ARG, why);
+	if ((flags & B2R_FLAG_LIGHT_TREE) && c->have_scene && !c->lt_valid) return fail(B2R_ERR_ARG, kLightsInvalid);
 	const SceneDev& sc = c->params.scene;
 	if ((flags & B2R_FLAG_SKY_LIGHT) && c->have_scene && sc.has_ambient && !c->sky_checked) {  // uploaded without the flag: the rule is checked on the texels now
 		std::vector<float4> tex(c->hdri_texels);
@@ -925,6 +963,17 @@ int b2r_set_flags(b2r_ctx* c, uint32_t flags) {
 		size_t len[LEN_COUNT] = {}; sky_table_lens(sc.hdri_w, sc.hdri_h, len);
 		if ((rc = reserve_tables(c, len)) || (rc = begin_scene_write(c, use_sides(c))) || (rc = launch_sky_build(c, sc.hdri_w, sc.hdri_h, sc.ambient)) || (rc = end_scene_write(c))) return rc;
 		c->sky_built = true; bind_tables(c->params, c->tables, sc.hdri != nullptr);
+	}
+	if ((flags & B2R_FLAG_LIGHT_TREE) && c->have_scene && !c->lt_built) {  // turned on over a scene: the tree, over the device's BVH-order spheres
+		std::vector<float4> prims(sc.n_prims); std::vector<int32_t> prim_mat(sc.n_prims);
+		CU(cudaMemcpyAsync(prims.data(), c->tables.prims.p, prims.size() * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+		CU(cudaMemcpyAsync(prim_mat.data(), c->tables.prim_mat.p, prim_mat.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream)); CU(sync_main(c));
+		LightTree lt; size_t len[LEN_COUNT] = {}; build_kept_light_tree(c, prims.data(), prim_mat.data(), sc.n_prims, lt, len);
+		if ((rc = reserve_tables(c, len)) || (rc = begin_scene_write(c, use_sides(c)))) return rc;
+		const UploadPart parts[] = {{c->tables.ltree_nodes.p, lt.nodes.data(), lt.nodes.size() * sizeof(float4)}, {c->tables.ltree_light.p, lt.light.data(), lt.light.size() * sizeof(int4)},
+		                            {c->tables.ltree_prim_light.p, lt.prim_light.data(), lt.prim_light.size() * sizeof(int32_t)}};
+		if ((rc = stage_upload(c, parts, 3)) || (rc = end_scene_write(c))) return rc;
+		c->lt_built = true; c->lt_nodes = static_cast<uint32_t>(lt.nodes.size() / 2u); bind_tables(c->params, c->tables, sc.hdri != nullptr);
 	}
 	c->cfg.flags = flags; c->params.frame.flags = flags;
 	set_sky_scalars(c);
@@ -941,7 +990,6 @@ namespace {
 // Host arrays -> device through ONE page-locked block, without stream synchronisation: the copies are ordered after the kernels
 // already enqueued (which may still read the old scene) and before the ones enqueued next; the block is only rewritten once the
 // previous upload's copies have completed (an event early in the previous frame, not its end).
-struct UploadPart { void* dst; const void* src; size_t bytes; };
 int stage_upload(b2r_ctx* c, const UploadPart* parts, size_t n_parts) {
 	size_t total = 0; for (size_t i = 0; i < n_parts; i++) total += (parts[i].bytes + 255) & ~static_cast<size_t>(255);
 	if (c->stage_busy) { CU(cudaEventSynchronize(c->ev_stage)); c->stage_busy = false; }
@@ -1007,6 +1055,9 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	bool sky_nonzero = false;
 	if (sky_checked && !sky_texels_valid(reinterpret_cast<const float4*>(hdri_rgba), static_cast<size_t>(hdri_w) * hdri_h, amb, &sky_nonzero)) return fail(B2R_ERR_ARG, kSkyInvalid);
 	const bool sky_build = sky_checked && sky_nonzero;
+	// B2R_FLAG_LIGHT_TREE: the input rule on the light list, refused here under the flag (otherwise when b2r_set_flags turns it on)
+	const bool lt_build = (c->cfg.flags & B2R_FLAG_LIGHT_TREE) != 0, lt_valid = light_list_valid(materials, light_geom_idx, n_lights, geometry);
+	if (lt_build && !lt_valid) return fail(B2R_ERR_ARG, kLightsInvalid);
 	if ((rc = ensure_device(c))) return rc;
 	// No stream synchronisation from here on: the copies below are ordered after the kernels already enqueued on the stream (which
 	// may still read the old scene) and before the ones enqueued next. The host side is staged in one page-locked block that is only
@@ -1065,11 +1116,15 @@ int b2r_upload_scene(b2r_ctx* c, const b2r_sphere* prims, const b2r_bvh_node* no
 	const size_t texels = has_ambient ? static_cast<size_t>(hdri_w) * hdri_h : 0;
 	size_t len[LEN_COUNT] = {n_prims, n_mat, ps.light_sphere.size(), c->n_wide, texels, 0, 0, 0};  // (no sky: the sky's tables are left alone)
 	if (sky_build) sky_table_lens(hdri_w, hdri_h, len);
+	keep_light_list(c, materials, light_geom_idx, n_lights, geometry, lt_valid);
+	LightTree lt; if (lt_build) build_kept_light_tree(c, ps.prims.data(), ps.prim_mat.data(), n_prims, lt, len);
 	if ((rc = reserve_tables(c, len))) return rc;
 	const bool bvh_next = (c->cfg.flags & B2R_FLAG_FORCE_BVH) ? true : (c->cfg.flags & B2R_FLAG_FORCE_BRUTE) ? false : n_prims > 32;
 	if ((rc = begin_scene_write(c, sides_for(c, bvh_next)))) return rc;
-	if ((rc = stage_packed(c, ps, {{c->tables.wide.p, c->wide_host.nodes.data(), gpu_tree ? 0 : c->wide_host.nodes.size() * sizeof(WideNode)}, {c->tables.hdri.p, hdri_rgba, texels * sizeof(float4)}}))) return rc;
-	c->hdri_texels = texels;
+	if ((rc = stage_packed(c, ps, {{c->tables.wide.p, c->wide_host.nodes.data(), gpu_tree ? 0 : c->wide_host.nodes.size() * sizeof(WideNode)}, {c->tables.hdri.p, hdri_rgba, texels * sizeof(float4)},
+	                               {c->tables.ltree_nodes.p, lt.nodes.data(), lt.nodes.size() * sizeof(float4)}, {c->tables.ltree_light.p, lt.light.data(), lt.light.size() * sizeof(int4)},
+	                               {c->tables.ltree_prim_light.p, lt.prim_light.data(), lt.prim_light.size() * sizeof(int32_t)}}))) return rc;
+	c->hdri_texels = texels; c->lt_built = lt_build; c->lt_nodes = static_cast<uint32_t>(lt.nodes.size() / 2u);
 	if (sky_build && (rc = launch_sky_build(c, hdri_w, hdri_h, amb))) return rc;
 	c->sky_built = sky_build; c->sky_checked = sky_checked; c->sky_valid = true; c->sky_nonzero = sky_nonzero;
 	c->wide_refit = false; c->cur_geom_of_prim.clear(); drop_speculation(c);
@@ -1120,6 +1175,8 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	if (n_lights && !light_geom_idx) return fail(B2R_ERR_ARG, "null light list");
 	bool diel_valid = true;
 	int rc = check_scene_refs(c, prims, geometry, n_prims, n_geom, materials, n_mat, light_geom_idx, n_lights, &diel_valid); if (rc) return rc;
+	const bool lt_build = (c->cfg.flags & B2R_FLAG_LIGHT_TREE) != 0, lt_valid = light_list_valid(materials, light_geom_idx, n_lights, geometry);
+	if (lt_build && !lt_valid) return fail(B2R_ERR_ARG, kLightsInvalid);
 	if ((rc = ensure_device(c))) return rc;
 	// The caller may have re-sorted its prims (the reference's constructor does on every rebuild, BVH.hpp:201-205): leaf links become
 	// indices into the NEW order. old index -> geometry index (known from the last upload / refit) -> new index (matched by value).
@@ -1142,11 +1199,16 @@ int b2r_refit_scene(b2r_ctx* c, const b2r_sphere* prims, uint32_t n_prims, const
 	}
 	PackedScene ps; pack_scene(prims, n_prims, materials, n_mat, light_geom_idx, n_lights, geometry, ps);
 	if ((rc = dev_reserve(&c->d_remap, &c->cap_remap, remap.size()))) return rc;
-	const size_t len[LEN_COUNT] = {0, n_mat, ps.light_sphere.size(), 0, 0, 0, 0, 0};  // the sphere count is kept: only the (small) material and light tables can grow
+	size_t len[LEN_COUNT] = {0, n_mat, ps.light_sphere.size(), 0, 0, 0, 0, 0};  // the sphere count is kept: only the (small) material and light tables can grow
+	keep_light_list(c, materials, light_geom_idx, n_lights, geometry, lt_valid);
+	LightTree lt; if (lt_build) build_kept_light_tree(c, ps.prims.data(), ps.prim_mat.data(), n_prims, lt, len);  // (the light list, and perhaps the BVH order, changed)
 	if ((rc = reserve_tables(c, len))) return rc;
 	if (!c->d_cost) { size_t cap = 0; if ((rc = dev_reserve(&c->d_cost, &cap, 1))) return rc; }
 	if ((rc = begin_scene_write(c, use_sides(c)))) return rc;
-	if ((rc = stage_packed(c, ps, {{c->d_remap, remap.data(), remap.size() * sizeof(uint32_t)}}))) return rc;
+	if ((rc = stage_packed(c, ps, {{c->d_remap, remap.data(), remap.size() * sizeof(uint32_t)},
+	                               {c->tables.ltree_nodes.p, lt.nodes.data(), lt.nodes.size() * sizeof(float4)}, {c->tables.ltree_light.p, lt.light.data(), lt.light.size() * sizeof(int4)},
+	                               {c->tables.ltree_prim_light.p, lt.prim_light.data(), lt.prim_light.size() * sizeof(int32_t)}}))) return rc;
+	c->lt_built = lt_build; c->lt_nodes = static_cast<uint32_t>(lt.nodes.size() / 2u);
 	if (!same_order) c->cur_geom_of_prim.swap(new_geom);
 	// boxes bottom-up on the device, for an origin box that holds the moved spheres
 	{
@@ -1503,7 +1565,7 @@ int b2r_write_buckets(b2r_ctx* c, const float* in_host) {
 namespace {
 struct CheckpointHeader { char magic[8]; uint32_t width, height, buckets, max_bounces, accumulations, result_flags; uint64_t payload_hash; uint64_t payload_bytes; uint32_t reserved[4]; };
 static_assert(sizeof(CheckpointHeader) == 64, "checkpoint header");
-constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT | B2R_FLAG_DIELECTRIC | B2R_FLAG_SKY_LIGHT;  // flags that change which image is being accumulated
+constexpr uint32_t kResultFlags = B2R_FLAG_NO_MIS | B2R_FLAG_REFERENCE_EXACT | B2R_FLAG_DIELECTRIC | B2R_FLAG_SKY_LIGHT | B2R_FLAG_LIGHT_TREE;  // flags that change which image is being accumulated
 uint64_t fnv1a64(const void* data, size_t bytes) { const unsigned char* b = static_cast<const unsigned char*>(data); uint64_t h = 1469598103934665603ull; for (size_t i = 0; i < bytes; i++) h = (h ^ b[i]) * 1099511628211ull; return h; }
 }  // namespace
 int b2r_save_checkpoint(b2r_ctx* c, const char* path) {
@@ -1768,6 +1830,20 @@ int b2r_read_sky_tables(b2r_ctx* c, float* marginal_out, float* conditional_out,
 	if (conditional_out) CU(cudaMemcpyAsync(conditional_out, c->tables.sky_cond.p, static_cast<size_t>(k.rows) * (k.cols + 1u) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 	if (pdf_out) CU(cudaMemcpyAsync(pdf_out, c->tables.sky_pdf.p, c->hdri_texels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 	CU(sync_main(c));
+	return B2R_OK;
+}
+int b2r_read_light_tree(b2r_ctx* c, float* nodes_out, int32_t* light_prim_out, uint32_t* n_nodes_out) {
+	if (!c || !n_nodes_out) return fail(B2R_ERR_ARG, "null argument");
+	if (!c->have_scene) return fail(B2R_ERR_STATE, "upload_scene first");
+	if (!c->lt_built || c->lt_nodes == 0u) return fail(B2R_ERR_STATE, "no light tree: B2R_FLAG_LIGHT_TREE over a scene with sphere lights builds it");
+	*n_nodes_out = c->lt_nodes;
+	int rc = ensure_device(c); if (rc) return rc;
+	c->main_reads_scene = true;
+	std::vector<int4> light(light_prim_out ? c->params.scene.n_lights : 0u);
+	if (nodes_out) CU(cudaMemcpyAsync(nodes_out, c->tables.ltree_nodes.p, 2u * static_cast<size_t>(c->lt_nodes) * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+	if (light_prim_out) CU(cudaMemcpyAsync(light.data(), c->tables.ltree_light.p, light.size() * sizeof(int4), cudaMemcpyDeviceToHost, c->stream));
+	CU(sync_main(c));
+	for (size_t i = 0; i < light.size(); i++) light_prim_out[i] = light[i].x;
 	return B2R_OK;
 }
 int b2r_get_origin_box(b2r_ctx* c, float out[6]) {

@@ -115,8 +115,9 @@ __device__ __forceinline__ bool finished_elsewhere(const Params& p, uint32_t bou
 // LENS (bounce 0 with a thin lens): every camera ray has its own origin, so there is no shared-origin sphere precompute (s_pre); phase 1
 // runs sphere_hit_closest per ray, and phase 2 regenerates a hit's camera ray from its path id instead of queueing its origin.
 // DIELECTRIC (B2R_FLAG_DIELECTRIC): the shading routines' smooth-dielectric path (b2r_shade.h dielectric_scatter); the same axis in k_brute_finish
-// and k_shade. SKY (B2R_FLAG_SKY_LIGHT): the sky as a light (b2r_shade.h sky_light_sample, shade_sky<true>); likewise.
-template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false, bool LENS = false, bool DIELECTRIC = false, bool SKY = false>
+// and k_shade. SKY (B2R_FLAG_SKY_LIGHT): the sky as a light (b2r_shade.h sky_light_sample, shade_sky<true>); likewise. LTREE
+// (B2R_FLAG_LIGHT_TREE): sphere lights picked from the light tree (b2r_shade.h light_tree_pick, light_tree_hit_pdf); likewise.
+template <bool FIRST, bool COUNT, bool EXACT, bool GGX = false, bool LENS = false, bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_brute(const Params p, const uint32_t bounce) {
 	constexpr int kQ = 2 * kBruteBlock;  // hit queue: up to kBruteBlock-1 waiting + kBruteBlock new
 	__shared__ float4 s_prim[kBruteTile];
@@ -250,11 +251,11 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 				c_hits++;
 				if (last) { rad_zero(p.rad, p.frame.npix, s.pid); c_drop++; }  // survivors of the last bounce lose their radiance (Q11)
 				else {
-					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, hprim, acc, seed, bounce, &sr, p.sky);
+					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY, LTREE>(sc, sf, s, hprim, acc, seed, bounce, &sr, p.sky, p.ltree);
 					if (sf.emissive) {
 						// light sample first, then emission (Renderer.hpp:304-353). The shadow test of an emissive hit (rare) is done
 						// right here so that order holds; every other shadow ray goes to the queue and is tested by dense warps.
-						const f3 e_add = shade_emission<DIELECTRIC, SKY>(sc, sf, s, depth, bounce, mis, p.sky);
+						const f3 e_add = shade_emission<DIELECTRIC, SKY, LTREE>(sc, sf, s, depth, bounce, mis, p.sky, p.ltree, hprim);
 						if (want_shadow) {
 							c_shadow++;
 							bool occluded = false;
@@ -268,7 +269,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 						} else rad_add(p.rad, p.frame.npix, s.pid, e_add, f3{0.0f, 0.0f, 0.0f}, true, false);
 						c_events++;
 					}
-					keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
+					keep = shade_continue<GGX, DIELECTRIC, SKY, LTREE>(sf, &s, acc, seed, bounce, p.sky, p.ltree);
 					if (!keep) c_term++;  // roulette: path ends here, radiance stays at the pixel (Renderer.hpp:379-381,424-430)
 				}
 			}
@@ -349,7 +350,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_bounce_br
 // lane; both sphere loops are warp-uniform (every lane walks all the spheres of the shared-memory copy), so the only divergence is paths
 // ending, and a lane whose path has ended picks up the next waiting path. Same routines, same RNG streams (a function of sample, pixel and
 // bounce), same order of a path's radiance additions (light sample, then emission) as k_bounce_brute: every path ends with the same bits.
-template <bool COUNT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
+template <bool COUNT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_brute_finish(const Params p, const uint32_t bounce0) {
 	__shared__ float4 s_prim[kBruteTile];
 	__shared__ int32_t s_prim_mat[kBruteTile];
@@ -418,9 +419,9 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_BRUTE_MIN_BLOCKS) k_brute_fin
 				c_hits++;
 				if (bounce + 1u >= mb) { rad_zero(p.rad, p.frame.npix, pid); c_drop++; }  // Q11
 				else {
-					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky);
-					if (sf.emissive) { emit = shade_emission<DIELECTRIC, SKY>(sc, sf, s, best, bounce, mis, p.sky); has_emit = true; }
-					keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
+					if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY, LTREE>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky, p.ltree);
+					if (sf.emissive) { emit = shade_emission<DIELECTRIC, SKY, LTREE>(sc, sf, s, best, bounce, mis, p.sky, p.ltree, prim); has_emit = true; }
+					keep = shade_continue<GGX, DIELECTRIC, SKY, LTREE>(sf, &s, acc, seed, bounce, p.sky, p.ltree);
 					if (!keep) c_term++;
 				}
 			}
@@ -794,7 +795,7 @@ __global__ void __launch_bounds__(kTravBlock) k_intersect_closest(const Params p
 }
 // shade the hit records: light sample -> shadow queue, emission, BRDF sample / roulette -> next path queue.
 // Same CTA structure as the brute-force kernel: hits are collected in a shared-memory queue and shaded a full CTA at a time.
-template <bool EXACT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
+template <bool EXACT, bool GGX = false, bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
 __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(const Params p, const uint32_t bounce) {
 	constexpr int kQ = 2 * kBruteBlock;
 	__shared__ uint32_t s_hit_i[kQ]; __shared__ float s_hit_t[kQ]; __shared__ int32_t s_hit_prim[kQ];
@@ -853,12 +854,12 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 			c_hits++;
 			if (last) { rad_zero(p.rad, p.frame.npix, s.pid); c_drop++; }  // Q11
 			else {
-				if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky);
+				if (mis) want_shadow = shade_light_sample<GGX, DIELECTRIC, SKY, LTREE>(sc, sf, s, prim, acc, seed, bounce, &sr, p.sky, p.ltree);
 				if (sf.emissive) {
 					// the reference adds the light sample first, then the emission (Renderer.hpp:304-353). For the (rare) emissive hit
 					// that also has a shadow ray the any-hit traversal is done right here so that order holds; every other shadow ray
 					// goes to the shadow queue and is traced by k_intersect_shadow.
-					const f3 emit = shade_emission<DIELECTRIC, SKY>(sc, sf, s, depth, bounce, mis, p.sky);
+					const f3 emit = shade_emission<DIELECTRIC, SKY, LTREE>(sc, sf, s, depth, bounce, mis, p.sky, p.ltree, prim);
 					if (want_shadow) {
 						uint32_t cs = 0, cb = 0;
 						const bool occluded = traverse_any<false>(sc.wide, Ray{sr.o.x, sr.o.y, sr.o.z, sr.d.x, sr.d.y, sr.d.z}, sr.tfar, &cs, &cb, sc.parent, 0u);
@@ -867,7 +868,7 @@ __global__ void __launch_bounds__(kBruteBlock, B2R_SHADE_MIN_BLOCKS) k_shade(con
 					} else rad_add(p.rad, p.frame.npix, s.pid, emit, f3{0.0f, 0.0f, 0.0f}, true, false);
 					c_events++;
 				}
-				keep = shade_continue<GGX, DIELECTRIC, SKY>(sf, &s, acc, seed, bounce, p.sky);
+				keep = shade_continue<GGX, DIELECTRIC, SKY, LTREE>(sf, &s, acc, seed, bounce, p.sky, p.ltree);
 				if (!keep) c_term++;
 			}
 		}

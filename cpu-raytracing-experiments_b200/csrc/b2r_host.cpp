@@ -673,6 +673,87 @@ void build_sky_tables(const float4* texels, int32_t w, int32_t h, const float am
 		for (uint32_t x = 0; x < static_cast<uint32_t>(w); x++) out.pdf[static_cast<size_t>(y) * w + x] = sky_texel_pdf(out.marg.data(), out.cond.data(), cols, rows, x, y);
 }
 
+namespace {
+// a sphere's 20 meaningful bytes (position, radius^2, material): "equal by value", as match_prims_to_geometry compares them
+std::array<uint32_t, 5> sphere_key(const float4 s, int32_t mat) { return {bits(s.x), bits(s.y), bits(s.z), bits(s.w), static_cast<uint32_t>(mat)}; }
+std::array<uint32_t, 5> sphere_key(const b2r_sphere& s) { return sphere_key(make_float4(s.position[0], s.position[1], s.position[2], s.radius_sq), s.material_ID); }
+}  // namespace
+
+bool light_list_valid(const b2r_material* materials, const int32_t* light_geom_idx, uint32_t n_lights, const b2r_sphere* geometry) {
+	std::vector<std::array<uint32_t, 5>> keys(n_lights);
+	for (uint32_t i = 0; i < n_lights; i++) {
+		const b2r_sphere& g = geometry[light_geom_idx[i]];
+		const float* e = materials[g.material_ID].emission;
+		for (int k = 0; k < 3; k++) if (!std::isfinite(e[k]) || !(e[k] >= 0.0f)) return false;
+		keys[i] = sphere_key(g);  // (the same index twice gives the same sphere)
+	}
+	std::sort(keys.begin(), keys.end());
+	return std::adjacent_find(keys.begin(), keys.end()) == keys.end();
+}
+
+void build_light_tree(const b2r_sphere* lights, const float* lum, uint32_t n_lights, const float4* prims, const int32_t* prim_mat, uint32_t n_prims, LightTree& out) {
+	out.nodes.clear(); out.lo.clear(); out.hi.clear(); out.depth = 0;
+	out.light.assign(n_lights, make_int4(-1, 0, 0, 0));
+	out.prim_light.assign(n_prims, -1);
+	// light -> BVH-order sphere (the lowest equal index) and back
+	std::vector<std::pair<std::array<uint32_t, 5>, uint32_t>> keys(n_lights);
+	for (uint32_t i = 0; i < n_lights; i++) keys[i] = {sphere_key(lights[i]), i};
+	std::sort(keys.begin(), keys.end());
+	for (uint32_t p = 0; p < n_prims && n_lights; p++) {
+		const auto k = sphere_key(prims[p], prim_mat[p]);
+		const auto it = std::lower_bound(keys.begin(), keys.end(), std::make_pair(k, 0u));
+		for (auto j = it; j != keys.end() && j->first == k; ++j)
+			if (out.light[j->second].x < 0) { out.light[j->second].x = static_cast<int32_t>(p); if (out.prim_light[p] < 0) out.prim_light[p] = static_cast<int32_t>(j->second); }
+	}
+	if (n_lights == 0u) return;
+	// topology: median splits, children allocated in pairs after their parent
+	std::vector<float> c(3 * static_cast<size_t>(n_lights));
+	for (uint32_t i = 0; i < n_lights; i++) for (int k = 0; k < 3; k++) c[3 * i + k] = lights[i].position[k];
+	std::vector<uint32_t> ord(n_lights); std::iota(ord.begin(), ord.end(), 0u);
+	struct Item { uint32_t node, a, b, bits, depth; };
+	std::vector<Item> work{{0u, 0u, n_lights, 0u, 0u}};
+	std::vector<int32_t> link(1, 0);
+	while (!work.empty()) {
+		const Item it = work.back(); work.pop_back();
+		if (it.b - it.a == 1u) {
+			const uint32_t l = ord[it.a];
+			link[it.node] = ~static_cast<int32_t>(l);
+			out.light[l].y = static_cast<int32_t>(it.bits); out.light[l].z = static_cast<int32_t>(it.depth); out.light[l].w = static_cast<int32_t>(it.node);
+			out.depth = std::max(out.depth, it.depth);
+			continue;
+		}
+		float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+		for (uint32_t j = it.a; j < it.b; j++) for (int k = 0; k < 3; k++) { lo[k] = std::min(lo[k], c[3 * ord[j] + k]); hi[k] = std::max(hi[k], c[3 * ord[j] + k]); }
+		int axis = 0;
+		for (int k = 1; k < 3; k++) if (hi[k] - lo[k] > hi[axis] - lo[axis]) axis = k;
+		std::sort(ord.begin() + it.a, ord.begin() + it.b, [&](uint32_t x, uint32_t y) { return c[3 * x + axis] < c[3 * y + axis] || (c[3 * x + axis] == c[3 * y + axis] && x < y); });
+		const uint32_t mid = it.a + (it.b - it.a) / 2u, kid = static_cast<uint32_t>(link.size());
+		link[it.node] = static_cast<int32_t>(kid); link.push_back(0); link.push_back(0);
+		work.push_back({kid + 1u, mid, it.b, it.bits | (1u << it.depth), it.depth + 1u});
+		work.push_back({kid, it.a, mid, it.bits, it.depth + 1u});
+	}
+	// boxes and energies bottom-up (children have higher indices than their parent)
+	const size_t n_nodes = link.size();
+	out.nodes.assign(2 * n_nodes, make_float4(0, 0, 0, 0)); out.lo.assign(3 * n_nodes, 0.0f); out.hi.assign(3 * n_nodes, 0.0f);
+	std::vector<float> E(n_nodes, 0.0f);
+	for (size_t n = n_nodes; n-- > 0;) {
+		float* lo = &out.lo[3 * n]; float* hi = &out.hi[3 * n];
+		if (link[n] < 0) {
+			const b2r_sphere& s = lights[~link[n]];
+			const float r = std::sqrt(s.radius_sq);
+			for (int k = 0; k < 3; k++) { lo[k] = s.position[k] - r; hi[k] = s.position[k] + r; }
+			E[n] = lum[~link[n]] * s.radius_sq;
+		} else {
+			const size_t l = static_cast<size_t>(link[n]);
+			for (int k = 0; k < 3; k++) { lo[k] = std::min(out.lo[3 * l + k], out.lo[3 * (l + 1) + k]); hi[k] = std::max(out.hi[3 * l + k], out.hi[3 * (l + 1) + k]); }
+			E[n] = E[l] + E[l + 1];
+		}
+		const float hx = (hi[0] - lo[0]) * 0.5f, hy = (hi[1] - lo[1]) * 0.5f, hz = (hi[2] - lo[2]) * 0.5f;
+		out.nodes[2 * n] = make_float4((lo[0] + hi[0]) * 0.5f, (lo[1] + hi[1]) * 0.5f, (lo[2] + hi[2]) * 0.5f, (hx * hx + hy * hy) + hz * hz);
+		out.nodes[2 * n + 1] = make_float4(E[n], int_as_float(link[n]), 0.0f, 0.0f);
+	}
+}
+
 }  // namespace b2r
 
 // ---------------------------------------------------------------------------------------------- C ABI (host-only part)

@@ -95,5 +95,26 @@ bool sky_texels_valid(const float4* texels, size_t n, const float ambient[3], bo
 // not zero everywhere. marg: rows + 1, cond: rows * (cols + 1), pdf: w * h floats (SkyDev).
 struct SkyTables { std::vector<float> marg, cond, pdf; uint32_t cols = 0, rows = 0; };
 void build_sky_tables(const float4* texels, int32_t w, int32_t h, const float ambient[3], SkyTables& out);
+// B2R_FLAG_LIGHT_TREE input rule: no light index appears twice, no two lights are spheres equal by value (they would be one sphere to the
+// renderer), and every light's material emission is finite and >= 0. Returns false when the light list breaks it.
+bool light_list_valid(const b2r_material* materials, const int32_t* light_geom_idx, uint32_t n_lights, const b2r_sphere* geometry);
+// B2R_FLAG_LIGHT_TREE (DESIGN §2): the binary tree over the light list that next-event estimation descends to pick a sphere light, and the
+// maps between lights and BVH-order spheres. Built on the host only (there is no device twin). Node layout (2 float4 per node, LightTreeDev):
+//   {c.xyz, R^2}  the box of the node's light spheres (centre +- r) as centre and squared half-diagonal
+//   {E, as_float(link), 0, 0}  E = sum of lum * r^2 over its lights (lum = mean of the emission rgb); link >= 0: the children are nodes link
+//   and link + 1; link < 0: a leaf holding light ~link
+// Node 0 is the root; children always follow their parent. Split at the median light centre along the box of the centres' largest extent (ties:
+// lowest axis, then light index), left half = floor(n / 2) lights: the depth is ceil(log2 n_lights), at most 32, so a leaf's root-to-leaf path
+// fits a 32-bit word.
+struct LightTree {
+	std::vector<float4> nodes;       // [2 * n_nodes]
+	std::vector<int4> light;         // [n_lights] {BVH-order sphere of the light (-1: none), path bits (bit d: right at depth d), depth, leaf node}
+	std::vector<int32_t> prim_light; // [n_prims] the light BVH-order sphere i is, -1: none
+	std::vector<float> lo, hi;       // [n_nodes][3] the box corners (host only: the tests' containment checks)
+	uint32_t depth = 0;
+};
+// lights[i] = geometry[light_geom_idx[i]] (position, radius^2, material), lum[i] its material's mean emission; prims / prim_mat: the spheres in
+// BVH order (SceneDev::prims). A light's sphere is the LOWEST BVH-order index equal to it by value: closest-hit ties go to the lowest index too.
+void build_light_tree(const b2r_sphere* lights, const float* lum, uint32_t n_lights, const float4* prims, const int32_t* prim_mat, uint32_t n_prims, LightTree& out);
 
 }  // namespace b2r

@@ -121,6 +121,13 @@ struct SkyDev {
 	float p_sky;          // probability that a light sample goes to the sky: 0 without a sky (nothing below reads the tables), 1 without sphere lights
 	float light_sel_pdf;  // (1 - p_sky) / n_lights: a sphere light's selection probability
 };
+// B2R_FLAG_LIGHT_TREE (DESIGN §2): the light tree of the host builder build_light_tree (node layout: b2r_host.h LightTree) and its maps.
+struct LightTreeDev {
+	const float4* nodes;       // [2 * n_nodes] {c.xyz, R^2}, {E, as_float(link), 0, 0}
+	const int4* light;         // [n_lights] {BVH-order sphere (-1: none), path bits, depth, leaf node}
+	const int32_t* prim_light; // [n_prims] the light BVH-order sphere i is (-1: none)
+	float sel_scale;           // 1 - p_sky: a sphere light's selection pdf is sel_scale * its tree pdf; 0 without sphere lights
+};
 struct Params {
 	SceneDev scene; FrameDev frame; QueueDev q; CountDev cnt; ExactDev ex;
 	const BatchDev* batch;
@@ -130,6 +137,7 @@ struct Params {
 	// A scene table, but kept here at the end rather than in SceneDev, so the parameter block of every other instantiation keeps its layout.
 	const float4* mat_diel;
 	SkyDev sky;  // read by the SKY instantiations only (B2R_FLAG_SKY_LIGHT); at the end for the same reason
+	LightTreeDev ltree;  // read by the LTREE instantiations only (B2R_FLAG_LIGHT_TREE); likewise
 };
 
 // ---------------------------------------------------------------------------------------------- small helpers
@@ -294,20 +302,77 @@ B2R_HD bool sky_light_sample(const SceneDev& sc, const SkyDev& sky, const Surfac
 	return true;
 }
 
+// ---------------------------------------------------------------------------------------------- the light tree (B2R_FLAG_LIGHT_TREE)
+// The probability of the LEFT child of the inner node whose children are link and link + 1, at the point P: I_l / (I_l + I_r) with a node's
+// importance I = E / max(|P - c|^2, R^2) (position only: the emissive-hit weight recomputes it from the path record, which keeps the previous
+// vertex's position but not its normal); 1/2 when that sum is 0 or not finite. The descent and light_tree_pdf both call this one routine.
+B2R_HD float light_tree_importance(const float4* nodes, uint32_t n, f3 P) {
+	const float4 a = ldg4(nodes + 2u * n), b = ldg4(nodes + 2u * n + 1u);
+	const float dx = P.x - a.x, dy = P.y - a.y, dz = P.z - a.z;
+	return b.x / sel_max((dx * dx + dy * dy) + dz * dz, a.w);
+}
+B2R_HD float light_tree_p_left(const float4* nodes, uint32_t link, f3 P) {
+	const float il = light_tree_importance(nodes, link, P), ir = light_tree_importance(nodes, link + 1u, P);
+	const float sum = il + ir;
+	return (sum > 0.0f && sum <= FLT_MAX) ? il / sum : 0.5f;
+}
+// The descent: at each inner node left when u < p_l (a branch of probability 0 is never taken, also at u = 1.0, which next_unit can return,
+// Q4), then u rescaled into the chosen branch and kept below 1. *pdf = the product of the branch probabilities, multiplied from the root down.
+// Returns the light. One light: the root is its leaf, pdf 1.
+B2R_HD uint32_t light_tree_pick(const LightTreeDev& lt, f3 P, float u, float* pdf) {
+	uint32_t node = 0u; float p = 1.0f;
+	for (;;) {
+		const int32_t link = as_int(ldg4(lt.nodes + 2u * node + 1u).y);
+		if (link < 0) { *pdf = p; return static_cast<uint32_t>(~link); }
+		const float pl = light_tree_p_left(lt.nodes, static_cast<uint32_t>(link), P), pr = 1.0f - pl;
+		const bool left = pr == 0.0f || (pl > 0.0f && u < pl);
+		if (left) { p = p * pl; u = u / pl; node = static_cast<uint32_t>(link); }
+		else { p = p * pr; u = (u - pl) / pr; node = static_cast<uint32_t>(link) + 1u; }
+		u = sel_min(u, 0x1.fffffep-1f);
+	}
+}
+// The probability light_tree_pick picks `light` at P, bit for bit the product it accumulates: the light's root-to-leaf path (LightTreeDev::light)
+// walked top-down with the same branch probabilities in the same order.
+B2R_HD float light_tree_pdf(const LightTreeDev& lt, f3 P, uint32_t light) {
+	const int4 li = lt.light[light];
+	uint32_t node = 0u; float p = 1.0f;
+	for (int32_t d = 0; d < li.z; d++) {
+		const uint32_t link = static_cast<uint32_t>(as_int(ldg4(lt.nodes + 2u * node + 1u).y));
+		const float pl = light_tree_p_left(lt.nodes, link, P), pr = 1.0f - pl;
+		if ((static_cast<uint32_t>(li.y) >> d) & 1u) { p = p * pr; node = link + 1u; }
+		else { p = p * pl; node = link; }
+	}
+	return p;
+}
+// The selection pdf an emissive hit of BVH-order sphere `prim`, reached from P, had as a light sample: sel_scale * its tree pdf, 0 when the sphere
+// is not a light (its MIS weight is then power_heuristic(pdf, 0), as for every emitter of a scene without lights).
+B2R_HD float light_tree_hit_pdf(const LightTreeDev& lt, f3 P, int32_t prim) {
+	const int32_t li = lt.prim_light[prim];
+	return li < 0 ? 0.0f : lt.sel_scale * light_tree_pdf(lt, P, static_cast<uint32_t>(li));
+}
+
 // next-event estimation, Renderer.hpp:249-298. Returns false when no shadow ray is produced; a dielectric surface (delta BSDF) never makes one.
 // SKY (B2R_FLAG_SKY_LIGHT): after u0, u1 and the sphere pick (drawn only when there are sphere lights), one draw chooses the sky when 0 < p_sky < 1
 // (sky when it is < p_sky); the sphere lights keep their estimator with selection pdf (1 - p_sky) / n_lights.
-template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
+// LTREE (B2R_FLAG_LIGHT_TREE): the sphere pick's draw descends the light tree instead (light_tree_pick at the surface point), the selection pdf is
+// (1 - p_sky) times the tree pdf, and the self test compares the light's BVH-order sphere with hit_prim (no Q9).
+template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
 B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const PathState& s, int32_t hit_prim,
-                                                   uint32_t acc, uint32_t seed, uint32_t bounce, ShadowRay* out, const SkyDev& sky = SkyDev{}) {
+                                                   uint32_t acc, uint32_t seed, uint32_t bounce, ShadowRay* out, const SkyDev& sky = SkyDev{},
+                                                   const LightTreeDev& lt = LightTreeDev{}) {
 	if (is_dielectric<DIELECTRIC>(sf)) return false;
 	if (sc.n_lights == 0u && !(SKY && sky.p_sky > 0.0f)) return false;  // undefined in the reference (Q15); defined here as "no light sampling"
 	Pcg rng{hash_2d(acc, seed + bounce * 2u)};  // Q3
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
-	const uint32_t pick = (!SKY || sc.n_lights != 0u) ? rng.next_below(sc.n_lights) : 0u;
+	const bool draw = !SKY || sc.n_lights != 0u;
+	const float ut = (LTREE && draw) ? rng.next_unit() : 0.0f;  // (the draw next_below consumes)
+	uint32_t pick = (!LTREE && draw) ? rng.next_below(sc.n_lights) : 0u;
 	if (SKY && (sky.p_sky >= 1.0f || (sky.p_sky > 0.0f && rng.next_unit() < sky.p_sky))) return sky_light_sample(sc, sky, sf, s, &rng, out);
+	float tree_sel = 0.0f;
+	if constexpr (LTREE) { pick = light_tree_pick(lt, sf.P, ut, &tree_sel); tree_sel = lt.sel_scale * tree_sel; }
 	const float4 ls = ld4(sc.light_sphere + pick), le = ld4(sc.light_emit + pick);
-	if (as_int(le.w) == hit_prim) return false;  // Q9: geometry index vs BVH-order index, as in the reference
+	if constexpr (LTREE) { if (lt.light[pick].x == hit_prim) return false; }  // the light's own BVH-order sphere
+	else if (as_int(le.w) == hit_prim) return false;  // Q9: geometry index vs BVH-order index, as in the reference
 	f3 wc{ls.x - sf.P.x, ls.y - sf.P.y, ls.z - sf.P.z};
 	const float d2 = dot3(wc, wc);
 	if (d2 <= ls.w) return false;
@@ -326,7 +391,7 @@ B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const Path
 		const float f = B2R_INV_PI * sel_max(0.0f, ll.z);  // Closure<Lambertian>::eval, DataStreams.hpp:169-172
 		rad = f3{rad.x * (sf.albedo.x * f), rad.y * (sf.albedo.y * f), rad.z * (sf.albedo.z * f)};
 	}
-	lpdf *= SKY ? sky.light_sel_pdf : sc.light_sel_pdf;
+	lpdf *= LTREE ? tree_sel : SKY ? sky.light_sel_pdf : sc.light_sel_pdf;
 	const float bpdf = GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, ll.z);  // Closure<GGX>::pdf is `return 0.0f; //TODO` in the reference (:196-198)
 	const float w = power_heuristic_over_f(lpdf, bpdf);
 	rad = scale3(rad, w);
@@ -335,15 +400,18 @@ B2R_HD bool shade_light_sample(const SceneDev& sc, const Surface& sf, const Path
 	return true;
 }
 // emissive-hit contribution, Renderer.hpp:319-353. DIELECTRIC: a path continued from a dielectric surface carries pdf = -1 (no light sample
-// competes with a delta BSDF), and its MIS weight is 1. SKY: the sphere's selection pdf is SkyDev::light_sel_pdf.
-template <bool DIELECTRIC = false, bool SKY = false>
-B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState& s, float depth, uint32_t bounce, bool mis, const SkyDev& sky = SkyDev{}) {
+// competes with a delta BSDF), and its MIS weight is 1. SKY: the sphere's selection pdf is SkyDev::light_sel_pdf. LTREE: the hit sphere's
+// selection pdf at the path record's origin (the point its light sample was taken from), light_tree_hit_pdf of BVH-order sphere `prim`.
+template <bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
+B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState& s, float depth, uint32_t bounce, bool mis, const SkyDev& sky = SkyDev{},
+                         const LightTreeDev& lt = LightTreeDev{}, int32_t prim = -1) {
 	const float4 em = ld4(sc.mat_emission + sf.mat);
 	if (!mis) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};  // this repo's MIS-off (Q23)
 	if (bounce == 0) return f3{em.x, em.y, em.z};
 	if (DIELECTRIC && s.pdf < 0.0f) return f3{s.tr * em.x, s.tg * em.y, s.tb * em.z};
 	const float d2 = depth * (depth + sf.n_dot_v * (2.0f * sqrtf(sf.r2))) + sf.r2;  // law of cosines, Renderer.hpp:331
-	const float w = power_heuristic(s.pdf, (SKY ? sky.light_sel_pdf : sc.light_sel_pdf) * sphere_light_pdf(sf.r2, d2));
+	const float sel = LTREE ? light_tree_hit_pdf(lt, f3{s.ox, s.oy, s.oz}, prim) : SKY ? sky.light_sel_pdf : sc.light_sel_pdf;
+	const float w = power_heuristic(s.pdf, sel * sphere_light_pdf(sf.r2, d2));
 	return f3{(s.tr * w) * em.x, (s.tg * w) * em.y, (s.tb * w) * em.z};
 }
 // BRDF sampling + Russian roulette, Renderer.hpp:359-403. Returns false when the path is terminated by roulette. A dielectric surface
@@ -351,8 +419,10 @@ B2R_HD f3 shade_emission(const SceneDev& sc, const Surface& sf, const PathState&
 // refraction scales the throughput by the transmission and leaves from P_in, and the path stores pdf = -1 (specular predecessor).
 // SKY with p_sky > 0 (the sky is sampled): the path stores the true pdf of the sampled direction, 1/pi times its LOCAL cosine, instead of Q10's
 // world-space one: the sky's MIS weights need the density the direction was drawn with, and the emissive-hit weight then reads it too.
-template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false>
-B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32_t seed, uint32_t bounce, const SkyDev& sky = SkyDev{}) {
+// LTREE with sphere lights (sel_scale > 0): likewise, so the sphere lights' two weights of a direction sum to 1 (no Q10).
+template <bool GGX = false, bool DIELECTRIC = false, bool SKY = false, bool LTREE = false>
+B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32_t seed, uint32_t bounce, const SkyDev& sky = SkyDev{},
+                           const LightTreeDev& lt = LightTreeDev{}) {
 	Pcg rng{hash_2d(acc, seed + bounce * 2u + 1u)};
 	const float u0 = rng.next_unit(), u1 = rng.next_unit();
 	f3 dl, est = sf.albedo, o = sf.P;
@@ -371,7 +441,7 @@ B2R_HD bool shade_continue(const Surface& sf, PathState* s, uint32_t acc, uint32
 	const f3 dw = frame_to_world(sf.T, dl);
 	s->ox = o.x; s->oy = o.y; s->oz = o.z; s->dx = dw.x; s->dy = dw.y; s->dz = dw.z;
 	s->tr = thr.x; s->tg = thr.y; s->tb = thr.z;
-	s->pdf = delta ? -1.0f : GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, (SKY && sky.p_sky > 0.0f) ? dl.z : dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
+	s->pdf = delta ? -1.0f : GGX ? 0.0f : B2R_INV_PI * sel_max(0.0f, ((SKY && sky.p_sky > 0.0f) || (LTREE && lt.sel_scale > 0.0f)) ? dl.z : dw.z);  // pdf of the world-space direction (Q10); Closure<GGX>::pdf returns 0
 	return true;
 }
 // miss shader with ambient sky, Renderer.hpp:411-420 + Sky::operator(), Primitives.hpp:35-46. SKY (B2R_FLAG_SKY_LIGHT): per channel, tr * L(d) * w

@@ -96,6 +96,21 @@ enum {
 	                                    * and B2R_FLAG_DIELECTRIC; B2R_ERR_ARG with B2R_FLAG_REFERENCE_EXACT, B2R_FLAG_NO_MIS or B2R_FLAG_GGX, at b2r_create
 	                                    * and b2r_set_flags. With the flag, b2r_upload_scene and b2r_set_flags refuse (B2R_ERR_ARG) a sky texel that is not
 	                                    * finite, or negative, in a channel whose ambient is > 0. A checkpoint does not load across the flag. */
+	B2R_FLAG_LIGHT_TREE = 1u << 14,    /* next-event estimation picks its sphere light by importance from a light tree instead of uniformly, in both
+	                                    * pipelines (DESIGN.md §2). The tree is a binary tree over the light list, built on the host (median splits of the
+	                                    * light centres, one light per leaf); a node keeps the box of its light spheres and its energy E = sum of
+	                                    * mean(emission) * r^2. The sample's draw descends it by the importance E / max(|P - c|^2, R^2) of each child at the
+	                                    * surface point; the light's selection pdf is (1 - p_sky) times the product of the branch probabilities, and an
+	                                    * emissive hit recomputes that pdf at the point its light sample was taken from. The self test compares the picked
+	                                    * light's BVH-order sphere with the hit sphere (quirk Q9 does not apply), the path record carries the local-cosine pdf
+	                                    * of its direction whenever there are sphere lights (quirk Q10 does not apply), and an emitter that is not in the
+	                                    * light list has selection pdf 0. Without sphere lights frames equal those without the flag. The tree is rebuilt at
+	                                    * b2r_upload_scene and b2r_refit_scene, or when b2r_set_flags turns the flag on (b2r_read_light_tree reads it).
+	                                    * Combines with B2R_FLAG_GGX, B2R_FLAG_DIELECTRIC, B2R_FLAG_SKY_LIGHT and a lens; B2R_ERR_ARG with
+	                                    * B2R_FLAG_REFERENCE_EXACT or B2R_FLAG_NO_MIS, at b2r_create and b2r_set_flags. With the flag, b2r_upload_scene,
+	                                    * b2r_refit_scene and b2r_set_flags refuse (B2R_ERR_ARG) a light list with a light index twice, or two lights that are
+	                                    * equal spheres (position, radius^2, material), or a light whose emission is not finite or is negative. A checkpoint
+	                                    * does not load across the flag. */
 };
 
 typedef struct b2r_config {
@@ -303,6 +318,12 @@ int  b2r_read_link_tables(b2r_ctx* ctx, uint32_t* parent_out, uint32_t* leaf_nod
  * (CDF over the rows), conditional_out[H'][W'+1] (CDF over the cells of each row), pdf_out[h][w] (solid-angle pdf of the cell each texel shows,
  * without the sky's selection probability). A null table pointer skips that table. B2R_ERR_STATE when no tables are built. Synchronises. */
 int  b2r_read_sky_tables(b2r_ctx* ctx, float* marginal_out, float* conditional_out, float* pdf_out, uint32_t* cols_out, uint32_t* rows_out);
+/* B2R_FLAG_LIGHT_TREE: the light tree as the device holds it. *n_nodes_out = its node count N (2 n_lights - 1); nodes_out[N][8] = per node
+ * {c.x, c.y, c.z, R^2, E, link, 0, 0}: the box of its light spheres as centre and squared half-diagonal, its energy, and `link` (an int32 stored
+ * in the float's bits): >= 0, the children are nodes link and link + 1; < 0, a leaf holding light ~link. Node 0 is the root.
+ * light_prim_out[n_lights] = the BVH-order sphere of each light (the lowest index equal to it by value; -1: none). A null table pointer skips
+ * that table. B2R_ERR_STATE when no tree is built (the flag is off, or the scene has no sphere lights). Synchronises. */
+int  b2r_read_light_tree(b2r_ctx* ctx, float* nodes_out, int32_t* light_prim_out, uint32_t* n_nodes_out);
 /* the box ray origins are assumed to lie in ({lo.xyz, hi.xyz}: sphere bounds, camera, origins passed to b2r_trace_*): the leaf slots of the
  * traversal tree are sized for it, so a host twin of the tree needs the same box (tests) */
 int  b2r_get_origin_box(b2r_ctx* ctx, float lo_hi_out[6]);
